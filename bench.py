@@ -9,8 +9,10 @@ Legs (DESIGN.md section 8): `value` = the shipped path (CUDA-graph replay on one
 and phase timers (roofline, phases), `e2e` through korali_b200.Engine().run(e) (k["Conduit"]["Devices"] = N), `parity_vs_n1` for N > 1,
 `cpu_baseline` on a bounded sample; `--impl reference` times REAL full-size generations of the reference algorithm on the host.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 Under torchrun (N > 1) every rank runs this file; rank 0 prints ONE JSON line.
+--dump-outputs DIR writes the solver state after the last timed generation as DIR/<name>.npy (float64), so that two builds can be
+compared output for output on the same seeded workload.
 """
 import argparse
 import json
@@ -82,6 +84,32 @@ class ClockSampler:
         return {"sm_mhz": float(np.median(sm)), "sm_max_mhz": float(max(mx)), "reasons": sorted(reasons), "samples": len(sm)}
 
 
+DUMP_ARRAYS = ["Covariance Matrix", "Covariance Eigenvector Matrix", "Axis Lengths", "Current Mean", "Evolution Path",
+               "Conjugate Evolution Path", "Best Ever Variables", "Value Vector"]
+DUMP_SCALARS = ["Sigma", "Best Ever Value", "Current Best Value", "Conjugate Evolution Path L2 Norm", "Current Generation"]
+DUMP_SAMPLE_ROWS = 2048        # the 65536 x 1000 population is 524 MB: a fixed, seeded sample of its rows is written instead
+
+
+def dump_outputs(s, out_dir):
+    """What a caller of the generation loop reads back after the last timed generation, as out_dir/<name>.npy (float64, about 34 MB
+    at config 3). The population ('BDZ Matrix', this rank's rows) is sampled at DUMP_SAMPLE_ROWS rows drawn with a fixed seed;
+    the drawn row numbers are written beside it."""
+    os.makedirs(out_dir, exist_ok=True)
+
+    def save(key, a):
+        np.save(os.path.join(out_dir, key.lower().replace(" ", "_") + ".npy"), np.asarray(a, dtype=np.float64))
+    for k in DUMP_ARRAYS:
+        a = s.get(k)
+        save(k, a.reshape(s.n, s.n) if k.endswith("Matrix") else a)
+    save("Sorting Index", s.get_index("Sorting Index"))
+    for k in DUMP_SCALARS:
+        save(k, [s.scalar(k)])
+    y = s.get("BDZ Matrix").reshape(-1, s.n)
+    rows = np.sort(np.random.default_rng(0).choice(y.shape[0], min(DUMP_SAMPLE_ROWS, y.shape[0]), replace=False))
+    save("BDZ Matrix Sample", y[rows])
+    save("BDZ Matrix Sample Rows", rows)
+
+
 # ---------------------------------------------------------------------------------------------------------
 def cpu_bounded_sample(steps, warmup, sample_lambda=1024):
     """cpu_baseline leg of the default run (about 10-20 s of host work): the C restatement in oracle/ (the reference itself needs
@@ -139,6 +167,8 @@ def reference_arm(args, rank):
         print("reference arm: generation %d  ask %.1f s  eval %.1f s  tell %.1f s" % (g + 1, t1 - t0, t2 - t1, t3 - t2), file=sys.stderr, flush=True)
         if (time.perf_counter() - t_begin) + max(times) > REF_TIME_BUDGET_S:
             break
+    if args.dump_outputs:
+        dump_outputs(o, args.dump_outputs)
     t_gen = float(np.mean(times))
     gps = 1.0 / t_gen
     ph = np.mean(np.array(phases), axis=0)
@@ -286,6 +316,8 @@ def ours_arm(args, rank, world):
         clocks.start()
     ms, launches = timed_leg(s, args.steps, False, torch, barrier)
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(s, args.dump_outputs)
     best = s.scalar("Best Ever Value")
     # ---- e2e through kcma_run (termination chain on the host every generation) on the same handle, next K generations
     barrier()
@@ -420,6 +452,8 @@ def main():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the state after the last timed generation as DIR/<name>.npy (float64)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
@@ -430,6 +464,8 @@ def main():
         # convenience: re-launch under torchrun
         cmd = [sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", str(args.gpus), "--master-addr", "127.0.0.1",
                "--master-port", "29511", os.path.abspath(__file__), "--gpus", str(args.gpus), "--steps", str(args.steps), "--warmup", str(args.warmup)]
+        if args.dump_outputs:
+            cmd += ["--dump-outputs", args.dump_outputs]
         sys.exit(subprocess.call(cmd))
     ours_arm(args, rank, world)
 
