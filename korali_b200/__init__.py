@@ -4,7 +4,8 @@
     e = korali.Experiment(); e["Solver"]["Type"] = "Optimizer/CMAES"; ...; korali.Engine().run(e)
 
 Served: `"Solver": {"Type": "Optimizer/CMAES"}` (the hot path) and its sibling population solvers `Optimizer/DEA`, `Optimizer/MOCMAES`
-of `"Problem": {"Type": "Optimization"}`, plus the float ask/tell class `fCMAES` (SURVEY.md scope).
+of `"Problem": {"Type": "Optimization"}`, the transitional MCMC sampler `Sampler/TMCMC` of `"Problem": {"Type": "Bayesian/Custom"}`
+(priors from `e["Distributions"]`), plus the float ask/tell class `fCMAES` (SURVEY.md scope).
 Layers: korali_b200._host (pybind11, C++: Engine / Experiment, mirrors python/korali/__init__.py:9-20 + source/engine.cpp:201-254)
  -> include/kcma.h (C ABI) -> korali_b200/libkcma.so (hand-written sm_100a CUDA). There is no CPU fallback.
 """

@@ -13,8 +13,8 @@ OBJ = os.path.join(HERE, "build")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-lineinfo", "-std=c++17", "-Xcompiler", "-fPIC", "-Xcompiler", "-Wall"] + ARCH
 # files whose arithmetic must round like the reference's scalar code (no fused multiply-add)
-NO_FMA = {"objective.cu", "update.cu", "constraints.cu", "dea.cu", "mocma.cu"}
-SOURCES = ["api.cu", "gemm.cu", "gemm_tma.cu", "rng.cu", "objective.cu", "sort.cu", "update.cu", "eigen.cu", "constraints.cu", "gemm_batched.cu", "tridiag.cu", "dc.cu", "dea.cu", "mocma.cu"]
+NO_FMA = {"objective.cu", "update.cu", "constraints.cu", "dea.cu", "mocma.cu", "tmcmc.cu"}
+SOURCES = ["api.cu", "gemm.cu", "gemm_tma.cu", "rng.cu", "objective.cu", "sort.cu", "update.cu", "eigen.cu", "constraints.cu", "gemm_batched.cu", "tridiag.cu", "dc.cu", "dea.cu", "mocma.cu", "tmcmc.cu"]
 
 
 def _newer(src, dst):
@@ -27,6 +27,7 @@ def build(force=False, verbose=False):
     headers.append(os.path.join(HERE, "..", "include", "kcma.h"))
     headers.append(os.path.join(HERE, "..", "include", "kdea.h"))
     headers.append(os.path.join(HERE, "..", "include", "kmocma.h"))
+    headers.append(os.path.join(HERE, "..", "include", "ktmcmc.h"))
     objs, rebuilt = [], False
     procs = []
     for s in SOURCES:
@@ -58,7 +59,8 @@ def build_host(force=False):
     import pybind11
     src = os.path.join(HERE, "host", "korali_host.cpp")
     out = os.path.join(HERE, "_host" + sysconfig.get_config_var("EXT_SUFFIX"))
-    if not (force or _newer(src, out) or _newer(OUT, out) or _newer(os.path.join(HERE, "..", "include", "kcma.h"), out)):
+    if not (force or _newer(src, out) or _newer(OUT, out) or
+            any(_newer(os.path.join(HERE, "..", "include", h), out) for h in ("kcma.h", "kdea.h", "kmocma.h", "ktmcmc.h"))):
         return out
     cmd = ["g++", "-O2", "-shared", "-fPIC", "-std=c++17", "-fvisibility=hidden", "-I", pybind11.get_include(),
            "-I", sysconfig.get_paths()["include"], src, "-o", out, "-L", HERE, "-lkcma", "-Wl,-rpath,$ORIGIN"]

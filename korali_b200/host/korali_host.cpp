@@ -32,6 +32,7 @@
 #include "../../include/kcma.h"
 #include "../../include/kdea.h"
 #include "../../include/kmocma.h"
+#include "../../include/ktmcmc.h"
 
 namespace py = pybind11;
 
@@ -1240,6 +1241,276 @@ class MOCMAES : public SolverBase {
   }
 };
 
+// ---- the solver plug-in: Sampler/TMCMC on libkcma (include/ktmcmc.h) for Bayesian/Custom problems ---------------------------------
+class TMCMC : public SolverBase {
+ public:
+  ktmcmc_t* h = nullptr;
+  ktmcmc_cfg cfg;
+  py::object distributions = py::none();   // the experiment's top-level "Distributions" (the priors)
+  std::vector<int32_t> prior_type;
+  std::vector<double> prior_a, prior_b;
+  std::vector<uint64_t> burn_in;
+  std::vector<std::string> prior_name;
+  std::string batched;
+  py::object model;
+  double tc_target = 1.0, tc_max_generations = 1e10, tc_max_model_evaluations = 1e9;
+
+  ~TMCMC() override { if (h) ktmcmc_destroy(h); }
+  const char* name() const override { return "Sampler/TMCMC"; }
+  size_t variableCount() const override { return cfg.n; }
+  void check(int rc) { if (rc) korali_error("%s", ktmcmc_last_error(h)); }
+  double scalar(const char* key) override { double v = NAN; check(ktmcmc_get_scalar(h, key, &v)); return v; }
+  std::vector<double> array(const char* key) override {
+    size_t n = 0;
+    check(ktmcmc_get_array(h, key, nullptr, 0, &n));
+    std::vector<double> v(n);
+    if (n) check(ktmcmc_get_array(h, key, v.data(), n, &n));
+    return v;
+  }
+
+  // generated TMCMC::setConfiguration (TMCMC.config) + Sampler:: + Solver:: (strict); priors from e["Distributions"]
+  void setConfiguration(py::dict solver, py::list variables, py::dict problem, uint64_t seed) override {
+    ktmcmc_cfg_defaults(&cfg);
+    Settings s(solver, "TMCMC");
+    s.take("Type");
+    const std::string version = s.str("Version", "TMCMC");
+    if (canon(version) == "mtmcmc") korali_error("Sampler/TMCMC: 'Version' mTMCMC is not built on the B200 path (only 'TMCMC')\n");
+    if (canon(version) != "tmcmc") korali_error(" + Object: [ TMCMC ] \n + Key:    ['Version']\n + Reason: unknown version '%s' (TMCMC)\n", version.c_str());
+    cfg.population_size = s.uint("Population Size", 0);
+    cfg.max_chain_length = s.uint("Max Chain Length", 1);
+    cfg.default_burn_in = s.uint("Default Burn In", 0);
+    if (s.has("Per Generation Burn In")) {
+      py::object b = s.take("Per Generation Burn In");
+      if (!py::isinstance<py::list>(b)) korali_error(" + Object: [ TMCMC ] \n + Key:    ['Per Generation Burn In']\n + Reason: an array was expected\n");
+      for (auto x : b) {
+        if (!is_number(x) || x.cast<double>() < 0) korali_error(" + Object: [ TMCMC ] \n + Key:    ['Per Generation Burn In']\n + Reason: unsigned integers were expected\n");
+        burn_in.push_back((uint64_t)x.cast<double>());
+      }
+    }
+    cfg.target_cov = s.num("Target Coefficient Of Variation", 1.0);
+    cfg.covariance_scaling = s.num("Covariance Scaling", 0.04);
+    cfg.min_annealing_update = s.num("Min Annealing Exponent Update", 1e-5);
+    cfg.max_annealing_update = s.num("Max Annealing Exponent Update", 1.0);
+    if (s.has("Termination Criteria")) {
+      py::object tco = s.take("Termination Criteria");
+      if (!py::isinstance<py::dict>(tco)) korali_error(" + Object: [ TMCMC ] \n + Key:    ['Termination Criteria']\n + Reason: not an object\n");
+      py::dict tcd;
+      for (auto kv : py::reinterpret_borrow<py::dict>(tco)) tcd[kv.first] = kv.second;
+      Settings tc(tcd, "TMCMC['Termination Criteria']");
+      tc_target = tc.num("Target Annealing Exponent", 1.0);
+      tc_max_generations = tc.num("Max Generations", 1e10);
+      tc_max_model_evaluations = tc.num("Max Model Evaluations", 1e9);
+      tc.finish();
+    }
+    for (const char* g : {"Multinormal Generator", "Uniform Generator", "Normal Generator"}) if (s.has(g)) s.take(g);
+    // the state a result file carries (getConfiguration); a run from such a file stops in restore()
+    for (const char* k : {"Annealing Exponent", "Previous Annealing Exponent", "Coefficient Of Variation", "LogEvidence", "Max Loglikelihood",
+                          "Proposals Acceptance Rate", "Selection Acceptance Rate", "Chain Count", "Model Evaluation Count", "Current Generation",
+                          "Covariance Matrix", "Mean Theta", "Sample Database", "Sample LogLikelihood Database", "Sample LogPrior Database"})
+      if (s.has(k)) s.take(k);
+    s.finish();
+    if (cfg.population_size < 2) korali_error("Sampler/TMCMC: 'Population Size' must be set to at least 2\n");
+    // problem (bayesian/custom.config)
+    py::dict pcopy;
+    for (auto kv : problem) pcopy[kv.first] = kv.second;
+    Settings p(pcopy, "Bayesian/Custom");
+    const std::string ptype = canon(p.str("Type", ""));
+    if (ptype != "bayesian/custom") korali_error("Sampler/TMCMC: only Problem Type 'Bayesian/Custom' is served (got '%s')\n", ptype.c_str());
+    if (!p.has("Likelihood Model")) korali_error(" + Object: [ Bayesian/Custom ] \n + Key:    ['Likelihood Model']\n + Reason: mandatory setting missing\n");
+    model = p.take("Likelihood Model");
+    p.finish();
+    if (py::isinstance<py::str>(model)) {
+      const std::string o = canon(model.cast<std::string>());
+      if (o == "negsphere" || o == "sphere") cfg.loglik = KCMA_OBJ_NEG_SPHERE;
+      else if (o == "negrosenbrock" || o == "rosenbrock") cfg.loglik = KCMA_OBJ_NEG_ROSENBROCK;
+      else if (o == "negackley" || o == "ackley") cfg.loglik = KCMA_OBJ_NEG_ACKLEY;
+      else if (o == "negellipsoid" || o == "ellipsoid") cfg.loglik = KCMA_OBJ_NEG_ELLIPSOID;
+      else if (o == "negsumsq") cfg.loglik = KCMA_OBJ_NEG_SUMSQ;
+      else if (o == "negspheresin2") cfg.loglik = KCMA_OBJ_NEG_SPHERE_SIN2;
+      else korali_error("Unknown device likelihood model '%s' (Sphere, Rosenbrock, Ackley, Ellipsoid, NegSumSq, NegSphereSin2)\n", o.c_str());
+    } else if (PyCallable_Check(model.ptr())) {
+      cfg.loglik = KCMA_OBJ_EXTERNAL;
+      batched = py::hasattr(model, "_korali_batched") ? model.attr("_korali_batched").cast<std::string>() : std::string();
+      if (!batched.empty() && batched != "numpy" && batched != "device") korali_error("Unknown batched model flavour '%s'\n", batched.c_str());
+    } else {
+      korali_error(" + Object: [ Bayesian/Custom ] \n + Key:    ['Likelihood Model']\n + Reason: neither a callable nor the name of a device model\n");
+    }
+    // priors: e["Distributions"][k] = {"Name", "Type", parameters}
+    std::vector<std::string> dname, dtype;
+    std::vector<double> da, db;
+    if (!distributions.is_none()) {
+      if (!py::isinstance<py::list>(distributions)) korali_error(" + Object: [ Experiment ] \n + Key:    ['Distributions']\n + Reason: an array was expected\n");
+      for (auto item : distributions) {
+        if (!py::isinstance<py::dict>(item)) korali_error("Distributions: every entry must be an object\n");
+        py::dict dcopy;
+        for (auto kv : py::reinterpret_borrow<py::dict>(item)) dcopy[kv.first] = kv.second;
+        Settings d(dcopy, "Distribution");
+        const std::string nm = d.str("Name", ""), ty = d.str("Type", "");
+        const std::string ct = canon(ty);
+        double a = NAN, b = NAN;
+        if (ct == "univariate/uniform") { a = d.num("Minimum", NAN); b = d.num("Maximum", NAN); dtype.push_back("uniform"); }
+        else if (ct == "univariate/normal") { a = d.num("Mean", NAN); b = d.num("Standard Deviation", NAN); dtype.push_back("normal"); }
+        else korali_error("Sampler/TMCMC: prior distribution type '%s' of '%s' is not built (Univariate/Uniform, Univariate/Normal)\n", ty.c_str(), nm.c_str());
+        if (d.has("Random Seed")) d.take("Random Seed");
+        d.finish();
+        if (!std::isfinite(a) || !std::isfinite(b)) korali_error("Distribution '%s' (%s): its parameters must be set to finite numbers\n", nm.c_str(), ty.c_str());
+        dname.push_back(nm); da.push_back(a); db.push_back(b);
+      }
+    }
+    const size_t n = py::len(variables);
+    if (n == 0) korali_error("Bayesian problems require at least one variable.\n");
+    lower.assign(n, -INFINITY); upper.assign(n, INFINITY);
+    prior_type.assign(n, 0); prior_a.assign(n, 0.0); prior_b.assign(n, 0.0); prior_name.assign(n, "");
+    for (size_t i = 0; i < n; i++) {
+      if (!py::isinstance<py::dict>(variables[i])) korali_error("Variable %zu is not an object\n", i);
+      py::dict vcopy;
+      for (auto kv : py::reinterpret_borrow<py::dict>(variables[i])) vcopy[kv.first] = kv.second;
+      Settings v(vcopy, "Variable");
+      const std::string vname = v.str("Name", "");
+      if (!v.has("Prior Distribution")) korali_error("Variable %zu ('%s') has no 'Prior Distribution'\n", i, vname.c_str());
+      const std::string pd = v.str("Prior Distribution", "");
+      v.num("Lower Bound", -INFINITY); v.num("Upper Bound", INFINITY);   // written back by getConfiguration
+      v.finish();
+      size_t k = 0;
+      while (k < dname.size() && dname[k] != pd) k++;
+      if (k == dname.size()) korali_error("Variable %zu ('%s'): prior distribution '%s' is not defined in e['Distributions']\n", i, vname.c_str(), pd.c_str());
+      prior_name[i] = pd;
+      prior_type[i] = dtype[k] == "uniform" ? KTMCMC_PRIOR_UNIFORM : KTMCMC_PRIOR_NORMAL;
+      prior_a[i] = da[k]; prior_b[i] = db[k];
+      if (prior_type[i] == KTMCMC_PRIOR_UNIFORM) { lower[i] = da[k]; upper[i] = db[k]; }
+    }
+    cfg.n = n; cfg.seed = seed;
+    cfg.prior_type = prior_type.data(); cfg.prior_a = prior_a.data(); cfg.prior_b = prior_b.data();
+    cfg.per_generation_burn_in = burn_in.empty() ? nullptr : burn_in.data(); cfg.burn_in_count = burn_in.size();
+  }
+
+  // Bayesian/Custom "Evaluate": the model sets sample["logLikelihood"]
+  static void host_loglik(void* user, const double* x, uint64_t rows, uint64_t n, double* l_out) {
+    TMCMC* self = (TMCMC*)user;
+    try {
+      if (self->batched == "numpy") {
+        py::array_t<double> X({(py::ssize_t)rows, (py::ssize_t)n}, {(py::ssize_t)(n * sizeof(double)), (py::ssize_t)sizeof(double)}, x, py::none());
+        py::array_t<double, py::array::c_style | py::array::forcecast> F(self->model(X));
+        if ((uint64_t)F.size() != rows) korali_error("The batched model returned %zu values for %zu samples\n", (size_t)F.size(), (size_t)rows);
+        for (uint64_t i = 0; i < rows; i++) l_out[i] = F.data()[i];
+        return;
+      }
+      for (uint64_t i = 0; i < rows; i++) {
+        py::dict sample;
+        py::list params;
+        for (uint64_t d = 0; d < n; d++) params.append(x[i * n + d]);
+        sample["Parameters"] = params;
+        sample["Sample Id"] = i;
+        sample["Module"] = "Problem";
+        sample["Operation"] = "Evaluate";
+        self->model(sample);
+        if (!sample.contains("logLikelihood")) korali_error("The model did not set 'logLikelihood' for sample %zu\n", (size_t)i);
+        l_out[i] = sample["logLikelihood"].cast<double>();
+      }
+    } catch (const std::exception& e) {
+      self->pending_error = e.what();
+      for (uint64_t i = 0; i < rows; i++) l_out[i] = 0.0;
+    }
+  }
+  static void device_loglik(void* user, const double* x_dev, uint64_t rows, uint64_t n, uint64_t ldx, double* f_dev, void* stream) {
+    TMCMC* self = (TMCMC*)user;
+    try {
+      self->model((uintptr_t)x_dev, rows, n, ldx, (uintptr_t)f_dev, (uintptr_t)stream);
+    } catch (const std::exception& e) {
+      self->pending_error = e.what();
+    }
+  }
+
+  void initialize(const std::vector<int>& device_ids) override {
+    if (device_ids.size() > 1) korali_error("Sampler/TMCMC runs on one device (k['Conduit']['Devices'] > 1 is built for Optimizer/CMAES)\n");
+    cfg.device = device_ids[0];
+    if (ktmcmc_create(&cfg, &h)) korali_error("%s", ktmcmc_last_error(nullptr));
+    if (cfg.loglik == KCMA_OBJ_EXTERNAL) {
+      if (batched == "device") check(ktmcmc_set_device_loglik(h, &TMCMC::device_loglik, this));
+      else check(ktmcmc_set_host_loglik(h, &TMCMC::host_loglik, this));
+    }
+    check(ktmcmc_set_scalar(h, "Termination Criteria/Target Annealing Exponent", tc_target));
+    check(ktmcmc_set_scalar(h, "Termination Criteria/Max Generations", tc_max_generations));
+    check(ktmcmc_set_scalar(h, "Termination Criteria/Max Model Evaluations", tc_max_model_evaluations));
+  }
+
+  void restore(uint64_t generation) override {
+    if (generation != 0) korali_error("Resuming a Sampler/TMCMC run from a result file is not built on the B200 path\n");
+  }
+
+  bool checkTermination() override {
+    int fin = 0;
+    const char* reason = "";
+    check(ktmcmc_check_termination(h, &fin, &reason));
+    if (fin) splitReasons(reason);
+    return fin != 0;
+  }
+
+  void runGeneration() override {
+    pending_error.clear();
+    int rc;
+    if (!needsPython()) { py::gil_scoped_release nogil; rc = ktmcmc_run_generation(h); }
+    else rc = ktmcmc_run_generation(h);
+    if (!pending_error.empty()) { std::string e = pending_error; pending_error.clear(); throw std::runtime_error(e); }
+    check(rc);
+  }
+  bool needsPython() const override { return cfg.loglik == KCMA_OBJ_EXTERNAL; }
+
+  py::list rowsOf(const std::vector<double>& flat, size_t width) {
+    py::list out;
+    for (size_t i = 0; width && (i + 1) * width <= flat.size(); i++) out.append(std::vector<double>(flat.begin() + i * width, flat.begin() + (i + 1) * width));
+    return out;
+  }
+
+  void printGeneration(const std::function<void(int, const char*)>& log) override {   // TMCMC::printGenerationAfter
+    char b[256];
+    snprintf(b, sizeof(b), "Acceptance Rate (proposals / selections): (%.2f%% / %.2f%%)\n", 100. * scalar("Proposals Acceptance Rate"),
+             100. * scalar("Selection Acceptance Rate"));
+    log(NORMAL, b);
+    snprintf(b, sizeof(b), "Coefficient of Variation: %.2f%%\n", 100. * scalar("Coefficient Of Variation")); log(NORMAL, b);
+    snprintf(b, sizeof(b), "Annealing Exponent:  %.3e.\n", scalar("Annealing Exponent")); log(NORMAL, b);
+    snprintf(b, sizeof(b), "Log Evidence: %.3e\n", scalar("LogEvidence")); log(DETAILED, b);
+  }
+
+  bool finalize(py::dict results, const std::function<void(int, const char*)>& log) override {
+    results["Posterior Sample Database"] = rowsOf(array("Sample Database"), cfg.n);
+    results["Posterior Sample LogLikelihood Database"] = array("Sample LogLikelihood Database");
+    results["Posterior Sample LogPrior Database"] = array("Sample LogPrior Database");
+    results["Log Evidence"] = scalar("LogEvidence");
+    char b[128];
+    log(MINIMAL, "--------------------------------------------------------------------\n");
+    snprintf(b, sizeof(b), "Log Evidence: %.4e\n", scalar("LogEvidence")); log(MINIMAL, b);
+    log(MINIMAL, "Sampler/TMCMC finished correctly.\n");
+    return true;
+  }
+
+  void getConfiguration(py::dict js) override {
+    js["Type"] = "Sampler/TMCMC";
+    js["Version"] = "TMCMC";
+    js["Population Size"] = cfg.population_size;
+    js["Max Chain Length"] = cfg.max_chain_length;
+    js["Default Burn In"] = cfg.default_burn_in;
+    js["Per Generation Burn In"] = burn_in;
+    js["Target Coefficient Of Variation"] = cfg.target_cov;
+    js["Covariance Scaling"] = cfg.covariance_scaling;
+    js["Min Annealing Exponent Update"] = cfg.min_annealing_update;
+    js["Max Annealing Exponent Update"] = cfg.max_annealing_update;
+    py::dict tc;
+    tc["Target Annealing Exponent"] = tc_target; tc["Max Generations"] = tc_max_generations; tc["Max Model Evaluations"] = tc_max_model_evaluations;
+    js["Termination Criteria"] = tc;
+    for (const char* k : {"Annealing Exponent", "Previous Annealing Exponent", "Coefficient Of Variation", "LogEvidence", "Max Loglikelihood",
+                          "Proposals Acceptance Rate", "Selection Acceptance Rate"})
+      js[k] = scalar(k);
+    for (const char* k : {"Chain Count", "Model Evaluation Count", "Current Generation"}) js[k] = (uint64_t)scalar(k);
+    const size_t n = cfg.n;
+    js["Covariance Matrix"] = rowsOf(array("Covariance Matrix"), n);
+    js["Mean Theta"] = array("Mean Theta");
+    js["Sample Database"] = rowsOf(array("Sample Database"), n);
+    js["Sample LogLikelihood Database"] = array("Sample LogLikelihood Database");
+    js["Sample LogPrior Database"] = array("Sample LogPrior Database");
+  }
+};
+
 class Experiment : public KoraliJson {
  public:
   std::unique_ptr<SolverBase> solver;
@@ -1304,13 +1575,16 @@ class Experiment : public KoraliJson {
     py::dict problem_js = py::reinterpret_borrow<py::dict>(top.take("Problem"));
     py::list variables = py::reinterpret_borrow<py::list>(top.take("Variables"));
     const std::string stype = canon(solver_js.contains("Type") && py::isinstance<py::str>(solver_js["Type"]) ? solver_js["Type"].cast<std::string>() : "");
-    if (stype != "optimizer/cmaes" && stype != "cmaes" && stype != "optimizer/dea" && stype != "dea" && stype != "optimizer/mocmaes" && stype != "mocmaes")
-      korali_error("Solver Type '%s' is not served by korali_b200: only 'Optimizer/CMAES', 'Optimizer/DEA' and 'Optimizer/MOCMAES' are built (SURVEY.md scope)\n", stype.c_str());
+    const bool tmcmc = stype == "sampler/tmcmc" || stype == "tmcmc";
+    if (stype != "optimizer/cmaes" && stype != "cmaes" && stype != "optimizer/dea" && stype != "dea" && stype != "optimizer/mocmaes" && stype != "mocmaes" && !tmcmc)
+      korali_error("Solver Type '%s' is not served by korali_b200: only 'Optimizer/CMAES', 'Optimizer/DEA', 'Optimizer/MOCMAES' and 'Sampler/TMCMC' are built (SURVEY.md scope)\n", stype.c_str());
     random_seed = top.uint("Random Seed", 0);
     if (random_seed == 0) random_seed = (uint64_t)std::chrono::system_clock::now().time_since_epoch().count();  // experiment.cpp.base:235-251
     top.boolean("Preserve Random Number Generator States", 0);
     top.boolean("Store Sample Information", 0);
     current_generation = top.uint("Current Generation", 0);
+    py::object distributions = py::none();   // the priors of Sampler/TMCMC; the optimizers ignore the key
+    if (tmcmc && top.has("Distributions")) distributions = top.take("Distributions");
     for (const char* k : {"Distributions", "Results", "Samples", "Globals", "Run ID", "Timestamp", "Type", "Is Finished"}) if (top.has(k)) top.take(k);
     if (top.has("Console Output")) {
       py::object co = top.take("Console Output");
@@ -1341,6 +1615,7 @@ class Experiment : public KoraliJson {
     top.finish();
     if (stype == "optimizer/dea" || stype == "dea") solver = std::make_unique<DEA>();
     else if (stype == "optimizer/mocmaes" || stype == "mocmaes") solver = std::make_unique<MOCMAES>();
+    else if (tmcmc) { auto t = std::make_unique<TMCMC>(); t->distributions = distributions; solver = std::move(t); }
     else solver = std::make_unique<CMAES>();
     solver->setConfiguration(solver_js, variables, problem_js, random_seed);   // Normal Generator gets seed S (distribution.cpp.base:36-37)
     solver->initialize(devices);
