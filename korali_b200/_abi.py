@@ -50,46 +50,53 @@ def _as_dp(a):
     return a.ctypes.data_as(_dp)
 
 
-class Handle:
-    """A solver handle of libkcma.so (prefix 'kcma_') — or of the oracle (prefix 'okcma_') in tests."""
+class HandleBase:
+    """A solver handle of one of the C ABIs of libkcma.so (kcma_, kdea_, kmocma_, ktmcmc_), or of a CPU oracle behind the same
+    vocabulary in tests (okcma_, odea_, omocma_, otmcmc_). The ABIs share the shape of their entry points; a subclass names its cfg
+    struct and how keyword arguments fill it:
+      CFG     the ctypes mirror of <prefix>cfg
+      ARRAYS  the double-array fields, broadcast to n values (None leaves the field NULL)
+      ENUMS   {field: {name: value}} for fields that also take a name
+    Any other keyword goes to _field, and then to the cfg field of its name."""
+    CFG = None
+    ARRAYS = ()
+    ENUMS = {}
 
     def __init__(self, lib, prefix, **kw):
-        self._lib, self._p = lib, prefix
-        self._keep = []
-        cfg = KcmaCfg()
-        self._fn("cfg_defaults", None, [C.POINTER(KcmaCfg)])(C.byref(cfg))
-        n = int(kw["n"])
+        self._lib, self._p, self._keep = lib, prefix, []
+        cfg = self.CFG()
+        self._fn("cfg_defaults", None, [C.POINTER(self.CFG)])(C.byref(cfg))
+        self.n = n = int(kw["n"])
         for k, v in kw.items():
-            if k in ("lower_bound", "upper_bound", "initial_value", "initial_stddev", "min_stddev_update",
-                     "objective_coef", "constraint_shift", "granularity"):
-                if v is None:
-                    continue
-                want = int(kw.get("n_constraints", 0)) if k == "constraint_shift" else n
-                arr = np.ascontiguousarray(np.broadcast_to(np.asarray(v, dtype=np.float64), (want,)))
-                self._keep.append(arr)
-                setattr(cfg, k, _as_dp(arr))
-            elif k == "mu_type":
-                cfg.mu_type = MU_TYPES[v] if isinstance(v, str) else int(v)
-            elif k == "objective":
-                cfg.objective = OBJECTIVES[v] if isinstance(v, str) else int(v)
-            elif k == "constraint_family":
-                cfg.constraint_family = CONSTRAINTS[v] if isinstance(v, str) else int(v)
-            else:
+            if k in self.ARRAYS:
+                if v is not None:
+                    setattr(cfg, k, self._array(v, n))
+            elif k in self.ENUMS:
+                setattr(cfg, k, self.ENUMS[k][v] if isinstance(v, str) else int(v))
+            elif not self._field(cfg, k, v, kw):
                 setattr(cfg, k, v)
-        self.n = n
         self._h = C.c_void_p()
-        create = self._fn("create", C.c_int, [C.POINTER(KcmaCfg), C.POINTER(C.c_void_p)])
-        if create(C.byref(cfg), C.byref(self._h)) != 0:
+        if self._fn("create", C.c_int, [C.POINTER(self.CFG), C.POINTER(C.c_void_p)])(C.byref(cfg), C.byref(self._h)) != 0:
             raise KcmaError(self._fn("last_error", C.c_char_p, [C.c_void_p])(None).decode())
+        self._created(cfg)
+
+    def _array(self, v, count, dtype=np.float64):
+        """A pointer to a contiguous copy of v broadcast to count values, kept alive with the handle."""
+        arr = np.ascontiguousarray(np.broadcast_to(np.asarray(v, dtype=dtype), (count,)))
+        self._keep.append(arr)
+        return arr.ctypes.data_as(C.POINTER(np.ctypeslib.as_ctypes_type(dtype)))
+
+    def _field(self, cfg, k, v, kw):
+        """Fills a cfg field that needs more than a plain assignment; returns whether it did."""
+        return False
+
+    def _created(self, cfg):
+        """Runs once the handle exists."""
 
     def _fn(self, name, restype, argtypes):
         f = getattr(self._lib, self._p + name)
         f.restype, f.argtypes = restype, argtypes
         return f
-
-    def _check(self, rc):
-        if rc != 0:
-            raise KcmaError(self._fn("last_error", C.c_char_p, [C.c_void_p])(self._live()).decode())
 
     def _live(self):
         """The handle, or an error instead of a NULL pointer into the library once close() was called."""
@@ -97,37 +104,55 @@ class Handle:
             raise KcmaError("the solver handle is closed")
         return self._h
 
+    def _check(self, rc):
+        if rc != 0:
+            raise KcmaError(self._fn("last_error", C.c_char_p, [C.c_void_p])(self._live()).decode())
+
     def close(self):
         if getattr(self, "_h", None):
             self._fn("destroy", None, [C.c_void_p])(self._h)
             self._h = None
 
-    __del__ = close
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
 
     # --- generation loop
-    def ask(self): self._check(self._fn("ask", C.c_int, [C.c_void_p])(self._live()))
-    def eval(self): self._check(self._fn("eval", C.c_int, [C.c_void_p])(self._live()))
-    def tell(self): self._check(self._fn("tell", C.c_int, [C.c_void_p])(self._live()))
-    def run_generation(self): self._check(self._fn("run_generation", C.c_int, [C.c_void_p])(self._live()))
+    def _call(self, name):
+        self._check(self._fn(name, C.c_int, [C.c_void_p])(self._live()))
+
+    def ask(self): self._call("ask")
+    def eval(self): self._call("eval")
+    def tell(self): self._call("tell")
+    def run_generation(self): self._call("run_generation")
 
     def run(self, max_generations):
         done = C.c_uint64(0)
         self._check(self._fn("run", C.c_int, [C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)])(
-            self._h, int(max_generations), C.byref(done)))
+            self._live(), int(max_generations), C.byref(done)))
         return done.value
 
     def check_termination(self):
         fin, reason = C.c_int(0), C.c_char_p()
         self._check(self._fn("check_termination", C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_char_p)])(
-            self._h, C.byref(fin), C.byref(reason)))
+            self._live(), C.byref(fin), C.byref(reason)))
         return bool(fin.value), (reason.value or b"").decode()
 
-    def take_warnings(self):
-        return self._fn("take_warnings", C.c_char_p, [C.c_void_p])(self._live()).decode()
-
-    def inject(self, kind, data):
+    def _inject(self, name, data):
         a = np.ascontiguousarray(data, dtype=np.float64).ravel()
-        self._check(self._fn("inject", C.c_int, [C.c_void_p, C.c_int, _dp, C.c_size_t])(self._live(), kind, _as_dp(a), a.size))
+        self._check(self._fn(name, C.c_int, [C.c_void_p, _dp, C.c_size_t])(self._live(), _as_dp(a), a.size))
+
+    def _set_callback(self, name, cb_t, fn, shape):
+        """Registers fn(X: ndarray[rows, n]) with <prefix><name> as the host callback cb_t(user, x, rows, n, out, *extra); fn's result
+        is written to out as an array of shape(rows, n, *extra)."""
+        def tramp(_u, x, rows, n, out, *extra):
+            s = shape(rows, n, *extra)
+            np.ctypeslib.as_array(out, shape=s)[:] = np.asarray(fn(np.ctypeslib.as_array(x, shape=(rows, n))), dtype=np.float64).reshape(s)
+        cb = cb_t(tramp)
+        self._keep.append(cb)
+        self._check(self._fn(name, C.c_int, [C.c_void_p, cb_t, C.c_void_p])(self._live(), cb, None))
 
     # --- state
     def get(self, key):
@@ -136,20 +161,13 @@ class Handle:
         cnt = C.c_size_t(0)
         self._check(f(self._live(), key.encode(), None, 0, C.byref(cnt)))
         out = np.empty(cnt.value, dtype=np.float64)
-        self._check(f(self._live(), key.encode(), _as_dp(out), out.size, C.byref(cnt)))
+        if cnt.value:
+            self._check(f(self._live(), key.encode(), _as_dp(out), out.size, C.byref(cnt)))
         return out
 
     def set(self, key, data):
         a = np.ascontiguousarray(data, dtype=np.float64).ravel()
         self._check(self._fn("set_array", C.c_int, [C.c_void_p, C.c_char_p, _dp, C.c_size_t])(self._live(), key.encode(), _as_dp(a), a.size))
-
-    def get_index(self, key):
-        f = self._fn("get_index_array", C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_uint64), C.c_size_t, C.POINTER(C.c_size_t)])
-        cnt = C.c_size_t(0)
-        self._check(f(self._live(), key.encode(), None, 0, C.byref(cnt)))
-        out = np.empty(cnt.value, dtype=np.uint64)
-        self._check(f(self._live(), key.encode(), out.ctypes.data_as(C.POINTER(C.c_uint64)), out.size, C.byref(cnt)))
-        return out
 
     def scalar(self, key):
         v = C.c_double(math.nan)
@@ -158,3 +176,35 @@ class Handle:
 
     def set_scalar(self, key, value):
         self._check(self._fn("set_scalar", C.c_int, [C.c_void_p, C.c_char_p, C.c_double])(self._live(), key.encode(), float(value)))
+
+    def launch_count(self):
+        return self._fn("launch_count", C.c_uint64, [C.c_void_p])(self._live())
+
+
+class Handle(HandleBase):
+    """A CMA-ES solver handle of libkcma.so (prefix 'kcma_') — or of the oracle (prefix 'okcma_') in tests."""
+    CFG = KcmaCfg
+    ARRAYS = ("lower_bound", "upper_bound", "initial_value", "initial_stddev", "min_stddev_update", "objective_coef", "granularity")
+    ENUMS = {"mu_type": MU_TYPES, "objective": OBJECTIVES, "constraint_family": CONSTRAINTS}
+
+    def _field(self, cfg, k, v, kw):
+        if k != "constraint_shift":
+            return False
+        if v is not None:
+            cfg.constraint_shift = self._array(v, int(kw.get("n_constraints", 0)))
+        return True
+
+    def take_warnings(self):
+        return self._fn("take_warnings", C.c_char_p, [C.c_void_p])(self._live()).decode()
+
+    def inject(self, kind, data):
+        a = np.ascontiguousarray(data, dtype=np.float64).ravel()
+        self._check(self._fn("inject", C.c_int, [C.c_void_p, C.c_int, _dp, C.c_size_t])(self._live(), kind, _as_dp(a), a.size))
+
+    def get_index(self, key):
+        f = self._fn("get_index_array", C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_uint64), C.c_size_t, C.POINTER(C.c_size_t)])
+        cnt = C.c_size_t(0)
+        self._check(f(self._live(), key.encode(), None, 0, C.byref(cnt)))
+        out = np.empty(cnt.value, dtype=np.uint64)
+        self._check(f(self._live(), key.encode(), out.ctypes.data_as(C.POINTER(C.c_uint64)), out.size, C.byref(cnt)))
+        return out

@@ -1,9 +1,7 @@
 """ctypes mirror of include/kdea.h (Differential Evolution on libkcma.so). Generic over the symbol prefix so that the CPU oracle
 (oracle/libokcma.so, prefix ``odea_``; test infrastructure only) can be driven with the same vocabulary. Nothing here loads the oracle."""
 import ctypes as C
-import math
-import numpy as np
-from ._abi import KcmaError, OBJECTIVES, _as_dp, _dp
+from ._abi import HandleBase, OBJECTIVES, _dp
 
 KDEA_ABI_VERSION = 1
 PARENT_RULES = {"Random": 0, "Best": 1}
@@ -23,102 +21,16 @@ class KdeaCfg(C.Structure):
     ]
 
 
-class DeaHandle:
-    def __init__(self, lib, prefix, **kw):
-        self._lib, self._p, self._keep = lib, prefix, []
-        cfg = KdeaCfg()
-        self._fn("cfg_defaults", None, [C.POINTER(KdeaCfg)])(C.byref(cfg))
-        n = int(kw["n"])
-        for k, v in kw.items():
-            if k in ("lower_bound", "upper_bound", "objective_coef"):
-                if v is None:
-                    continue
-                arr = np.ascontiguousarray(np.broadcast_to(np.asarray(v, dtype=np.float64), (n,)))
-                self._keep.append(arr)
-                setattr(cfg, k, _as_dp(arr))
-            elif k == "objective":
-                cfg.objective = OBJECTIVES[v] if isinstance(v, str) else int(v)
-            elif k == "parent_selection_rule":
-                cfg.parent_selection_rule = PARENT_RULES[v] if isinstance(v, str) else int(v)
-            elif k == "accept_rule":
-                cfg.accept_rule = ACCEPT_RULES[v] if isinstance(v, str) else int(v)
-            elif k == "mutation_rule":
-                cfg.mutation_rule = MUTATION_RULES[v] if isinstance(v, str) else int(v)
-            else:
-                setattr(cfg, k, v)
-        self.n, self.population_size = n, int(cfg.population_size)
-        self._h = C.c_void_p()
-        if self._fn("create", C.c_int, [C.POINTER(KdeaCfg), C.POINTER(C.c_void_p)])(C.byref(cfg), C.byref(self._h)) != 0:
-            raise KcmaError(self._fn("last_error", C.c_char_p, [C.c_void_p])(None).decode())
+class DeaHandle(HandleBase):
+    CFG = KdeaCfg
+    ARRAYS = ("lower_bound", "upper_bound", "objective_coef")
+    ENUMS = {"objective": OBJECTIVES, "parent_selection_rule": PARENT_RULES, "accept_rule": ACCEPT_RULES, "mutation_rule": MUTATION_RULES}
 
-    def _fn(self, name, restype, argtypes):
-        f = getattr(self._lib, self._p + name)
-        f.restype, f.argtypes = restype, argtypes
-        return f
-
-    def _live(self):
-        if not getattr(self, "_h", None):
-            raise KcmaError("the solver handle is closed")
-        return self._h
-
-    def _check(self, rc):
-        if rc != 0:
-            raise KcmaError(self._fn("last_error", C.c_char_p, [C.c_void_p])(self._live()).decode())
-
-    def close(self):
-        if getattr(self, "_h", None):
-            self._fn("destroy", None, [C.c_void_p])(self._h)
-            self._h = None
-
-    __del__ = close
-
-    def ask(self): self._check(self._fn("ask", C.c_int, [C.c_void_p])(self._live()))
-    def eval(self): self._check(self._fn("eval", C.c_int, [C.c_void_p])(self._live()))
-    def tell(self): self._check(self._fn("tell", C.c_int, [C.c_void_p])(self._live()))
-    def run_generation(self): self._check(self._fn("run_generation", C.c_int, [C.c_void_p])(self._live()))
-
-    def run(self, max_generations):
-        done = C.c_uint64(0)
-        self._check(self._fn("run", C.c_int, [C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)])(self._live(), int(max_generations), C.byref(done)))
-        return done.value
-
-    def check_termination(self):
-        fin, reason = C.c_int(0), C.c_char_p()
-        self._check(self._fn("check_termination", C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_char_p)])(
-            self._live(), C.byref(fin), C.byref(reason)))
-        return bool(fin.value), (reason.value or b"").decode()
+    def _created(self, cfg):
+        self.population_size = int(cfg.population_size)
 
     def inject_f(self, f):
-        a = np.ascontiguousarray(f, dtype=np.float64).ravel()
-        self._check(self._fn("inject_f", C.c_int, [C.c_void_p, _dp, C.c_size_t])(self._live(), _as_dp(a), a.size))
-
-    def get(self, key):
-        f = self._fn("get_array", C.c_int, [C.c_void_p, C.c_char_p, _dp, C.c_size_t, C.POINTER(C.c_size_t)])
-        cnt = C.c_size_t(0)
-        self._check(f(self._live(), key.encode(), None, 0, C.byref(cnt)))
-        out = np.empty(cnt.value, dtype=np.float64)
-        self._check(f(self._live(), key.encode(), _as_dp(out), out.size, C.byref(cnt)))
-        return out
-
-    def set(self, key, data):
-        a = np.ascontiguousarray(data, dtype=np.float64).ravel()
-        self._check(self._fn("set_array", C.c_int, [C.c_void_p, C.c_char_p, _dp, C.c_size_t])(self._live(), key.encode(), _as_dp(a), a.size))
-
-    def scalar(self, key):
-        v = C.c_double(math.nan)
-        self._check(self._fn("get_scalar", C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_double)])(self._live(), key.encode(), C.byref(v)))
-        return v.value
-
-    def set_scalar(self, key, value):
-        self._check(self._fn("set_scalar", C.c_int, [C.c_void_p, C.c_char_p, C.c_double])(self._live(), key.encode(), float(value)))
-
-    def launch_count(self):
-        return self._fn("launch_count", C.c_uint64, [C.c_void_p])(self._live())
-
-
-DEA_EXPORTS = ["kdea_cfg_defaults", "kdea_create", "kdea_destroy", "kdea_last_error", "kdea_run_generation", "kdea_ask", "kdea_eval", "kdea_tell",
-               "kdea_set_host_objective", "kdea_inject_f", "kdea_check_termination", "kdea_run", "kdea_get_array", "kdea_set_array",
-               "kdea_get_scalar", "kdea_set_scalar", "kdea_launch_count"]
+        self._inject("inject_f", f)
 
 
 class Solver(DeaHandle):
@@ -130,10 +42,5 @@ class Solver(DeaHandle):
 
     def set_host_objective(self, fn):
         """fn(X: ndarray[rows, n]) -> ndarray[rows]; the batched host conduit."""
-        cb_t = C.CFUNCTYPE(None, C.c_void_p, _dp, C.c_uint64, C.c_uint64, _dp)
-
-        def tramp(_u, x, rows, n, out):
-            xs = np.ctypeslib.as_array(x, shape=(rows, n))
-            np.ctypeslib.as_array(out, shape=(rows,))[:] = np.asarray(fn(xs), dtype=np.float64)
-        self._host_obj = cb_t(tramp)
-        self._check(self._fn("set_host_objective", C.c_int, [C.c_void_p, cb_t, C.c_void_p])(self._live(), self._host_obj, None))
+        self._set_callback("set_host_objective", C.CFUNCTYPE(None, C.c_void_p, _dp, C.c_uint64, C.c_uint64, _dp), fn,
+                           lambda rows, n: (rows,))

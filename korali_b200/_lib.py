@@ -70,18 +70,10 @@ class Solver(Handle):
             self._h, phase.encode(), C.byref(ms), C.byref(calls))
         return ms.value, calls.value
 
-    def launch_count(self):
-        return self._fn("launch_count", C.c_uint64, [C.c_void_p])(self._live())
-
     def set_host_objective(self, fn):
         """fn(X: ndarray[rows, n]) -> ndarray[rows]; the batched host conduit (needs keep_population=1)."""
-        cb_t = C.CFUNCTYPE(None, C.c_void_p, _dp, C.c_uint64, C.c_uint64, _dp)
-
-        def tramp(_u, x, rows, n, out):
-            xs = np.ctypeslib.as_array(x, shape=(rows, n))
-            np.ctypeslib.as_array(out, shape=(rows,))[:] = np.asarray(fn(xs), dtype=np.float64)
-        self._host_obj = cb_t(tramp)
-        self._check(self._fn("set_host_objective", C.c_int, [C.c_void_p, cb_t, C.c_void_p])(self._live(), self._host_obj, None))
+        self._set_callback("set_host_objective", C.CFUNCTYPE(None, C.c_void_p, _dp, C.c_uint64, C.c_uint64, _dp), fn,
+                           lambda rows, n: (rows,))
 
     def set_host_objective_grad(self, fn):
         """fn(X: ndarray[rows, n]) -> (F: ndarray[rows], dF/dX: ndarray[rows, n]); needs use_gradient_information=1."""
@@ -97,13 +89,8 @@ class Solver(Handle):
 
     def set_host_constraints(self, fn):
         """fn(X: ndarray[rows, n]) -> ndarray[n_constraints, rows]."""
-        cb_t = C.CFUNCTYPE(None, C.c_void_p, _dp, C.c_uint64, C.c_uint64, _dp, C.c_uint64)
-
-        def tramp(_u, x, rows, n, out, nc):
-            xs = np.ctypeslib.as_array(x, shape=(rows, n))
-            np.ctypeslib.as_array(out, shape=(nc, rows))[:] = np.asarray(fn(xs), dtype=np.float64).reshape(nc, rows)
-        self._host_con = cb_t(tramp)
-        self._check(self._fn("set_host_constraints", C.c_int, [C.c_void_p, cb_t, C.c_void_p])(self._live(), self._host_con, None))
+        self._set_callback("set_host_constraints", C.CFUNCTYPE(None, C.c_void_p, _dp, C.c_uint64, C.c_uint64, _dp, C.c_uint64), fn,
+                           lambda rows, n, nc: (nc, rows))
 
     def flush_l2(self):
         self._check(self._fn("flush_l2", C.c_int, [C.c_void_p])(self._live()))

@@ -1,8 +1,7 @@
 """ctypes mirror of include/kmocma.h (multi-objective CMA-ES on libkcma.so). Generic over the symbol prefix so that the CPU oracle
 (oracle/libokcma.so, prefix ``omocma_``; test infrastructure only) can be driven with the same vocabulary. Nothing here loads the oracle."""
 import ctypes as C
-import numpy as np
-from ._abi import KcmaError, _as_dp, _dp
+from ._abi import HandleBase, _dp
 
 KMOCMA_ABI_VERSION = 1
 OBJECTIVES = {"External": 0, "NegRosenbrockAndSphere": 1, "NegRosenbrockAndTwoSpheres": 2}
@@ -21,100 +20,21 @@ class KmocmaCfg(C.Structure):
     ]
 
 
-class MocmaHandle:
-    def __init__(self, lib, prefix, **kw):
-        self._lib, self._p, self._keep = lib, prefix, []
-        cfg = KmocmaCfg()
-        self._fn("cfg_defaults", None, [C.POINTER(KmocmaCfg)])(C.byref(cfg))
-        n = int(kw["n"])
-        for k, v in kw.items():
-            if k in ("lower_bound", "upper_bound", "initial_value", "initial_stddev"):
-                if v is None:
-                    continue
-                arr = np.ascontiguousarray(np.broadcast_to(np.asarray(v, dtype=np.float64), (n,)))
-                self._keep.append(arr)
-                setattr(cfg, k, _as_dp(arr))
-            elif k == "objective":
-                cfg.objective = OBJECTIVES[v] if isinstance(v, str) else int(v)
-            else:
-                setattr(cfg, k, v)
-        self._h = C.c_void_p()
-        if self._fn("create", C.c_int, [C.POINTER(KmocmaCfg), C.POINTER(C.c_void_p)])(C.byref(cfg), C.byref(self._h)) != 0:
-            raise KcmaError(self._fn("last_error", C.c_char_p, [C.c_void_p])(None).decode())
-        self.n, self.num_objectives = n, int(cfg.num_objectives)
+class MocmaHandle(HandleBase):
+    CFG = KmocmaCfg
+    ARRAYS = ("lower_bound", "upper_bound", "initial_value", "initial_stddev")
+    ENUMS = {"objective": OBJECTIVES}
+
+    def _created(self, cfg):
+        self.num_objectives = int(cfg.num_objectives)
         self.population_size, self.mu_value = int(self.scalar("Population Size")), int(self.scalar("Mu Value"))
 
-    def _fn(self, name, restype, argtypes):
-        f = getattr(self._lib, self._p + name)
-        f.restype, f.argtypes = restype, argtypes
-        return f
-
-    def _live(self):
-        if not getattr(self, "_h", None):
-            raise KcmaError("the solver handle was closed")
-        return self._h
-
-    def _check(self, rc):
-        if rc != 0:
-            raise KcmaError(self._fn("last_error", C.c_char_p, [C.c_void_p])(self._h).decode())
-
-    def close(self):
-        if getattr(self, "_h", None):
-            self._fn("destroy", None, [C.c_void_p])(self._h)
-            self._h = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def ask(self): self._check(self._fn("ask", C.c_int, [C.c_void_p])(self._live()))
-    def eval(self): self._check(self._fn("eval", C.c_int, [C.c_void_p])(self._live()))
-    def tell(self): self._check(self._fn("tell", C.c_int, [C.c_void_p])(self._live()))
-    def run_generation(self): self._check(self._fn("run_generation", C.c_int, [C.c_void_p])(self._live()))
-
-    def run(self, max_generations):
-        done = C.c_uint64(0)
-        self._check(self._fn("run", C.c_int, [C.c_void_p, C.c_uint64, C.POINTER(C.c_uint64)])(self._live(), int(max_generations), C.byref(done)))
-        return done.value
-
-    def check_termination(self):
-        fin, why = C.c_int(0), C.c_char_p()
-        self._check(self._fn("check_termination", C.c_int, [C.c_void_p, C.POINTER(C.c_int), C.POINTER(C.c_char_p)])(self._live(), C.byref(fin), C.byref(why)))
-        return bool(fin.value), (why.value or b"").decode()
-
     def inject_f(self, f):
-        f = np.ascontiguousarray(f, dtype=np.float64).reshape(-1)
-        self._check(self._fn("inject_f", C.c_int, [C.c_void_p, _dp, C.c_size_t])(self._live(), _as_dp(f), f.size))
+        self._inject("inject_f", f)
 
     def set_host_objective(self, fn):
         """fn(X: ndarray[rows, n]) -> ndarray[rows, num_objectives]."""
-        def tramp(_u, x, rows, n, out, k):
-            xs = np.ctypeslib.as_array(x, shape=(rows, n))
-            np.ctypeslib.as_array(out, shape=(rows, k))[:] = np.asarray(fn(xs), dtype=np.float64).reshape(rows, k)
-        self._cb = HOST_CB(tramp)
-        self._check(self._fn("set_host_objective", C.c_int, [C.c_void_p, HOST_CB, C.c_void_p])(self._live(), self._cb, None))
-
-    def get(self, key):
-        cnt = C.c_size_t(0)
-        f = self._fn("get_array", C.c_int, [C.c_void_p, C.c_char_p, _dp, C.c_size_t, C.POINTER(C.c_size_t)])
-        self._check(f(self._live(), key.encode(), None, 0, C.byref(cnt)))
-        out = np.empty(cnt.value, dtype=np.float64)
-        if cnt.value:
-            self._check(f(self._h, key.encode(), _as_dp(out), out.size, C.byref(cnt)))
-        return out
-
-    def scalar(self, key):
-        v = C.c_double(0)
-        self._check(self._fn("get_scalar", C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_double)])(self._live(), key.encode(), C.byref(v)))
-        return v.value
-
-    def set_scalar(self, key, value):
-        self._check(self._fn("set_scalar", C.c_int, [C.c_void_p, C.c_char_p, C.c_double])(self._live(), key.encode(), float(value)))
-
-    def launch_count(self):
-        return self._fn("launch_count", C.c_uint64, [C.c_void_p])(self._live())
+        self._set_callback("set_host_objective", HOST_CB, fn, lambda rows, n, k: (rows, k))
 
 
 def Solver(**kw):

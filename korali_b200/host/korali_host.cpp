@@ -185,11 +185,131 @@ struct Settings {
   }
 };
 
+// a strict reader over a copy of the object v (consumed keys are erased from the copy, the experiment's tree is left as it is)
+Settings object(py::handle v, std::string module, const std::string& not_an_object) {
+  if (!py::isinstance<py::dict>(v)) korali_error("%s", not_an_object.c_str());
+  py::dict d;
+  for (auto kv : py::reinterpret_borrow<py::dict>(v)) d[kv.first] = kv.second;
+  return Settings(d, std::move(module));
+}
+
+Settings variable(py::list variables, size_t i) { return object(variables[i], "Variable", "Variable " + std::to_string(i) + " is not an object\n"); }
+
 std::string canon(std::string s) {  // module types are compared case-insensitively with spaces stripped (module.cpp:103)
   std::string o;
   for (char c : s) if (c != ' ') o += (char)std::tolower((unsigned char)c);
   return o;
 }
+
+// the built-in device objectives by name (CMAES, DEA objectives and TMCMC log-likelihood models); noun names the setting in errors
+int32_t deviceObjective(const std::string& name, const char* noun) {
+  static const std::pair<const char*, int32_t> kObjectives[] = {
+      {"negsphere", KCMA_OBJ_NEG_SPHERE}, {"sphere", KCMA_OBJ_NEG_SPHERE}, {"negrosenbrock", KCMA_OBJ_NEG_ROSENBROCK},
+      {"rosenbrock", KCMA_OBJ_NEG_ROSENBROCK}, {"negackley", KCMA_OBJ_NEG_ACKLEY}, {"ackley", KCMA_OBJ_NEG_ACKLEY},
+      {"negellipsoid", KCMA_OBJ_NEG_ELLIPSOID}, {"ellipsoid", KCMA_OBJ_NEG_ELLIPSOID}, {"negsumsq", KCMA_OBJ_NEG_SUMSQ},
+      {"negspheresin2", KCMA_OBJ_NEG_SPHERE_SIN2}};
+  const std::string o = canon(name);
+  for (const auto& e : kObjectives) if (o == e.first) return e.second;
+  korali_error("Unknown device %s '%s' (Sphere, Rosenbrock, Ackley, Ellipsoid, NegSumSq, NegSphereSin2)\n", noun, o.c_str());
+}
+
+// rows of `width` values of a flat row-major array, as a JSON array of arrays
+py::list rowsOf(const std::vector<double>& flat, size_t width) {
+  py::list out;
+  for (size_t i = 0; width && (i + 1) * width <= flat.size(); i++) out.append(std::vector<double>(flat.begin() + i * width, flat.begin() + (i + 1) * width));
+  return out;
+}
+
+// the inverse of rowsOf for a saved state: an array of arrays (or of numbers) read back row-major
+std::vector<double> flatten(py::handle o) {
+  std::vector<double> v;
+  for (auto row : o) {
+    if (py::isinstance<py::list>(row) || py::isinstance<py::tuple>(row)) for (auto x : row) v.push_back(x.cast<double>());
+    else v.push_back(row.cast<double>());
+  }
+  return v;
+}
+
+// the sample a per-sample Python model receives (Sample Id, Module and Operation as the reference's conduit sets them)
+py::dict sampleOf(py::object params, uint64_t id, const char* operation) {
+  py::dict sample;
+  sample["Parameters"] = params;
+  sample["Sample Id"] = id;
+  sample["Module"] = "Problem";
+  sample["Operation"] = operation;
+  return sample;
+}
+
+py::list paramsOf(const double* x, uint64_t n) {
+  py::list params;
+  for (uint64_t d = 0; d < n; d++) params.append(x[d]);
+  return params;
+}
+
+// A Python model behind the host and device conduits of the C ABIs. Per sample, the model is called with a sample dict and sets
+// sample[output] (a list of K values for "Evaluate Multiple"); korali_b200.batched(fn) gets the whole population as a (rows x N)
+// NumPy view and returns rows x K values; korali_b200.batched_device(fn) gets raw device pointers. A Python exception is kept in
+// *pending (rethrown after the generation) and the outputs are filled with `fill`.
+struct Model {
+  py::object fn;
+  std::string flavour;                  // "", "numpy" or "device"
+  const char* operation = "Evaluate";   // or "Evaluate Multiple"
+  const char* output = "F(x)";
+  double fill = NAN;
+  std::string* pending = nullptr;
+
+  void set(py::object f, std::string* pending_error) {
+    fn = std::move(f);
+    pending = pending_error;
+    flavour = py::hasattr(fn, "_korali_batched") ? fn.attr("_korali_batched").cast<std::string>() : std::string();
+    if (!flavour.empty() && flavour != "numpy" && flavour != "device") korali_error("Unknown batched model flavour '%s'\n", flavour.c_str());
+  }
+
+  void evaluate(const double* x, uint64_t rows, uint64_t n, double* out, uint64_t K) {
+    const bool multiple = !strcmp(operation, "Evaluate Multiple");
+    try {
+      if (flavour == "numpy") {
+        py::array_t<double> X({(py::ssize_t)rows, (py::ssize_t)n}, {(py::ssize_t)(n * sizeof(double)), (py::ssize_t)sizeof(double)}, x, py::none());
+        py::array_t<double, py::array::c_style | py::array::forcecast> F(fn(X));
+        if ((uint64_t)F.size() != rows * K) {
+          if (multiple) korali_error("The batched model returned %zu values for %zu samples x %zu objectives\n", (size_t)F.size(), (size_t)rows, (size_t)K);
+          korali_error("The batched model returned %zu values for %zu samples\n", (size_t)F.size(), (size_t)rows);
+        }
+        const double* f = F.data();
+        for (uint64_t i = 0; i < rows * K; i++) out[i] = f[i];
+        return;
+      }
+      for (uint64_t i = 0; i < rows; i++) {
+        py::dict sample = sampleOf(paramsOf(x + i * n, n), i, operation);
+        fn(sample);
+        if (!sample.contains(output)) korali_error("The model did not set '%s' for sample %zu\n", output, (size_t)i);
+        py::object fx = sample[output];
+        if (!multiple) { out[i] = fx.cast<double>(); continue; }
+        if (!(py::isinstance<py::list>(fx) || py::isinstance<py::tuple>(fx)) || (uint64_t)py::len(fx) != K)
+          korali_error("Multi-objective model: 'F(x)' of sample %zu must be a list of %zu values ('Num Objectives')\n", (size_t)i, (size_t)K);
+        uint64_t k = 0;
+        for (auto v : fx) out[i * K + k++] = v.cast<double>();
+      }
+    } catch (const std::exception& e) {
+      *pending = e.what();
+      for (uint64_t i = 0; i < rows * K; i++) out[i] = fill;
+    }
+  }
+
+  // kcma_host_objective_fn / ktmcmc_host_loglik_fn: one value per sample
+  static void host(void* user, const double* x, uint64_t rows, uint64_t n, double* out) { ((Model*)user)->evaluate(x, rows, n, out, 1); }
+  // kmocma_host_objective_fn: K values per sample
+  static void hostMultiple(void* user, const double* x, uint64_t rows, uint64_t n, double* out, uint64_t K) { ((Model*)user)->evaluate(x, rows, n, out, K); }
+  // kcma_device_objective_fn: the wrapper of korali_b200.batched_device builds zero-copy tensor views itself
+  static void device(void* user, const double* x_dev, uint64_t rows, uint64_t n, uint64_t ldx, double* f_dev, void* stream) {
+    Model* self = (Model*)user;
+    try {
+      self->fn((uintptr_t)x_dev, rows, n, ldx, (uintptr_t)f_dev, (uintptr_t)stream);
+    } catch (const std::exception& e) {
+      *self->pending = e.what();
+    }
+  }
+};
 
 enum Verbosity { SILENT = 0, MINIMAL = 1, NORMAL = 2, DETAILED = 3 };
 
@@ -277,23 +397,125 @@ class RankPool {
   bool stop_ = false;
 };
 
-// ---- the solver plug-in: Optimizer/CMAES on libkcma ----------------------------------------------------------
-class CMAES : public SolverBase {
+// The entry points every solver ABI has (include/kcma.h, kdea.h, kmocma.h, ktmcmc.h): the same signatures over its own handle type
+template <class H, class Cfg>
+struct Abi {
+  int (*create)(const Cfg*, H**);
+  void (*destroy)(H*);
+  const char* (*last_error)(const H*);
+  int (*run_generation)(H*);
+  int (*check_termination)(H*, int*, const char**);
+  int (*get_array)(H*, const char*, double*, size_t, size_t*);
+  int (*get_scalar)(H*, const char*, double*);
+  int (*set_scalar)(H*, const char*, double);
+};
+
+// A termination criterion of a solver's "Termination Criteria" object: its default, whether it is read as an unsigned integer, and
+// whether it is set on the handle as "Termination Criteria/<key>" (the others are passed through the cfg, or only written back).
+struct Criterion {
+  const char* key;
+  double dflt;
+  bool is_uint;
+  bool pushed;
+};
+
+// The part of a solver plug-in that only drives its C ABI: the handles (one per device; every solver but CMAES has one), errors,
+// state getters, termination criteria and the generation call.
+template <class H, class Cfg>
+class Plugin : public SolverBase {
  public:
-  kcma_t* h = nullptr;                  // rank 0 (the replicated state is read from it)
-  std::vector<kcma_t*> hs;              // all ranks, one per device
+  const Abi<H, Cfg> abi;
+  const std::vector<Criterion> criteria;   // in the order they are parsed and written back
+  std::vector<double> tc;                  // their values
+  Cfg cfg;
+  H* h = nullptr;                          // rank 0 (the replicated state is read from it)
+  std::vector<H*> hs;                      // all ranks, one per device
+
+  Plugin(Abi<H, Cfg> a, std::vector<Criterion> c) : abi(a), criteria(std::move(c)) {
+    for (const Criterion& x : criteria) tc.push_back(x.dflt);
+  }
+  ~Plugin() override { for (H* x : hs) if (x) abi.destroy(x); }
+
+  void check(int rc) { if (rc) korali_error("%s", abi.last_error(h)); }
+  void each(const std::function<int(H*)>& fn) { for (H* x : hs) if (fn(x)) korali_error("%s", abi.last_error(x)); }
+  double scalar(const char* key) override { double v = NAN; check(abi.get_scalar(h, key, &v)); return v; }
+  std::vector<double> array(const char* key) override {
+    size_t n = 0;
+    check(abi.get_array(h, key, nullptr, 0, &n));
+    std::vector<double> v(n);
+    if (n) check(abi.get_array(h, key, v.data(), n, &n));
+    return v;
+  }
+
+  void requireOneDevice(const std::vector<int>& device_ids) {
+    if (device_ids.size() > 1) korali_error("%s runs on one device (k['Conduit']['Devices'] > 1 is built for Optimizer/CMAES)\n", name());
+  }
+  // appends the handle of cfg on `device` (cfg.device is set here, the rest of cfg by the caller)
+  void create(int device) {
+    cfg.device = device;
+    H* x = nullptr;
+    if (abi.create(&cfg, &x)) korali_error("%s", abi.last_error(nullptr));
+    hs.push_back(x);
+    h = hs[0];
+  }
+
+  // s["Termination Criteria"], strictly, into tc
+  void parseCriteria(Settings& s) {
+    if (!s.has("Termination Criteria")) return;
+    Settings t = object(s.take("Termination Criteria"), s.module + "['Termination Criteria']",
+                        " + Object: [ " + s.module + " ] \n + Key:    ['Termination Criteria']\n + Reason: not an object\n");
+    for (size_t i = 0; i < criteria.size(); i++)
+      tc[i] = criteria[i].is_uint ? (double)t.uint(criteria[i].key, (uint64_t)criteria[i].dflt) : t.num(criteria[i].key, criteria[i].dflt);
+    t.finish();
+  }
+  void pushCriteria() {
+    for (size_t i = 0; i < criteria.size(); i++)
+      if (criteria[i].pushed) each([&](H* x) { return abi.set_scalar(x, (std::string("Termination Criteria/") + criteria[i].key).c_str(), tc[i]); });
+  }
+  void emitCriteria(py::dict js) {
+    py::dict t;
+    for (size_t i = 0; i < criteria.size(); i++) t[criteria[i].key] = tc[i];
+    js["Termination Criteria"] = t;
+  }
+
+  bool checkTermination() override {
+    int fin = 0;
+    const char* reason = "";
+    check(abi.check_termination(h, &fin, &reason));
+    if (fin) splitReasons(reason);
+    return fin != 0;
+  }
+
+  void runGeneration() override {
+    pending_error.clear();
+    int rc;
+    if (!needsPython()) { py::gil_scoped_release nogil; rc = abi.run_generation(h); }   // other experiments' threads run meanwhile
+    else rc = abi.run_generation(h);
+    if (!pending_error.empty()) { std::string e = pending_error; pending_error.clear(); throw std::runtime_error(e); }
+    check(rc);
+  }
+};
+
+// ---- the solver plug-in: Optimizer/CMAES on libkcma ----------------------------------------------------------
+class CMAES : public Plugin<kcma_t, kcma_cfg> {
+ public:
   std::unique_ptr<RankPool> pool;
-  kcma_cfg cfg;
   std::string mu_type = "Logarithmic";
   std::vector<double> init_val, init_sd, min_sd, gran;
   std::vector<std::string> names;
-  py::object objective;                 // Python callable, or a string naming a built-in device objective
+  Model objective;                      // the Python model when cfg.objective is KCMA_OBJ_EXTERNAL
   std::vector<py::object> constraints;  // Python callables
-  // termination criteria as given
-  double tc_max_generations = 1e10, tc_max_model_evaluations = 1e9, tc_max_value = INFINITY, tc_min_value_diff = -INFINITY;
-  double tc_max_infeasible = 0, tc_max_condition = INFINITY, tc_min_sd = -INFINITY, tc_max_sd = INFINITY;
-  int devices = 1;
 
+  CMAES() : Plugin({kcma_create, kcma_destroy, kcma_last_error, kcma_run_generation, kcma_check_termination, kcma_get_array, kcma_get_scalar,
+                    kcma_set_scalar},
+                   {{"Max Infeasible Resamplings", 0, true, false},   // a cfg field
+                    {"Max Condition Covariance Matrix", INFINITY, false, true},
+                    {"Min Standard Deviation", -INFINITY, false, true},
+                    {"Max Standard Deviation", INFINITY, false, true},
+                    {"Max Value", INFINITY, false, true},
+                    {"Min Value Difference Threshold", -INFINITY, false, true},
+                    {"Max Model Evaluations", 1e9, false, true},
+                    {"Max Generations", 1e10, false, true}}) {}
   const char* name() const override { return "Optimizer/CMAES"; }
   size_t variableCount() const override { return cfg.n; }
   std::string takeWarnings() override { const char* w = kcma_take_warnings(h); return w ? w : ""; }
@@ -310,27 +532,6 @@ class CMAES : public SolverBase {
     snprintf(b, sizeof(b), "Covariance Eigenvalues: Min = %+6.3e -  Max = %+6.3e\n", scalar("Minimum Covariance Eigenvalue"), scalar("Maximum Covariance Eigenvalue"));
     log(NORMAL, b);
     snprintf(b, sizeof(b), "Number of Infeasible Samples: %zu\n", (size_t)scalar("Infeasible Sample Count")); log(DETAILED, b);
-  }
-
-  ~CMAES() {
-    pool.reset();
-    for (kcma_t* x : hs) if (x) kcma_destroy(x);
-  }
-  void each(const std::function<int(kcma_t*)>& fn) {
-    for (kcma_t* x : hs) if (fn(x)) korali_error("%s", kcma_last_error(x));
-  }
-
-  void check(int rc) {
-    if (rc) korali_error("%s", kcma_last_error(h));
-  }
-
-  double scalar(const char* key) override { double v = NAN; check(kcma_get_scalar(h, key, &v)); return v; }
-  std::vector<double> array(const char* key) override {
-    size_t n = 0;
-    check(kcma_get_array(h, key, nullptr, 0, &n));
-    std::vector<double> v(n);
-    if (n) check(kcma_get_array(h, key, v.data(), n, &n));
-    return v;
   }
 
   // generated CMAES::setConfiguration + Optimizer:: + Solver:: (strict)
@@ -361,23 +562,8 @@ class CMAES : public SolverBase {
     cfg.covariance_matrix_adaption_strength = s.num("Covariance Matrix Adaption Strength", 0.1);
     cfg.normal_vector_learning_rate = s.num("Normal Vector Learning Rate", -1.0);
     cfg.global_success_learning_rate = s.num("Global Success Learning Rate", 0.2);
-    if (s.has("Termination Criteria")) {
-      py::object tco = s.take("Termination Criteria");
-      if (!py::isinstance<py::dict>(tco)) korali_error(" + Object: [ CMAES ] \n + Key:    ['Termination Criteria']\n + Reason: not an object\n");
-      py::dict tcd;
-      for (auto kv : py::reinterpret_borrow<py::dict>(tco)) tcd[kv.first] = kv.second;
-      Settings tc(tcd, "CMAES['Termination Criteria']");
-      tc_max_infeasible = (double)tc.uint("Max Infeasible Resamplings", 0);
-      tc_max_condition = tc.num("Max Condition Covariance Matrix", INFINITY);
-      tc_min_sd = tc.num("Min Standard Deviation", -INFINITY);
-      tc_max_sd = tc.num("Max Standard Deviation", INFINITY);
-      tc_max_value = tc.num("Max Value", INFINITY);
-      tc_min_value_diff = tc.num("Min Value Difference Threshold", -INFINITY);
-      tc_max_model_evaluations = tc.num("Max Model Evaluations", 1e9);
-      tc_max_generations = tc.num("Max Generations", 1e10);
-      tc.finish();
-    }
-    cfg.max_infeasible_resamplings = (uint64_t)tc_max_infeasible;
+    parseCriteria(s);
+    cfg.max_infeasible_resamplings = (uint64_t)tc[0];   // "Max Infeasible Resamplings"
     // generators are part of the module defaults (CMAES.config:510-519). A saved state carries the Normal Generator's own
     // "Random Seed" (distribution.cpp.base:36-37): resuming with it continues the counter-based Philox stream exactly.
     for (const char* g : {"Normal Generator", "Uniform Generator"}) {
@@ -421,10 +607,7 @@ class CMAES : public SolverBase {
     gran.assign(n, 0.0);
     names.assign(n, "");
     for (size_t i = 0; i < n; i++) {
-      if (!py::isinstance<py::dict>(variables[i])) korali_error("Variable %zu is not an object\n", i);
-      py::dict vcopy;
-      for (auto kv : py::reinterpret_borrow<py::dict>(variables[i])) vcopy[kv.first] = kv.second;
-      Settings v(vcopy, "Variable");
+      Settings v = variable(variables, i);
       names[i] = v.str("Name", "");
       lower[i] = v.num("Lower Bound", -INFINITY);
       upper[i] = v.num("Upper Bound", INFINITY);
@@ -442,13 +625,11 @@ class CMAES : public SolverBase {
     cfg.initial_stddev = init_sd.data(); cfg.min_stddev_update = min_sd.data(); cfg.granularity = gran.data();
     cfg.seed = seed;
     // problem (optimization.config)
-    py::dict pcopy;
-    for (auto kv : problem) pcopy[kv.first] = kv.second;
-    Settings p(pcopy, "Optimization");
+    Settings p = object(problem, "Optimization", "'Problem' is not an object\n");
     const std::string ptype = canon(p.str("Type", ""));
     if (ptype != "optimization") korali_error("Only Problem Type 'Optimization' is served by the B200 CMA-ES path (got '%s')\n", ptype.c_str());
     if (!p.has("Objective Function")) korali_error(" + Object: [ Optimization ] \n + Key:    ['Objective Function']\n + Reason: mandatory setting missing\n");
-    objective = p.take("Objective Function");
+    py::object objective_fn = p.take("Objective Function");
     p.uint("Num Objectives", 1);
     p.boolean("Has Discrete Variables", 0);
     constraints.clear();
@@ -460,23 +641,15 @@ class CMAES : public SolverBase {
     p.finish();
     cfg.n_constraints = constraints.size();
     cfg.constraint_family = constraints.empty() ? KCMA_CON_NONE : KCMA_CON_EXTERNAL;
-    if (py::isinstance<py::str>(objective)) {
-      const std::string o = canon(objective.cast<std::string>());
-      if (o == "negsphere" || o == "sphere") cfg.objective = KCMA_OBJ_NEG_SPHERE;
-      else if (o == "negrosenbrock" || o == "rosenbrock") cfg.objective = KCMA_OBJ_NEG_ROSENBROCK;
-      else if (o == "negackley" || o == "ackley") cfg.objective = KCMA_OBJ_NEG_ACKLEY;
-      else if (o == "negellipsoid" || o == "ellipsoid") cfg.objective = KCMA_OBJ_NEG_ELLIPSOID;
-      else if (o == "negsumsq") cfg.objective = KCMA_OBJ_NEG_SUMSQ;
-      else if (o == "negspheresin2") cfg.objective = KCMA_OBJ_NEG_SPHERE_SIN2;
-      else korali_error("Unknown device objective '%s' (Sphere, Rosenbrock, Ackley, Ellipsoid, NegSumSq, NegSphereSin2)\n", o.c_str());
+    if (py::isinstance<py::str>(objective_fn)) {
+      cfg.objective = deviceObjective(objective_fn.cast<std::string>(), "objective");
       cfg.keep_population = constraints.empty() ? 0 : 1;
-    } else if (PyCallable_Check(objective.ptr())) {
+    } else if (PyCallable_Check(objective_fn.ptr())) {
       cfg.objective = KCMA_OBJ_EXTERNAL;
       cfg.keep_population = 1;
       // korali_b200.batched(fn) / korali_b200.batched_device(fn): the model takes the whole population in one call
-      batched = py::hasattr(objective, "_korali_batched") ? objective.attr("_korali_batched").cast<std::string>() : std::string();
-      if (!batched.empty() && batched != "numpy" && batched != "device") korali_error("Unknown batched model flavour '%s'\n", batched.c_str());
-      if (!batched.empty() && cfg.use_gradient_information) korali_error("Batched models do not return gradients: use a per-sample model with 'Use Gradient Information'\n");
+      objective.set(objective_fn, &pending_error);
+      if (!objective.flavour.empty() && cfg.use_gradient_information) korali_error("Batched models do not return gradients: use a per-sample model with 'Use Gradient Information'\n");
     } else {
       korali_error(" + Object: [ Optimization ] \n + Key:    ['Objective Function']\n + Reason: neither a callable nor the name of a device objective\n");
     }
@@ -484,65 +657,14 @@ class CMAES : public SolverBase {
   }
 
   py::dict saved_internal;
-  std::string batched;   // "", "numpy" or "device"
 
-  // korali_b200.batched(fn): ONE call per generation with X as a (rows x N) NumPy view of the host copy of the population
-  static void host_objective_batched(void* user, const double* x, uint64_t rows, uint64_t n, double* f_out) {
-    CMAES* self = (CMAES*)user;
-    try {
-      py::array_t<double> X({(py::ssize_t)rows, (py::ssize_t)n}, {(py::ssize_t)(n * sizeof(double)), (py::ssize_t)sizeof(double)}, x, py::none());
-      py::array_t<double, py::array::c_style | py::array::forcecast> F(self->objective(X));
-      if ((uint64_t)F.size() != rows) korali_error("The batched model returned %zu values for %zu samples\n", (size_t)F.size(), (size_t)rows);
-      const double* f = F.data();
-      for (uint64_t i = 0; i < rows; i++) f_out[i] = f[i];
-    } catch (const std::exception& e) {
-      self->pending_error = e.what();
-      for (uint64_t i = 0; i < rows; i++) f_out[i] = NAN;
-    }
-  }
-  // korali_b200.batched_device(fn): the wrapper receives raw device pointers and builds zero-copy tensor views itself
-  static void device_objective(void* user, const double* x_dev, uint64_t rows, uint64_t n, uint64_t ldx, double* f_dev, void* stream) {
-    CMAES* self = (CMAES*)user;
-    try {
-      self->objective((uintptr_t)x_dev, rows, n, ldx, (uintptr_t)f_dev, (uintptr_t)stream);
-    } catch (const std::exception& e) {
-      self->pending_error = e.what();
-    }
-  }
-
-  static void host_objective(void* user, const double* x, uint64_t rows, uint64_t n, double* f_out) {
-    CMAES* self = (CMAES*)user;
-    try {
-      for (uint64_t i = 0; i < rows; i++) {
-        py::dict sample;
-        py::list params;
-        for (uint64_t d = 0; d < n; d++) params.append(x[i * n + d]);
-        sample["Parameters"] = params;
-        sample["Sample Id"] = i;
-        sample["Module"] = "Problem";
-        sample["Operation"] = "Evaluate";
-        self->objective(sample);
-        if (!sample.contains("F(x)")) korali_error("The model did not set 'F(x)' for sample %zu\n", (size_t)i);
-        f_out[i] = sample["F(x)"].cast<double>();
-      }
-    } catch (const std::exception& e) {
-      self->pending_error = e.what();
-      for (uint64_t i = 0; i < rows; i++) f_out[i] = NAN;
-    }
-  }
   // operation "Evaluate With Gradients" (CMAES.cpp.base:199-200, 226-228): the model sets "F(x)" and "Gradient"
   static void host_objective_grad(void* user, const double* x, uint64_t rows, uint64_t n, double* f_out, double* grad_out) {
     CMAES* self = (CMAES*)user;
     try {
       for (uint64_t i = 0; i < rows; i++) {
-        py::dict sample;
-        py::list params;
-        for (uint64_t d = 0; d < n; d++) params.append(x[i * n + d]);
-        sample["Parameters"] = params;
-        sample["Sample Id"] = i;
-        sample["Module"] = "Problem";
-        sample["Operation"] = "Evaluate With Gradients";
-        self->objective(sample);
+        py::dict sample = sampleOf(paramsOf(x + i * n, n), i, "Evaluate With Gradients");
+        self->objective.fn(sample);
         if (!sample.contains("F(x)")) korali_error("The model did not set 'F(x)' for sample %zu\n", (size_t)i);
         if (!sample.contains("Gradient")) korali_error("The model did not set 'Gradient' for sample %zu ('Use Gradient Information' is on)\n", (size_t)i);
         f_out[i] = sample["F(x)"].cast<double>();
@@ -560,14 +682,9 @@ class CMAES : public SolverBase {
     CMAES* self = (CMAES*)user;
     try {
       for (uint64_t i = 0; i < rows; i++) {
-        py::list params;
-        for (uint64_t d = 0; d < n; d++) params.append(x[i * n + d]);
+        py::list params = paramsOf(x + i * n, n);
         for (uint64_t c = 0; c < nc; c++) {
-          py::dict sample;
-          sample["Parameters"] = params;
-          sample["Sample Id"] = 0;
-          sample["Module"] = "Problem";
-          sample["Operation"] = "Evaluate Constraints";
+          py::dict sample = sampleOf(params, 0, "Evaluate Constraints");
           self->constraints[c](sample);
           g_out[c * rows + i] = sample["F(x)"].cast<double>();
         }
@@ -584,32 +701,20 @@ class CMAES : public SolverBase {
       korali_error("k['Conduit']['Devices'] > 1 shards the population over several GPUs of this process: it needs a device objective "
                    "(e['Problem']['Objective Function'] = 'Ellipsoid' ...) and no constraints; Python models run on one device\n");
     for (int r = 0; r < G; r++) {
-      cfg.device = device_ids[r]; cfg.rank = r; cfg.nranks = G;
-      kcma_t* x = nullptr;
-      if (kcma_create(&cfg, &x)) korali_error("%s", kcma_last_error(nullptr));
-      hs.push_back(x);
+      cfg.rank = r; cfg.nranks = G;
+      create(device_ids[r]);
     }
-    h = hs[0];
     if (G > 1) {
       if (kcma_comm_init_all(hs.data(), G)) korali_error("%s", kcma_last_error(h));
       pool = std::make_unique<RankPool>(G);
     }
     if (cfg.objective == KCMA_OBJ_EXTERNAL) {
       if (cfg.use_gradient_information) check(kcma_set_host_objective_grad(h, &CMAES::host_objective_grad, this));
-      else if (batched == "device") check(kcma_set_device_objective(h, &CMAES::device_objective, this));
-      else if (batched == "numpy") check(kcma_set_host_objective(h, &CMAES::host_objective_batched, this));
-      else check(kcma_set_host_objective(h, &CMAES::host_objective, this));
+      else if (objective.flavour == "device") check(kcma_set_device_objective(h, &Model::device, &objective));
+      else check(kcma_set_host_objective(h, &Model::host, &objective));
     }
     if (!constraints.empty()) check(kcma_set_host_constraints(h, &CMAES::host_constraints, this));
-    each([&](kcma_t* x) {
-      return kcma_set_scalar(x, "Termination Criteria/Max Condition Covariance Matrix", tc_max_condition) ||
-             kcma_set_scalar(x, "Termination Criteria/Min Standard Deviation", tc_min_sd) ||
-             kcma_set_scalar(x, "Termination Criteria/Max Standard Deviation", tc_max_sd) ||
-             kcma_set_scalar(x, "Termination Criteria/Max Value", tc_max_value) ||
-             kcma_set_scalar(x, "Termination Criteria/Min Value Difference Threshold", tc_min_value_diff) ||
-             kcma_set_scalar(x, "Termination Criteria/Max Model Evaluations", tc_max_model_evaluations) ||
-             kcma_set_scalar(x, "Termination Criteria/Max Generations", tc_max_generations);
-    });
+    pushCriteria();
   }
 
   // restore "Internal Settings" of a loaded state (CMAES.cpp:1042-1560): resume continues from the saved generation
@@ -634,8 +739,7 @@ class CMAES : public SolverBase {
     if (!constraints.empty()) {
       for (const char* k : {"Viability Boundaries", "Best Constraint Evaluations"}) arr(k);
       if (saved_internal.contains("Normal Constraint Approximation")) {   // saved as a C x N array of arrays
-        std::vector<double> flat;
-        for (auto row : saved_internal["Normal Constraint Approximation"]) for (auto x : row) flat.push_back(x.cast<double>());
+        std::vector<double> flat = flatten(saved_internal["Normal Constraint Approximation"]);
         if (!flat.empty()) each([&](kcma_t* x) { return kcma_set_array(x, "Normal Constraint Approximation", flat.data(), flat.size()); });
       }
       for (const char* k : {"Global Success Rate", "Resampled Parameter Count", "Covariance Matrix Adaptation Count",
@@ -651,26 +755,11 @@ class CMAES : public SolverBase {
     each([&](kcma_t* x) { return kcma_set_scalar(x, "Current Generation", (double)generation); });
   }
 
-  bool checkTermination() override {
-    int fin = 0;
-    const char* reason = "";
-    check(kcma_check_termination(h, &fin, &reason));
-    if (fin) splitReasons(reason);
-    return fin != 0;
-  }
-
   void runGeneration() override {
+    if (!pool) return Plugin::runGeneration();
     pending_error.clear();
-    if (pool) {   // one call per device, in flight together
-      const int failed = pool->run([this](int r) { return kcma_run_generation(hs[r]); });
-      if (failed) korali_error("%s", kcma_last_error(hs[failed - 1]));
-      return;
-    }
-    int rc;
-    if (!needsPython()) { py::gil_scoped_release nogil; rc = kcma_run_generation(h); }   // other experiments' threads run meanwhile
-    else rc = kcma_run_generation(h);
-    if (!pending_error.empty()) { std::string e = pending_error; pending_error.clear(); throw std::runtime_error(e); }
-    check(rc);
+    const int failed = pool->run([this](int r) { return kcma_run_generation(hs[r]); });   // one call per device, in flight together
+    if (failed) korali_error("%s", kcma_last_error(hs[failed - 1]));
   }
   bool needsPython() const override { return cfg.objective == KCMA_OBJ_EXTERNAL || !constraints.empty(); }
 
@@ -696,16 +785,7 @@ class CMAES : public SolverBase {
     js["Covariance Matrix Adaption Strength"] = cfg.covariance_matrix_adaption_strength;
     js["Normal Vector Learning Rate"] = cfg.normal_vector_learning_rate;
     js["Global Success Learning Rate"] = cfg.global_success_learning_rate;
-    py::dict tc;
-    tc["Max Infeasible Resamplings"] = tc_max_infeasible;
-    tc["Max Condition Covariance Matrix"] = tc_max_condition;
-    tc["Min Standard Deviation"] = tc_min_sd;
-    tc["Max Standard Deviation"] = tc_max_sd;
-    tc["Max Value"] = tc_max_value;
-    tc["Min Value Difference Threshold"] = tc_min_value_diff;
-    tc["Max Model Evaluations"] = tc_max_model_evaluations;
-    tc["Max Generations"] = tc_max_generations;
-    js["Termination Criteria"] = tc;
+    emitCriteria(js);
     py::dict ng, ug;
     ng["Type"] = "Univariate/Normal"; ng["Mean"] = 0.0; ng["Standard Deviation"] = 1.0; ng["Random Seed"] = cfg.seed;
     ug["Type"] = "Univariate/Uniform"; ug["Minimum"] = 0.0; ug["Maximum"] = 1.0; ug["Random Seed"] = cfg.seed + 1;
@@ -738,46 +818,33 @@ class CMAES : public SolverBase {
       std::vector<uint64_t> idx(lam);
       if (scalar("Current Generation") > 0 && !kcma_get_index_array(h, "Sorting Index", idx.data(), lam, &cnt)) js["Sorting Index"] = idx;
     }
-    if (cfg.keep_population && lam * n <= (1u << 22)) {
-      std::vector<double> flat = array("Sample Population");
-      py::list pop;
-      for (uint64_t i = 0; i * n < flat.size(); i++) pop.append(std::vector<double>(flat.begin() + i * n, flat.begin() + (i + 1) * n));
-      js["Sample Population"] = pop;
-    }
+    if (cfg.keep_population && lam * n <= (1u << 22)) js["Sample Population"] = rowsOf(array("Sample Population"), n);
     if (!constraints.empty()) {
       js["Viability Boundaries"] = array("Viability Boundaries");
       js["Best Constraint Evaluations"] = array("Best Constraint Evaluations");
-      std::vector<double> flat = array("Normal Constraint Approximation");
-      py::list rows;
-      for (size_t c = 0; c * n < flat.size(); c++) rows.append(std::vector<double>(flat.begin() + c * n, flat.begin() + (c + 1) * n));
-      js["Normal Constraint Approximation"] = rows;
+      js["Normal Constraint Approximation"] = rowsOf(array("Normal Constraint Approximation"), n);
     }
   }
 };
 
 // ---- the solver plug-in: Optimizer/DEA on libkcma (include/kdea.h) -------------------------------------------------
-class DEA : public SolverBase {
+class DEA : public Plugin<kdea_t, kdea_cfg> {
  public:
-  kdea_t* h = nullptr;
-  kdea_cfg cfg;
-  std::string mutation_rule = "Fixed", parent_rule = "Random", accept_rule = "Greedy", batched;
-  py::object objective;
-  double tc_max_generations = 1e10, tc_max_model_evaluations = 1e9, tc_max_value = INFINITY, tc_min_value_diff = -INFINITY;
-  double tc_max_infeasible = 1e7, tc_min_value = -INFINITY, tc_min_step = -INFINITY;
+  std::string mutation_rule = "Fixed", parent_rule = "Random", accept_rule = "Greedy";
+  Model objective;   // the Python model when cfg.objective is KCMA_OBJ_EXTERNAL
   py::dict saved_internal;
 
-  ~DEA() override { if (h) kdea_destroy(h); }
+  DEA() : Plugin({kdea_create, kdea_destroy, kdea_last_error, kdea_run_generation, kdea_check_termination, kdea_get_array, kdea_get_scalar,
+                  kdea_set_scalar},
+                 {{"Max Infeasible Resamplings", 1e7, false, true},
+                  {"Min Value", -INFINITY, false, true},
+                  {"Min Step Size", -INFINITY, false, true},
+                  {"Max Value", INFINITY, false, true},
+                  {"Min Value Difference Threshold", -INFINITY, false, true},
+                  {"Max Model Evaluations", 1e9, false, true},
+                  {"Max Generations", 1e10, false, true}}) {}
   const char* name() const override { return "Optimizer/DEA"; }
   size_t variableCount() const override { return cfg.n; }
-  void check(int rc) { if (rc) korali_error("%s", kdea_last_error(h)); }
-  double scalar(const char* key) override { double v = NAN; check(kdea_get_scalar(h, key, &v)); return v; }
-  std::vector<double> array(const char* key) override {
-    size_t n = 0;
-    check(kdea_get_array(h, key, nullptr, 0, &n));
-    std::vector<double> v(n);
-    if (n) check(kdea_get_array(h, key, v.data(), n, &n));
-    return v;
-  }
 
   // generated DEA::setConfiguration (DEA.config) + Optimizer:: + Solver:: (strict)
   void setConfiguration(py::dict solver, py::list variables, py::dict problem, uint64_t seed) override {
@@ -803,21 +870,7 @@ class DEA : public SolverBase {
     else if (accept_rule == "Improved") cfg.accept_rule = KDEA_ACCEPT_IMPROVED;
     else if (accept_rule == "Iterative") cfg.accept_rule = KDEA_ACCEPT_ITERATIVE;
     else korali_error("Accept Rule (%s) not recognized.\n", accept_rule.c_str());
-    if (s.has("Termination Criteria")) {
-      py::object tco = s.take("Termination Criteria");
-      if (!py::isinstance<py::dict>(tco)) korali_error(" + Object: [ DEA ] \n + Key:    ['Termination Criteria']\n + Reason: not an object\n");
-      py::dict tcd;
-      for (auto kv : py::reinterpret_borrow<py::dict>(tco)) tcd[kv.first] = kv.second;
-      Settings tc(tcd, "DEA['Termination Criteria']");
-      tc_max_infeasible = tc.num("Max Infeasible Resamplings", 1e7);
-      tc_min_value = tc.num("Min Value", -INFINITY);
-      tc_min_step = tc.num("Min Step Size", -INFINITY);
-      tc_max_value = tc.num("Max Value", INFINITY);
-      tc_min_value_diff = tc.num("Min Value Difference Threshold", -INFINITY);
-      tc_max_model_evaluations = tc.num("Max Model Evaluations", 1e9);
-      tc_max_generations = tc.num("Max Generations", 1e10);
-      tc.finish();
-    }
+    parseCriteria(s);
     for (const char* g : {"Normal Generator", "Uniform Generator"}) {
       if (!s.has(g)) continue;
       py::object go = s.take(g);
@@ -837,10 +890,7 @@ class DEA : public SolverBase {
     if (n == 0) korali_error("Optimization Evaluation problems require at least one variable.\n");
     lower.assign(n, -INFINITY); upper.assign(n, INFINITY);
     for (size_t i = 0; i < n; i++) {
-      if (!py::isinstance<py::dict>(variables[i])) korali_error("Variable %zu is not an object\n", i);
-      py::dict vcopy;
-      for (auto kv : py::reinterpret_borrow<py::dict>(variables[i])) vcopy[kv.first] = kv.second;
-      Settings v(vcopy, "Variable");
+      Settings v = variable(variables, i);
       v.str("Name", "");
       lower[i] = v.num("Lower Bound", -INFINITY);
       upper[i] = v.num("Upper Bound", INFINITY);
@@ -850,13 +900,11 @@ class DEA : public SolverBase {
     }
     cfg.n = n; cfg.lower_bound = lower.data(); cfg.upper_bound = upper.data();
     cfg.seed = uniform_seed ? uniform_seed : seed + 1;   // Uniform Generator = S + 1 (distribution.cpp.base:36-37: Normal S, Uniform S + 1); a saved state carries its own
-    py::dict pcopy;
-    for (auto kv : problem) pcopy[kv.first] = kv.second;
-    Settings p(pcopy, "Optimization");
+    Settings p = object(problem, "Optimization", "'Problem' is not an object\n");
     const std::string ptype = canon(p.str("Type", ""));
     if (ptype != "optimization") korali_error("Only Problem Type 'Optimization' is served by the B200 path (got '%s')\n", ptype.c_str());
     if (!p.has("Objective Function")) korali_error(" + Object: [ Optimization ] \n + Key:    ['Objective Function']\n + Reason: mandatory setting missing\n");
-    objective = p.take("Objective Function");
+    py::object objective_fn = p.take("Objective Function");
     p.uint("Num Objectives", 1);
     p.boolean("Has Discrete Variables", 0);
     if (p.has("Constraints")) {
@@ -864,102 +912,36 @@ class DEA : public SolverBase {
       if (py::isinstance<py::list>(c) && py::len(c) > 0) korali_error("Optimizer/DEA does not take constraints\n");
     }
     p.finish();
-    if (py::isinstance<py::str>(objective)) {
-      const std::string o = canon(objective.cast<std::string>());
-      if (o == "negsphere" || o == "sphere") cfg.objective = KCMA_OBJ_NEG_SPHERE;
-      else if (o == "negrosenbrock" || o == "rosenbrock") cfg.objective = KCMA_OBJ_NEG_ROSENBROCK;
-      else if (o == "negackley" || o == "ackley") cfg.objective = KCMA_OBJ_NEG_ACKLEY;
-      else if (o == "negellipsoid" || o == "ellipsoid") cfg.objective = KCMA_OBJ_NEG_ELLIPSOID;
-      else if (o == "negsumsq") cfg.objective = KCMA_OBJ_NEG_SUMSQ;
-      else if (o == "negspheresin2") cfg.objective = KCMA_OBJ_NEG_SPHERE_SIN2;
-      else korali_error("Unknown device objective '%s' (Sphere, Rosenbrock, Ackley, Ellipsoid, NegSumSq, NegSphereSin2)\n", o.c_str());
-    } else if (PyCallable_Check(objective.ptr())) {
+    if (py::isinstance<py::str>(objective_fn)) {
+      cfg.objective = deviceObjective(objective_fn.cast<std::string>(), "objective");
+    } else if (PyCallable_Check(objective_fn.ptr())) {
       cfg.objective = KCMA_OBJ_EXTERNAL;
-      batched = py::hasattr(objective, "_korali_batched") ? objective.attr("_korali_batched").cast<std::string>() : std::string();
-      if (batched == "device") korali_error("Optimizer/DEA takes per-sample models and korali.batched(fn) models (not device-tensor models)\n");
+      objective.set(objective_fn, &pending_error);
+      if (objective.flavour == "device") korali_error("Optimizer/DEA takes per-sample models and korali.batched(fn) models (not device-tensor models)\n");
     } else {
       korali_error(" + Object: [ Optimization ] \n + Key:    ['Objective Function']\n + Reason: neither a callable nor the name of a device objective\n");
     }
     s.finish();
   }
 
-  static void host_objective(void* user, const double* x, uint64_t rows, uint64_t n, double* f_out) {
-    DEA* self = (DEA*)user;
-    try {
-      if (self->batched == "numpy") {
-        py::array_t<double> X({(py::ssize_t)rows, (py::ssize_t)n}, {(py::ssize_t)(n * sizeof(double)), (py::ssize_t)sizeof(double)}, x, py::none());
-        py::array_t<double, py::array::c_style | py::array::forcecast> F(self->objective(X));
-        if ((uint64_t)F.size() != rows) korali_error("The batched model returned %zu values for %zu samples\n", (size_t)F.size(), (size_t)rows);
-        for (uint64_t i = 0; i < rows; i++) f_out[i] = F.data()[i];
-        return;
-      }
-      for (uint64_t i = 0; i < rows; i++) {
-        py::dict sample;
-        py::list params;
-        for (uint64_t d = 0; d < n; d++) params.append(x[i * n + d]);
-        sample["Parameters"] = params;
-        sample["Sample Id"] = i;
-        sample["Module"] = "Problem";
-        sample["Operation"] = "Evaluate";
-        self->objective(sample);
-        if (!sample.contains("F(x)")) korali_error("The model did not set 'F(x)' for sample %zu\n", (size_t)i);
-        f_out[i] = sample["F(x)"].cast<double>();
-      }
-    } catch (const std::exception& e) {
-      self->pending_error = e.what();
-      for (uint64_t i = 0; i < rows; i++) f_out[i] = NAN;
-    }
-  }
-
   void initialize(const std::vector<int>& device_ids) override {
-    if (device_ids.size() > 1) korali_error("Optimizer/DEA runs on one device (k['Conduit']['Devices'] > 1 is built for Optimizer/CMAES)\n");
-    cfg.device = device_ids[0];
-    if (kdea_create(&cfg, &h)) korali_error("%s", kdea_last_error(nullptr));
-    if (cfg.objective == KCMA_OBJ_EXTERNAL) check(kdea_set_host_objective(h, &DEA::host_objective, this));
-    check(kdea_set_scalar(h, "Termination Criteria/Max Infeasible Resamplings", tc_max_infeasible));
-    check(kdea_set_scalar(h, "Termination Criteria/Min Value", tc_min_value));
-    check(kdea_set_scalar(h, "Termination Criteria/Min Step Size", tc_min_step));
-    check(kdea_set_scalar(h, "Termination Criteria/Max Value", tc_max_value));
-    check(kdea_set_scalar(h, "Termination Criteria/Min Value Difference Threshold", tc_min_value_diff));
-    check(kdea_set_scalar(h, "Termination Criteria/Max Model Evaluations", tc_max_model_evaluations));
-    check(kdea_set_scalar(h, "Termination Criteria/Max Generations", tc_max_generations));
+    requireOneDevice(device_ids);
+    create(device_ids[0]);
+    if (cfg.objective == KCMA_OBJ_EXTERNAL) check(kdea_set_host_objective(h, &Model::host, &objective));
+    pushCriteria();
   }
 
   void restore(uint64_t generation) override {
     if (generation == 0) return;
-    auto flat = [&](py::handle o) {
-      std::vector<double> v;
-      for (auto row : o) {
-        if (py::isinstance<py::list>(row) || py::isinstance<py::tuple>(row)) for (auto x : row) v.push_back(x.cast<double>());
-        else v.push_back(row.cast<double>());
-      }
-      return v;
-    };
     for (const char* k : {"Sample Population", "Candidate Population", "Value Vector", "Previous Value Vector", "Current Mean", "Previous Mean",
                           "Best Ever Variables", "Current Best Variables", "Max Distances"})
-      if (saved_internal.contains(k)) { std::vector<double> v = flat(saved_internal[k]); check(kdea_set_array(h, k, v.data(), v.size())); }
+      if (saved_internal.contains(k)) { std::vector<double> v = flatten(saved_internal[k]); check(kdea_set_array(h, k, v.data(), v.size())); }
     for (const char* k : {"Best Ever Value", "Previous Best Ever Value", "Current Best Value", "Previous Best Value", "Best Sample Index",
                           "Infeasible Sample Count", "Model Evaluation Count"})
       if (saved_internal.contains(k)) check(kdea_set_scalar(h, k, saved_internal[k].cast<double>()));
     check(kdea_set_scalar(h, "Current Generation", (double)generation));
   }
 
-  bool checkTermination() override {
-    int fin = 0;
-    const char* reason = "";
-    check(kdea_check_termination(h, &fin, &reason));
-    if (fin) splitReasons(reason);
-    return fin != 0;
-  }
-
-  void runGeneration() override {
-    pending_error.clear();
-    int rc;
-    if (!needsPython()) { py::gil_scoped_release nogil; rc = kdea_run_generation(h); }
-    else rc = kdea_run_generation(h);
-    if (!pending_error.empty()) { std::string e = pending_error; pending_error.clear(); throw std::runtime_error(e); }
-    check(rc);
-  }
   bool needsPython() const override { return cfg.objective == KCMA_OBJ_EXTERNAL; }
 
   void printGeneration(const std::function<void(int, const char*)>& log) override {   // DEA::printGenerationAfter :290-299
@@ -978,11 +960,7 @@ class DEA : public SolverBase {
     js["Parent Selection Rule"] = parent_rule;
     js["Accept Rule"] = accept_rule;
     js["Fix Infeasible"] = cfg.fix_infeasible;
-    py::dict tc;
-    tc["Max Infeasible Resamplings"] = tc_max_infeasible; tc["Min Value"] = tc_min_value; tc["Min Step Size"] = tc_min_step;
-    tc["Max Value"] = tc_max_value; tc["Min Value Difference Threshold"] = tc_min_value_diff;
-    tc["Max Model Evaluations"] = tc_max_model_evaluations; tc["Max Generations"] = tc_max_generations;
-    js["Termination Criteria"] = tc;
+    emitCriteria(js);
     py::dict ng, ug;
     ng["Type"] = "Univariate/Normal"; ng["Mean"] = 0.0; ng["Standard Deviation"] = 1.0; ng["Random Seed"] = cfg.seed - 1;
     ug["Type"] = "Univariate/Uniform"; ug["Minimum"] = 0.0; ug["Maximum"] = 1.0; ug["Random Seed"] = cfg.seed;
@@ -995,41 +973,31 @@ class DEA : public SolverBase {
       js[k] = array(k);
     const uint64_t n = cfg.n, lam = cfg.population_size;
     if (lam * n <= (1u << 22))
-      for (const char* k : {"Sample Population", "Candidate Population"}) {
-        std::vector<double> flat = array(k);
-        py::list pop;
-        for (uint64_t i = 0; i * n < flat.size(); i++) pop.append(std::vector<double>(flat.begin() + i * n, flat.begin() + (i + 1) * n));
-        js[k] = pop;
-      }
+      for (const char* k : {"Sample Population", "Candidate Population"}) js[k] = rowsOf(array(k), n);
   }
 };
 
-// ---- Experiment ------------------------------------------------------------------------------------------------
 // ---- the solver plug-in: Optimizer/MOCMAES on libkcma (include/kmocma.h) ----------------------------------------------
-class MOCMAES : public SolverBase {
+class MOCMAES : public Plugin<kmocma_t, kmocma_cfg> {
  public:
-  kmocma_t* h = nullptr;
-  kmocma_cfg cfg;
   std::vector<double> init_val, init_sd;
-  std::string batched;
-  py::object objective;
-  double tc_max_generations = 1e10, tc_max_model_evaluations = 1e9, tc_max_value = INFINITY, tc_min_value_diff = -INFINITY;
-  double tc_min_max_value_diff = -INFINITY, tc_min_var_diff = -INFINITY, tc_min_sd = -INFINITY, tc_max_sd = INFINITY;
+  Model objective;   // the Python model when cfg.objective is KMOCMA_OBJ_EXTERNAL
 
-  ~MOCMAES() override { if (h) kmocma_destroy(h); }
+  MOCMAES() : Plugin({kmocma_create, kmocma_destroy, kmocma_last_error, kmocma_run_generation, kmocma_check_termination, kmocma_get_array,
+                      kmocma_get_scalar, kmocma_set_scalar},
+                     {{"Min Max Value Difference Threshold", -INFINITY, false, false},   // parsed, but the criterion reads the base threshold
+                      {"Min Variable Difference Threshold", -INFINITY, false, true},
+                      {"Min Standard Deviation", -INFINITY, false, true},
+                      {"Max Standard Deviation", INFINITY, false, true},
+                      {"Max Value", INFINITY, false, false},
+                      {"Min Value Difference Threshold", -INFINITY, false, true},
+                      {"Max Model Evaluations", 1e9, false, true},
+                      {"Max Generations", 1e10, false, true}}) {}
   const char* name() const override { return "Optimizer/MOCMAES"; }
   size_t variableCount() const override { return cfg.n; }
-  void check(int rc) { if (rc) korali_error("%s", kmocma_last_error(h)); }
   double scalar(const char* key) override {
     if (!strcmp(key, "Best Ever Value")) return NAN;    // the base-class scalars are disabled by MOCMAES (:64-66)
-    double v = NAN; check(kmocma_get_scalar(h, key, &v)); return v;
-  }
-  std::vector<double> array(const char* key) override {
-    size_t n = 0;
-    check(kmocma_get_array(h, key, nullptr, 0, &n));
-    std::vector<double> v(n);
-    if (n) check(kmocma_get_array(h, key, v.data(), n, &n));
-    return v;
+    return Plugin::scalar(key);
   }
 
   // generated MOCMAES::setConfiguration (MOCMAES.config) + Optimizer:: + Solver:: (strict)
@@ -1044,31 +1012,13 @@ class MOCMAES : public SolverBase {
     cfg.target_success_rate = s.num("Target Success Rate", 0.175);
     cfg.threshold_probability = s.num("Threshold Probability", 0.44);
     cfg.success_learning_rate = s.num("Success Learning Rate", 0.08);
-    if (s.has("Termination Criteria")) {
-      py::object tco = s.take("Termination Criteria");
-      if (!py::isinstance<py::dict>(tco)) korali_error(" + Object: [ MOCMAES ] \n + Key:    ['Termination Criteria']\n + Reason: not an object\n");
-      py::dict tcd;
-      for (auto kv : py::reinterpret_borrow<py::dict>(tco)) tcd[kv.first] = kv.second;
-      Settings tc(tcd, "MOCMAES['Termination Criteria']");
-      tc_min_max_value_diff = tc.num("Min Max Value Difference Threshold", -INFINITY);   // parsed, but the criterion reads the base threshold
-      tc_min_var_diff = tc.num("Min Variable Difference Threshold", -INFINITY);
-      tc_min_sd = tc.num("Min Standard Deviation", -INFINITY);
-      tc_max_sd = tc.num("Max Standard Deviation", INFINITY);
-      tc_max_value = tc.num("Max Value", INFINITY);
-      tc_min_value_diff = tc.num("Min Value Difference Threshold", -INFINITY);
-      tc_max_model_evaluations = tc.num("Max Model Evaluations", 1e9);
-      tc_max_generations = tc.num("Max Generations", 1e10);
-      tc.finish();
-    }
+    parseCriteria(s);
     for (const char* g : {"Multinormal Generator", "Uniform Generator", "Normal Generator"}) if (s.has(g)) s.take(g);
     const size_t n = py::len(variables);
     if (n == 0) korali_error("Optimization Evaluation problems require at least one variable.\n");
     lower.assign(n, -INFINITY); upper.assign(n, INFINITY); init_val.assign(n, NAN); init_sd.assign(n, NAN);
     for (size_t i = 0; i < n; i++) {
-      if (!py::isinstance<py::dict>(variables[i])) korali_error("Variable %zu is not an object\n", i);
-      py::dict vcopy;
-      for (auto kv : py::reinterpret_borrow<py::dict>(variables[i])) vcopy[kv.first] = kv.second;
-      Settings v(vcopy, "Variable");
+      Settings v = variable(variables, i);
       v.str("Name", "");
       lower[i] = v.num("Lower Bound", -INFINITY);
       upper[i] = v.num("Upper Bound", INFINITY);
@@ -1080,13 +1030,11 @@ class MOCMAES : public SolverBase {
     }
     cfg.n = n; cfg.lower_bound = lower.data(); cfg.upper_bound = upper.data(); cfg.initial_value = init_val.data(); cfg.initial_stddev = init_sd.data();
     cfg.seed = seed;
-    py::dict pcopy;
-    for (auto kv : problem) pcopy[kv.first] = kv.second;
-    Settings p(pcopy, "Optimization");
+    Settings p = object(problem, "Optimization", "'Problem' is not an object\n");
     const std::string ptype = canon(p.str("Type", ""));
     if (ptype != "optimization") korali_error("Korali problem incompatible with MO-CMAES, must be of type 'Optimization'.\n");
     if (!p.has("Objective Function")) korali_error(" + Object: [ Optimization ] \n + Key:    ['Objective Function']\n + Reason: mandatory setting missing\n");
-    objective = p.take("Objective Function");
+    py::object objective_fn = p.take("Objective Function");
     cfg.num_objectives = p.uint("Num Objectives", 1);
     p.boolean("Has Discrete Variables", 0);
     if (p.has("Constraints")) {
@@ -1094,94 +1042,34 @@ class MOCMAES : public SolverBase {
       if (py::isinstance<py::list>(c) && py::len(c) > 0) korali_error("Optimizer/MOCMAES does not take constraints\n");
     }
     p.finish();
-    if (py::isinstance<py::str>(objective)) {
-      const std::string o = canon(objective.cast<std::string>());
+    if (py::isinstance<py::str>(objective_fn)) {
+      const std::string o = canon(objective_fn.cast<std::string>());
       if (o == "negrosenbrockandsphere" || o == "rosenbrockandsphere") cfg.objective = KMOCMA_OBJ_NEG_ROSENBROCK_AND_SPHERE;
       else if (o == "negrosenbrockandtwospheres" || o == "rosenbrockandtwospheres") cfg.objective = KMOCMA_OBJ_NEG_ROSENBROCK_AND_TWO_SPHERES;
       else korali_error("Unknown multi-objective device model '%s' (RosenbrockAndSphere, RosenbrockAndTwoSpheres)\n", o.c_str());
-    } else if (PyCallable_Check(objective.ptr())) {
+    } else if (PyCallable_Check(objective_fn.ptr())) {
       cfg.objective = KMOCMA_OBJ_EXTERNAL;
-      batched = py::hasattr(objective, "_korali_batched") ? objective.attr("_korali_batched").cast<std::string>() : std::string();
-      if (batched == "device") korali_error("Optimizer/MOCMAES takes per-sample models and korali.batched(fn) models (not device-tensor models)\n");
+      objective.set(objective_fn, &pending_error);
+      objective.operation = "Evaluate Multiple";   // sample["F(x)"] is a list of Num Objectives values (optimization.cpp.base)
+      if (objective.flavour == "device") korali_error("Optimizer/MOCMAES takes per-sample models and korali.batched(fn) models (not device-tensor models)\n");
     } else {
       korali_error(" + Object: [ Optimization ] \n + Key:    ['Objective Function']\n + Reason: neither a callable nor the name of a device model\n");
     }
     s.finish();
   }
 
-  // operation "Evaluate Multiple": sample["F(x)"] is a list of Num Objectives values (optimization.cpp.base)
-  static void host_objective(void* user, const double* x, uint64_t rows, uint64_t n, double* f_out, uint64_t K) {
-    MOCMAES* self = (MOCMAES*)user;
-    try {
-      if (self->batched == "numpy") {
-        py::array_t<double> X({(py::ssize_t)rows, (py::ssize_t)n}, {(py::ssize_t)(n * sizeof(double)), (py::ssize_t)sizeof(double)}, x, py::none());
-        py::array_t<double, py::array::c_style | py::array::forcecast> F(self->objective(X));
-        if ((uint64_t)F.size() != rows * K) korali_error("The batched model returned %zu values for %zu samples x %zu objectives\n", (size_t)F.size(), (size_t)rows, (size_t)K);
-        for (uint64_t i = 0; i < rows * K; i++) f_out[i] = F.data()[i];
-        return;
-      }
-      for (uint64_t i = 0; i < rows; i++) {
-        py::dict sample;
-        py::list params;
-        for (uint64_t d = 0; d < n; d++) params.append(x[i * n + d]);
-        sample["Parameters"] = params;
-        sample["Sample Id"] = i;
-        sample["Module"] = "Problem";
-        sample["Operation"] = "Evaluate Multiple";
-        self->objective(sample);
-        if (!sample.contains("F(x)")) korali_error("The model did not set 'F(x)' for sample %zu\n", (size_t)i);
-        py::object fx = sample["F(x)"];
-        if (!(py::isinstance<py::list>(fx) || py::isinstance<py::tuple>(fx)) || (uint64_t)py::len(fx) != K)
-          korali_error("Multi-objective model: 'F(x)' of sample %zu must be a list of %zu values ('Num Objectives')\n", (size_t)i, (size_t)K);
-        uint64_t k = 0;
-        for (auto v : fx) f_out[i * K + k++] = v.cast<double>();
-      }
-    } catch (const std::exception& e) {
-      self->pending_error = e.what();
-      for (uint64_t i = 0; i < rows * K; i++) f_out[i] = NAN;
-    }
-  }
-
   void initialize(const std::vector<int>& device_ids) override {
-    if (device_ids.size() > 1) korali_error("Optimizer/MOCMAES runs on one device (k['Conduit']['Devices'] > 1 is built for Optimizer/CMAES)\n");
-    cfg.device = device_ids[0];
-    if (kmocma_create(&cfg, &h)) korali_error("%s", kmocma_last_error(nullptr));
-    if (cfg.objective == KMOCMA_OBJ_EXTERNAL) check(kmocma_set_host_objective(h, &MOCMAES::host_objective, this));
-    check(kmocma_set_scalar(h, "Termination Criteria/Min Value Difference Threshold", tc_min_value_diff));
-    check(kmocma_set_scalar(h, "Termination Criteria/Min Variable Difference Threshold", tc_min_var_diff));
-    check(kmocma_set_scalar(h, "Termination Criteria/Min Standard Deviation", tc_min_sd));
-    check(kmocma_set_scalar(h, "Termination Criteria/Max Standard Deviation", tc_max_sd));
-    check(kmocma_set_scalar(h, "Termination Criteria/Max Model Evaluations", tc_max_model_evaluations));
-    check(kmocma_set_scalar(h, "Termination Criteria/Max Generations", tc_max_generations));
+    requireOneDevice(device_ids);
+    create(device_ids[0]);
+    if (cfg.objective == KMOCMA_OBJ_EXTERNAL) check(kmocma_set_host_objective(h, &Model::hostMultiple, &objective));
+    pushCriteria();
   }
 
   void restore(uint64_t generation) override {
     if (generation != 0) korali_error("Resuming an Optimizer/MOCMAES run from a result file is not built on the B200 path\n");
   }
 
-  bool checkTermination() override {
-    int fin = 0;
-    const char* reason = "";
-    check(kmocma_check_termination(h, &fin, &reason));
-    if (fin) splitReasons(reason);
-    return fin != 0;
-  }
-
-  void runGeneration() override {
-    pending_error.clear();
-    int rc;
-    if (!needsPython()) { py::gil_scoped_release nogil; rc = kmocma_run_generation(h); }
-    else rc = kmocma_run_generation(h);
-    if (!pending_error.empty()) { std::string e = pending_error; pending_error.clear(); throw std::runtime_error(e); }
-    check(rc);
-  }
   bool needsPython() const override { return cfg.objective == KMOCMA_OBJ_EXTERNAL; }
-
-  py::list rowsOf(const std::vector<double>& flat, size_t width) {
-    py::list out;
-    for (size_t i = 0; width && (i + 1) * width <= flat.size(); i++) out.append(std::vector<double>(flat.begin() + i * width, flat.begin() + (i + 1) * width));
-    return out;
-  }
 
   void printGeneration(const std::function<void(int, const char*)>& log) override {   // MOCMAES::printGenerationAfter :524-537
     char b[256];
@@ -1215,12 +1103,7 @@ class MOCMAES : public SolverBase {
     js["Target Success Rate"] = cfg.target_success_rate;
     js["Threshold Probability"] = cfg.threshold_probability;
     js["Success Learning Rate"] = cfg.success_learning_rate;
-    py::dict tc;
-    tc["Min Max Value Difference Threshold"] = tc_min_max_value_diff; tc["Min Variable Difference Threshold"] = tc_min_var_diff;
-    tc["Min Standard Deviation"] = tc_min_sd; tc["Max Standard Deviation"] = tc_max_sd; tc["Max Value"] = tc_max_value;
-    tc["Min Value Difference Threshold"] = tc_min_value_diff; tc["Max Model Evaluations"] = tc_max_model_evaluations;
-    tc["Max Generations"] = tc_max_generations;
-    js["Termination Criteria"] = tc;
+    emitCriteria(js);
     const size_t n = cfg.n, K = cfg.num_objectives;
     js["Num Objectives"] = K;
     js["Current Non Dominated Sample Count"] = (uint64_t)scalar("Current Non Dominated Sample Count");
@@ -1242,31 +1125,22 @@ class MOCMAES : public SolverBase {
 };
 
 // ---- the solver plug-in: Sampler/TMCMC on libkcma (include/ktmcmc.h) for Bayesian/Custom problems ---------------------------------
-class TMCMC : public SolverBase {
+class TMCMC : public Plugin<ktmcmc_t, ktmcmc_cfg> {
  public:
-  ktmcmc_t* h = nullptr;
-  ktmcmc_cfg cfg;
   py::object distributions = py::none();   // the experiment's top-level "Distributions" (the priors)
   std::vector<int32_t> prior_type;
   std::vector<double> prior_a, prior_b;
   std::vector<uint64_t> burn_in;
   std::vector<std::string> prior_name;
-  std::string batched;
-  py::object model;
-  double tc_target = 1.0, tc_max_generations = 1e10, tc_max_model_evaluations = 1e9;
+  Model model;   // the Python likelihood model when cfg.loglik is KCMA_OBJ_EXTERNAL
 
-  ~TMCMC() override { if (h) ktmcmc_destroy(h); }
+  TMCMC() : Plugin({ktmcmc_create, ktmcmc_destroy, ktmcmc_last_error, ktmcmc_run_generation, ktmcmc_check_termination, ktmcmc_get_array,
+                    ktmcmc_get_scalar, ktmcmc_set_scalar},
+                   {{"Target Annealing Exponent", 1.0, false, true},
+                    {"Max Generations", 1e10, false, true},
+                    {"Max Model Evaluations", 1e9, false, true}}) {}
   const char* name() const override { return "Sampler/TMCMC"; }
   size_t variableCount() const override { return cfg.n; }
-  void check(int rc) { if (rc) korali_error("%s", ktmcmc_last_error(h)); }
-  double scalar(const char* key) override { double v = NAN; check(ktmcmc_get_scalar(h, key, &v)); return v; }
-  std::vector<double> array(const char* key) override {
-    size_t n = 0;
-    check(ktmcmc_get_array(h, key, nullptr, 0, &n));
-    std::vector<double> v(n);
-    if (n) check(ktmcmc_get_array(h, key, v.data(), n, &n));
-    return v;
-  }
 
   // generated TMCMC::setConfiguration (TMCMC.config) + Sampler:: + Solver:: (strict); priors from e["Distributions"]
   void setConfiguration(py::dict solver, py::list variables, py::dict problem, uint64_t seed) override {
@@ -1291,17 +1165,7 @@ class TMCMC : public SolverBase {
     cfg.covariance_scaling = s.num("Covariance Scaling", 0.04);
     cfg.min_annealing_update = s.num("Min Annealing Exponent Update", 1e-5);
     cfg.max_annealing_update = s.num("Max Annealing Exponent Update", 1.0);
-    if (s.has("Termination Criteria")) {
-      py::object tco = s.take("Termination Criteria");
-      if (!py::isinstance<py::dict>(tco)) korali_error(" + Object: [ TMCMC ] \n + Key:    ['Termination Criteria']\n + Reason: not an object\n");
-      py::dict tcd;
-      for (auto kv : py::reinterpret_borrow<py::dict>(tco)) tcd[kv.first] = kv.second;
-      Settings tc(tcd, "TMCMC['Termination Criteria']");
-      tc_target = tc.num("Target Annealing Exponent", 1.0);
-      tc_max_generations = tc.num("Max Generations", 1e10);
-      tc_max_model_evaluations = tc.num("Max Model Evaluations", 1e9);
-      tc.finish();
-    }
+    parseCriteria(s);
     for (const char* g : {"Multinormal Generator", "Uniform Generator", "Normal Generator"}) if (s.has(g)) s.take(g);
     // the state a result file carries (getConfiguration); a run from such a file stops in restore()
     for (const char* k : {"Annealing Exponent", "Previous Annealing Exponent", "Coefficient Of Variation", "LogEvidence", "Max Loglikelihood",
@@ -1311,27 +1175,19 @@ class TMCMC : public SolverBase {
     s.finish();
     if (cfg.population_size < 2) korali_error("Sampler/TMCMC: 'Population Size' must be set to at least 2\n");
     // problem (bayesian/custom.config)
-    py::dict pcopy;
-    for (auto kv : problem) pcopy[kv.first] = kv.second;
-    Settings p(pcopy, "Bayesian/Custom");
+    Settings p = object(problem, "Bayesian/Custom", "'Problem' is not an object\n");
     const std::string ptype = canon(p.str("Type", ""));
     if (ptype != "bayesian/custom") korali_error("Sampler/TMCMC: only Problem Type 'Bayesian/Custom' is served (got '%s')\n", ptype.c_str());
     if (!p.has("Likelihood Model")) korali_error(" + Object: [ Bayesian/Custom ] \n + Key:    ['Likelihood Model']\n + Reason: mandatory setting missing\n");
-    model = p.take("Likelihood Model");
+    py::object model_fn = p.take("Likelihood Model");
     p.finish();
-    if (py::isinstance<py::str>(model)) {
-      const std::string o = canon(model.cast<std::string>());
-      if (o == "negsphere" || o == "sphere") cfg.loglik = KCMA_OBJ_NEG_SPHERE;
-      else if (o == "negrosenbrock" || o == "rosenbrock") cfg.loglik = KCMA_OBJ_NEG_ROSENBROCK;
-      else if (o == "negackley" || o == "ackley") cfg.loglik = KCMA_OBJ_NEG_ACKLEY;
-      else if (o == "negellipsoid" || o == "ellipsoid") cfg.loglik = KCMA_OBJ_NEG_ELLIPSOID;
-      else if (o == "negsumsq") cfg.loglik = KCMA_OBJ_NEG_SUMSQ;
-      else if (o == "negspheresin2") cfg.loglik = KCMA_OBJ_NEG_SPHERE_SIN2;
-      else korali_error("Unknown device likelihood model '%s' (Sphere, Rosenbrock, Ackley, Ellipsoid, NegSumSq, NegSphereSin2)\n", o.c_str());
-    } else if (PyCallable_Check(model.ptr())) {
+    if (py::isinstance<py::str>(model_fn)) {
+      cfg.loglik = deviceObjective(model_fn.cast<std::string>(), "likelihood model");
+    } else if (PyCallable_Check(model_fn.ptr())) {
       cfg.loglik = KCMA_OBJ_EXTERNAL;
-      batched = py::hasattr(model, "_korali_batched") ? model.attr("_korali_batched").cast<std::string>() : std::string();
-      if (!batched.empty() && batched != "numpy" && batched != "device") korali_error("Unknown batched model flavour '%s'\n", batched.c_str());
+      model.set(model_fn, &pending_error);
+      model.output = "logLikelihood";   // Bayesian/Custom "Evaluate": the model sets sample["logLikelihood"]
+      model.fill = 0.0;
     } else {
       korali_error(" + Object: [ Bayesian/Custom ] \n + Key:    ['Likelihood Model']\n + Reason: neither a callable nor the name of a device model\n");
     }
@@ -1341,10 +1197,7 @@ class TMCMC : public SolverBase {
     if (!distributions.is_none()) {
       if (!py::isinstance<py::list>(distributions)) korali_error(" + Object: [ Experiment ] \n + Key:    ['Distributions']\n + Reason: an array was expected\n");
       for (auto item : distributions) {
-        if (!py::isinstance<py::dict>(item)) korali_error("Distributions: every entry must be an object\n");
-        py::dict dcopy;
-        for (auto kv : py::reinterpret_borrow<py::dict>(item)) dcopy[kv.first] = kv.second;
-        Settings d(dcopy, "Distribution");
+        Settings d = object(item, "Distribution", "Distributions: every entry must be an object\n");
         const std::string nm = d.str("Name", ""), ty = d.str("Type", "");
         const std::string ct = canon(ty);
         double a = NAN, b = NAN;
@@ -1362,10 +1215,7 @@ class TMCMC : public SolverBase {
     lower.assign(n, -INFINITY); upper.assign(n, INFINITY);
     prior_type.assign(n, 0); prior_a.assign(n, 0.0); prior_b.assign(n, 0.0); prior_name.assign(n, "");
     for (size_t i = 0; i < n; i++) {
-      if (!py::isinstance<py::dict>(variables[i])) korali_error("Variable %zu is not an object\n", i);
-      py::dict vcopy;
-      for (auto kv : py::reinterpret_borrow<py::dict>(variables[i])) vcopy[kv.first] = kv.second;
-      Settings v(vcopy, "Variable");
+      Settings v = variable(variables, i);
       const std::string vname = v.str("Name", "");
       if (!v.has("Prior Distribution")) korali_error("Variable %zu ('%s') has no 'Prior Distribution'\n", i, vname.c_str());
       const std::string pd = v.str("Prior Distribution", "");
@@ -1384,83 +1234,21 @@ class TMCMC : public SolverBase {
     cfg.per_generation_burn_in = burn_in.empty() ? nullptr : burn_in.data(); cfg.burn_in_count = burn_in.size();
   }
 
-  // Bayesian/Custom "Evaluate": the model sets sample["logLikelihood"]
-  static void host_loglik(void* user, const double* x, uint64_t rows, uint64_t n, double* l_out) {
-    TMCMC* self = (TMCMC*)user;
-    try {
-      if (self->batched == "numpy") {
-        py::array_t<double> X({(py::ssize_t)rows, (py::ssize_t)n}, {(py::ssize_t)(n * sizeof(double)), (py::ssize_t)sizeof(double)}, x, py::none());
-        py::array_t<double, py::array::c_style | py::array::forcecast> F(self->model(X));
-        if ((uint64_t)F.size() != rows) korali_error("The batched model returned %zu values for %zu samples\n", (size_t)F.size(), (size_t)rows);
-        for (uint64_t i = 0; i < rows; i++) l_out[i] = F.data()[i];
-        return;
-      }
-      for (uint64_t i = 0; i < rows; i++) {
-        py::dict sample;
-        py::list params;
-        for (uint64_t d = 0; d < n; d++) params.append(x[i * n + d]);
-        sample["Parameters"] = params;
-        sample["Sample Id"] = i;
-        sample["Module"] = "Problem";
-        sample["Operation"] = "Evaluate";
-        self->model(sample);
-        if (!sample.contains("logLikelihood")) korali_error("The model did not set 'logLikelihood' for sample %zu\n", (size_t)i);
-        l_out[i] = sample["logLikelihood"].cast<double>();
-      }
-    } catch (const std::exception& e) {
-      self->pending_error = e.what();
-      for (uint64_t i = 0; i < rows; i++) l_out[i] = 0.0;
-    }
-  }
-  static void device_loglik(void* user, const double* x_dev, uint64_t rows, uint64_t n, uint64_t ldx, double* f_dev, void* stream) {
-    TMCMC* self = (TMCMC*)user;
-    try {
-      self->model((uintptr_t)x_dev, rows, n, ldx, (uintptr_t)f_dev, (uintptr_t)stream);
-    } catch (const std::exception& e) {
-      self->pending_error = e.what();
-    }
-  }
-
   void initialize(const std::vector<int>& device_ids) override {
-    if (device_ids.size() > 1) korali_error("Sampler/TMCMC runs on one device (k['Conduit']['Devices'] > 1 is built for Optimizer/CMAES)\n");
-    cfg.device = device_ids[0];
-    if (ktmcmc_create(&cfg, &h)) korali_error("%s", ktmcmc_last_error(nullptr));
+    requireOneDevice(device_ids);
+    create(device_ids[0]);
     if (cfg.loglik == KCMA_OBJ_EXTERNAL) {
-      if (batched == "device") check(ktmcmc_set_device_loglik(h, &TMCMC::device_loglik, this));
-      else check(ktmcmc_set_host_loglik(h, &TMCMC::host_loglik, this));
+      if (model.flavour == "device") check(ktmcmc_set_device_loglik(h, &Model::device, &model));
+      else check(ktmcmc_set_host_loglik(h, &Model::host, &model));
     }
-    check(ktmcmc_set_scalar(h, "Termination Criteria/Target Annealing Exponent", tc_target));
-    check(ktmcmc_set_scalar(h, "Termination Criteria/Max Generations", tc_max_generations));
-    check(ktmcmc_set_scalar(h, "Termination Criteria/Max Model Evaluations", tc_max_model_evaluations));
+    pushCriteria();
   }
 
   void restore(uint64_t generation) override {
     if (generation != 0) korali_error("Resuming a Sampler/TMCMC run from a result file is not built on the B200 path\n");
   }
 
-  bool checkTermination() override {
-    int fin = 0;
-    const char* reason = "";
-    check(ktmcmc_check_termination(h, &fin, &reason));
-    if (fin) splitReasons(reason);
-    return fin != 0;
-  }
-
-  void runGeneration() override {
-    pending_error.clear();
-    int rc;
-    if (!needsPython()) { py::gil_scoped_release nogil; rc = ktmcmc_run_generation(h); }
-    else rc = ktmcmc_run_generation(h);
-    if (!pending_error.empty()) { std::string e = pending_error; pending_error.clear(); throw std::runtime_error(e); }
-    check(rc);
-  }
   bool needsPython() const override { return cfg.loglik == KCMA_OBJ_EXTERNAL; }
-
-  py::list rowsOf(const std::vector<double>& flat, size_t width) {
-    py::list out;
-    for (size_t i = 0; width && (i + 1) * width <= flat.size(); i++) out.append(std::vector<double>(flat.begin() + i * width, flat.begin() + (i + 1) * width));
-    return out;
-  }
 
   void printGeneration(const std::function<void(int, const char*)>& log) override {   // TMCMC::printGenerationAfter
     char b[256];
@@ -1495,9 +1283,7 @@ class TMCMC : public SolverBase {
     js["Covariance Scaling"] = cfg.covariance_scaling;
     js["Min Annealing Exponent Update"] = cfg.min_annealing_update;
     js["Max Annealing Exponent Update"] = cfg.max_annealing_update;
-    py::dict tc;
-    tc["Target Annealing Exponent"] = tc_target; tc["Max Generations"] = tc_max_generations; tc["Max Model Evaluations"] = tc_max_model_evaluations;
-    js["Termination Criteria"] = tc;
+    emitCriteria(js);
     for (const char* k : {"Annealing Exponent", "Previous Annealing Exponent", "Coefficient Of Variation", "LogEvidence", "Max Loglikelihood",
                           "Proposals Acceptance Rate", "Selection Acceptance Rate"})
       js[k] = scalar(k);
@@ -1575,23 +1361,26 @@ class Experiment : public KoraliJson {
     py::dict problem_js = py::reinterpret_borrow<py::dict>(top.take("Problem"));
     py::list variables = py::reinterpret_borrow<py::list>(top.take("Variables"));
     const std::string stype = canon(solver_js.contains("Type") && py::isinstance<py::str>(solver_js["Type"]) ? solver_js["Type"].cast<std::string>() : "");
-    const bool tmcmc = stype == "sampler/tmcmc" || stype == "tmcmc";
-    if (stype != "optimizer/cmaes" && stype != "cmaes" && stype != "optimizer/dea" && stype != "dea" && stype != "optimizer/mocmaes" && stype != "mocmaes" && !tmcmc)
+    // the solver types, by canonical name and short name; TMCMC reads its priors from e["Distributions"], the optimizers ignore the key
+    using Factory = std::unique_ptr<SolverBase> (*)(py::object distributions);
+    static const struct { const char* type; const char* alias; Factory make; } kSolvers[] = {
+        {"optimizer/cmaes", "cmaes", [](py::object) -> std::unique_ptr<SolverBase> { return std::make_unique<CMAES>(); }},
+        {"optimizer/dea", "dea", [](py::object) -> std::unique_ptr<SolverBase> { return std::make_unique<DEA>(); }},
+        {"optimizer/mocmaes", "mocmaes", [](py::object) -> std::unique_ptr<SolverBase> { return std::make_unique<MOCMAES>(); }},
+        {"sampler/tmcmc", "tmcmc", [](py::object d) -> std::unique_ptr<SolverBase> { auto t = std::make_unique<TMCMC>(); t->distributions = d; return t; }}};
+    Factory make = nullptr;
+    for (const auto& t : kSolvers) if (stype == t.type || stype == t.alias) make = t.make;
+    if (!make)
       korali_error("Solver Type '%s' is not served by korali_b200: only 'Optimizer/CMAES', 'Optimizer/DEA', 'Optimizer/MOCMAES' and 'Sampler/TMCMC' are built (SURVEY.md scope)\n", stype.c_str());
     random_seed = top.uint("Random Seed", 0);
     if (random_seed == 0) random_seed = (uint64_t)std::chrono::system_clock::now().time_since_epoch().count();  // experiment.cpp.base:235-251
     top.boolean("Preserve Random Number Generator States", 0);
     top.boolean("Store Sample Information", 0);
     current_generation = top.uint("Current Generation", 0);
-    py::object distributions = py::none();   // the priors of Sampler/TMCMC; the optimizers ignore the key
-    if (tmcmc && top.has("Distributions")) distributions = top.take("Distributions");
-    for (const char* k : {"Distributions", "Results", "Samples", "Globals", "Run ID", "Timestamp", "Type", "Is Finished"}) if (top.has(k)) top.take(k);
+    py::object distributions = top.has("Distributions") ? top.take("Distributions") : py::none();
+    for (const char* k : {"Results", "Samples", "Globals", "Run ID", "Timestamp", "Type", "Is Finished"}) if (top.has(k)) top.take(k);
     if (top.has("Console Output")) {
-      py::object co = top.take("Console Output");
-      if (!py::isinstance<py::dict>(co)) korali_error("'Console Output' is not an object\n");
-      py::dict cd;
-      for (auto kv : py::reinterpret_borrow<py::dict>(co)) cd[kv.first] = kv.second;
-      Settings c(cd, "Experiment['Console Output']");
+      Settings c = object(top.take("Console Output"), "Experiment['Console Output']", "'Console Output' is not an object\n");
       const std::string v = c.str("Verbosity", "Normal");
       if (v == "Silent") verbosity = SILENT; else if (v == "Minimal") verbosity = MINIMAL; else if (v == "Normal") verbosity = NORMAL;
       else if (v == "Detailed") verbosity = DETAILED; else korali_error("Unknown Console Output Verbosity '%s'\n", v.c_str());
@@ -1599,11 +1388,7 @@ class Experiment : public KoraliJson {
       c.finish();
     }
     if (top.has("File Output")) {
-      py::object fo = top.take("File Output");
-      if (!py::isinstance<py::dict>(fo)) korali_error("'File Output' is not an object\n");
-      py::dict fd;
-      for (auto kv : py::reinterpret_borrow<py::dict>(fo)) fd[kv.first] = kv.second;
-      Settings f(fd, "Experiment['File Output']");
+      Settings f = object(top.take("File Output"), "Experiment['File Output']", "'File Output' is not an object\n");
       file_enabled = f.boolean("Enabled", 1);
       file_path = f.str("Path", "_korali_result");
       file_frequency = f.uint("Frequency", 1);
@@ -1613,10 +1398,7 @@ class Experiment : public KoraliJson {
       f.finish();
     }
     top.finish();
-    if (stype == "optimizer/dea" || stype == "dea") solver = std::make_unique<DEA>();
-    else if (stype == "optimizer/mocmaes" || stype == "mocmaes") solver = std::make_unique<MOCMAES>();
-    else if (tmcmc) { auto t = std::make_unique<TMCMC>(); t->distributions = distributions; solver = std::move(t); }
-    else solver = std::make_unique<CMAES>();
+    solver = make(distributions);
     solver->setConfiguration(solver_js, variables, problem_js, random_seed);   // Normal Generator gets seed S (distribution.cpp.base:36-37)
     solver->initialize(devices);
     solver->restore(current_generation);

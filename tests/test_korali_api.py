@@ -75,6 +75,7 @@ def base_mo():
     (lambda e: e["Problem"].__setitem__("Objective Function", "Ellipsoid"), "Unknown multi-objective device model"),
     (lambda e: e["Problem"].__setitem__("Num Objectives", 3), "the built-in objective has 2 objectives"),
     (lambda e: e["Variables"][0].__setitem__("Upper Bound", float("inf")), "cannot be inferred"),                # :70-82
+    (lambda e: e["Solver"].__setitem__("Termination Criteria", 5), r"MOCMAES \] \n \+ Key:    \['Termination Criteria'\]\n \+ Reason: not an object"),
 ])
 def test_mocmaes_configuration_errors(mod, match):
     """The configuration checks of MOCMAES::setInitialConfiguration (tests/unit/modules/solver/optimizers.cpp:2112-2180) are raised
@@ -82,6 +83,28 @@ def test_mocmaes_configuration_errors(mod, match):
     e = base_mo()
     mod(e)
     e["Solver"]["Type"]
+    with pytest.raises(RuntimeError, match=match):
+        korali.Engine().run(e)
+
+
+@pytest.mark.parametrize("mod,match", [
+    (lambda e: e["Solver"].__setitem__("Bogus Key", 3), "Unrecognized settings for Korali module: DEA"),
+    (lambda e: e["Solver"]["Termination Criteria"].__setitem__("Max Fun", 1), r"Unrecognized settings for Korali module: DEA\['Termination Criteria'\]"),
+    (lambda e: e["Solver"].__setitem__("Termination Criteria", 5), r"DEA \] \n \+ Key:    \['Termination Criteria'\]\n \+ Reason: not an object"),
+    (lambda e: e["Solver"].__setitem__("Accept Rule", "Sideways"), r"Accept Rule \(Sideways\) not recognized"),
+    (lambda e: e["Solver"].__setitem__("Parent Selection Rule", "Worst"), r"Invalid setting of Parent Selection Rule \(Worst\)"),
+    (lambda e: e["Solver"].__setitem__("Mutation Rule", "Self Adaptive"), "Mutation Rule 'Self Adaptive' is not built"),
+    (lambda e: e["Problem"].__setitem__("Objective Function", "Banana"), "Unknown device objective 'banana'"),
+    (lambda e: e["Problem"].__setitem__("Constraints", [evalmodel]), "Optimizer/DEA does not take constraints"),
+    (lambda e: e["Problem"].__setitem__("Objective Function", korali.batched_device(lambda X: X.sum(1))),
+     r"Optimizer/DEA takes per-sample models and korali.batched\(fn\) models"),
+])
+def test_dea_configuration_errors(mod, match):
+    """DEA's strict configuration (termination criteria, rules, objective, constraints) is checked before any device work."""
+    e = base_1d()
+    e["Solver"]["Type"] = "Optimizer/DEA"
+    mod(e)
+    e["Solver"]["Type"]     # reset the cursor after the chained access above
     with pytest.raises(RuntimeError, match=match):
         korali.Engine().run(e)
 

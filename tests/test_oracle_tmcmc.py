@@ -118,6 +118,7 @@ def without_likelihood_model():
     (lambda e: e["Problem"].__setitem__("Type", "Optimization"), "only Problem Type 'Bayesian/Custom'"),
     (lambda e: e["Solver"].__setitem__("Bogus Key", 1), "Unrecognized settings for Korali module: TMCMC"),
     (lambda e: e["Problem"].__setitem__("Likelihood Model", "Banana"), "Unknown device likelihood model"),
+    (lambda e: e["Solver"].__setitem__("Termination Criteria", 5), r"TMCMC \] \n \+ Key:    \['Termination Criteria'\]\n \+ Reason: not an object"),
 ])
 def test_configuration_errors(mod, match):
     e = base()
