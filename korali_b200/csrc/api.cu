@@ -124,11 +124,6 @@ struct kcma {
   std::vector<double> hX, hF, hG;
   // tridiagonalisation-based eigensolver (created on first use)
   kc::TridiagWs* tri = nullptr;
-  // Philox draws of the generation issued on a side stream beside the divide & conquer stage of the eigensolver (they need only
-  // seed + generation, VERDICT r01 weak #10); never beside sytrd_kernel, whose cooperative launch needs every SM for itself
-  cudaStream_t rng_stream = nullptr;
-  cudaEvent_t ev_rng_fork = nullptr, ev_rng_done = nullptr;
-  bool rng_prelaunched = false;
   // nccl
   ncclComm_t comm = nullptr;
   bool comm_in_process = false;   // kcma_comm_init_all: the ranks are threads of one process (no graph replay there, see graph_eligible)
@@ -421,36 +416,16 @@ int ensure_vt(kcma* h) {
   return 0;
 }
 
-// Which eigensolver runs above the single-CTA size: KCMA_EIGEN=tridiag (default) | jacobi (the round-1 warm-started one-sided
-// Jacobi kernels, kept for A/B runs). Read per call so that one process can time both.
+// Which eigensolver runs above the single-CTA size: the tridiagonal one, or the warm-started one-sided Jacobi kernels on the
+// constraint path and beyond the tridiagonal solver's size. KCMA_EIGEN=tridiag | jacobi forces one of the two, so that tests can
+// compare them on the same input; read per call so that one process can run both.
 bool eigen_use_tridiag(const kcma* h) {
   const char* e = getenv("KCMA_EIGEN");
   if (e && !strcmp(e, "jacobi")) return false;
   // The constraint path decomposes C_aux once per correction round (handleConstraints :774-832): nearly the same matrix again and
   // again, which the warm-started one-sided Jacobi finishes in a sweep or two (config 5: 3.9 instead of 6.1 ms per generation)
   if (h->has_constraints && h->N <= 1184 && !(e && !strcmp(e, "tridiag"))) return false;
-  return h->N >= 4 && (size_t)h->N * 5 * sizeof(double) + 4096 <= 226 * 1024;
-}
-
-unsigned gen_arg(const kcma* h);
-uint64_t local_zrows(const kcma* h);
-
-// The draws can be issued early when nothing is injected for this generation and no phase timers run (they would not see the side stream).
-bool rng_overlap_ok(kcma* h) {
-  // measured on config 3 (profiles/r02_bench_v6_rng_overlap.log): 11.21 ms per generation with and without — the draws do not hide
-  // behind the small launches of the eigensolver's second stage, so this stays an opt-in (KCMA_RNG_OVERLAP=1)
-  static const int on = getenv("KCMA_RNG_OVERLAP") ? atoi(getenv("KCMA_RNG_OVERLAP")) : 0;
-  if (!on || h->timing || h->inj_z || h->inj_y || h->inj_x || h->cfg.diagonal_covariance) return false;
-  if (!h->rng_stream) {
-    if (cudaStreamCreateWithFlags(&h->rng_stream, cudaStreamNonBlocking) != cudaSuccess ||
-        cudaEventCreateWithFlags(&h->ev_rng_fork, cudaEventDisableTiming) != cudaSuccess ||
-        cudaEventCreateWithFlags(&h->ev_rng_done, cudaEventDisableTiming) != cudaSuccess) {
-      cudaGetLastError();
-      h->rng_stream = nullptr;
-      return false;
-    }
-  }
-  return true;
+  return eigen_tridiag_fits(h->N);
 }
 
 // updateEigensystem (CMAES.cpp.base:869-890) + eigen (:896-938)
@@ -467,8 +442,7 @@ int update_eigensystem(kcma* h, const double* dM) {
   ensure_vt(h);
   const double tol = 4.0 * 2.220446049250313e-16 * sqrt((double)N);
   const int max_sweeps = 40;
-  static const int small_max = getenv("KCMA_EIGEN_SMALL_MAX") ? atoi(getenv("KCMA_EIGEN_SMALL_MAX")) : 24;
-  if (eigen_small_fits(N) && N <= small_max) {  // the whole solver in one launch, everything in one SM's shared memory
+  if (eigen_use_small(N)) {  // the whole solver in one launch, everything in one SM's shared memory
     launch_eigen_small(h->stream, dM, ld, N, h->dVT, h->dGT, h->dB, h->dA, h->dD, tol, max_sweeps, h->dSc);
     h->launches += 2;
     h->scalars_fresh = false;
@@ -485,16 +459,6 @@ int update_eigensystem(kcma* h, const double* dM) {
     bool ok;
     { PhaseTimer t1(h, "eigen_sytrd"); ok = tridiag_stage_sytrd(h->stream, h->tri, dM); }
     if (ok) ok = tridiag_stage_back_fork(h->stream, h->tri, &l);   // Q accumulation on the side stream, next to stage 2
-    if (ok && dM == h->dC && rng_overlap_ok(h)) {
-      const long long zrows = (long long)local_zrows(h);
-      const unsigned long long zrow_begin = h->cfg.mirrored_sampling ? h->shard_lo / 2 : h->shard_lo;
-      cudaEventRecord(h->ev_rng_fork, h->stream);
-      cudaStreamWaitEvent(h->rng_stream, h->ev_rng_fork, 0);
-      launch_philox_normal(h->rng_stream, h->dZ, ld, zrows, N, h->cfg.seed, gen_arg(h), zrow_begin, nullptr, nullptr, h->num_sms, h->dSc);
-      cudaEventRecord(h->ev_rng_done, h->rng_stream);
-      h->rng_prelaunched = true;
-      h->launches++;
-    }
     if (ok) { PhaseTimer t2(h, "eigen_dc"); ok = tridiag_stage_dc(h->stream, h->tri, &l); }
     if (ok) { PhaseTimer t3(h, "eigen_back"); ok = tridiag_stage_back_join(h->stream, h->tri, &l); }
     if (!ok) return fail(h, "the tridiagonal eigensolver could not be launched: %s", cudaGetErrorString(cudaGetLastError()));
@@ -690,9 +654,7 @@ int sample_population(kcma* h) {
   const long long zrows = (long long)local_zrows(h);
   const unsigned long long zrow_begin = h->cfg.mirrored_sampling ? h->shard_lo / 2 : h->shard_lo;
   if (!h->inj_y && !h->inj_x) {
-    if (h->rng_prelaunched) {   // drawn on the side stream beside the eigensolver's second stage
-      cudaStreamWaitEvent(h->stream, h->ev_rng_done, 0);
-    } else if (!h->inj_z) {
+    if (!h->inj_z) {
       PhaseTimer t(h, "rng");
       launch_philox_normal(h->stream, h->dZ, ld, zrows, N, h->cfg.seed, gen_arg(h), zrow_begin, nullptr, nullptr, h->num_sms, h->dSc);
       h->launches++;
@@ -706,8 +668,6 @@ int sample_population(kcma* h) {
     }
     h->launches++;
   }
-  if (h->rng_prelaunched && (h->inj_y || h->inj_x)) cudaStreamWaitEvent(h->stream, h->ev_rng_done, 0);   // (cannot happen: see rng_overlap_ok)
-  h->rng_prelaunched = false;
   copy_sigma_kernel<<<1, 1, 0, h->stream>>>(h->dSc, h->dSigmaSampling);
   h->launches++;
   CUDA_OK(h, cudaMemsetAsync(h->dAttempt, 0, sizeof(unsigned) * (size_t)(zrows > 0 ? zrows : 1), h->stream));
@@ -892,7 +852,6 @@ int update_and_handle_constraints(kcma* h) {
 }
 
 int do_ask(kcma* h) {
-  h->rng_prelaunched = false;
   if (h->has_constraints && check_mean_and_set_regime(h)) return 1;
   if (update_eigensystem(h, h->dC)) return 1;
   if (sample_population(h)) return 1;
@@ -1149,9 +1108,6 @@ void kcma_destroy(kcma_t* h) {
   if (h->cap_stream) cudaStreamDestroy(h->cap_stream);
   if (h->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(h->comm);
   kc::tridiag_ws_destroy(h->tri);
-  if (h->rng_stream) { cudaStreamSynchronize(h->rng_stream); cudaStreamDestroy(h->rng_stream); }
-  if (h->ev_rng_fork) cudaEventDestroy(h->ev_rng_fork);
-  if (h->ev_rng_done) cudaEventDestroy(h->ev_rng_done);
   void* ptrs[] = {h->dC, h->dB, h->dA, h->dD, h->dVT, h->dVTw, h->dGT, h->dEv, h->dPerm, h->dMean, h->dMeanOld, h->dMeanUpd, h->dT,
                   h->dPs, h->dPc, h->dZ, h->dY, h->dX, h->dF, h->dIdx, h->dSortWs, h->dW, h->dSelW, h->dSelS, h->dCount, h->dS,
                   h->dPartial, h->dWsplit, h->dRed, h->dBestEver, h->dCurBest, h->dLower, h->dUpper, h->dMinSd, h->dCoef, h->dShift,

@@ -8,11 +8,10 @@
 // lambda_i = v_i . g_i (Rayleigh quotient, signed). Vectors are stored as ROWS (VT, GT) so rotations touch contiguous memory.
 // Kernels: eigen_small_kernel (tiny N, everything in one launch), jacobi_pipe_kernel (24 < N <= 1184: persistent cooperative,
 // warp-specialised Gram-update steps on the DMMA pipe, 4-row blocks), jacobi_big_step_kernel (larger N: one launch per
-// tournament step, 16-row blocks, V updated one launch late), jacobi_gram_step_kernel (4-row blocks per launch, A/B only).
+// tournament step, 16-row blocks, V updated one launch late).
 // DESIGN.md section 6.
 #include <cooperative_groups.h>
 #include <stdlib.h>
-#include <string.h>
 
 #include "common.cuh"
 #include "jacobi_inner.cuh"
@@ -61,17 +60,13 @@ __device__ __forceinline__ void stcg_256(double* p, double a, double b, double c
 //   * V group (the last NWV warps, none on warp 0's scheduler) applies the same R to the V rows behind it, decoupled:
 //     R travels through a small ring in shared memory, V blocks have their own ready flags, nothing on the G path waits for V.
 // ------------------------------------------------------------------------------------------------------
-template <int NT, int ORDER /* 0: round-robin, 1: ring (nb = power of two), 2: ring + the slot's first block resident in shared memory */>
+template <int NT, int ORDER /* 0: round-robin, 1: ring (nb = power of two) */>
 __global__ void __launch_bounds__(NT, 1)
 jacobi_pipe_kernel(double* GT, double* VT, int ld, int n, int nb, double tol, int max_sweeps, DevScalars* sc, unsigned* readyG,
                    unsigned* readyV, long long* dbg /* nullable: phase timestamps (profiles/microbench/jacobi_phases.py) */, int dbg_sweep, int dbg_step0) {
   cg::grid_group grid = cg::this_grid();
 #define KCMA_TS(slot) do { if (dbg && blockIdx.x == 1 && tid == 0 && sweep == dbg_sweep && step >= dbg_step0 && step < dbg_step0 + 32) dbg[(step - dbg_step0) * 16 + (slot)] = clock64(); } while (0)
 #define KCMA_TSV(slot) do { if (dbg && blockIdx.x == 1 && tid == NWG * 32 && sweep == dbg_sweep && step >= dbg_step0 && step < dbg_step0 + 32) dbg[(step - dbg_step0) * 16 + (slot)] = clock64(); } while (0)
-  // ORDER 2 (experimental): in the ring order the first block I of a slot stays the same for all but log2(nb) - 1 of the
-  // nb - 2 step transitions of a sweep. Its 4 rows of G (and of V) then stay in rows 0-3 of Gs (Vs) from step to step: they are
-  // neither re-fetched nor written back nor flagged while the slot keeps them; only the travelling block J goes through L2.
-  constexpr bool ANCHOR = (ORDER == 2);
   constexpr int NW = NT / 32;                       // 8: warp 0 | data warps 1..4 | V warps 5..7
   constexpr int NWV = 3;                            // V warps on schedulers 1, 2, 3 (none shares the FP64 pipe of warp 0)
   constexpr int NWG = NW - NWV;                     // G group: warp 0 (flags, rotations) + NWD data warps
@@ -95,7 +90,6 @@ jacobi_pipe_kernel(double* GT, double* VT, int ld, int n, int nb, double tol, in
   const int nspans = ld >> 4;
   const double tol2 = tol * tol;
   unsigned epoch = 0;                               // steps completed by this group of this CTA
-  bool g_dirty = false, v_valid = false, v_dirty = false;   // ORDER 2: resident anchor rows newer than global / present in Vs
   if (tid == 0) { g_head = 0; v_tail = 0; }
   __syncthreads();
 
@@ -111,18 +105,11 @@ jacobi_pipe_kernel(double* GT, double* VT, int ld, int n, int nb, double tol, in
       for (int step = 0; step < nb - 1; step++) {
         int I, J;
         tournament_pair<ORDER>(nb, step, blockIdx.x, I, J);
-        bool keep_prev = false, keep_next = false;    // block I was / stays this slot's first block: its rows are / stay in Gs[0..3]
-        if (ANCHOR) {
-          int Ia, Ja;
-          if (step > 0) { ring_pair(nb, step - 1, blockIdx.x, Ia, Ja); keep_prev = (Ia == I); }
-          if (step + 2 < nb) { ring_pair(nb, step + 1, blockIdx.x, Ia, Ja); keep_next = (Ia == I); }
-          if (!keep_prev) g_dirty = false;
-        }
         const int slot = epoch & (RING - 1);
         KCMA_TS(0);
         if (dbg && blockIdx.x == 1 && tid == 0 && sweep == dbg_sweep && step < 1024) dbg[512 + step] = clock64();
         if (warp == 0) {   // lanes 0 and 1 each watch one flag (acquire loads: no fence, no serialised round trips)
-          if (lane < 2 && !(ANCHOR && lane == 0 && keep_prev)) {
+          if (lane < 2) {
             const unsigned* f = readyG + (lane == 0 ? I : J);
             unsigned v;
             do { asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(f) : "memory"); } while (v < epoch);
@@ -144,20 +131,12 @@ jacobi_pipe_kernel(double* GT, double* VT, int ld, int n, int nb, double tol, in
             for (int k = 0; k < BG; k++) {
               const int h = dw + (kb + k) * NWD;
               xs[k].a = xs[k].b = xs[k].c = xs[k].d = 0.0;
-              if (rvalid && h < nspans) {
-                if (ANCHOR && keep_prev && g < 4) {   // resident anchor rows: from shared memory
-                  const double* sp = Gs + g * S + 16 * h + 4 * t;
-                  const double2 u = *reinterpret_cast<const double2*>(sp), v = *reinterpret_cast<const double2*>(sp + 2);
-                  xs[k].a = u.x; xs[k].b = u.y; xs[k].c = v.x; xs[k].d = v.y;
-                } else {
-                  xs[k] = ldcg_256(grow + 16 * h + 4 * t);
-                }
-              }
+              if (rvalid && h < nspans) xs[k] = ldcg_256(grow + 16 * h + 4 * t);
             }
 #pragma unroll
             for (int k = 0; k < BG; k++) {   // two independent accumulator chains
               const int h = dw + (kb + k) * NWD;
-              if (h < nspans && !(ANCHOR && keep_prev && g < 4)) {
+              if (h < nspans) {
                 double* dst = Gs + g * S + 16 * h + 4 * t;
                 *reinterpret_cast<double2*>(dst) = make_double2(xs[k].a, xs[k].b);
                 *reinterpret_cast<double2*>(dst + 2) = make_double2(xs[k].c, xs[k].d);
@@ -218,36 +197,13 @@ jacobi_pipe_kernel(double* GT, double* VT, int ld, int n, int nb, double tol, in
               bA0[k] = ok ? src[0] : 0.0;         bB0[k] = ok ? src[2] : 0.0;
               bA1[k] = ok ? src[4 * S] : 0.0;     bB1[k] = ok ? src[4 * S + 2] : 0.0;
             }
-            if (ANCHOR) __syncwarp();   // every operand of the batch is read before a resident row of these spans is overwritten
 #pragma unroll
             for (int k = 0; k < 8; k++) {
               const int h = h0 + k * NWD;
               double d0 = 0.0, d1 = 0.0, e0 = 0.0, e1 = 0.0;
               dmma884(d0, d1, a_lo, bA0[k]); dmma884(e0, e1, a_lo, bB0[k]);
               dmma884(d0, d1, a_hi, bA1[k]); dmma884(e0, e1, a_hi, bB1[k]);
-              if (h < nspans && rvalid) {
-                if (ANCHOR && keep_next && g < 4) {   // the anchor block stays: update it in place in shared memory
-                  double* dst = Gs + g * S + 16 * h + 4 * t;
-                  *reinterpret_cast<double2*>(dst) = make_double2(d0, d1);
-                  *reinterpret_cast<double2*>(dst + 2) = make_double2(e0, e1);
-                } else {
-                  stcg_256(gout + 16 * h + 4 * t, d0, d1, e0, e1);
-                }
-              }
-            }
-          }
-        }
-        if (ANCHOR) {
-          // kept: newer than global; released: written to global just now. While the block is kept, rotation-free steps leave
-          // the flag alone: the copy in shared memory stays ahead of global until the block is released.
-          if (rot != 0) g_dirty = keep_next;
-          else if (!keep_next && g_dirty && warp != 0 && g < 4 && rvalid) {
-            // released without a rotation in this step, but updated in shared memory since it was fetched: write it back
-            double* gout = GT + (size_t)rowg * ld;
-            for (int h = warp - 1; h < nspans; h += NWD) {
-              const double* sp = Gs + g * S + 16 * h + 4 * t;
-              const double2 u = *reinterpret_cast<const double2*>(sp), v = *reinterpret_cast<const double2*>(sp + 2);
-              stcg_256(gout + 16 * h + 4 * t, u.x, u.y, v.x, v.y);
+              if (h < nspans && rvalid) stcg_256(gout + 16 * h + 4 * t, d0, d1, e0, e1);
             }
           }
         }
@@ -256,7 +212,7 @@ jacobi_pipe_kernel(double* GT, double* VT, int ld, int n, int nb, double tol, in
         if (tid == 0) {
           __threadfence();                          // gpu scope: the G rows; also orders Rring before g_head for the V group
           volatile unsigned* rg = readyG;
-          if (!(ANCHOR && keep_next)) rg[I] = epoch + 1;
+          rg[I] = epoch + 1;
           rg[J] = epoch + 1;
           g_head = epoch + 1;
         }
@@ -269,13 +225,6 @@ jacobi_pipe_kernel(double* GT, double* VT, int ld, int n, int nb, double tol, in
       for (int step = 0; step < nb - 1; step++) {
         int I, J;
         tournament_pair<ORDER>(nb, step, blockIdx.x, I, J);
-        bool keep_prev = false, keep_next = false;
-        if (ANCHOR) {
-          int Ia, Ja;
-          if (step > 0) { ring_pair(nb, step - 1, blockIdx.x, Ia, Ja); keep_prev = (Ia == I); }
-          if (step + 2 < nb) { ring_pair(nb, step + 1, blockIdx.x, Ia, Ja); keep_next = (Ia == I); }
-          if (!keep_prev) { v_valid = false; v_dirty = false; }
-        }
         const int slot = epoch & (RING - 1);
         KCMA_TSV(9);
         if (dbg && blockIdx.x == 1 && tid == NWG * 32 && sweep == dbg_sweep && step < 1024) dbg[512 + 1024 + step] = clock64();
@@ -286,7 +235,7 @@ jacobi_pipe_kernel(double* GT, double* VT, int ld, int n, int nb, double tol, in
         asm volatile("bar.sync 2, %0;" ::"n"(NWV * 32));
         KCMA_TSV(10);
         const int rot = rot_ring[slot];
-        if (vtid < 2 && !(ANCHOR && vtid == 0 && keep_prev)) {   // the previous owners are done with these V blocks (also when nothing rotates here:
+        if (vtid < 2) {   // the previous owners are done with these V blocks (also when nothing rotates here:
           const unsigned* f = readyV + (vtid == 0 ? I : J);   // publishing them early would let the next owner overtake a pending update)
           unsigned v;
           do { asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(f) : "memory"); } while (v < epoch);
@@ -296,7 +245,7 @@ jacobi_pipe_kernel(double* GT, double* VT, int ld, int n, int nb, double tol, in
           asm volatile("bar.sync 2, %0;" ::"n"(NWV * 32));
           const int chunks = ld >> 1;   // 16-byte chunks per row
 #pragma unroll
-          for (int r = (ANCHOR && v_valid) ? 4 : 0; r < 8; r++) {   // (resident anchor rows are not fetched again)
+          for (int r = 0; r < 8; r++) {
             const int row = (r < 4 ? I * 4 + r : J * 4 + (r - 4));
             const bool ok = row < n;
             const double* src = VT + (ok ? (size_t)row * ld : 0);
@@ -321,34 +270,13 @@ jacobi_pipe_kernel(double* GT, double* VT, int ld, int n, int nb, double tol, in
               bA0[k] = ok ? src[0] : 0.0;         bB0[k] = ok ? src[2] : 0.0;
               bA1[k] = ok ? src[4 * S] : 0.0;     bB1[k] = ok ? src[4 * S + 2] : 0.0;
             }
-            if (ANCHOR) __syncwarp();
 #pragma unroll
             for (int k = 0; k < 8; k++) {
               const int h = h0 + k * NWV;
               double d0 = 0.0, d1 = 0.0, e0 = 0.0, e1 = 0.0;
               dmma884(d0, d1, a_lo, bA0[k]); dmma884(e0, e1, a_lo, bB0[k]);
               dmma884(d0, d1, a_hi, bA1[k]); dmma884(e0, e1, a_hi, bB1[k]);
-              if (h < nspans && prow < n) {
-                if (ANCHOR && keep_next && g < 4) {
-                  double* dst = Vs + g * S + 16 * h + 4 * t;
-                  *reinterpret_cast<double2*>(dst) = make_double2(d0, d1);
-                  *reinterpret_cast<double2*>(dst + 2) = make_double2(e0, e1);
-                } else {
-                  stcg_256(vout + 16 * h + 4 * t, d0, d1, e0, e1);
-                }
-              }
-            }
-          }
-          if (ANCHOR) { v_valid = keep_next; v_dirty = keep_next; }   // (released: rows 0-3 of Vs hold the pre-rotation rows)
-        } else if (ANCHOR && !keep_next && v_dirty) {
-          // released without a rotation in this step, but updated in shared memory since it was fetched: write it back
-          const int prow = I * 4 + g;
-          if (g < 4 && prow < n) {
-            double* vout = VT + (size_t)prow * ld;
-            for (int h = vw; h < nspans; h += NWV) {
-              const double* sp = Vs + g * S + 16 * h + 4 * t;
-              const double2 u = *reinterpret_cast<const double2*>(sp), v = *reinterpret_cast<const double2*>(sp + 2);
-              stcg_256(vout + 16 * h + 4 * t, u.x, u.y, v.x, v.y);
+              if (h < nspans && prow < n) stcg_256(vout + 16 * h + 4 * t, d0, d1, e0, e1);
             }
           }
         }
@@ -357,7 +285,7 @@ jacobi_pipe_kernel(double* GT, double* VT, int ld, int n, int nb, double tol, in
         if (vtid == 0) {
           __threadfence();   // release: our stores, and (when nothing rotated here) the previous owners' rows we acquired above
           volatile unsigned* rv = readyV;
-          if (!(ANCHOR && keep_next)) rv[I] = epoch + 1;
+          rv[I] = epoch + 1;
           rv[J] = epoch + 1;
           v_tail = epoch + 1;
         }
@@ -377,102 +305,6 @@ jacobi_pipe_kernel(double* GT, double* VT, int ld, int n, int nb, double tol, in
   }
 #undef KCMA_TS
 #undef KCMA_TSV
-}
-
-// One Gram-update step per launch (N too large for one co-resident CTA per block pair, e.g. N = 4096: 512 pairs).
-// Same algebra as jacobi_pipe_kernel, no pipelining: every step streams G and V through HBM (they exceed L2 at that size).
-template <int NT>
-__global__ void __launch_bounds__(NT, 1)
-jacobi_gram_step_kernel(double* GT, double* VT, int ld, int n, int nb, int step, double tol, DevScalars* sc) {
-  constexpr int NW = NT / 32;
-  __shared__ double part[NW][64];
-  __shared__ double Gam[8][9];
-  __shared__ double Rm[8][9];
-  __shared__ int s_rot;
-  __shared__ unsigned long long s_max;
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31, g = lane >> 2, t = lane & 3;
-  const int ngroups = ld >> 3;
-  int I, J;
-  rr_pair(nb, step, blockIdx.x, I, J);
-  const int rowg = (g < 4 ? I * 4 + g : J * 4 + (g - 4));
-  const bool rvalid = rowg < n;
-  const double* grow = GT + (size_t)rowg * ld;
-  double c0 = 0.0, c1 = 0.0, c2 = 0.0, c3 = 0.0;
-  for (int grp0 = warp; grp0 < ngroups; grp0 += NW * 8) {   // 8 groups in flight per warp
-    double2 xs[8];
-#pragma unroll
-    for (int k = 0; k < 8; k++) {
-      const int grp = grp0 + k * NW;
-      xs[k] = make_double2(0.0, 0.0);
-      if (rvalid && grp < ngroups) xs[k] = *reinterpret_cast<const double2*>(grow + 8 * grp + 2 * t);
-    }
-#pragma unroll
-    for (int k = 0; k < 8; k++) { dmma884(c0, c1, xs[k].x, xs[k].x); dmma884(c2, c3, xs[k].y, xs[k].y); }
-  }
-  part[warp][g * 8 + 2 * t] = c0 + c2;
-  part[warp][g * 8 + 2 * t + 1] = c1 + c3;
-  if (tid == 0) { s_rot = 0; s_max = 0ull; }
-  __syncthreads();
-  if (tid < 64) {
-    double a = 0.0;
-#pragma unroll
-    for (int w = 0; w < NW; w++) a += part[w][tid];
-    Gam[tid >> 3][tid & 7] = a;
-    Rm[tid >> 3][tid & 7] = ((tid >> 3) == (tid & 7)) ? 1.0 : 0.0;
-  }
-  __syncthreads();
-  if (warp == 0) {   // the step's rotations on Gamma, in registers (jacobi_inner.cuh)
-    Inner8 m;
-#pragma unroll
-    for (int a = 0; a < 8; a++) {
-#pragma unroll
-      for (int b = a; b < 8; b++) m.g[a][b] = Gam[a][b];
-    }
-#pragma unroll
-    for (int a = 0; a < 8; a++) m.rc[a] = (a == (lane & 7)) ? 1.0 : 0.0;
-    m.rotations = 0; m.big = 0;
-    if (step == 0) inner_full(m, tol * tol); else inner_cross(m, tol * tol);
-    if (lane < 8) {
-#pragma unroll
-      for (int a = 0; a < 8; a++) Rm[a][lane] = m.rc[a];
-    }
-    if (lane == 0) { s_rot = m.rotations; s_max = m.big ? 0x3ff0000000000000ull : 0ull; }   // "max cos^2" collapsed to {0, 1.0}
-  }
-  __syncthreads();
-  if (s_rot == 0) return;
-  const double a_lo = Rm[g][t], a_hi = Rm[g][4 + t];
-  const int r0 = I * 4 + t, r1 = J * 4 + t;
-  const bool v0 = r0 < n, v1 = r1 < n;
-  double* gout = GT + (size_t)rowg * ld;
-  double* vout = VT + (size_t)rowg * ld;
-  // every warp owns whole 8-column groups: it reads all 8 rows of a group before writing them, so in-place is safe
-  for (int grp0 = warp; grp0 < ngroups; grp0 += NW * 4) {   // 4 groups (16 loads) in flight per warp
-    double bg0[4], bg1[4], bv0[4], bv1[4];
-#pragma unroll
-    for (int k = 0; k < 4; k++) {
-      const int grp = grp0 + k * NW;
-      const int col = 8 * grp + g;
-      const bool ok = grp < ngroups;
-      bg0[k] = (ok && v0) ? GT[(size_t)r0 * ld + col] : 0.0; bg1[k] = (ok && v1) ? GT[(size_t)r1 * ld + col] : 0.0;
-      bv0[k] = (ok && v0) ? VT[(size_t)r0 * ld + col] : 0.0; bv1[k] = (ok && v1) ? VT[(size_t)r1 * ld + col] : 0.0;
-    }
-    __syncwarp();   // the whole warp has read its 8-column groups before any lane overwrites them (in place)
-#pragma unroll
-    for (int k = 0; k < 4; k++) {
-      const int grp = grp0 + k * NW;
-      double d0 = 0.0, d1 = 0.0, e0 = 0.0, e1 = 0.0;
-      dmma884(d0, d1, a_lo, bg0[k]); dmma884(d0, d1, a_hi, bg1[k]);
-      dmma884(e0, e1, a_lo, bv0[k]); dmma884(e0, e1, a_hi, bv1[k]);
-      if (rvalid && grp < ngroups) {
-        *reinterpret_cast<double2*>(gout + 8 * grp + 2 * t) = make_double2(d0, d1);
-        *reinterpret_cast<double2*>(vout + 8 * grp + 2 * t) = make_double2(e0, e1);
-      }
-    }
-  }
-  if (tid == 0) {
-    atomicAdd(&sc->jacobi_rotations, s_rot);
-    atomicMax(&sc->jacobi_max_rel_bits, s_max);
-  }
 }
 
 // ------------------------------------------------------------------------------------------------------
@@ -731,8 +563,9 @@ void launch_set_identity(cudaStream_t st, double* M, int ld, int n) {
 }
 
 constexpr size_t kMaxDynSmem = 227 * 1024 - 2048;  // leave room for the kernels' static shared memory
+constexpr int kEigenSmallMax = 24;                 // largest N for eigen_small_kernel
 size_t eigen_small_smem_bytes(int n) { return sizeof(double) * (2 * (size_t)n * (n | 1) + 2 * n) + sizeof(int) * n + 16; }
-bool eigen_small_fits(int n) { return eigen_small_smem_bytes(n) <= kMaxDynSmem; }
+bool eigen_use_small(int n) { return n <= kEigenSmallMax && eigen_small_smem_bytes(n) <= kMaxDynSmem; }
 void launch_eigen_small(cudaStream_t st, const double* C, int ld, int n, double* VT, double* GT, double* B, double* A, double* D,
                         double tol, int max_sweeps, DevScalars* sc) {
   launch_gemm_tn(st, n, n, n, VT, ld, C, ld, GT, ld);   // GT[i][j] = sum_k VT[i][k] C[j][k]
@@ -744,23 +577,20 @@ void launch_eigen_small(cudaStream_t st, const double* C, int ld, int n, double*
 long long* g_jacobi_dbg = nullptr;   // device buffer of phase timestamps (KCMA_JACOBI_DEBUG=1)
 
 // All sweeps in one cooperative launch: one CTA per pair of 4-row blocks, so the whole tournament round must be
-// co-resident. Returns false when it is not (N > 8*num_sms, or rows longer than the kernel's register tile covers);
-// the caller then launches one jacobi_gram_step_kernel per tournament round.
+// co-resident. Returns false when it is not (N > 8*num_sms, or rows longer than the kernel's register tile covers) or when the
+// cooperative launch fails; the caller then launches one jacobi_big_step_kernel per tournament step.
 bool launch_jacobi_persistent(cudaStream_t st, double* GT, double* VT, int ld, int n, double tol, int max_sweeps, DevScalars* sc,
                               int num_sms, unsigned* ready) {
   int nb = ((n + 3) / 4 + 1) & ~1;
   if (nb / 2 > num_sms || ld > 1280) return false;
-  const char* e = getenv("KCMA_JACOBI_PERSISTENT");
-  if (e && atoi(e) == 0) return false;
-  // Tournament order (read per call so that one process can A/B both): the ring order needs a power-of-two block count;
-  // it is used when the phantom blocks that pads in cost less than the sweep it saves (<= 1/8 more steps) and the padded
-  // round is still co-resident; otherwise, or with KCMA_JACOBI_ORDER=rr, the round-robin order. Measured on config 3 (same box,
-  // profiles/r01_jacobi_order_ab.log): 7.80 instead of 8.65 sweeps per decomposition, 13.2 instead of 14.6 ms.
+  // Tournament order: the ring order needs a power-of-two block count; it is used when the phantom blocks that pads in cost less
+  // than the sweep it saves (<= 1/8 more steps) and the padded round is still co-resident; otherwise the round-robin order.
+  // Measured on config 3 (same box, profiles/r01_jacobi_order_ab.log): 7.80 instead of 8.65 sweeps per decomposition, 13.2
+  // instead of 14.6 ms. (Keeping the ring order's first block of a slot resident in shared memory was measured and dropped: 14.30
+  // instead of 13.23 ms, profiles/r02_jacobi_anchor_ab.log.)
   int nb_ring = 2;
   while (nb_ring < nb) nb_ring <<= 1;
-  const char* oe = getenv("KCMA_JACOBI_ORDER");
-  const bool ring = !(oe && strcmp(oe, "rr") == 0) && nb_ring / 2 <= num_sms && (nb_ring - nb) * 8 <= nb && 2 * nb_ring <= ld;
-  bool anchor = ring && oe && strcmp(oe, "anchor") == 0;   // EXPERIMENTAL, opt-in only: ring order + resident first block (ORDER 2)
+  const bool ring = nb_ring / 2 <= num_sms && (nb_ring - nb) * 8 <= nb && 2 * nb_ring <= ld;
   if (ring) nb = nb_ring;
   static int coop = -1;
   static std::atomic<unsigned long long> attr{0};
@@ -774,14 +604,6 @@ bool launch_jacobi_persistent(cudaStream_t st, double* GT, double* VT, int ld, i
     if (coop != 0) coop = c;
   }
   if (coop <= 0) return false;
-  if (anchor) {   // set up lazily so that the experimental instantiation can never disable the product path
-    static int anchor_ok = -1;
-    if (anchor_ok < 0) {
-      anchor_ok = cudaFuncSetAttribute(jacobi_pipe_kernel<256, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kMaxDynSmem - 16 * 1024) == cudaSuccess;
-      if (!anchor_ok) cudaGetLastError();
-    }
-    anchor = anchor_ok == 1;
-  }
   static long long* dbg = nullptr;   // phase timestamps, only with KCMA_JACOBI_DEBUG=<sweep to trace>
   const char* de = getenv("KCMA_JACOBI_DEBUG");
   if (de && !dbg) {
@@ -795,7 +617,7 @@ bool launch_jacobi_persistent(cudaStream_t st, double* GT, double* VT, int ld, i
   cudaMemsetAsync(ready, 0, sizeof(unsigned) * 2 * nb, st);
   unsigned* ready_v = ready + nb;
   void* args[] = {&GT, &VT, &ld, &n, &nb, &tol, &max_sweeps, &sc, &ready, &ready_v, &dbg, &dbg_sweep, &dbg_step0};
-  const void* fn = anchor ? (const void*)jacobi_pipe_kernel<256, 2> : ring ? (const void*)jacobi_pipe_kernel<256, 1> : (const void*)jacobi_pipe_kernel<256, 0>;
+  const void* fn = ring ? (const void*)jacobi_pipe_kernel<256, 1> : (const void*)jacobi_pipe_kernel<256, 0>;
   if (cudaLaunchCooperativeKernel(fn, dim3(nb / 2), dim3(256), args, smem, st) == cudaSuccess) return true;
   cudaGetLastError();
   return false;
@@ -1048,18 +870,13 @@ BigState& big_state() {
   return g_big[dev & 63];
 }
 size_t big_smem_bytes() { return sizeof(double) * ((BIG_NT / 64) * BIG_TILES * 64 + 3 * BIG_R * BIG_LDS); }
-bool big_enabled() {
-  static const int big = getenv("KCMA_JACOBI_BIG") ? atoi(getenv("KCMA_JACOBI_BIG")) : 1;
-  return big != 0;
-}
 // Block count and tournament order of the 16-row-block path: the ring order (jacobi_inner.cuh) when padding the block count
-// to a power of two costs <= 1/8 more steps (N = 4096: 256 blocks, no padding), else (or KCMA_JACOBI_ORDER=rr) round-robin.
+// to a power of two costs <= 1/8 more steps (N = 4096: 256 blocks, no padding), else round-robin.
 int big_blocks(int n, int* order) {
   int nsb = ((n + BIG_B - 1) / BIG_B + 1) & ~1;
   int nsb_ring = 2;
   while (nsb_ring < nsb) nsb_ring <<= 1;
-  const char* oe = getenv("KCMA_JACOBI_ORDER");
-  const bool ring = !(oe && strcmp(oe, "rr") == 0) && (nsb_ring - nsb) * 8 <= nsb;
+  const bool ring = (nsb_ring - nsb) * 8 <= nsb;
   *order = ring ? 1 : 0;
   return ring ? nsb_ring : nsb;
 }
@@ -1075,31 +892,25 @@ void big_launch(cudaStream_t st, double* GT, double* VT, int ld, int n, int nsb,
 
 void launch_jacobi_block_sweep(cudaStream_t st, double* GT, double* VT, int ld, int n, double tol, DevScalars* sc, int* launches) {
   reset_rotations_kernel<<<1, 1, 0, st>>>(sc);
-  if (big_enabled()) {   // 16-row blocks: N/16 - 1 steps per sweep
-    int order = 0;
-    const int nsb = big_blocks(n, &order);
-    static std::atomic<unsigned long long> attr{0};
-    if (first_call_on_device(attr)) cudaFuncSetAttribute(jacobi_big_step_kernel<BIG_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)big_smem_bytes());
-    BigState& b = big_state();
-    if ((size_t)(nsb / 2) > b.pairs) {
-      cudaStreamSynchronize(st);
-      if (b.rlog) cudaFree(b.rlog);
-      b.pairs = (size_t)(nsb / 2);
-      cudaMalloc(&b.rlog, sizeof(double) * 2 * b.pairs * BIG_RLOG);
-      b.pending = -1;
-    }
-    for (int step = 0; step < nsb - 1; step++) big_launch(st, GT, VT, ld, n, nsb, order, step, 1, tol, sc);
-    if (launches) *launches += nsb;
-    return;
+  int order = 0;
+  const int nsb = big_blocks(n, &order);   // 16-row blocks: N/16 - 1 steps per sweep
+  static std::atomic<unsigned long long> attr{0};
+  if (first_call_on_device(attr)) cudaFuncSetAttribute(jacobi_big_step_kernel<BIG_NT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)big_smem_bytes());
+  BigState& b = big_state();
+  if ((size_t)(nsb / 2) > b.pairs) {
+    cudaStreamSynchronize(st);
+    if (b.rlog) cudaFree(b.rlog);
+    b.pairs = (size_t)(nsb / 2);
+    cudaMalloc(&b.rlog, sizeof(double) * 2 * b.pairs * BIG_RLOG);
+    b.pending = -1;
   }
-  const int nb = ((n + 3) / 4 + 1) & ~1;
-  for (int step = 0; step < nb - 1; step++) jacobi_gram_step_kernel<512><<<nb / 2, 512, 0, st>>>(GT, VT, ld, n, nb, step, tol, sc);
-  if (launches) *launches += nb;
+  for (int step = 0; step < nsb - 1; step++) big_launch(st, GT, VT, ld, n, nsb, order, step, 1, tol, sc);
+  if (launches) *launches += nsb;
 }
 
 // The V update of the last step is still pending after the last sweep.
 void launch_jacobi_block_flush(cudaStream_t st, double* GT, double* VT, int ld, int n, double tol, DevScalars* sc, int* launches) {
-  if (!big_enabled() || big_state().pending < 0) return;
+  if (big_state().pending < 0) return;
   int order = 0;
   const int nsb = big_blocks(n, &order);
   big_launch(st, GT, VT, ld, n, nsb, order, 0, 0, tol, sc);

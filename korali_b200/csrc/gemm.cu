@@ -7,7 +7,6 @@
 //
 // Version 1 staging: 16-byte cp.async (LDGSTS) into padded shared-memory tiles whose row stride is
 // == 32 B (mod 128 B), which makes every LDS.64 fragment read of a half-warp hit 16 distinct bank pairs.
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "kernels.h"
@@ -225,16 +224,10 @@ static void ensure_attrs() {
 size_t gemm_tn_smem_bytes() { return sizeof(double) * STAGES * (BM + BN) * PADK; }
 size_t syrk_tt_smem_bytes() { return sizeof(double) * STAGES * 2 * BK * PADN; }
 
-// KCMA_GEMM=cpasync selects the version-1 staging (LDGSTS) for A/B comparisons; the default is the TMA pipeline.
-static bool want_tma() {
-  const char* e = getenv("KCMA_GEMM");
-  return !(e && e[0] == 'c');
-}
-
 void launch_gemm_tn(cudaStream_t st, int M, int Nc, int K, const double* A, int lda, const double* B, int ldb,
                     double* C, int ldc) {
   if (M <= 0 || Nc <= 0) return;
-  if (want_tma() && launch_gemm_tn_tma(st, M, Nc, K, A, lda, B, ldb, C, ldc)) return;
+  if (launch_gemm_tn_tma(st, M, Nc, K, A, lda, B, ldb, C, ldc)) return;   // the cp.async kernel when no tensor map can be built
   ensure_attrs();
   dim3 grid((Nc + BN - 1) / BN, (M + BM - 1) / BM);
   gemm_tn_kernel<<<grid, THREADS, gemm_tn_smem_bytes(), st>>>(M, Nc, K, A, lda, B, ldb, C, ldc);
@@ -262,21 +255,18 @@ int syrk_pick_splits(int n, int K, int num_sms, int max_splits) {
 
 void launch_syrk_tt(cudaStream_t st, int n, int K, const int* kptr, const double* S, int lds, long long s_rows, double* W, int ldw,
                     int splits) {
-  if (want_tma() && launch_syrk_tt_tma(st, n, K, kptr, S, lds, s_rows, W, ldw, splits)) return;
+  if (launch_syrk_tt_tma(st, n, K, kptr, S, lds, s_rows, W, ldw, splits)) return;
   ensure_attrs();
   dim3 grid(syrk_tiles(n), splits);
   syrk_tt_kernel<<<grid, THREADS, syrk_tt_smem_bytes(), st>>>(n, K, kptr, S, lds, W, ldw);
 }
 
-// The rank-mu product with the scheduling chosen here: stream-K over the triangular tiles (gemm_tma.cu) by default, the split-K
-// kernels with KCMA_SYRK=splitk (A/B runs) or when the TMA path is unavailable. Returns the number of slabs of W to sum.
+// The rank-mu product with the scheduling chosen here: stream-K over the triangular tiles (gemm_tma.cu), or the split-K kernels when
+// the TMA path is unavailable. Returns the number of slabs of W to sum.
 int launch_syrk(cudaStream_t st, int n, int K, const int* kptr, const double* S, int lds, long long s_rows, double* W, int ldw,
                 int expect_rows, int num_sms, int max_splits) {
-  const char* e = getenv("KCMA_SYRK");
-  if (want_tma() && !(e && !strcmp(e, "splitk"))) {
-    const int parts = launch_syrk_sk_tma(st, n, K, kptr, S, lds, s_rows, W, ldw, num_sms, max_splits);
-    if (parts > 0) return parts;
-  }
+  const int parts = launch_syrk_sk_tma(st, n, K, kptr, S, lds, s_rows, W, ldw, num_sms, max_splits);
+  if (parts > 0) return parts;
   const int splits = syrk_pick_splits(n, expect_rows, num_sms, max_splits);
   launch_syrk_tt(st, n, K, kptr, S, lds, s_rows, W, ldw, splits);
   return splits;

@@ -70,6 +70,9 @@ void tridiag_get_tridiagonal(TridiagWs* ws, double* d, double* e, double* tau, d
 void tridiag_set_tridiagonal(TridiagWs* ws, const double* d, const double* e);
 void tridiag_dump_prof(TridiagWs* ws);   // KCMA_SYTRD_PROF=step0[,cta]: prints the phase stamps of sytrd_kernel to stderr
 void launch_eig_sign(cudaStream_t st, const double* VT, int ld, int n, double* sign);
+// The size policy of the symmetric eigensolvers, one rule for CMA-ES (api.cu) and TMCMC (tmcmc.cu): eigen_use_small (eigen.cu),
+// else the tridiagonal solver while its shared-memory vectors fit.
+bool eigen_tridiag_fits(int n);
 
 // rng.cu
 void launch_philox_normal(cudaStream_t st, double* Z, int ldz, long long rows, int n, unsigned long long seed, unsigned generation,
@@ -136,7 +139,7 @@ void launch_viability_boundaries(cudaStream_t st, const double* G, long long ldg
 
 // eigen.cu
 void launch_set_identity(cudaStream_t st, double* M, int ld, int n);
-bool eigen_small_fits(int n);
+bool eigen_use_small(int n);   // N <= 24: launch_eigen_small, the whole solver in one CTA
 void launch_eigen_small(cudaStream_t st, const double* C, int ld, int n, double* VT, double* GT, double* B, double* A, double* D,
                         double tol, int max_sweeps, DevScalars* sc);
 bool launch_jacobi_persistent(cudaStream_t st, double* GT, double* VT, int ld, int n, double tol, int max_sweeps, DevScalars* sc,

@@ -6,7 +6,6 @@
 // block comes from warp-striped ownership + __match_any_sync ranks, so equal keys keep ascending index.
 // The whole sorted order is produced (weights depend on the rank of every one of the top-mu samples).
 #include <cooperative_groups.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "kernels.h"
@@ -262,8 +261,7 @@ __global__ void __launch_bounds__(256) sort_rank_scatter_kernel(const unsigned* 
 
 int launch_sort_index(cudaStream_t st, const double* f, int n, void* workspace, unsigned* sorted_idx, int num_sms) {
   if (n <= 0) return 0;
-  static const int rank_max = getenv("KCMA_SORT_RANK_MAX") ? atoi(getenv("KCMA_SORT_RANK_MAX")) : RANK_MAX_N;
-  if (n <= rank_max) {
+  if (n <= RANK_MAX_N) {
     unsigned* rank = (unsigned*)workspace;
     cudaMemsetAsync(rank, 0, sizeof(unsigned) * (size_t)n, st);
     dim3 grid((n + 255) / 256, (n + RANK_CHUNK - 1) / RANK_CHUNK);
@@ -278,8 +276,7 @@ int launch_sort_index(cudaStream_t st, const double* f, int n, void* workspace, 
   unsigned* v0 = (unsigned*)w; w += sizeof(unsigned) * (size_t)n;
   unsigned* v1 = (unsigned*)w; w += sizeof(unsigned) * (size_t)n;
   unsigned* hist = (unsigned*)w;
-  static const int fused_on = getenv("KCMA_SORT_FUSED") ? atoi(getenv("KCMA_SORT_FUSED")) : 1;
-  if (fused_on && nblocks <= num_sms) {   // one cooperative launch (every CTA must be resident: one tile per SM at most)
+  if (nblocks <= num_sms) {   // one cooperative launch (every CTA must be resident: one tile per SM at most)
     const double* fp = f;
     void* args[] = {&fp, &n, &k0, &k1, &v0, &v1, &sorted_idx, &hist};
     if (cudaLaunchCooperativeKernel((const void*)sort_fused_kernel, dim3(nblocks), dim3(SORT_THREADS), args, 0, st) == cudaSuccess) return 1;

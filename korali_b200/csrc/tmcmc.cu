@@ -475,8 +475,6 @@ int tm_pull(ktmcmc* h) {
   TM_CUDA(h, cudaGetLastError());
   return 0;
 }
-bool tm_use_tridiag(int N) { return N > 24 || !eigen_small_fits(N); }
-bool tm_tridiag_fits(int N) { return N >= 4 && (size_t)N * 5 * sizeof(double) + 4096 <= 226 * 1024; }
 int tm_check_flags(ktmcmc* h) {
   if (h->hSc->nan_flag) return tm_fail(h, "A NaN log-likelihood was produced by the likelihood model\n");
   if (h->hSc->allinf_flag) return tm_fail(h, "Every sample of the population has a log-likelihood of -inf: the annealing step is undefined\n");
@@ -534,7 +532,7 @@ int ktmcmc_create(const ktmcmc_cfg* cfg, ktmcmc_t** out) {
   }
   if (cfg->loglik != KCMA_OBJ_EXTERNAL && (cfg->loglik < KCMA_OBJ_NEG_SPHERE || cfg->loglik > KCMA_OBJ_NEG_SPHERE_SIN2))
     return tm_fail(nullptr, "unknown log-likelihood model id %d", cfg->loglik);
-  if (N > 24 && !tm_tridiag_fits(N)) return tm_fail(nullptr, "Sampler/TMCMC: n = %d is above the tridiagonal eigensolver's size\n", N);
+  if (!eigen_use_small(N) && !eigen_tridiag_fits(N)) return tm_fail(nullptr, "Sampler/TMCMC: n = %d is above the tridiagonal eigensolver's size\n", N);
   int ndev = 0;
   if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) return tm_fail(nullptr, "no CUDA device: korali_b200 has no CPU fallback");
   if (cfg->device < 0 || cfg->device >= ndev) return tm_fail(nullptr, "invalid device %d", cfg->device);
@@ -572,7 +570,7 @@ int ktmcmc_create(const ktmcmc_cfg* cfg, ktmcmc_t** out) {
   CREATE_CUDA(cudaMemcpy(h->dDsc, &ds, sizeof(ds), cudaMemcpyHostToDevice));
   launch_set_identity(h->stream, h->dVT, (int)ld, N);
   launch_set_identity(h->stream, h->dB, (int)ld, N);
-  if (tm_use_tridiag(N)) {
+  if (!eigen_use_small(N)) {
     char msg[512] = "";
     h->tri = tridiag_ws_create(N, (int)ld, h->num_sms, msg, sizeof(msg));
     if (!h->tri) { tm_fail(nullptr, "%s", msg); ktmcmc_destroy(h); return 1; }

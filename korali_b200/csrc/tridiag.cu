@@ -71,17 +71,6 @@ __device__ __forceinline__ double block_sum(double v, double* slot) {
   return s;
 }
 
-template <int NW>
-__device__ __forceinline__ double block_sum_n(double v, double* slot) {
-  v = warp_sum_butterfly(v);
-  if ((threadIdx.x & 31) == 0) slot[threadIdx.x >> 5] = v;
-  __syncthreads();
-  double s = 0.0;
-#pragma unroll
-  for (int k = 0; k < NW; k++) s += slot[k];
-  return s;
-}
-
 // The two element formulas of a step, with explicit roundings: they are evaluated per row by the row's thread AND for rows i, i+1
 // by every thread (scalars), and both must give the same bits.
 __device__ __forceinline__ double w_of(double tau, double p, double alpha, double v) { return __fma_rn(tau, p, __dmul_rn(alpha, v)); }
@@ -286,39 +275,8 @@ __device__ __forceinline__ void ll_load2(const LL* p, unsigned long long (&q)[4]
   asm volatile(KC_LL_LD ".v4.u64 {%0, %1, %2, %3}, [%4];" : "=l"(q[0]), "=l"(q[1]), "=l"(q[2]), "=l"(q[3]) : "l"(p) : "memory");
 }
 
-// ---- thread-block clusters (CL > 1): only the leader CTA of a cluster polls the L2 slots and pushes what it received into its
-// peers' shared memory (distributed shared memory) — 148 CTAs polling the same 2 n slots is what stretches the exchange of a step
-__device__ __forceinline__ unsigned cluster_ctarank() { unsigned r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ unsigned map_to_cta(const void* local_smem, unsigned cta) {
-  unsigned la = (unsigned)__cvta_generic_to_shared(local_smem), ra;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(ra) : "r"(la), "r"(cta));
-  return ra;
-}
-__device__ __forceinline__ void st_cluster_f64x2(unsigned raddr, double a, double b) {
-  asm volatile("st.shared::cluster.v2.f64 [%0], {%1, %2};" ::"r"(raddr), "d"(a), "d"(b) : "memory");
-}
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, unsigned count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(bar)), "r"(count) : "memory");
-  asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-}
-__device__ __forceinline__ void mbar_arrive_remote(unsigned raddr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(raddr) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, unsigned parity) {
-  const unsigned a = (unsigned)__cvta_generic_to_shared(bar);
-  asm volatile("{\n\t.reg .pred p;\n\tWAIT_%=:\n\tmbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%0], %1;\n\t@!p bra WAIT_%=;\n\t}" ::"r"(a), "r"(parity)
-               : "memory");
-}
-
-// PF (column prefetch): column c travels ONE STEP EARLIER than it is needed — its owner publishes it in the pass of step c-2 (with the
-// rank-2 updates of the steps <= c-3), every CTA reads it in the pass of step c-1 (long after it was stored: one polling round,
-// off the critical path, its latency hidden behind the pass arithmetic) and applies the updates of the steps c-2 and c-1 itself.
-// The exchange a step waits for is then p = A v alone: half the polled bytes, and the column's stores leave the chain.
-template <int KU, int NC, int CL = 1, int NT = SY_NT, bool PF = false>
-__global__ void __launch_bounds__(NT, 1)
+template <int KU, int NC>
+__global__ void __launch_bounds__(SY_NT, 1)
 sytrd_reg_kernel(const double* __restrict__ M, int ld, int n, int ns /* n rounded up to even: LL stride per parity, vector stride */,
                  LL* __restrict__ xP, LL* __restrict__ xC, double* __restrict__ dT, double* __restrict__ eT, double* __restrict__ tauv,
                  double* __restrict__ VR, long long* __restrict__ prof, int prof_step0, int prof_cta, int opt, int copies) {
@@ -327,23 +285,14 @@ sytrd_reg_kernel(const double* __restrict__ M, int ld, int n, int ns /* n rounde
   double* vs_old = sm;             // reflector v_{i-1} by index (lookups v[c], v[i+1])
   double* vs_new = sm + ns;
   double* wsm = sm + 2 * ns;       // w_{i-1} by index (lookups w[c])
-  double* red = sm + 3 * ns;       // 4 slots x (NT / 32)
+  double* red = sm + 3 * ns;       // 4 slots x SY_NW
   double* bc = red + 64;           // 2 parities x {c_i, p_i, c_{i+1}, p_{i+1}}
-  double* pp = red + 80;           // NC x NT partial products of the pass
-  double* cbuf = pp + NC * NT;  // CL > 1: received column / product entries pushed by the cluster leader, 2 parities x ns each
-  double* pbuf = cbuf + 2 * ns;
-  __shared__ __align__(8) unsigned long long mbar;
-  static_assert(!(PF && CL > 1), "the prefetch variant has no cluster path");
-  const unsigned crank = CL > 1 ? cluster_ctarank() : 0u;
-  if (CL > 1) {
-    if (tid == 0) mbar_init(&mbar, (NT / 32));   // one arrival per warp of the leader and step
-    cluster_sync_all();
-  }
+  double* pp = red + 80;           // NC x SY_NT partial products of the pass
   const int nloc = b < n ? (n - b + G - 1) / G : 0;
   double A[KU][NC][2], v[2 * KU], w[2 * KU], vnw[2 * KU];
 #pragma unroll
   for (int k = 0; k < KU; k++) {
-    const int r = 2 * (tid + NT * k);
+    const int r = 2 * (tid + SY_NT * k);
 #pragma unroll
     for (int s = 0; s < NC; s++) {
       const double* src = M + (size_t)(b + s * G) * ld;   // column c of a symmetric matrix = its row c
@@ -352,7 +301,7 @@ sytrd_reg_kernel(const double* __restrict__ M, int ld, int n, int ns /* n rounde
     }
     v[2 * k] = v[2 * k + 1] = w[2 * k] = w[2 * k + 1] = vnw[2 * k] = vnw[2 * k + 1] = 0.0;
   }
-  for (int r = tid; r < ns; r += NT) { vs_old[r] = 0.0; vs_new[r] = 0.0; wsm[r] = 0.0; }
+  for (int r = tid; r < ns; r += SY_NT) { vs_old[r] = 0.0; vs_new[r] = 0.0; wsm[r] = 0.0; }
   // Every slot exists `copies` times (stride cstride): all CTAs poll the same 2 n slots, and 148 requests per 128-byte line and
   // polling round serialise in the L2 slice that owns the line; CTA b reads copy b % copies, the producers write all copies.
   const size_t cstride = 4 * (size_t)ns;
@@ -360,14 +309,8 @@ sytrd_reg_kernel(const double* __restrict__ M, int ld, int n, int ns /* n rounde
   // owner n stores per copy, a product entry one)
   const int ccop = copies & 255, pcop = (copies >> 8) ? (copies >> 8) : ccop;
   const size_t my_copy = (size_t)(b % ccop) * cstride, my_copy_p = (size_t)(b % pcop) * cstride;
-  double cn[2 * KU];   // PF: column i with the updates of the steps <= i-2, this thread's rows (columns 0 and 1 come from M itself)
-#pragma unroll
-  for (int j = 0; j < 2 * KU; j++) {
-    const int r = 2 * (tid + NT * (j >> 1)) + (j & 1);
-    cn[j] = (PF && r < n) ? M[r] : 0.0;
-  }
-  if (!PF && b == 0)   // owner of column 0 publishes it for step 0
-    for (int r = tid; r < n; r += NT)
+  if (b == 0)   // owner of column 0 publishes it for step 0
+    for (int r = tid; r < n; r += SY_NT)
       for (int q = 0; q < ccop; q++) ll_store(xC + q * cstride + r, M[r], 1ull);
   __syncthreads();
   double tau_old = 0.0;
@@ -384,11 +327,11 @@ sytrd_reg_kernel(const double* __restrict__ M, int ld, int n, int ns /* n rounde
     unsigned need = 0;
 #pragma unroll
     for (int j = 0; j < 2 * KU; j++) {
-      const int r = 2 * (tid + NT * (j >> 1)) + (j & 1);
+      const int r = 2 * (tid + SY_NT * (j >> 1)) + (j & 1);
       if (r >= i && r < n) need |= 1u << j;
-      cv[j] = (PF && r >= i && r < n) ? cn[j] : 0.0; pq[j] = 0.0;
+      cv[j] = 0.0; pq[j] = 0.0;
     }
-    if (have_p && (opt & 4) && crank == 0) {
+    if (have_p && (opt & 4)) {
       // Gate: a few lanes spin on ONE slot per producer — the products of the last G columns (every CTA that still owns a column
       // publishes exactly one of them), plus the last row of the column when it travels in this step — and only then does the
       // block read its 2 x 16 KB of slots, once. A round of everybody polling everything is ~1000 cycles of L2 traffic
@@ -400,68 +343,35 @@ sytrd_reg_kernel(const double* __restrict__ M, int ld, int n, int ns /* n rounde
         const bool n0 = r0 >= i && r0 < n, n1 = r0 + 1 < n;
         unsigned long long q[4];
         do { ll_load2(Pin + r0, q); } while ((n0 && q[1] != tag) || (n1 && q[3] != tag));
-      } else if (!PF && tid == NT - 1) {
+      } else if (tid == SY_NT - 1) {
         unsigned long long q[4];
         const bool n0 = ns - 2 >= i, n1 = ns - 1 < n;
         do { ll_load2(Cin + ns - 2, q); } while ((n0 && q[1] != tag) || (n1 && q[3] != tag));
       }
       __syncthreads();
-    } else if (have_p && (opt & 1) && crank == 0) {   // one lane per warp spins on one slot first: 148 x 256 threads polling everything back to back saturate the L2
+    } else if (have_p && (opt & 1)) {   // one lane per warp spins on one slot first: 148 x 256 threads polling everything back to back saturate the L2
       if (lane == 0 && need) {
         const int j0 = __ffs(need) - 1;
-        (void)ll_wait(Pin + 2 * (tid + NT * (j0 >> 1)) + (j0 & 1), tag);
+        (void)ll_wait(Pin + 2 * (tid + SY_NT * (j0 >> 1)) + (j0 & 1), tag);
       }
       __syncwarp();
     }
-    if (crank == 0) {
-      unsigned pc = PF ? 0u : need, ppn = have_p ? need : 0u;
-      while (pc | ppn) {
-        unsigned long long qc[KU][4], qp[KU][4];
+    unsigned pc = need, ppn = have_p ? need : 0u;
+    while (pc | ppn) {
+      unsigned long long qc[KU][4], qp[KU][4];
 #pragma unroll
-        for (int k = 0; k < KU; k++) {
-          if ((pc >> (2 * k)) & 3u) ll_load2(Cin + 2 * (tid + NT * k), qc[k]);
-          if ((ppn >> (2 * k)) & 3u) ll_load2(Pin + 2 * (tid + NT * k), qp[k]);
-        }
-#pragma unroll
-        for (int k = 0; k < KU; k++)
-#pragma unroll
-          for (int h = 0; h < 2; h++) {
-            const unsigned bit = 1u << (2 * k + h);
-            if ((pc & bit) && qc[k][2 * h + 1] == tag) { cv[2 * k + h] = __longlong_as_double((long long)qc[k][2 * h]); pc &= ~bit; }
-            if ((ppn & bit) && qp[k][2 * h + 1] == tag) { pq[2 * k + h] = __longlong_as_double((long long)qp[k][2 * h]); ppn &= ~bit; }
-          }
-        if ((pc | ppn) && (opt & 2)) __nanosleep(100);
+      for (int k = 0; k < KU; k++) {
+        if ((pc >> (2 * k)) & 3u) ll_load2(Cin + 2 * (tid + SY_NT * k), qc[k]);
+        if ((ppn >> (2 * k)) & 3u) ll_load2(Pin + 2 * (tid + SY_NT * k), qp[k]);
       }
-    }
-    if (CL > 1) {
-      if (crank == 0) {   // push to the peers; the buffer of this parity was last read two steps ago (same argument as for the LL slots)
 #pragma unroll
-        for (unsigned q = 1; q < (unsigned)CL; q++)
+      for (int k = 0; k < KU; k++)
 #pragma unroll
-          for (int k = 0; k < KU; k++) {
-            const int r = 2 * (tid + NT * k);
-            if (r < ns) {
-              st_cluster_f64x2(map_to_cta(cbuf + par * ns + r, q), cv[2 * k], cv[2 * k + 1]);
-              st_cluster_f64x2(map_to_cta(pbuf + par * ns + r, q), pq[2 * k], pq[2 * k + 1]);
-            }
-          }
-        asm volatile("fence.acq_rel.cluster;" ::: "memory");
-        __syncwarp();
-        if (lane == 0)
-#pragma unroll
-          for (unsigned q = 1; q < (unsigned)CL; q++) mbar_arrive_remote(map_to_cta(&mbar, q));
-      } else {
-        mbar_wait(&mbar, (unsigned)(i & 1));
-#pragma unroll
-        for (int k = 0; k < KU; k++) {
-          const int r = 2 * (tid + NT * k);
-          if (r < ns) {
-            const double2 c2 = *reinterpret_cast<const double2*>(cbuf + par * ns + r);
-            const double2 p2 = *reinterpret_cast<const double2*>(pbuf + par * ns + r);
-            cv[2 * k] = c2.x; cv[2 * k + 1] = c2.y; pq[2 * k] = p2.x; pq[2 * k + 1] = p2.y;
-          }
+        for (int h = 0; h < 2; h++) {
+          const unsigned bit = 1u << (2 * k + h);
+          if ((pc & bit) && qc[k][2 * h + 1] == tag) { cv[2 * k + h] = __longlong_as_double((long long)qc[k][2 * h]); pc &= ~bit; }
+          if ((ppn & bit) && qp[k][2 * h + 1] == tag) { pq[2 * k + h] = __longlong_as_double((long long)qp[k][2 * h]); ppn &= ~bit; }
         }
-      }
     }
     if (pr) prof[(i - prof_step0) * 8 + 1] = clock64();
     // ---- p.v over the own rows; the four scalars every thread needs
@@ -469,19 +379,19 @@ sytrd_reg_kernel(const double* __restrict__ M, int ld, int n, int ns /* n rounde
     double* bcp = bc + par * 4;
 #pragma unroll
     for (int j = 0; j < 2 * KU; j++) {
-      const int r = 2 * (tid + NT * (j >> 1)) + (j & 1);
+      const int r = 2 * (tid + SY_NT * (j >> 1)) + (j & 1);
       if (need & (1u << j)) part = __fma_rn(pq[j], v[j], part);
       if (r == i) { bcp[0] = cv[j]; bcp[1] = pq[j]; }
       if (r == i + 1 && r < n) { bcp[2] = cv[j]; bcp[3] = pq[j]; }
     }
-    const double pv = block_sum_n<NT / 32>(part, red + (par * 2 + 0) * (NT / 32));
+    const double pv = block_sum(part, red + (par * 2 + 0) * SY_NW);
     const double alpha = -0.5 * tau_old * (tau_old * pv);
     const double vi = vs_old[i];
     const double wi = w_of(tau_old, bcp[1], alpha, vi);
     double xpart = 0.0;
 #pragma unroll
     for (int j = 0; j < 2 * KU; j++) {
-      const int r = 2 * (tid + NT * (j >> 1)) + (j & 1);
+      const int r = 2 * (tid + SY_NT * (j >> 1)) + (j & 1);
       if (need & (1u << j)) {
         w[j] = w_of(tau_old, pq[j], alpha, v[j]);
         wsm[r] = w[j];
@@ -498,7 +408,7 @@ sytrd_reg_kernel(const double* __restrict__ M, int ld, int n, int ns /* n rounde
     }
     const double vi1 = vs_old[i + 1];
     const double alph = col_upd(bcp[2], vi1, wi, w_of(tau_old, bcp[3], alpha, vi1), vi);
-    const double xn2 = block_sum_n<NT / 32>(xpart, red + (par * 2 + 1) * (NT / 32));
+    const double xn2 = block_sum(xpart, red + (par * 2 + 1) * SY_NW);
     double tau = 0.0, scale = 0.0, ei = alph;
     if (xn2 > 0.0) {
       const double beta = -copysign(sqrt(alph * alph + xn2), alph);
@@ -508,38 +418,19 @@ sytrd_reg_kernel(const double* __restrict__ M, int ld, int n, int ns /* n rounde
     }
 #pragma unroll
     for (int j = 0; j < 2 * KU; j++) {
-      const int r = 2 * (tid + NT * (j >> 1)) + (j & 1);
+      const int r = 2 * (tid + SY_NT * (j >> 1)) + (j & 1);
       vnw[j] = (r == i + 1) ? 1.0 : ((r >= i + 2 && r < n) ? cv[j] * scale : 0.0);
       if (r < ns) vs_new[r] = vnw[j];
     }
     if (b == i % G && tid == 0) { dT[i] = di; eT[i] = ei; tauv[i] = tau; }   // the owner of the retired column records the step
     // no barrier here: wsm (read by column index in the pass) was written in front of the second block sum's barrier, and vs_new
-    // is first read — as vs_old — behind the first block sum's barrier of the next step; the cluster variant keeps its barrier
-    if (CL > 1) __syncthreads();
+    // is first read — as vs_old — behind the first block sum's barrier of the next step
     if (pr) prof[(i - prof_step0) * 8 + 2] = clock64();
     // ---- pass over this CTA's columns c >= i+1 (registers): rank-2 update of step i-1, partial p = A v_i, publication of column i+1
     LL* Pout = xP + (size_t)(par ^ 1) * ns;
-    LL* Cout = xC + (size_t)(PF ? par : (par ^ 1)) * ns;     // PF: column i+2 (tag i+3) goes where column i was
+    LL* Cout = xC + (size_t)(par ^ 1) * ns;
     const unsigned long long otag = tag + 1ull;
-    const unsigned long long ctag = PF ? tag + 2ull : otag;
-    const int cpub = PF ? i + 2 : i + 1;
     const int s0 = (i + 1 > b) ? (i + 1 - b + G - 1) / G : 0;
-    // PF: column i+1 (published one step ago, tag i+2) — the loads fly during the pass
-    unsigned long long qn[KU][4];
-    unsigned pn = 0;
-    if (PF) {
-#pragma unroll
-      for (int j = 0; j < 2 * KU; j++) {
-        const int r = 2 * (tid + NT * (j >> 1)) + (j & 1);
-        if (r >= i + 1 && r < n) pn |= 1u << j;
-      }
-      if (i > 0) {
-        const LL* Cnx = xC + my_copy + (size_t)(par ^ 1) * ns;
-#pragma unroll
-        for (int k = 0; k < KU; k++)
-          if ((pn >> (2 * k)) & 3u) ll_load2(Cnx + 2 * (tid + NT * k), qn[k]);
-      }
-    }
 #pragma unroll
     for (int s = 0; s < NC; s++) {
       if (s >= s0 && s < nloc) {
@@ -554,56 +445,23 @@ sytrd_reg_kernel(const double* __restrict__ M, int ld, int n, int ns /* n rounde
           A[k][s][0] = a0; A[k][s][1] = a1;
           dot = __fma_rn(a0, vnw[2 * k], dot);
           dot = __fma_rn(a1, vnw[2 * k + 1], dot);
-          if (c == cpub) {
-            const int r = 2 * (tid + NT * k);
+          if (c == i + 1) {
+            const int r = 2 * (tid + SY_NT * k);
             for (int q = 0; q < ccop; q++) {
-              if (r > i && r < n) ll_store(Cout + q * cstride + r, a0, ctag);
-              if (r + 1 > i && r + 1 < n) ll_store(Cout + q * cstride + r + 1, a1, ctag);
+              if (r > i && r < n) ll_store(Cout + q * cstride + r, a0, otag);
+              if (r + 1 > i && r + 1 < n) ll_store(Cout + q * cstride + r + 1, a1, otag);
             }
           }
         }
-        pp[s * NT + tid] = dot;
-      }
-    }
-    if (PF) {   // column i+1 for the next step: received with the updates <= i-2, update i-1 applied here (v, w still hold step i-1)
-      const double wc1 = wsm[i + 1], vc1 = vs_old[i + 1];
-      if (i == 0) {
-        const double* src = M + (size_t)ld;
-#pragma unroll
-        for (int j = 0; j < 2 * KU; j++) {
-          const int r = 2 * (tid + NT * (j >> 1)) + (j & 1);
-          cn[j] = (pn & (1u << j)) ? src[r] : 0.0;
-        }
-      } else {
-        const LL* Cnx = xC + my_copy + (size_t)(par ^ 1) * ns;
-        unsigned left = pn;
-        for (;;) {
-#pragma unroll
-          for (int k = 0; k < KU; k++)
-#pragma unroll
-            for (int h = 0; h < 2; h++) {
-              const unsigned bit = 1u << (2 * k + h);
-              if ((left & bit) && qn[k][2 * h + 1] == otag) {
-                cn[2 * k + h] = col_upd(__longlong_as_double((long long)qn[k][2 * h]), v[2 * k + h], wc1, w[2 * k + h], vc1);
-                left &= ~bit;
-              }
-            }
-          if (!left) break;
-#pragma unroll
-          for (int k = 0; k < KU; k++)
-            if ((left >> (2 * k)) & 3u) ll_load2(Cnx + 2 * (tid + NT * k), qn[k]);
-        }
-#pragma unroll
-        for (int j = 0; j < 2 * KU; j++)
-          if (!(pn & (1u << j))) cn[j] = 0.0;
+        pp[s * SY_NT + tid] = dot;
       }
     }
     __syncthreads();
-    for (int s = warp; s < NC; s += (NT / 32))   // a warp finishes column s: 256 partials in a fixed order
+    for (int s = warp; s < NC; s += SY_NW)   // a warp finishes column s: 256 partials in a fixed order
       if (s >= s0 && s < nloc) {
         double x = 0.0;
 #pragma unroll
-        for (int j = 0; j < (NT / 32); j++) x += pp[s * NT + lane + 32 * j];
+        for (int j = 0; j < SY_NW; j++) x += pp[s * SY_NT + lane + 32 * j];
         x = warp_sum_butterfly(x);
         if (lane < pcop) ll_store(Pout + lane * cstride + b + s * G, x, otag);
       }
@@ -612,7 +470,7 @@ sytrd_reg_kernel(const double* __restrict__ M, int ld, int n, int ns /* n rounde
       double* vr = VR + (size_t)i * ld;
 #pragma unroll
       for (int j = 0; j < 2 * KU; j++) {
-        const int r = 2 * (tid + NT * (j >> 1)) + (j & 1);
+        const int r = 2 * (tid + SY_NT * (j >> 1)) + (j & 1);
         if (r > i && r < n) vr[r] = vnw[j];
       }
     }
@@ -621,55 +479,18 @@ sytrd_reg_kernel(const double* __restrict__ M, int ld, int n, int ns /* n rounde
     double* t = vs_old; vs_old = vs_new; vs_new = t;
     tau_old = tau;
   }
-  if (CL > 1) cluster_sync_all();   // no CTA may exit while a peer can still write into its shared memory
 }
 
 // (A single-CTA variant for N <= 128 — the whole matrix in the registers of one CTA, no exchange, four block barriers per step — was
 // built and measured at N = 100: 0.338 ms against 0.294 ms for the 25-CTA exchange kernel (profiles/r02_eigen_ab13.log); not kept.)
 // ---- compact-WY panel factor (dlarft, forward / columnwise): T upper triangular, nb x nb, from G = V^T V and tau ------------
-// Column p: T[0:p, p] = -tau_p T[0:p, 0:p] G[0:p, p]. The columns are sequential; inside a column two threads share a row's
-// inner product (interleaved terms, one shuffle). G arrives as `gsplits` split-K slabs (summed here in a fixed order) and is read
-// by rows (G is symmetric), one row per step, prefetched one step ahead.
-constexpr int LARFT_NT = 256;
-__global__ void __launch_bounds__(LARFT_NT)
-larft_kernel(const double* __restrict__ Gbuf, long long gstride, int gsplits, const double* __restrict__ tauv, int n_refl, int nb,
-             double* __restrict__ Tbuf) {
-  extern __shared__ __align__(16) double sm[];
-  double* T = sm;                 // nb x (nb+1)
-  double* grow = sm + nb * (nb + 1);
-  const double* __restrict__ G = Gbuf + (size_t)blockIdx.x * nb * nb;
-  const int panel = blockIdx.x, p0 = panel * nb, kb = min(nb, n_refl - p0), tid = threadIdx.x, lt = nb + 1;
-  const int q = tid >> 1, h = tid & 1;
-  auto gload = [&](int row) {
-    double g = 0.0;
-    for (int k = 0; k < gsplits; k++) g += G[(size_t)k * gstride + (size_t)row * nb + tid];
-    return g;
-  };
-  for (int i = tid; i < nb * lt; i += LARFT_NT) T[i] = 0.0;
-  double gn = (tid < nb && kb > 0) ? gload(0) : 0.0, gn2 = (tid < nb && kb > 1) ? gload(1) : 0.0;   // two rows ahead: an L2 round trip outlasts a step
-  __syncthreads();
-  for (int p = 0; p < kb; p++) {
-    if (tid < nb) grow[tid] = gn;
-    __syncthreads();
-    gn = gn2;
-    if (tid < nb && p + 2 < kb) gn2 = gload(p + 2);
-    const double tp = tauv[p0 + p];
-    double sacc = 0.0;
-    if (q < p)
-      for (int m = q + h; m < p; m += 2) sacc += T[q * lt + m] * grow[m];
-    sacc += __shfl_xor_sync(0xffffffffu, sacc, 1);
-    if (h == 0 && q < p) T[q * lt + p] = -tp * sacc;
-    if (tid == 0) T[p * lt + p] = tp;
-    __syncthreads();
-  }
-  for (int i = tid; i < nb * nb; i += LARFT_NT) Tbuf[(size_t)panel * nb * nb + i] = T[(i / nb) * lt + (i % nb)];
-}
-
-// The same factor, all columns at once: T is the inverse of the upper triangular S = striu(G) + diag(1 / tau) (the column recurrence of
-// dlarft is the column-by-column inverse of S), so column j follows from S t_j = e_j by back substitution on its own:
+// T is the inverse of the upper triangular S = striu(G) + diag(1 / tau) (the column recurrence of dlarft,
+// T[0:p, p] = -tau_p T[0:p, 0:p] G[0:p, p], is the column-by-column inverse of S), so column j follows from S t_j = e_j by back
+// substitution on its own:
 //   t_jj = tau_j,   t_ij = -tau_i sum_{k = i+1 .. j} G_ik t_kj   (i = j-1 .. 0).
 // One WARP per column (lane l keeps t_k for k = l mod 32), rows of G prefetched four steps ahead: nb dependent steps of one shuffle
-// reduction each, instead of nb block-wide steps of two barriers each (0.20 ms -> ~0.02 ms per decomposition at N = 1000).
+// reduction each. (The column recurrence with one CTA per panel, nb block-wide steps of two barriers each, took 0.20 ms instead of
+// ~0.02 ms per decomposition at N = 1000.)
 // tau_j = 0 (H_j = I) gives a zero row and column like the recurrence does. Needs nb <= 128, nb % 32 == 0.
 __global__ void __launch_bounds__(256)
 larft_cols_kernel(const double* __restrict__ Gbuf, const double* __restrict__ tauv, int n_refl, int nb, double* __restrict__ Tbuf) {
@@ -748,6 +569,8 @@ void launch_eig_sign(cudaStream_t st, const double* VT, int ld, int n, double* s
   eig_sign_kernel<<<(n * 32 + 255) / 256, 256, 0, st>>>(VT, ld, n, sign);
 }
 
+bool eigen_tridiag_fits(int n) { return n >= 4 && (size_t)n * 5 * sizeof(double) + 4096 <= 226 * 1024; }
+
 TridiagWs* tridiag_ws_create(int n, int ld, int num_sms, char* err, size_t errlen) {
   TridiagWs* ws = new TridiagWs();
   ws->n = n; ws->ld = ld; ws->num_sms = num_sms;
@@ -756,7 +579,6 @@ TridiagWs* tridiag_ws_create(int n, int ld, int num_sms, char* err, size_t errle
   // ---- stage 1 geometry
   const int ns = (n + 1) & ~1;
   int grid = num_sms < 1 ? 1 : num_sms;
-  if (const char* ge = getenv("KCMA_SYTRD_GRID")) { const int g = atoi(ge); if (g >= 1 && g <= grid) grid = g; }   // A/B runs
   if (grid > (n + 3) / 4) grid = (n + 3) / 4;        // at least ~4 columns per CTA: fewer slices to collect per step at small N
   if (grid < 1) grid = 1;
   const int nloc_max = (n + grid - 1) / grid;
@@ -772,46 +594,23 @@ TridiagWs* tridiag_ws_create(int n, int ld, int num_sms, char* err, size_t errle
     else if (units <= 2 * SY_NT && nloc_max <= 14) ws->reg_variant = 4;
     else if (units <= 3 * SY_NT && nloc_max <= 11) ws->reg_variant = 3;
   }
-  ws->sy_threads = SY_NT;   // (74 CTAs x 512 threads, <1, 14, 1, 512>, was measured and dropped: 6.1 instead of 4.3 ms, profiles/r02_eigen_ab10.log)
+  // (74 CTAs x 512 threads, <KU, NC> = <1, 14>, was measured and dropped: 6.1 instead of 4.3 ms, profiles/r02_eigen_ab10.log)
   ws->resident = ws->reg_variant != 0;
   ws->sy_grid = grid;
   static const int kNC[5] = {0, 4, 7, 11, 14};
-  ws->sy_smem = ws->resident ? sizeof(double) * (3 * (size_t)ns + 80 + (size_t)kNC[ws->reg_variant] * ws->sy_threads) : vec_bytes;
-  // thread-block clusters (KCMA_SYTRD_CLUSTER=2|4): only for the <2,7> instantiation, and only when enough clusters are co-resident
-  ws->cluster = 1;
-  if (const char* cle = getenv("KCMA_SYTRD_CLUSTER")) {
-    const int cl = atoi(cle);
-    if ((cl == 2 || cl == 4) && ws->reg_variant == 2) {
-      const void* cfn = cl == 4 ? (const void*)sytrd_reg_kernel<2, 7, 4> : (const void*)sytrd_reg_kernel<2, 7, 2>;
-      const size_t smem = ws->sy_smem + sizeof(double) * 4 * (size_t)ns;
-      cudaLaunchConfig_t cfg;
-      memset(&cfg, 0, sizeof(cfg));
-      cfg.gridDim = dim3((grid / cl) * cl); cfg.blockDim = dim3(SY_NT); cfg.dynamicSmemBytes = smem;
-      cudaLaunchAttribute attr;
-      attr.id = cudaLaunchAttributeClusterDimension;
-      attr.val.clusterDim.x = cl; attr.val.clusterDim.y = 1; attr.val.clusterDim.z = 1;
-      cfg.attrs = &attr; cfg.numAttrs = 1;
-      int max_clusters = 0;
-      if (cudaFuncSetAttribute(cfn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) == cudaSuccess &&
-          cudaOccupancyMaxActiveClusters(&max_clusters, cfn, &cfg) == cudaSuccess) {
-        const int g = std::min(max_clusters, grid / cl) * cl;
-        if (g > 0 && (n + g - 1) / g <= 7) { ws->cluster = cl; ws->sy_grid = g; ws->sy_smem = smem; }
-      }
-      cudaGetLastError();
-    }
-  }
+  ws->sy_smem = ws->resident ? sizeof(double) * (3 * (size_t)ns + 80 + (size_t)kNC[ws->reg_variant] * SY_NT) : vec_bytes;
+  // (thread-block clusters of 2 or 4 CTAs for <2, 7>, whose leader polled the slots and pushed the entries into its peers' shared
+  // memory, were measured and dropped: config 3, sytrd 4.30 ms without, 4.44 / 4.30 ms with, profiles/r02_eigen_ab9_cluster.log)
   bool ok = true;
   if (!ws->resident) ok = ok && ws_alloc(ws, &ws->Awork, mat);
   ok = ok && ws_alloc(ws, &ws->dT, n) && ws_alloc(ws, &ws->eT, n) && ws_alloc(ws, &ws->tau, n) && ws_alloc(ws, &ws->VR, mat) &&
        ws_alloc(ws, &ws->VC, mat);
   LL* xb = nullptr;
   ws->ll_copies = 2;
-  if (const char* ce = getenv("KCMA_SYTRD_COPIES")) { const int c = atoi(ce); if (c >= 1 && c <= 16) ws->ll_copies = c; }
   // product slots: four copies at large N (a copy costs a producer one more 16-byte store per entry; 37 pollers per line instead of 74:
   // sytrd 4.17 -> 4.05 ms at N = 1000; three, six or eight copies, or more than two copies of the COLUMN slots, lose again:
   // profiles/r02_eigen_ab15.log, r02_eigen_ab16.log)
   ws->ll_pcopies = n > 512 ? 4 : ws->ll_copies;
-  if (const char* ce = getenv("KCMA_SYTRD_PCOPIES")) { const int c = atoi(ce); if (c >= 1 && c <= 16) ws->ll_pcopies = c; }
   ok = ok && ws_alloc(ws, &xb, (size_t)std::max(ws->ll_copies, ws->ll_pcopies) * 4 * (size_t)ns);
   ws->xbuf = xb;
   if (const char* pe = getenv("KCMA_SYTRD_PROF")) {   // "step0[,cta]": clock64 stamps of 32 steps of one CTA (tridiag_dump_prof)
@@ -821,10 +620,9 @@ TridiagWs* tridiag_ws_create(int n, int ld, int num_sms, char* err, size_t errle
   }
   // ---- stage 2 tree: uniform depth, even leaf boundaries, leaves of 2..32 rows
   int levels = 0;
-  // largest leaf: 12 rows (KCMA_DC_LEAF=<4..30> for A/B runs). Smaller leaves = cheaper Jacobi leaves, more merge levels: at N = 100 the
+  // largest leaf: 12 rows. Smaller leaves = cheaper Jacobi leaves, more merge levels: at N = 100 the
   // stage takes 0.38 ms with leaves of 25 rows, 0.25 with 6; at N = 1000 0.79 ms with 16 rows, 0.75 with 8 (profiles/r02_eigen_ab12.log)
-  int leaf_rows = 12;
-  if (const char* le = getenv("KCMA_DC_LEAF")) { const int v = atoi(le); if (v >= 4 && v <= 30) leaf_rows = v; }
+  const int leaf_rows = 12;
   if (n > 32)
     while ((n + (1 << levels) - 1) / (1 << levels) > leaf_rows) levels++;
   const int leaves = 1 << levels;
@@ -869,9 +667,7 @@ TridiagWs* tridiag_ws_create(int n, int ld, int num_sms, char* err, size_t errle
   cudaMemcpy(ws->d_row2node, row2node.data(), sizeof(int) * row2node.size(), cudaMemcpyHostToDevice);
   // ---- stage 3 geometry
   const int n_refl = n - 1;     // reflectors 0 .. n-2 (the last one is the identity, tau = 0)
-  const char* nbe = getenv("KCMA_WY_NB");
-  ws->nb = nbe ? atoi(nbe) : 128;
-  if (ws->nb < 16 || ws->nb > 128 || (ws->nb & 1)) ws->nb = 128;
+  ws->nb = 128;
   ws->nbld = ws->nb;
   ws->npanels = n_refl > 0 ? (n_refl + ws->nb - 1) / ws->nb : 0;
   const int row_tiles = (n + 127) / 128;
@@ -889,8 +685,7 @@ TridiagWs* tridiag_ws_create(int n, int ld, int num_sms, char* err, size_t errle
     // (the slabs are summed over the diagonal blocks only, dc_reduce_blocks_kernel). Bounded by 256 MB of slabs.
     ws->lvl_split.assign(std::max(levels, 1), 1);
     int max_split = ws->splitF;
-    static const int lvl_split_on = getenv("KCMA_DC_SPLIT") ? atoi(getenv("KCMA_DC_SPLIT")) : 1;
-    for (int l = 1; l < levels && lvl_split_on; l++) {
+    for (int l = 1; l < levels; l++) {
       int nmax = 0;
       for (const DcNode& nd : ws->lvl[l - 1]) nmax = std::max(nmax, nd.n);
       const int t = (nmax + 127) / 128, ctas = (int)ws->lvl[l - 1].size() * t * t;
@@ -981,8 +776,7 @@ TridiagWs* tridiag_ws_create(int n, int ld, int num_sms, char* err, size_t errle
   cudaError_t e1 = cudaFuncSetAttribute(sytrd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemCap);
   cudaError_t e2 = cudaFuncSetAttribute(sytrd_reg_kernel<3, 11>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
   if (e2 == cudaSuccess) e2 = cudaFuncSetAttribute(sytrd_reg_kernel<2, 14>, cudaFuncAttributeMaxDynamicSharedMemorySize, 96 * 1024);
-  cudaError_t e3 = cudaFuncSetAttribute(larft_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(sizeof(double) * (128 * 129 + 128)));
-  if (e1 != cudaSuccess || e2 != cudaSuccess || e3 != cudaSuccess) return fail("cudaFuncSetAttribute failed");
+  if (e1 != cudaSuccess || e2 != cudaSuccess) return fail("cudaFuncSetAttribute failed");
   if (cudaDeviceSynchronize() != cudaSuccess) return fail("CUDA error while building the workspace");
   return ws;
 }
@@ -1010,33 +804,14 @@ bool tridiag_stage_sytrd(cudaStream_t st, TridiagWs* ws, const double* M) {
   // exchange: 1 = one lane per warp spins on one slot before the block polls everything; 4 = a gate on one slot per producer first
   // (same time at N = 1000, 0.33 -> 0.28 ms at N = 100 where a step is short: profiles/r02_sytrd_exchange_ab.log)
   int opt = n <= 512 ? 4 : 1;
-  if (const char* oe = getenv("KCMA_SYTRD_OPT")) opt = atoi(oe);
   int copies = ws->ll_copies | (ws->ll_pcopies != ws->ll_copies ? ws->ll_pcopies << 8 : 0);
   void* rargs[] = {&M, &ld, &n, &ns, &xP, &xC, &dT, &eT, &tau, &VR, &prof, &prof_step0, &prof_cta, &opt, &copies};
   const void* fn = ws->reg_variant == 1 ? (const void*)sytrd_reg_kernel<1, 4> : ws->reg_variant == 2 ? (const void*)sytrd_reg_kernel<2, 7>
                    : ws->reg_variant == 3 ? (const void*)sytrd_reg_kernel<3, 11> : ws->reg_variant == 4 ? (const void*)sytrd_reg_kernel<2, 14>
                    : (const void*)sytrd_kernel;
-  // column prefetch (sytrd_reg_kernel<..., PF = true>): measured and NOT adopted (config 3: sytrd 4.67 against 4.30 ms — the column's
-  // loads come back late inside the pass, profiles/r02_sytrd_exchange_ab.log); KCMA_SYTRD_PREFETCH=1 selects it for A/B runs
-  bool pf = false;
-  if (const char* pe = getenv("KCMA_SYTRD_PREFETCH")) pf = atoi(pe) != 0;
-  if (pf && ws->cluster <= 1) {
-    if (ws->reg_variant == 1) fn = (const void*)sytrd_reg_kernel<1, 4, 1, SY_NT, true>;
-    else if (ws->reg_variant == 2) fn = (const void*)sytrd_reg_kernel<2, 7, 1, SY_NT, true>;
-  }
-  if (ws->cluster > 1) {   // <2,7> with a cluster leader that polls for its peers (geometry checked in tridiag_ws_create)
-    const void* cfn = ws->cluster == 4 ? (const void*)sytrd_reg_kernel<2, 7, 4> : (const void*)sytrd_reg_kernel<2, 7, 2>;
-    cudaLaunchConfig_t cfg;
-    memset(&cfg, 0, sizeof(cfg));
-    cfg.gridDim = dim3(ws->sy_grid); cfg.blockDim = dim3(SY_NT); cfg.dynamicSmemBytes = ws->sy_smem; cfg.stream = st;
-    cudaLaunchAttribute attrs[2];
-    attrs[0].id = cudaLaunchAttributeClusterDimension;
-    attrs[0].val.clusterDim.x = ws->cluster; attrs[0].val.clusterDim.y = 1; attrs[0].val.clusterDim.z = 1;
-    attrs[1].id = cudaLaunchAttributeCooperative;
-    attrs[1].val.cooperative = 1;
-    cfg.attrs = attrs; cfg.numAttrs = 2;
-    if (cudaLaunchKernelExC(&cfg, cfn, rargs) != cudaSuccess) return false;
-  } else if (cudaLaunchCooperativeKernel(fn, dim3(ws->sy_grid), dim3(ws->sy_threads), ws->resident ? rargs : args, ws->sy_smem, st) != cudaSuccess) return false;
+  // (column prefetch, where column c travels one step early and the exchange a step waits for is p = A v alone, was measured and
+  // dropped: config 3, sytrd 4.67 against 4.30 ms — the column's loads come back late inside the pass, profiles/r02_sytrd_exchange_ab.log)
+  if (cudaLaunchCooperativeKernel(fn, dim3(ws->sy_grid), dim3(SY_NT), ws->resident ? rargs : args, ws->sy_smem, st) != cudaSuccess) return false;
   // row n-1 of VR (no reflector) and tau[n-1] stay zero from the allocation; VC = VR^T
   launch_transpose(st, ws->VR, ws->VC, ld, n);
   return cudaGetLastError() == cudaSuccess;
@@ -1060,14 +835,12 @@ bool tridiag_stage_back_fork(cudaStream_t st, TridiagWs* ws, int* launches) {
   launch_set_identity(s2, ws->QT, ld, n);
   launch_gemm_batched(s2, ws->d_desc + ws->desc_g, ws->npanels, nb, nb, ws->gsplits);
   const double* G = ws->Gbuf;
-  if (ws->gsplits > 1) {   // sum the split-K slabs once (fixed order) instead of gsplits dependent loads per step of larft_kernel
+  if (ws->gsplits > 1) {   // sum the split-K slabs once (fixed order)
     launch_reduce_slabs(s2, ws->Gbuf, (long long)ws->npanels * nb * nb, ws->gsplits, ws->npanels * nb, nb, nb, ws->Gred, ws->num_sms);
     G = ws->Gred;
     *launches += 1;
   }
-  static const int larft_cols = getenv("KCMA_LARFT_COLS") ? atoi(getenv("KCMA_LARFT_COLS")) : 1;
-  if (larft_cols && nb <= 128 && nb % 32 == 0) larft_cols_kernel<<<dim3((nb + 7) / 8, ws->npanels), 256, 0, s2>>>(G, ws->tau, n_refl, nb, ws->Tbuf);
-  else larft_kernel<<<ws->npanels, LARFT_NT, sizeof(double) * (nb * (nb + 1) + nb), s2>>>(G, 0, 1, ws->tau, n_refl, nb, ws->Tbuf);
+  larft_cols_kernel<<<dim3((nb + 7) / 8, ws->npanels), 256, 0, s2>>>(G, ws->tau, n_refl, nb, ws->Tbuf);
   launch_gemm_batched(s2, ws->d_desc + ws->desc_vtil, ws->npanels, nb, n, 1);
   *launches += 4;
   for (int p = ws->npanels - 1; p >= 0; p--) {

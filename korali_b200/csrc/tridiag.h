@@ -12,16 +12,15 @@ struct TridiagWs {
   int n = 0, ld = 0, num_sms = 148;
   // ---- stage 1: Householder tridiagonalisation (sytrd_kernel)
   bool resident = false;       // this CTA's columns live in REGISTERS (N <= 1536: sytrd_reg_kernel), else in the global working copy
-  int cluster = 1;             // thread-block cluster size of the register variant (leader polls, peers receive through DSMEM)
-  int reg_variant = 0;         // 1, 2, 3 = sytrd_reg_kernel<1,4>, <2,7>, <3,11>
-  int sy_grid = 0, sy_threads = 256; size_t sy_smem = 0;
+  int reg_variant = 0;         // 1, 2, 3, 4 = sytrd_reg_kernel<1,4>, <2,7>, <3,11>, <2,14>
+  int sy_grid = 0; size_t sy_smem = 0;
   double* Awork = nullptr;     // n x ld working copy (global variant only)
   double *dT = nullptr, *eT = nullptr, *tau = nullptr;   // diagonal, off-diagonal, reflector scalars
   double *VR = nullptr;        // row i = reflector v_i (support i+1.., v_i[i+1] = 1)
   double *VC = nullptr;        // VR^T (column i = v_i)
   void* xbuf = nullptr;        // LL exchange slots: copies x [P | C] x 2 parities x n x 16 B
   int ll_copies = 2;           // replicas of every slot (spreads the polling of 148 CTAs over several L2 lines)
-  int ll_pcopies = 2;          // copies of the product slots (KCMA_SYTRD_PCOPIES; default = ll_copies)
+  int ll_pcopies = 2;          // copies of the product slots (four above N = 512, else ll_copies)
   long long* prof = nullptr; int prof_step0 = 0, prof_cta = 0;   // optional clock64 phase stamps of 32 steps (KCMA_SYTRD_PROF)
   // ---- stage 2: divide & conquer on (dT, eT)
   int levels = 0, leaf_count = 0;

@@ -1,5 +1,5 @@
 """One stand-alone eigendecomposition (kcma_k_eigen) of a CMA-ES-like covariance, for `ncu --metrics gpu__time_duration.sum`
-launch lists of the tridiagonalisation path (sytrd_kernel, dc_*, gemm_tn_batched_kernel, larft_kernel ...).
+launch lists of the tridiagonalisation path (sytrd_kernel, dc_*, gemm_tn_batched_kernel, larft_cols_kernel ...).
 
     python profiles/microbench/eigen_once.py [n] [repeats]
 """

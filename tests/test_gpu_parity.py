@@ -4,7 +4,6 @@ CPU oracle (oracle/okcma.c) or with the reference's own saved trajectory (tests/
 Bars (BASELINE.json north_star): ranking / selection indices bit-exact; mean, paths, sigma and C within a relative
 1e-11 in FP64 (TOL below); polynomial objectives bit-exact; optimum within 1e-8.
 """
-import os
 
 import numpy as np
 import pytest
@@ -167,12 +166,12 @@ def test_eigen_clustered_and_repeated_spectrum(n):
     assert np.abs(v2.T @ v2 - np.eye(n)).max() < 1e-12
 
 
-@pytest.mark.parametrize("order", ["rr", "ring"])
-@pytest.mark.parametrize("n", [31, 120, 1000])
-def test_eigen_tournament_orders(order, n, monkeypatch):
-    """Both tournament orders of jacobi_pipe_kernel (KCMA_JACOBI_ORDER, read per launch; the ring order is the default at
-    these sizes: 8, 32 and 256 blocks) give a decomposition of the same quality; the eigenvalues agree to round-off."""
-    monkeypatch.setenv("KCMA_JACOBI_ORDER", order)
+@pytest.mark.parametrize("n,order", [(31, "ring"), (120, "ring"), (1000, "ring"), (200, "rr"), (300, "rr"), (600, "rr")])
+def test_eigen_tournament_orders(n, order, monkeypatch):
+    """Both tournament orders of jacobi_pipe_kernel, each reached by size: the ring order when padding the block count to a power
+    of two costs <= 1/8 more steps (8, 32 and 256 blocks), else round-robin (50, 76 and 150 blocks). KCMA_EIGEN=jacobi, because
+    without constraints these sizes go to the tridiagonal solver. Same decomposition quality; the eigenvalues agree to round-off."""
+    monkeypatch.setenv("KCMA_EIGEN", "jacobi")
     rng = np.random.default_rng(77 + n)
     q, _ = np.linalg.qr(rng.standard_normal((n, n)))
     lam = np.sort(10.0 ** rng.uniform(0, 3, n))
@@ -185,13 +184,13 @@ def test_eigen_tournament_orders(order, n, monkeypatch):
     assert np.abs(w - lam).max() < 1e-11 * lam.max()
 
 
-@pytest.mark.parametrize("order", ["rr", "ring"])
-def test_eigen_tournament_orders_large_n_path(order, monkeypatch):
-    """N = 2000 runs on the one-launch-per-step path with 16-row blocks (126 blocks, 128 with the ring order's two phantom
-    blocks): both orders must deliver the decomposition; clustered CMA-ES-like spectrum."""
-    monkeypatch.setenv("KCMA_JACOBI_ORDER", order)
-    n = 2000
-    rng = np.random.default_rng(2000)
+@pytest.mark.parametrize("n,order", [(2000, "ring"), (1300, "rr")])
+def test_eigen_tournament_orders_large_n_path(n, order, monkeypatch):
+    """Rows longer than 1280 run on the one-launch-per-step path with 16-row blocks, in both orders by size: N = 2000 has 126
+    blocks, 128 with the ring order's two phantom blocks; N = 1300 has 82 blocks and takes the round-robin order. KCMA_EIGEN=jacobi
+    as above; both must deliver the decomposition of a clustered CMA-ES-like spectrum."""
+    monkeypatch.setenv("KCMA_EIGEN", "jacobi")
+    rng = np.random.default_rng(n)
     z = rng.standard_normal((2 * n, n))
     c = 0.965 * np.eye(n) + 0.035 * (z.T @ z) / (2 * n)
     c = 0.5 * (c + c.T)
@@ -200,26 +199,6 @@ def test_eigen_tournament_orders_large_n_path(order, monkeypatch):
     assert np.abs(v @ np.diag(w) @ v.T - c).max() < 1e-12 * np.abs(c).max()
     assert np.abs(v.T @ v - np.eye(n)).max() < 1e-12
     assert np.abs(w - np.linalg.eigvalsh(c)).max() < 1e-12 * np.abs(w).max()
-
-
-@pytest.mark.skipif(os.environ.get("KCMA_TEST_EXPERIMENTAL") != "1",
-                    reason="experimental kernel variant, written and compiled in round 1 but not yet run on a GPU: KCMA_TEST_EXPERIMENTAL=1")
-@pytest.mark.parametrize("n", [31, 64, 120, 1000])
-def test_eigen_resident_anchor_variant(n, monkeypatch):
-    """KCMA_JACOBI_ORDER=anchor: ring order with the slot's first block resident in shared memory (jacobi_pipe_kernel<256, 2>).
-    Same decomposition quality as the product path; the eigenvalues agree with it to round-off."""
-    rng = np.random.default_rng(99 + n)
-    q, _ = np.linalg.qr(rng.standard_normal((n, n)))
-    lam = np.sort(10.0 ** rng.uniform(0, 3, n))
-    c = (q * lam) @ q.T
-    c = 0.5 * (c + c.T)
-    w0, _ = _lib.k_eigen(c)
-    monkeypatch.setenv("KCMA_JACOBI_ORDER", "anchor")
-    w, v = _lib.k_eigen(c)
-    assert np.all(np.diff(w) >= 0)
-    assert np.abs(v @ np.diag(w) @ v.T - c).max() < 1e-12 * np.abs(c).max()
-    assert np.abs(v.T @ v - np.eye(n)).max() < 1e-12
-    assert np.abs(w - w0).max() < 1e-12 * lam.max()
 
 
 def test_eigen_identity_and_rejection():

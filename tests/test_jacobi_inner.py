@@ -126,7 +126,7 @@ def test_inner_solver_quadratic_tail_and_noop(inner):
 def test_tournament_schedules_are_one_factorisations(inner, order, sizes):
     """Both tournament orders of jacobi_pipe_kernel (rr_pair / ring_pair, the code the kernel runs): every step pairs every
     block exactly once, every pair of blocks meets exactly once per sweep, p < q. The ring order additionally keeps the
-    first block of slot k in place for all but log2(np) - 1 of the step transitions (what a resident-anchor kernel needs)."""
+    first block of slot k in place for all but log2(np) - 1 of the step transitions."""
     so = inner.lib
     for nb in sizes:
         seen = set()
@@ -149,35 +149,3 @@ def test_tournament_schedules_are_one_factorisations(inner, order, sizes):
         if order == 1 and nb >= 8:
             # slot k changes its first block only when a sub-tournament hands it a block of the B half: at most once per level
             assert stays >= (nb - 2) * (nb // 2) - (nb // 2) * (int(np.log2(nb)) - 1)
-
-
-@pytest.mark.parametrize("nb,p_rot0", [(8, 0.0), (16, 0.3), (16, 0.9), (32, 0.5)])
-def test_resident_anchor_protocol_emulation(nb, p_rot0):
-    """The dataflow protocol of the experimental resident-anchor variant (KCMA_JACOBI_ORDER=anchor, eigen.cu ORDER = 2), emulated
-    on the CPU under random interleavings of every CTA's G and V group: no deadlock, every combined block value is the current
-    one, global memory is current after every sweep (asserted inside the emulation), and the variant saves what it claims."""
-    import importlib.util
-    spec = importlib.util.spec_from_file_location(
-        "jacobi_anchor_protocol_sim", os.path.join(HERE, "..", "profiles", "microbench", "jacobi_anchor_protocol_sim.py"))
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    sim = mod.run(nb, 2, 11 + nb, p_rot0)
-    pair_steps = 2 * (nb - 1) * (nb // 2)
-    assert sim.G == sim.truthG and sim.V == sim.truthV
-    assert sim.stats["steps"] == pair_steps
-    assert sim.stats["g_loads"] < 1.5 * pair_steps          # 2 per pair-step without the resident block
-    # the emulated schedule is the one the kernel runs
-    for step in range(nb - 1):
-        for k in range(nb // 2):
-            assert mod.ring_pair(nb, step, k) == _pair(1, nb, step, k)
-
-
-def _pair(order, nb, step, k, _cache={}):
-    if "lib" not in _cache:
-        import tempfile
-        so = os.path.join(tempfile.mkdtemp(prefix="jinner"), "libjinner.so")
-        subprocess.check_call(["g++", "-O2", "-ffp-contract=off", "-shared", "-fPIC", "-o", so, os.path.join(HERE, "helpers", "jacobi_inner_host.cpp")])
-        _cache["lib"] = C.CDLL(so)
-    p, q = C.c_int(-1), C.c_int(-1)
-    _cache["lib"].jacobi_pair_host(order, nb, step, k, C.byref(p), C.byref(q))
-    return p.value, q.value

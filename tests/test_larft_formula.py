@@ -2,8 +2,8 @@
 Householder reflectors H_0 H_1 ... H_{k-1} = I - V T V^T (dlarft, forward / columnwise) is the inverse of the upper triangular
 S = striu(V^T V) + diag(1 / tau), so every column of T follows from a back substitution of its own,
     t_jj = tau_j,   t_ij = -tau_i sum_{k = i+1 .. j} G_ik t_kj   (i = j-1 .. 0),
-which is what one warp per column computes on the device. Checked against the column recurrence of dlarft (the predecessor
-larft_kernel) and against the product of the reflectors; tau_j = 0 (H_j = I) gives a zero row and column in both."""
+which is what one warp per column computes on the device. Checked against the column recurrence of dlarft (what a
+column-sequential kernel computes) and against the product of the reflectors; tau_j = 0 (H_j = I) gives a zero row and column in both."""
 import numpy as np
 
 
