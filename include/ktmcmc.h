@@ -41,6 +41,23 @@
  *   resampling uniform of draw k                  : ctr { 0, k, 0, generation }, first uniform;
  *   accept uniform of chain k at step t           : ctr { 1, k, t, generation }, first uniform;
  *   z of chain k at step t, components 2p, 2p+1   : ctr { 2^20 + p, k, t, generation } -> Box-Muller pair.
+ *
+ * Bayesian/Reference (ktmcmc_set_reference): the log-likelihood of an evaluated row is reduced on the device from M model outputs.
+ * d_j = reference datum j (j < M), g_j = the computational model's prediction, p_j = its per-point parameter, r_j = d_j - g_j:
+ *   KTMCMC_LIK_NORMAL           p = sigma ("Standard Deviation") > 0:  t_j = -log(2 pi)/2 - log sigma - (r / sigma)^2 / 2
+ *   KTMCMC_LIK_POSITIVE_NORMAL  p = sigma > 0, the normal truncated to d >= 0:  t_j = the Normal term - log Phi(g / sigma), with
+ *                               log Phi(u) = log(erfc(-u / sqrt 2) / 2) for u >= -1, else log(erfcx(-u / sqrt 2) / 2) - u^2 / 2
+ *                               (finite for every finite u); a term that rounds to NaN (only when |g / sigma| overflows) is -inf
+ *   KTMCMC_LIK_STUDENT_T        p = nu ("Degrees Of Freedom") > 0, the standard t of the residual:
+ *                               t_j = lgamma((nu + 1) / 2) - lgamma(nu / 2) - log(nu pi) / 2 - (nu + 1) / 2 log1p(r^2 / nu); for nu >= 50
+ *                               the first three terms are evaluated as their asymptotic series in x = nu / 2,
+ *                               -log(2 pi) / 2 + (1 / x)(-1/8 + y (1/192 + y (-1/640 + y 17/14336))), y = 1 / x^2 (exact to double
+ *                               precision there; the difference of two lgamma values would cancel)
+ *   KTMCMC_LIK_POISSON          no parameter, g = the mean >= 0:  t_j = d log g - g - lgamma(d + 1) (lgamma(d + 1) computed once on the
+ *                               host from the data); t_j = -g when d = 0 and -inf when g = 0 < d
+ * l = sum_j t_j: lane k of one warp per row sums j = k, k + 32, ... ascending, then the xor butterfly (the order of the log-prior).
+ * Errors (reported after the step with the evaluation row): a non-finite g, a parameter <= 0 or non-finite, a Poisson mean < 0.
+ * A finite model output can give l = -inf (weight 0), never +inf or NaN.
  */
 #ifndef KTMCMC_H
 #define KTMCMC_H
@@ -108,13 +125,31 @@ int ktmcmc_inject_factor(ktmcmc_t* h, const double* a, size_t count);
 int ktmcmc_set_host_loglik(ktmcmc_t* h, ktmcmc_host_loglik_fn fn, void* user);
 int ktmcmc_set_device_loglik(ktmcmc_t* h, kcma_device_objective_fn fn, void* user);
 
+/* Bayesian/Reference: the log-likelihood is reduced on the device from the outputs of a computational model (definitions above). */
+enum { KTMCMC_LIK_NORMAL = 1, KTMCMC_LIK_POSITIVE_NORMAL = 2, KTMCMC_LIK_STUDENT_T = 3, KTMCMC_LIK_POISSON = 4 };
+/* Once, after create and before generation 1; cfg.loglik must be KCMA_OBJ_EXTERNAL. Copies data[m]. Allocates the model outputs
+ * (lambda x m, and as many per-point parameters unless the likelihood has none); an allocation failure names the GiB needed. */
+int ktmcmc_set_reference(ktmcmc_t* h, int32_t likelihood, const double* data, uint64_t m);
+/* g_out / p_out: rows x m, row-major, packed; p_out is NULL for a likelihood without a per-point parameter (Poisson) */
+typedef void (*ktmcmc_host_reference_fn)(void* user, const double* x, uint64_t rows, uint64_t n, double* g_out, double* p_out, uint64_t m);
+/* x_dev: rows x n with leading dimension ldx; g_dev / p_dev: rows x m with leading dimension ldm (p_dev NULL as above); the model
+ * writes them on `stream` (a cudaStream_t) */
+typedef void (*ktmcmc_device_reference_fn)(void* user, const double* x_dev, uint64_t rows, uint64_t n, uint64_t ldx,
+                                           double* g_dev, double* p_dev, uint64_t m, uint64_t ldm, void* stream);
+int ktmcmc_set_host_reference_model(ktmcmc_t* h, ktmcmc_host_reference_fn fn, void* user);
+int ktmcmc_set_device_reference_model(ktmcmc_t* h, ktmcmc_device_reference_fn fn, void* user);
+/* The model outputs of the rows the next ktmcmc_eval evaluates (parity tests); count = rows * m; p is NULL for Poisson. */
+int ktmcmc_inject_reference(ktmcmc_t* h, const double* g, const double* p, size_t count);
+
 int ktmcmc_check_termination(ktmcmc_t* h, int* finished, const char** reason);
 int ktmcmc_run(ktmcmc_t* h, uint64_t max_generations, uint64_t* done);
 
 /* State by Korali key name. Arrays: "Sample Database" (lambda x n), "Sample LogLikelihood Database", "Sample LogPrior Database",
  * "Covariance Matrix" (n x n), "Proposal Factor" (A = B D, n x n), "Mean Theta" (n), "Weights" (w~), "Selection Counts" (c_i),
  * "Chain Leaders", "Chain Lengths" (chain count each), "Evaluation Rows" (rows of the next evaluation, packed),
- * "Proposal Support" (per chain: 1 = the last proposal was inside the priors' support), "Accept Flags" (per chain, last step).
+ * "Proposal Support" (per chain: 1 = the last proposal was inside the priors' support), "Accept Flags" (per chain, last step),
+ * "Evaluation LogLikelihoods" (the log-likelihoods the last ktmcmc_eval produced, packed like "Evaluation Rows"; read it before the
+ * next ktmcmc_propose).
  * Scalars: "Annealing Exponent", "Previous Annealing Exponent", "Annealing Exponent Update", "Coefficient Of Variation",
  * "LogEvidence", "Max Loglikelihood", "Chain Count", "Max Chain Steps", "Current Step", "Proposals Acceptance Rate",
  * "Selection Acceptance Rate", "Model Evaluation Count", "Current Generation", "Population Size", "Burn In",

@@ -5,7 +5,9 @@
 
 Served: `"Solver": {"Type": "Optimizer/CMAES"}` (the hot path) and its sibling population solvers `Optimizer/DEA`, `Optimizer/MOCMAES`
 of `"Problem": {"Type": "Optimization"}`, the transitional MCMC sampler `Sampler/TMCMC` of `"Problem": {"Type": "Bayesian/Custom"}`
-(priors from `e["Distributions"]`), plus the float ask/tell class `fCMAES` (SURVEY.md scope).
+and `"Bayesian/Reference"` (priors from `e["Distributions"]`; Reference: "Reference Data", a "Computational Model" that sets
+`sample["Reference Evaluations"]`, and the Normal, Positive Normal, StudentT or Poisson "Likelihood Model", reduced on the device),
+plus the float ask/tell class `fCMAES` (SURVEY.md scope).
 Layers: korali_b200._host (pybind11, C++: Engine / Experiment, mirrors python/korali/__init__.py:9-20 + source/engine.cpp:201-254)
  -> include/kcma.h (C ABI) -> korali_b200/libkcma.so (hand-written sm_100a CUDA). There is no CPU fallback.
 """
@@ -40,6 +42,12 @@ def batched(fn):
     at a time (conduit.cpp.base:29-88); per-sample models still work, this is the fast path for Python models.
 
         e["Problem"]["Objective Function"] = korali.batched(lambda X: -np.sum(X * X, axis=1))
+
+    As a Bayesian/Reference "Computational Model", ``fn(X)`` returns a dict keyed like the sample, each value broadcast to
+    ``samples x M`` (a bare array of predictions is accepted for Poisson):
+
+        e["Problem"]["Computational Model"] = korali.batched(lambda X: {"Reference Evaluations": X[:, :1] + X[:, 1:2] * t,
+                                                                         "Standard Deviation": X[:, 2:3]})
     """
     def model(X):
         return fn(X)
@@ -60,6 +68,10 @@ def batched_device(fn):
     population never leaves the device.
 
         e["Problem"]["Objective Function"] = korali.batched_device(lambda X: -(X * X).sum(dim=1))
+
+    As a Bayesian/Reference "Computational Model", ``fn(X)`` returns a dict of CUDA tensors keyed like the sample ("Reference
+    Evaluations" and the likelihood's per-point parameter; a bare tensor for Poisson), each broadcast to ``samples x M`` by ``copy_``
+    straight into the solver's buffers on its stream.
     """
     def model(x_ptr, rows, n, ldx, f_ptr, stream):
         import torch
@@ -70,8 +82,34 @@ def batched_device(fn):
                 F.copy_(fn(X).to(torch.float64).reshape(rows))
         else:       # the solver runs on the legacy default stream, which is also torch's default stream
             F.copy_(fn(X).to(torch.float64).reshape(rows))
+
+    def reference(x_ptr, rows, n, ldx, g_ptr, p_ptr, m, ldm, stream, g_key, p_key):
+        import contextlib
+        import torch
+        X = torch.as_tensor(_DeviceArray(x_ptr, (rows, n), (ldx * 8, 8)), device="cuda")
+        with torch.cuda.stream(torch.cuda.ExternalStream(stream)) if stream else contextlib.nullcontext():
+            r = fn(X)
+            if not isinstance(r, dict):
+                if p_key is not None:
+                    raise ValueError("The batched computational model must return a dict with '%s' and '%s' (a bare tensor is accepted "
+                                     "for Poisson only)" % (g_key, p_key))
+                r = {g_key: r}
+            for key, ptr in ((g_key, g_ptr), (p_key, p_ptr)):
+                if key is None:
+                    continue
+                if key not in r:
+                    raise KeyError("The batched computational model did not return '%s'" % key)
+                v = torch.as_tensor(r[key], dtype=torch.float64, device="cuda")
+                dst = torch.as_tensor(_DeviceArray(ptr, (rows, m), (ldm * 8, 8)), device="cuda")
+                try:
+                    dst.copy_(v)
+                except RuntimeError:
+                    raise ValueError("The batched computational model's '%s' has shape %s, which does not broadcast to %d samples x %d "
+                                     "reference points" % (key, tuple(v.shape), rows, m)) from None
     model._korali_batched = "device"
+    model._korali_reference = reference     # Bayesian/Reference: the outputs go to the solver's prediction / parameter buffers
     return model
+
 
 
 def fCMAES(nVars, populationSize=0, muSize=0, device=0):

@@ -2,19 +2,22 @@
 (oracle/libokcma.so, prefix ``otmcmc_``; test infrastructure only) can be driven with the same vocabulary. Nothing here loads the oracle."""
 import ctypes as C
 import numpy as np
-from ._abi import HandleBase, OBJECTIVES, _dp
+from ._abi import HandleBase, OBJECTIVES, _as_dp, _dp
 
 KTMCMC_ABI_VERSION = 1
 KCMA_OBJ_EXTERNAL = 100
 PRIORS = {"Uniform": 0, "Normal": 1}
+LIKELIHOODS = {"Normal": 1, "Positive Normal": 2, "StudentT": 3, "Poisson": 4}   # KTMCMC_LIK_* of Bayesian/Reference
 HOST_CB = C.CFUNCTYPE(None, C.c_void_p, _dp, C.c_uint64, C.c_uint64, _dp)
+HOST_REFERENCE_CB = C.CFUNCTYPE(None, C.c_void_p, _dp, C.c_uint64, C.c_uint64, _dp, _dp, C.c_uint64)
 
 # every symbol include/ktmcmc.h declares
 EXPORTS = [
     "ktmcmc_cfg_defaults", "ktmcmc_create", "ktmcmc_destroy", "ktmcmc_last_error", "ktmcmc_run_generation", "ktmcmc_anneal",
     "ktmcmc_resample", "ktmcmc_propose", "ktmcmc_eval", "ktmcmc_accept", "ktmcmc_inject_loglik", "ktmcmc_inject_factor",
     "ktmcmc_set_host_loglik", "ktmcmc_set_device_loglik", "ktmcmc_check_termination", "ktmcmc_run", "ktmcmc_get_array",
-    "ktmcmc_get_scalar", "ktmcmc_set_scalar", "ktmcmc_launch_count",
+    "ktmcmc_get_scalar", "ktmcmc_set_scalar", "ktmcmc_launch_count", "ktmcmc_set_reference", "ktmcmc_set_host_reference_model",
+    "ktmcmc_set_device_reference_model", "ktmcmc_inject_reference",
 ]
 
 
@@ -32,10 +35,12 @@ class KtmcmcCfg(C.Structure):
 
 class TmcmcHandle(HandleBase):
     """kw: n, population_size, priors = [(type, a, b)] * n (type "Uniform" | "Normal"), loglik (a KCMA_OBJ name such as "NegSphere",
-    or "External"), per_generation_burn_in (list), loglik_coef, and the scalar fields of ktmcmc_cfg."""
+    or "External"), per_generation_burn_in (list), loglik_coef, reference = (likelihood name of LIKELIHOODS, data) for
+    Bayesian/Reference (the log-likelihood must be External, the default), and the scalar fields of ktmcmc_cfg."""
     CFG = KtmcmcCfg
     ARRAYS = ("loglik_coef",)
     ENUMS = {"loglik": OBJECTIVES}
+    reference = None
 
     def _field(self, cfg, k, v, kw):
         if k == "priors":
@@ -43,12 +48,19 @@ class TmcmcHandle(HandleBase):
             cfg.prior_a, cfg.prior_b = self._array([p[1] for p in v], len(v)), self._array([p[2] for p in v], len(v))
         elif k == "per_generation_burn_in":
             cfg.per_generation_burn_in, cfg.burn_in_count = self._array(v, len(v), np.uint64), len(v)
+        elif k == "reference":
+            self.reference = v
         else:
             return False
         return True
 
     def _created(self, cfg):
         self.population_size = int(cfg.population_size)
+        if self.reference is not None:
+            name, data = self.reference
+            d = np.ascontiguousarray(data, dtype=np.float64).ravel()
+            self.likelihood, self.m = LIKELIHOODS[name], d.size
+            self._check(self._fn("set_reference", C.c_int, [C.c_void_p, C.c_int32, _dp, C.c_uint64])(self._live(), self.likelihood, _as_dp(d), d.size))
 
     def anneal(self): self._call("anneal")
     def resample(self): self._call("resample")
@@ -60,6 +72,26 @@ class TmcmcHandle(HandleBase):
     def set_host_loglik(self, fn):
         """fn(X: ndarray[rows, n]) -> ndarray[rows] of log-likelihoods."""
         self._set_callback("set_host_loglik", HOST_CB, fn, lambda rows, n: (rows,))
+
+    def set_host_reference(self, fn):
+        """Bayesian/Reference: fn(X: ndarray[rows, n]) -> (G, P) of rows x m predictions and per-point parameters (broadcast), or G
+        alone for Poisson."""
+        def tramp(_u, x, rows, n, g_out, p_out, m):
+            out = fn(np.ctypeslib.as_array(x, shape=(rows, n)))
+            g, p = (out, None) if not p_out else out
+            np.ctypeslib.as_array(g_out, shape=(rows, m))[:] = np.broadcast_to(np.asarray(g, dtype=np.float64), (rows, m))
+            if p_out:
+                np.ctypeslib.as_array(p_out, shape=(rows, m))[:] = np.broadcast_to(np.asarray(p, dtype=np.float64), (rows, m))
+        cb = HOST_REFERENCE_CB(tramp)
+        self._keep.append(cb)
+        self._check(self._fn("set_host_reference_model", C.c_int, [C.c_void_p, HOST_REFERENCE_CB, C.c_void_p])(self._live(), cb, None))
+
+    def inject_reference(self, g, p=None):
+        """The model outputs (rows x m, and the parameters unless Poisson) of the rows the next eval evaluates."""
+        g = np.ascontiguousarray(g, dtype=np.float64).ravel()
+        p = None if p is None else np.ascontiguousarray(p, dtype=np.float64).ravel()
+        self._check(self._fn("inject_reference", C.c_int, [C.c_void_p, _dp, _dp, C.c_size_t])(
+            self._live(), _as_dp(g), None if p is None else _as_dp(p), g.size))
 
 
 def Solver(**kw):

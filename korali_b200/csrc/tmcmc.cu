@@ -13,7 +13,8 @@
 //                    tm_chain_init_kernel    chains start at their leader's (x, l, p)
 //   ktmcmc_propose   tm_z_kernel + launch_gemm_tn (x' = x + A z for every chain) + tm_epilogue_kernel (log-prior, support flag)
 //                    + tm_compact_kernel / tm_gather_kernel (the in-support proposals of active chains, packed in chain order)
-//   ktmcmc_eval      launch_objective (built-in models) or the host / device conduit on the packed rows
+//   ktmcmc_eval      launch_objective (built-in models) or the host / device conduit on the packed rows; Bayesian/Reference: the
+//                    host / device computational model writes G (and P), then tm_reference_loglik_kernel<LIK> reduces them to l
 //   ktmcmc_accept    tm_accept_kernel        Metropolis test, database append, acceptance statistics
 // Compiled with --fmad=false: the arithmetic rounds like oracle/otmcmc.c (the device's exp / log / sincospi may differ from libm in
 // the last bit; the GEMM and the SYRK sum in their own order).
@@ -69,8 +70,10 @@ struct TmScalars {
   unsigned long long step_evals;     // rows of the current evaluation
   unsigned long long accepted, proposals;   // this generation
   int chain_count, max_len, leaders, last_pos;
-  int nan_flag, allinf_flag, pad0, pad1;
+  int nan_flag, allinf_flag;
+  unsigned long long ref_err;        // Bayesian/Reference: ~(row << 2 | code) of the first bad model output (atomicMax), 0 = none
 };
+enum { kRefNonFinite = 0, kRefParameter = 1, kRefPoissonMean = 2 };
 
 __device__ __forceinline__ double prior_term(int type, double a, double b, double x) {
   if (type == KTMCMC_PRIOR_UNIFORM) return (x >= a && x <= b) ? -log(b - a) : -INFINITY;
@@ -416,6 +419,61 @@ __global__ void tm_check_nan_kernel(const double* __restrict__ F, int count, TmS
   if (i < count && F[i] != F[i]) sc->nan_flag = 1;
 }
 
+// Bayesian/Reference terms (include/ktmcmc.h; tests/helpers/otmcmc_reference.c restates them in the same operation order)
+constexpr double kInvSqrt2 = 0.70710678118654752440;
+constexpr double kPi = 3.14159265358979323846;
+__device__ __forceinline__ double log_ndtr(double u) {
+  if (u >= -1.0) return log(0.5 * erfc(-u * kInvSqrt2));
+  return log(0.5 * erfcx(-u * kInvSqrt2)) - 0.5 * (u * u);
+}
+__device__ __forceinline__ double student_t_const(double nu) {   // lgamma((nu + 1) / 2) - lgamma(nu / 2) - log(nu pi) / 2
+  if (nu < 50.0) return lgamma(0.5 * (nu + 1.0)) - lgamma(0.5 * nu) - 0.5 * log(nu * kPi);
+  const double ix = 1.0 / (0.5 * nu), y = ix * ix;
+  return ix * (-0.125 + y * (1.0 / 192.0 + y * (-1.0 / 640.0 + y * (17.0 / 14336.0)))) - kHalfLog2Pi;
+}
+// l of each evaluated row from its M predictions G (and parameters P): one warp per row, lane k sums j = k, k + 32, ... ascending,
+// then the xor butterfly. Reads rows * M * 8 bytes of G (and of P) once, coalesced; the data (and, for Poisson, lgamma(d + 1) in
+// DC) through the read-only path. A bad output is recorded in sc->ref_err and leaves its term NaN.
+template <int LIK>
+__global__ void __launch_bounds__(256)
+tm_reference_loglik_kernel(int rows, int m, long long ldm, const double* __restrict__ G, const double* __restrict__ P,
+                           const double* __restrict__ D, const double* __restrict__ DC, double* __restrict__ EF, TmScalars* __restrict__ sc) {
+  const int lane = threadIdx.x & 31;
+  const long long i = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5;
+  if (i >= rows) return;
+  const double* g = G + i * ldm;
+  const double* p = LIK == KTMCMC_LIK_POISSON ? nullptr : P + i * ldm;
+  double s = 0.0;
+  int bad = 4;
+  for (int j = lane; j < m; j += 32) {
+    const double gj = g[j], dj = __ldg(D + j);
+    double t;
+    if (!isfinite(gj)) { bad = min(bad, (int)kRefNonFinite); t = NAN; }
+    else if (LIK == KTMCMC_LIK_POISSON) {
+      if (gj < 0.0) { bad = min(bad, (int)kRefPoissonMean); t = NAN; }
+      else t = dj == 0.0 ? -gj : (gj == 0.0 ? -INFINITY : dj * log(gj) - gj - __ldg(DC + j));
+    } else {
+      const double pj = p[j], r = dj - gj;
+      if (!(pj > 0.0) || !isfinite(pj)) { bad = min(bad, (int)kRefParameter); t = NAN; }
+      else if (LIK == KTMCMC_LIK_STUDENT_T) t = student_t_const(pj) - 0.5 * (pj + 1.0) * log1p(r * r / pj);
+      else {
+        const double z = r / pj;
+        t = -kHalfLog2Pi - log(pj) - 0.5 * (z * z);
+        if (LIK == KTMCMC_LIK_POSITIVE_NORMAL) { t = t - log_ndtr(gj / pj); if (t != t) t = -INFINITY; }
+      }
+    }
+    s = s + t;
+  }
+  if (bad < 4) atomicMax(&sc->ref_err, ~(((unsigned long long)i << 2) | (unsigned)bad));
+  s = warp_sum_butterfly(s);
+  if (lane == 0) EF[i] = s;
+}
+template <int LIK>
+void launch_reference(cudaStream_t st, int rows, int m, long long ldm, const double* G, const double* P, const double* D, const double* DC,
+                      double* EF, TmScalars* sc) {
+  tm_reference_loglik_kernel<LIK><<<(unsigned)(((long long)rows * 32 + 255) / 256), 256, 0, st>>>(rows, m, ldm, G, P, D, DC, EF, sc);
+}
+
 unsigned grid_for(long long threads, int per) { return (unsigned)std::max<long long>(1, (threads + per - 1) / per); }
 
 }  // namespace
@@ -447,7 +505,14 @@ struct ktmcmc {
   double tc_target = 1.0, tc_max_generations = 1e10, tc_max_model_evaluations = 1e9;
   ktmcmc_host_loglik_fn host_fn = nullptr; void* host_user = nullptr;
   kcma_device_objective_fn dev_fn = nullptr; void* dev_user = nullptr;
-  std::vector<double> hX, hF;
+  // Bayesian/Reference (lik = 0: Bayesian/Custom): data, lgamma(data + 1) for Poisson, model outputs G and parameters Pr (s_rows x ldm)
+  int lik = 0, ef_rows = 0;
+  long long m = 0, ldm = 0;
+  double *dData = nullptr, *dDataC = nullptr, *dG = nullptr, *dPr = nullptr;
+  bool have_ref_inj = false;
+  ktmcmc_host_reference_fn host_ref_fn = nullptr; void* host_ref_user = nullptr;
+  ktmcmc_device_reference_fn dev_ref_fn = nullptr; void* dev_ref_user = nullptr;
+  std::vector<double> hX, hF, hG, hP;
   std::string err, reason;
   std::vector<void*> allocs;
 };
@@ -475,7 +540,18 @@ int tm_pull(ktmcmc* h) {
   TM_CUDA(h, cudaGetLastError());
   return 0;
 }
+const char* tm_param_key(int lik) { return lik == KTMCMC_LIK_STUDENT_T ? "Degrees Of Freedom" : "Standard Deviation"; }
 int tm_check_flags(ktmcmc* h) {
+  if (h->hSc->ref_err) {
+    const unsigned long long e = ~h->hSc->ref_err;
+    const long long row = (long long)(e >> 2);
+    const int code = (int)(e & 3);
+    if (code == kRefNonFinite)
+      return tm_fail(h, "Bayesian/Reference: 'Reference Evaluations' of sample %lld contains a non-finite value\n", row);
+    if (code == kRefParameter)
+      return tm_fail(h, "Bayesian/Reference: '%s' of sample %lld contains a value that is not positive and finite\n", tm_param_key(h->lik), row);
+    return tm_fail(h, "Bayesian/Reference: 'Reference Evaluations' of sample %lld contains a negative Poisson mean\n", row);
+  }
   if (h->hSc->nan_flag) return tm_fail(h, "A NaN log-likelihood was produced by the likelihood model\n");
   if (h->hSc->allinf_flag) return tm_fail(h, "Every sample of the population has a log-likelihood of -inf: the annealing step is undefined\n");
   return 0;
@@ -593,6 +669,51 @@ int ktmcmc_set_device_loglik(ktmcmc_t* h, kcma_device_objective_fn fn, void* use
   return 0;
 }
 
+int ktmcmc_set_reference(ktmcmc_t* h, int32_t likelihood, const double* data, uint64_t m) {
+  if (!h) return tm_fail(nullptr, "null solver handle");
+  if (h->lik) return tm_fail(h, "set_reference: the reference data are already set");
+  if (h->gen != 1 || h->proposed) return tm_fail(h, "set_reference: call it before generation 1");
+  if (h->cfg.loglik != KCMA_OBJ_EXTERNAL) return tm_fail(h, "set_reference: the log-likelihood must be External (KCMA_OBJ_EXTERNAL)");
+  if (likelihood < KTMCMC_LIK_NORMAL || likelihood > KTMCMC_LIK_POISSON) return tm_fail(h, "set_reference: unknown likelihood %d", likelihood);
+  if (!data || m < 1 || m > (uint64_t)INT32_MAX) return tm_fail(h, "set_reference: need 1 <= m < 2^31 reference data (got %zu)", (size_t)m);
+  std::vector<double> dc(m, 0.0);
+  for (uint64_t j = 0; j < m; j++) {
+    const double d = data[j];
+    if (!std::isfinite(d)) return tm_fail(h, "Bayesian/Reference: 'Reference Data' %zu is not finite\n", (size_t)j);
+    if (likelihood == KTMCMC_LIK_POISSON && (d < 0.0 || d != floor(d)))
+      return tm_fail(h, "Bayesian/Reference: 'Reference Data' %zu (%g) must be a non-negative integer for the Poisson likelihood\n", (size_t)j, d);
+    if (likelihood == KTMCMC_LIK_POSITIVE_NORMAL && d < 0.0)
+      return tm_fail(h, "Bayesian/Reference: 'Reference Data' %zu (%g) must be >= 0 for the Positive Normal likelihood\n", (size_t)j, d);
+    if (likelihood == KTMCMC_LIK_POISSON) dc[j] = lgamma(d + 1.0);
+  }
+  TM_CUDA(h, cudaSetDevice(h->device));
+  const long long ldm = ((long long)m + 3) / 4 * 4;   // 32-byte aligned rows
+  const bool param = likelihood != KTMCMC_LIK_POISSON;
+  const size_t each = (size_t)h->s_rows * ldm;
+  const double gib = (double)each * sizeof(double) * (param ? 2 : 1) / (double)(1ull << 30);
+  if (tm_alloc(h, &h->dG, each) != cudaSuccess || (param && tm_alloc(h, &h->dPr, each) != cudaSuccess)) {
+    cudaGetLastError();
+    return tm_fail(h, "Bayesian/Reference: cannot allocate the model outputs of %d samples x %zu reference points (%.2f GiB)\n", h->lambda,
+                   (size_t)m, gib);
+  }
+  TM_CUDA(h, tm_alloc(h, &h->dData, m));
+  TM_CUDA(h, tm_alloc(h, &h->dDataC, m));
+  TM_CUDA(h, cudaMemcpy(h->dData, data, sizeof(double) * m, cudaMemcpyHostToDevice));
+  TM_CUDA(h, cudaMemcpy(h->dDataC, dc.data(), sizeof(double) * m, cudaMemcpyHostToDevice));
+  h->lik = likelihood; h->m = (long long)m; h->ldm = ldm;
+  return 0;
+}
+int ktmcmc_set_host_reference_model(ktmcmc_t* h, ktmcmc_host_reference_fn fn, void* user) {
+  if (!h) return tm_fail(nullptr, "null solver handle");
+  h->host_ref_fn = fn; h->host_ref_user = user;
+  return 0;
+}
+int ktmcmc_set_device_reference_model(ktmcmc_t* h, ktmcmc_device_reference_fn fn, void* user) {
+  if (!h) return tm_fail(nullptr, "null solver handle");
+  h->dev_ref_fn = fn; h->dev_ref_user = user;
+  return 0;
+}
+
 // steps 1-3
 int ktmcmc_anneal(ktmcmc_t* h) {
   if (!h) return tm_fail(nullptr, "null solver handle");
@@ -691,6 +812,24 @@ int ktmcmc_inject_loglik(ktmcmc_t* h, const double* l, size_t count) {
   return 0;
 }
 
+int ktmcmc_inject_reference(ktmcmc_t* h, const double* g, const double* p, size_t count) {
+  if (!h) return tm_fail(nullptr, "null solver handle");
+  if (!h->lik) return tm_fail(h, "inject_reference: no reference data (ktmcmc_set_reference)");
+  if (!h->proposed || h->evaluated) return tm_fail(h, "inject_reference: no proposals waiting for an evaluation");
+  if (!g || (h->lik != KTMCMC_LIK_POISSON) != (p != nullptr)) return tm_fail(h, "inject_reference: need g, and p exactly when the likelihood has a parameter");
+  TM_CUDA(h, cudaSetDevice(h->device));
+  if (h->eval_rows < 0) { if (tm_pull(h)) return 1; h->eval_rows = (int)h->hSc->step_evals; }
+  if (count != (size_t)h->eval_rows * h->m) return tm_fail(h, "inject_reference: %zu values for %d evaluation rows x %lld", count, h->eval_rows, h->m);
+  const size_t row = sizeof(double) * h->m, pitch = sizeof(double) * h->ldm;
+  if (count) {
+    TM_CUDA(h, cudaMemcpy2DAsync(h->dG, pitch, g, row, row, h->eval_rows, cudaMemcpyHostToDevice, h->stream));
+    if (p) TM_CUDA(h, cudaMemcpy2DAsync(h->dPr, pitch, p, row, row, h->eval_rows, cudaMemcpyHostToDevice, h->stream));
+  }
+  TM_CUDA(h, cudaStreamSynchronize(h->stream));
+  h->have_ref_inj = true;
+  return 0;
+}
+
 int ktmcmc_inject_factor(ktmcmc_t* h, const double* a, size_t count) {
   if (!h) return tm_fail(nullptr, "null solver handle");
   if (count != (size_t)h->N * h->N) return tm_fail(h, "inject_factor: %zu values for %d x %d", count, h->N, h->N);
@@ -706,8 +845,39 @@ int ktmcmc_eval(ktmcmc_t* h) {
   TM_CUDA(h, cudaSetDevice(h->device));
   const int N = h->N, ld = h->ld;
   cudaStream_t st = h->stream;
+  h->ef_rows = h->eval_rows;
   if (h->have_inj) {
     h->have_inj = false;
+  } else if (h->lik) {
+    // Bayesian/Reference: injected outputs, or the device / host computational model, then the likelihood kernel
+    if (h->eval_rows < 0) { if (tm_pull(h)) return 1; h->eval_rows = (int)h->hSc->step_evals; }
+    const int rows = h->ef_rows = h->eval_rows;
+    const long long m = h->m, ldm = h->ldm;
+    double* dp = h->lik == KTMCMC_LIK_POISSON ? nullptr : h->dPr;
+    if (h->have_ref_inj) {
+      h->have_ref_inj = false;
+    } else if (rows > 0 && h->dev_ref_fn) {
+      h->dev_ref_fn(h->dev_ref_user, h->dEX, (uint64_t)rows, (uint64_t)N, (uint64_t)ld, h->dG, dp, (uint64_t)m, (uint64_t)ldm, (void*)st);
+    } else if (rows > 0 && h->host_ref_fn) {
+      const size_t row = sizeof(double) * m, pitch = sizeof(double) * ldm;
+      h->hX.resize((size_t)rows * N); h->hG.resize((size_t)rows * m); h->hP.resize(dp ? (size_t)rows * m : 0);
+      TM_CUDA(h, cudaMemcpy2DAsync(h->hX.data(), sizeof(double) * N, h->dEX, sizeof(double) * ld, sizeof(double) * N, rows, cudaMemcpyDeviceToHost, st));
+      TM_CUDA(h, cudaStreamSynchronize(st));
+      h->host_ref_fn(h->host_ref_user, h->hX.data(), (uint64_t)rows, (uint64_t)N, h->hG.data(), dp ? h->hP.data() : nullptr, (uint64_t)m);
+      TM_CUDA(h, cudaMemcpy2DAsync(h->dG, pitch, h->hG.data(), row, row, rows, cudaMemcpyHostToDevice, st));
+      if (dp) TM_CUDA(h, cudaMemcpy2DAsync(dp, pitch, h->hP.data(), row, row, rows, cudaMemcpyHostToDevice, st));
+    } else if (rows > 0) {
+      return tm_fail(h, "Bayesian/Reference: inject the model outputs or set a host / device computational model before eval");
+    }
+    if (rows > 0) {
+      switch (h->lik) {
+        case KTMCMC_LIK_NORMAL: launch_reference<KTMCMC_LIK_NORMAL>(st, rows, (int)m, ldm, h->dG, dp, h->dData, h->dDataC, h->dEF, h->dSc); break;
+        case KTMCMC_LIK_POSITIVE_NORMAL: launch_reference<KTMCMC_LIK_POSITIVE_NORMAL>(st, rows, (int)m, ldm, h->dG, dp, h->dData, h->dDataC, h->dEF, h->dSc); break;
+        case KTMCMC_LIK_STUDENT_T: launch_reference<KTMCMC_LIK_STUDENT_T>(st, rows, (int)m, ldm, h->dG, dp, h->dData, h->dDataC, h->dEF, h->dSc); break;
+        default: launch_reference<KTMCMC_LIK_POISSON>(st, rows, (int)m, ldm, h->dG, dp, h->dData, h->dDataC, h->dEF, h->dSc); break;
+      }
+      h->launches++;
+    }
   } else if (h->cfg.loglik != KCMA_OBJ_EXTERNAL) {
     const long long rows = h->gen == 1 ? h->lambda : h->chains;   // rows past the packed ones are evaluated and never read
     launch_objective(st, h->cfg.loglik, h->dEX, ld, rows, N, 0, 1, nullptr, h->dDsc, h->dCoef, h->dEF, h->num_sms);
@@ -824,6 +994,9 @@ int ktmcmc_get_array(ktmcmc_t* h, const char* key, double* out, size_t cap, size
   else if (!strcmp(key, "Evaluation Rows")) {
     if (h->proposed && h->eval_rows < 0) { if (tm_pull(h)) return 1; h->eval_rows = (int)h->hSc->step_evals; }
     src = h->dEX; rows = h->proposed ? (size_t)h->eval_rows : 0; width = N; pitch = ld;
+  } else if (!strcmp(key, "Evaluation LogLikelihoods")) {
+    if (h->ef_rows < 0) { if (tm_pull(h)) return 1; h->ef_rows = (int)h->hSc->step_evals; }
+    src = h->dEF; rows = (size_t)h->ef_rows;
   } else return tm_fail(h, "unknown array key '%s'", key);
   const size_t n = rows * width;
   if (count) *count = n;

@@ -250,11 +250,15 @@ py::list paramsOf(const double* x, uint64_t n) {
 // sample[output] (a list of K values for "Evaluate Multiple"); korali_b200.batched(fn) gets the whole population as a (rows x N)
 // NumPy view and returns rows x K values; korali_b200.batched_device(fn) gets raw device pointers. A Python exception is kept in
 // *pending (rethrown after the generation) and the outputs are filled with `fill`.
+// A Bayesian/Reference computational model has two outputs per sample: sample[output] ("Reference Evaluations") and, unless param
+// is null, sample[param] (the per-point parameter), each a list of M values; a batched model returns them as a dict keyed like the
+// sample, broadcast to rows x M (evaluateReference, hostReference, deviceReference).
 struct Model {
   py::object fn;
   std::string flavour;                  // "", "numpy" or "device"
   const char* operation = "Evaluate";   // or "Evaluate Multiple"
   const char* output = "F(x)";
+  const char* param = nullptr;          // Bayesian/Reference: "Standard Deviation", "Degrees Of Freedom", or null (Poisson)
   double fill = NAN;
   std::string* pending = nullptr;
 
@@ -293,6 +297,74 @@ struct Model {
     } catch (const std::exception& e) {
       *pending = e.what();
       for (uint64_t i = 0; i < rows * K; i++) out[i] = fill;
+    }
+  }
+
+  // one output of a per-sample computational model: a list of m values
+  static void sampleValues(py::dict sample, const char* key, uint64_t i, uint64_t m, double* out) {
+    if (!sample.contains(key)) korali_error("The computational model did not set '%s' for sample %zu\n", key, (size_t)i);
+    py::object v = sample[key];
+    if (py::isinstance<py::str>(v) || !py::hasattr(v, "__len__") || (uint64_t)py::len(v) != m)
+      korali_error("The computational model's '%s' of sample %zu must be a list of %zu values (one per 'Reference Data' point)\n", key, (size_t)i, (size_t)m);
+    uint64_t k = 0;
+    for (auto x : v) out[k++] = x.cast<double>();
+  }
+  // one output of a batched computational model, broadcast to rows x m
+  static void batchValues(py::object v, const char* key, uint64_t rows, uint64_t m, double* out) {
+    py::module_ np = py::module_::import("numpy");
+    py::object a = np.attr("asarray")(v, "float64");
+    py::array_t<double, py::array::c_style | py::array::forcecast> b;
+    try {
+      b = np.attr("ascontiguousarray")(np.attr("broadcast_to")(a, py::make_tuple(rows, m)));
+    } catch (const py::error_already_set&) {
+      const std::string shape = py::str(a.attr("shape")).cast<std::string>();
+      korali_error("The batched computational model's '%s' has shape %s, which does not broadcast to %zu samples x %zu reference points\n", key,
+                   shape.c_str(), (size_t)rows, (size_t)m);
+    }
+    memcpy(out, b.data(), sizeof(double) * rows * m);
+  }
+  void evaluateReference(const double* x, uint64_t rows, uint64_t n, double* g, double* p, uint64_t m) {
+    try {
+      if (flavour == "numpy") {
+        py::array_t<double> X({(py::ssize_t)rows, (py::ssize_t)n}, {(py::ssize_t)(n * sizeof(double)), (py::ssize_t)sizeof(double)}, x, py::none());
+        py::object r = fn(X);
+        if (!py::isinstance<py::dict>(r)) {
+          if (param) korali_error("The batched computational model must return a dict with '%s' and '%s' (a bare array is accepted for Poisson only)\n", output, param);
+          batchValues(r, output, rows, m, g);
+          return;
+        }
+        py::dict d = py::reinterpret_borrow<py::dict>(r);
+        for (const char* key : {output, param}) {
+          if (!key) continue;
+          if (!d.contains(key)) korali_error("The batched computational model did not return '%s'\n", key);
+          batchValues(d[key], key, rows, m, key == output ? g : p);
+        }
+        return;
+      }
+      for (uint64_t i = 0; i < rows; i++) {
+        py::dict sample = sampleOf(paramsOf(x + i * n, n), i, operation);
+        fn(sample);
+        sampleValues(sample, output, i, m, g + i * m);
+        if (param) sampleValues(sample, param, i, m, p + i * m);
+      }
+    } catch (const std::exception& e) {
+      *pending = e.what();
+      for (uint64_t i = 0; i < rows * m; i++) { g[i] = 0.0; if (p) p[i] = 1.0; }   // valid outputs: the pending error is the one raised
+    }
+  }
+  // ktmcmc_host_reference_fn
+  static void hostReference(void* user, const double* x, uint64_t rows, uint64_t n, double* g, double* p, uint64_t m) {
+    ((Model*)user)->evaluateReference(x, rows, n, g, p, m);
+  }
+  // ktmcmc_device_reference_fn: the second entry point of korali_b200.batched_device copies the model's tensors into g_dev / p_dev
+  static void deviceReference(void* user, const double* x_dev, uint64_t rows, uint64_t n, uint64_t ldx, double* g_dev, double* p_dev, uint64_t m,
+                              uint64_t ldm, void* stream) {
+    Model* self = (Model*)user;
+    try {
+      self->fn.attr("_korali_reference")((uintptr_t)x_dev, rows, n, ldx, (uintptr_t)g_dev, (uintptr_t)p_dev, m, ldm, (uintptr_t)stream,
+                                         self->output, self->param ? py::object(py::str(self->param)) : py::object(py::none()));
+    } catch (const std::exception& e) {
+      *self->pending = e.what();
     }
   }
 
@@ -1124,7 +1196,7 @@ class MOCMAES : public Plugin<kmocma_t, kmocma_cfg> {
   }
 };
 
-// ---- the solver plug-in: Sampler/TMCMC on libkcma (include/ktmcmc.h) for Bayesian/Custom problems ---------------------------------
+// ---- the solver plug-in: Sampler/TMCMC on libkcma (include/ktmcmc.h) for Bayesian/Custom and Bayesian/Reference problems ----
 class TMCMC : public Plugin<ktmcmc_t, ktmcmc_cfg> {
  public:
   py::object distributions = py::none();   // the experiment's top-level "Distributions" (the priors)
@@ -1132,7 +1204,9 @@ class TMCMC : public Plugin<ktmcmc_t, ktmcmc_cfg> {
   std::vector<double> prior_a, prior_b;
   std::vector<uint64_t> burn_in;
   std::vector<std::string> prior_name;
-  Model model;   // the Python likelihood model when cfg.loglik is KCMA_OBJ_EXTERNAL
+  Model model;   // the Python likelihood model when cfg.loglik is KCMA_OBJ_EXTERNAL, or the Bayesian/Reference computational model
+  int32_t likelihood = 0;          // Bayesian/Reference: KTMCMC_LIK_*, 0 for Bayesian/Custom
+  std::vector<double> ref_data;    // its "Reference Data"
 
   TMCMC() : Plugin({ktmcmc_create, ktmcmc_destroy, ktmcmc_last_error, ktmcmc_run_generation, ktmcmc_check_termination, ktmcmc_get_array,
                     ktmcmc_get_scalar, ktmcmc_set_scalar},
@@ -1141,6 +1215,65 @@ class TMCMC : public Plugin<ktmcmc_t, ktmcmc_cfg> {
                     {"Max Model Evaluations", 1e9, false, true}}) {}
   const char* name() const override { return "Sampler/TMCMC"; }
   size_t variableCount() const override { return cfg.n; }
+
+  // bayesian/custom.config: "Likelihood Model" is a callable setting sample["logLikelihood"] or the name of a device model
+  void setCustom(Settings& p) {
+    if (!p.has("Likelihood Model")) korali_error(" + Object: [ Bayesian/Custom ] \n + Key:    ['Likelihood Model']\n + Reason: mandatory setting missing\n");
+    py::object model_fn = p.take("Likelihood Model");
+    p.finish();
+    if (py::isinstance<py::str>(model_fn)) {
+      cfg.loglik = deviceObjective(model_fn.cast<std::string>(), "likelihood model");
+    } else if (PyCallable_Check(model_fn.ptr())) {
+      cfg.loglik = KCMA_OBJ_EXTERNAL;
+      model.set(model_fn, &pending_error);
+      model.output = "logLikelihood";   // Bayesian/Custom "Evaluate": the model sets sample["logLikelihood"]
+      model.fill = 0.0;
+    } else {
+      korali_error(" + Object: [ Bayesian/Custom ] \n + Key:    ['Likelihood Model']\n + Reason: neither a callable nor the name of a device model\n");
+    }
+  }
+
+  // bayesian/reference.config: "Likelihood Model", "Reference Data" and a "Computational Model" that sets sample["Reference
+  // Evaluations"] (and the likelihood's per-point parameter); the log-likelihood is reduced on the device (include/ktmcmc.h)
+  void setReference(Settings& p) {
+    p.module = "Bayesian/Reference";
+    for (const char* k : {"Likelihood Model", "Reference Data", "Computational Model"})
+      if (!p.has(k)) korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['%s']\n + Reason: mandatory setting missing\n", k);
+    const std::string name = p.str("Likelihood Model", "");
+    const std::string lik = canon(name);
+    if (lik == "normal") likelihood = KTMCMC_LIK_NORMAL;
+    else if (lik == "positivenormal") likelihood = KTMCMC_LIK_POSITIVE_NORMAL;
+    else if (lik == "studentt") likelihood = KTMCMC_LIK_STUDENT_T;
+    else if (lik == "poisson") likelihood = KTMCMC_LIK_POISSON;
+    else if (lik == "positivestudentt" || lik == "geometric" || lik == "negativebinomial")
+      korali_error("Bayesian/Reference: 'Likelihood Model' '%s' is not built on the B200 path (Normal, Positive Normal, StudentT and Poisson are)\n", name.c_str());
+    else korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Likelihood Model']\n + Reason: unknown value '%s' (Normal, Positive Normal, StudentT, Poisson)\n", name.c_str());
+    py::object data = p.take("Reference Data");
+    if (!py::isinstance<py::list>(data) || py::len(data) == 0)
+      korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Reference Data']\n + Reason: a non-empty array of numbers was expected\n");
+    ref_data.clear();
+    for (auto x : data) {
+      const size_t j = ref_data.size();
+      if (!is_number(x) || !std::isfinite(x.cast<double>()))
+        korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Reference Data']\n + Reason: entry %zu is not a finite number\n", j);
+      const double d = x.cast<double>();
+      if (likelihood == KTMCMC_LIK_POISSON && (d < 0.0 || d != std::floor(d)))
+        korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Reference Data']\n + Reason: entry %zu (%g) must be a non-negative integer for the Poisson likelihood\n", j, d);
+      if (likelihood == KTMCMC_LIK_POSITIVE_NORMAL && d < 0.0)
+        korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Reference Data']\n + Reason: entry %zu (%g) must be >= 0 for the Positive Normal likelihood\n", j, d);
+      ref_data.push_back(d);
+    }
+    py::object model_fn = p.take("Computational Model");
+    if (py::isinstance<py::str>(model_fn))
+      korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Computational Model']\n + Reason: a callable was expected (there is no built-in device computational model)\n");
+    if (!PyCallable_Check(model_fn.ptr()))
+      korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Computational Model']\n + Reason: a callable was expected\n");
+    p.finish();
+    cfg.loglik = KCMA_OBJ_EXTERNAL;
+    model.set(model_fn, &pending_error);
+    model.output = "Reference Evaluations";
+    model.param = likelihood == KTMCMC_LIK_POISSON ? nullptr : likelihood == KTMCMC_LIK_STUDENT_T ? "Degrees Of Freedom" : "Standard Deviation";
+  }
 
   // generated TMCMC::setConfiguration (TMCMC.config) + Sampler:: + Solver:: (strict); priors from e["Distributions"]
   void setConfiguration(py::dict solver, py::list variables, py::dict problem, uint64_t seed) override {
@@ -1174,23 +1307,12 @@ class TMCMC : public Plugin<ktmcmc_t, ktmcmc_cfg> {
       if (s.has(k)) s.take(k);
     s.finish();
     if (cfg.population_size < 2) korali_error("Sampler/TMCMC: 'Population Size' must be set to at least 2\n");
-    // problem (bayesian/custom.config)
+    // problem (bayesian/custom.config, bayesian/reference.config)
     Settings p = object(problem, "Bayesian/Custom", "'Problem' is not an object\n");
     const std::string ptype = canon(p.str("Type", ""));
-    if (ptype != "bayesian/custom") korali_error("Sampler/TMCMC: only Problem Type 'Bayesian/Custom' is served (got '%s')\n", ptype.c_str());
-    if (!p.has("Likelihood Model")) korali_error(" + Object: [ Bayesian/Custom ] \n + Key:    ['Likelihood Model']\n + Reason: mandatory setting missing\n");
-    py::object model_fn = p.take("Likelihood Model");
-    p.finish();
-    if (py::isinstance<py::str>(model_fn)) {
-      cfg.loglik = deviceObjective(model_fn.cast<std::string>(), "likelihood model");
-    } else if (PyCallable_Check(model_fn.ptr())) {
-      cfg.loglik = KCMA_OBJ_EXTERNAL;
-      model.set(model_fn, &pending_error);
-      model.output = "logLikelihood";   // Bayesian/Custom "Evaluate": the model sets sample["logLikelihood"]
-      model.fill = 0.0;
-    } else {
-      korali_error(" + Object: [ Bayesian/Custom ] \n + Key:    ['Likelihood Model']\n + Reason: neither a callable nor the name of a device model\n");
-    }
+    if (ptype == "bayesian/reference") setReference(p);
+    else if (ptype == "bayesian/custom") setCustom(p);
+    else korali_error("Sampler/TMCMC: only Problem Type 'Bayesian/Custom' or 'Bayesian/Reference' is served (got '%s')\n", ptype.c_str());
     // priors: e["Distributions"][k] = {"Name", "Type", parameters}
     std::vector<std::string> dname, dtype;
     std::vector<double> da, db;
@@ -1237,7 +1359,11 @@ class TMCMC : public Plugin<ktmcmc_t, ktmcmc_cfg> {
   void initialize(const std::vector<int>& device_ids) override {
     requireOneDevice(device_ids);
     create(device_ids[0]);
-    if (cfg.loglik == KCMA_OBJ_EXTERNAL) {
+    if (likelihood) {
+      check(ktmcmc_set_reference(h, likelihood, ref_data.data(), ref_data.size()));
+      if (model.flavour == "device") check(ktmcmc_set_device_reference_model(h, &Model::deviceReference, &model));
+      else check(ktmcmc_set_host_reference_model(h, &Model::hostReference, &model));
+    } else if (cfg.loglik == KCMA_OBJ_EXTERNAL) {
       if (model.flavour == "device") check(ktmcmc_set_device_loglik(h, &Model::device, &model));
       else check(ktmcmc_set_host_loglik(h, &Model::host, &model));
     }
