@@ -4,7 +4,6 @@
 #include <dlfcn.h>
 #include <math.h>
 #include <nccl.h>
-#include <stdarg.h>
 #include <stdio.h>
 #include <string.h>
 
@@ -15,14 +14,13 @@
 
 #include "../../include/kcma.h"
 #include "common.cuh"
+#include "handle.cuh"
 #include "kernels.h"
 
 using namespace kc;
 namespace kc { extern long long* g_jacobi_dbg; }
 
 namespace {
-
-char g_create_err[1024] = "";
 
 // ---- NCCL through dlopen: no link-time dependency; prefers the copy torch already loaded ---------------
 struct NcclApi {
@@ -53,10 +51,9 @@ struct Phase { double ms = 0; uint64_t calls = 0; };
 
 }  // namespace
 
-struct kcma {
+struct kcma : Handle<kcma, DevScalars> {
   kcma_cfg cfg;
-  int N = 0, ld = 0, device = 0, num_sms = 148;
-  cudaStream_t stream = 0;
+  int N = 0, ld = 0, num_sms = 148;
   std::vector<double> lower, upper, init_val, init_sd, min_sd, coef, con_shift;
   bool has_bounds = false, any_min_sd = false;
   uint64_t lambda = 0, mu = 0, vlambda = 0, vmu = 0, cur_lambda = 0, cur_mu = 0, s_max = 0, mu_max = 0;
@@ -71,7 +68,7 @@ struct kcma {
   std::vector<double> h_weights;
   double tc_max_condition = INFINITY, tc_min_sd = -INFINITY, tc_max_sd = INFINITY, tc_max_value = INFINITY,
          tc_min_value_diff = -INFINITY, tc_max_model_evaluations = 1e9, tc_max_generations = 1e10;
-  uint64_t gen = 1, model_evals = 0;
+  uint64_t model_evals = 0;
   int is_viability = 0, has_constraints = 0;
   uint64_t n_con = 0;
   // device state
@@ -85,7 +82,7 @@ struct kcma {
   std::vector<double> gran;
   double *dGran = nullptr, *dMask = nullptr, *dMaskSigma = nullptr, *dDiscMut = nullptr;
   unsigned* dIdx = nullptr;
-  void* dSortWs = nullptr;
+  unsigned char* dSortWs = nullptr;
   double *dW = nullptr, *dSelW = nullptr;
   int *dSelS = nullptr, *dCount = nullptr;
   double *dS = nullptr, *dPartial = nullptr, *dWsplit = nullptr, *dRed = nullptr;
@@ -105,12 +102,9 @@ struct kcma {
   unsigned* dAttempt = nullptr;
   long long ldg = 0; int u_rows = 0;
   double normal_lr = -1.0, cov_adaption_factor = -1.0;
-  void* dFlush = nullptr; size_t flush_bytes = 0;
-  DevScalars* dSc = nullptr;
-  DevScalars* hSc = nullptr;  // pinned mirror
+  double* dFlush = nullptr; size_t flush_bytes = 0;
   int* hCount = nullptr;      // pinned
   int s_rows_padded = 0, rows_per_cta = 64, max_splits = 16, cur_splits = 1;
-  bool scalars_fresh = false;
   bool sampled_pending = false;  // ask done, tell not yet: X uses (mean, sigma); afterwards (mean_old, sigma_sampling)
   // injections
   bool inj_z = false, inj_bd = false, inj_y = false, inj_x = false, inj_f = false, inj_grad = false;
@@ -133,7 +127,6 @@ struct kcma {
   struct Pending { std::string name; cudaEvent_t a, b; };
   std::vector<Pending> pending;
   std::vector<cudaEvent_t> event_pool;
-  uint64_t launches = 0;
   uint64_t sweeps_base = 0;   // DevScalars::jacobi_sweeps_total at the last kcma_timing_reset
   // CUDA graph of one whole generation (ask + eval + tell) for the launch-latency-bound configurations
   cudaStream_t cap_stream = nullptr;
@@ -141,35 +134,12 @@ struct kcma {
   bool capturing = false, graph_failed = false;
   uint64_t dev_gen = ~0ull;   // value DevScalars::gen is known to hold on the device (~0 = unknown): the graph replay reads it
   uint64_t g_launches = 0, g_evals = 0;   // host-side counters one replay stands for
-  std::string err, warn, reason;
+  std::string warn;
   char warn_out[4096];
+  ~kcma();
 };
 
 namespace {
-
-int fail(kcma* h, const char* fmt, ...) {
-  char buf[1024];
-  va_list ap;
-  va_start(ap, fmt);
-  vsnprintf(buf, sizeof(buf), fmt, ap);
-  va_end(ap);
-  if (h) h->err = buf;
-  else strncpy(g_create_err, buf, sizeof(g_create_err) - 1);
-  return 1;
-}
-
-#define CUDA_OK(h, call)                                                                      \
-  do {                                                                                        \
-    cudaError_t e_ = (call);                                                                  \
-    if (e_ != cudaSuccess) return fail(h, "CUDA error %s at %s:%d (%s)", cudaGetErrorString(e_), __FILE__, __LINE__, #call); \
-  } while (0)
-
-template <typename T>
-cudaError_t dmalloc(T** p, size_t count) {
-  cudaError_t e = cudaMalloc((void**)p, sizeof(T) * (count ? count : 1));
-  if (e == cudaSuccess) e = cudaMemset(*p, 0, sizeof(T) * (count ? count : 1));
-  return e;
-}
 
 struct PhaseTimer {
   kcma* h; const char* name; cudaEvent_t a = nullptr, b = nullptr;
@@ -270,17 +240,9 @@ int nccl_check(kcma* h, ncclResult_t r, const char* what) {
   return fail(h, "NCCL error in %s: %s", what, g_nccl.GetErrorString ? g_nccl.GetErrorString(r) : "?");
 }
 
-int pull_scalars(kcma* h) {
-  if (h->scalars_fresh) return 0;
-  CUDA_OK(h, cudaMemcpyAsync(h->hSc, h->dSc, sizeof(DevScalars), cudaMemcpyDeviceToHost, h->stream));
-  CUDA_OK(h, cudaStreamSynchronize(h->stream));
-  h->scalars_fresh = true;
-  return 0;
-}
 int push_scalars(kcma* h) {
   h->hSc->gen = h->gen - 1;   // device copy of the generation counter = last completed generation
-  CUDA_OK(h, cudaMemcpyAsync(h->dSc, h->hSc, sizeof(DevScalars), cudaMemcpyHostToDevice, h->stream));
-  CUDA_OK(h, cudaStreamSynchronize(h->stream));
+  if (push(h)) return 1;
   h->dev_gen = h->gen - 1;
   return 0;
 }
@@ -487,7 +449,7 @@ int update_eigensystem(kcma* h, const double* dM) {
     launch_jacobi_block_sweep(h->stream, h->dGT, h->dVTw, ld, N, tol, h->dSc, &l);
     h->launches += l;
     h->scalars_fresh = false;
-    if (pull_scalars(h)) return 1;
+    if (pull_cached(h)) return 1;
     if (h->hSc->jacobi_rotations == 0) break;
     // quadratic convergence: once every pair of the sweep was already orthogonal to 1e-8 (KC_QUAD_TAIL), what is left after
     // this sweep is ~1e-16 * lambda / gap and the confirmation sweep (a full pass that rotates nothing) can be skipped
@@ -598,7 +560,7 @@ int settle_resampling_budget(kcma* h, long long ls, unsigned long long zrow_begi
     CUDA_OK(h, cudaStreamSynchronize(h->stream));   // `att` / `rows` are host vectors
   }
   h->scalars_fresh = false;
-  if (pull_scalars(h)) return 1;
+  if (pull_cached(h)) return 1;
   h->hSc->infeasible_sample_count = total;
   return push_scalars(h);
 }
@@ -613,7 +575,7 @@ int resample_infeasible(kcma* h, long long ls, unsigned long long zrow_begin) {
   if (dFresh) CUDA_OK(h, cudaMemsetAsync(dFresh, 1, local_zrows(h), h->stream));
   unsigned long long count_before = 0, local_counted = 0;
   if (maxres != 0) {
-    if (pull_scalars(h)) return 1;
+    if (pull_cached(h)) return 1;
     count_before = h->hSc->infeasible_sample_count;
   }
   // no sample needs more redraws than the budget holds; the hard cap keeps a never-feasible sample from spinning forever
@@ -630,7 +592,7 @@ int resample_infeasible(kcma* h, long long ls, unsigned long long zrow_begin) {
     if (maxres == 0) return 0;  // reference release build: size_t(Infinity) == 0 -> never resamples (SURVEY Q2)
     CUDA_OK(h, cudaMemcpyAsync(h->hCount, h->dCount, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
     CUDA_OK(h, cudaMemcpyAsync(h->hRound, h->dRound, 2 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, h->stream));
-    if (pull_scalars(h)) return 1;
+    if (pull_cached(h)) return 1;
     local_counted += h->hSc->infeasible_this_round;
     const int cnt = *h->hCount;
     if (h->hRound[1] == 0 || round >= cap) break;
@@ -746,7 +708,7 @@ int check_mean_and_set_regime(kcma* h) {
     CUDA_OK(h, cudaMemcpyAsync(m.data(), h->dMean, sizeof(double) * h->N, cudaMemcpyDeviceToHost, h->stream));
     CUDA_OK(h, cudaStreamSynchronize(h->stream));
     h->host_con(h->host_con_user, m.data(), 1, (uint64_t)h->N, g.data(), h->n_con);
-    if (pull_scalars(h)) return 1;
+    if (pull_cached(h)) return 1;
     h->hSc->constraint_evaluation_count += 1;
     int ok = 1;
     for (uint64_t c = 0; c < h->n_con; c++) {
@@ -760,7 +722,7 @@ int check_mean_and_set_regime(kcma* h) {
     launch_constraints_mean(h->stream, h->dMean, h->dShift, h->N, (int)h->n_con, h->dSc);
     h->launches++;
     h->scalars_fresh = false;
-    if (pull_scalars(h)) return 1;
+    if (pull_cached(h)) return 1;
   }
   if (h->hSc->nonfinite) return fail(h, "Non finite value of constraint evaluation detected\n");
   if (!h->hSc->mean_feasible) return 0;
@@ -803,7 +765,7 @@ int update_and_handle_constraints(kcma* h) {
     h->scalars_fresh = false;
   }
   for (int iter = 0; iter < 100000; iter++) {
-    if (pull_scalars(h)) return 1;
+    if (pull_cached(h)) return 1;
     if (h->hSc->nonfinite) return fail(h, "Non finite value of constraint evaluation detected\n");
     if (h->hSc->max_violation_count == 0) break;
     int J, nv, aborted;
@@ -814,7 +776,7 @@ int update_and_handle_constraints(kcma* h) {
       h->launches++;
       h->scalars_fresh = false;
       CUDA_OK(h, cudaMemcpyAsync(h->hCount, h->dCount, 2 * sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-      if (pull_scalars(h)) return 1;
+      if (pull_cached(h)) return 1;
       J = h->hCount[0]; nv = h->hCount[1]; aborted = h->hSc->adaptation_abort;
       int splits = 1;
       if (J > 0) {
@@ -902,7 +864,7 @@ int do_eval(kcma* h) {
     for (size_t i = 0; i < ls; i++)  // ref: optimization.cpp.base:32-33
       if (!std::isfinite(h->hF[i])) {
         if (h->cfg.nranks == 1) return fail(h, "Non finite value of function evaluation detected: %f\n", h->hF[i]);
-        if (pull_scalars(h)) return 1;      // several ranks: fail collectively at the end of the generation (flag in the all-reduce)
+        if (pull_cached(h)) return 1;      // several ranks: fail collectively at the end of the generation (flag in the all-reduce)
         h->hSc->nonfinite = 1;
         if (push_scalars(h)) return 1;
         h->hF[i] = -1e300;
@@ -1029,7 +991,7 @@ int do_tell(kcma* h) {
 }
 
 int end_of_generation(kcma* h) {
-  if (pull_scalars(h)) return 1;
+  if (pull_cached(h)) return 1;
   if (h->timing) resolve_timers(h);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return fail(h, "CUDA error after generation: %s", cudaGetErrorString(e));
@@ -1089,7 +1051,7 @@ void kcma_shard_range(uint64_t population, int mirrored, int rank, int nranks, u
   *end = e * unit;
 }
 
-const char* kcma_last_error(const kcma_t* h) { return h ? h->err.c_str() : g_create_err; }
+const char* kcma_last_error(const kcma_t* h) { return h ? h->err.c_str() : kcma::create_err; }
 
 const char* kcma_take_warnings(kcma_t* h) {
   strncpy(h->warn_out, h->warn.c_str(), sizeof(h->warn_out) - 1);
@@ -1100,46 +1062,29 @@ const char* kcma_take_warnings(kcma_t* h) {
 
 namespace { void invalidate_graph(kcma* h); }
 
-void kcma_destroy(kcma_t* h) {
-  if (!h) return;
-  cudaSetDevice(h->device);
-  cudaStreamSynchronize(h->stream);
-  invalidate_graph(h);
-  if (h->cap_stream) cudaStreamDestroy(h->cap_stream);
-  if (h->comm && g_nccl.CommDestroy) g_nccl.CommDestroy(h->comm);
-  kc::tridiag_ws_destroy(h->tri);
-  void* ptrs[] = {h->dC, h->dB, h->dA, h->dD, h->dVT, h->dVTw, h->dGT, h->dEv, h->dPerm, h->dMean, h->dMeanOld, h->dMeanUpd, h->dT,
-                  h->dPs, h->dPc, h->dZ, h->dY, h->dX, h->dF, h->dIdx, h->dSortWs, h->dW, h->dSelW, h->dSelS, h->dCount, h->dS,
-                  h->dPartial, h->dWsplit, h->dRed, h->dBestEver, h->dCurBest, h->dLower, h->dUpper, h->dMinSd, h->dCoef, h->dShift,
-                  h->dSigmaSampling, h->dInfeasible, h->dFlush, h->dSc, h->dG, h->dBounds, h->dNormal, h->dCaux, h->dBestCon, h->dU, h->dViol,
-                  h->dIndicator, h->dEvSample, h->dEvCon, h->dVioRows, h->dAttempt, h->dGrad, h->dGran, h->dMask,
-                  h->dMaskSigma, h->dDiscMut};
-  for (void* p : ptrs) if (p) cudaFree(p);
-  if (h->hSc) cudaFreeHost(h->hSc);
-  if (h->hCount) cudaFreeHost(h->hCount);
-  if (h->hRound) cudaFreeHost(h->hRound);
-  cudaFree(h->dFresh); cudaFree(h->dRound); cudaFree(h->dRoundV);
-  for (auto& p : h->pending) { cudaEventDestroy(p.a); cudaEventDestroy(p.b); }
-  for (auto e : h->event_pool) cudaEventDestroy(e);
-  delete h;
+kcma::~kcma() {
+  cudaSetDevice(device);
+  cudaStreamSynchronize(stream);
+  invalidate_graph(this);
+  if (cap_stream) cudaStreamDestroy(cap_stream);
+  if (comm && g_nccl.CommDestroy) g_nccl.CommDestroy(comm);
+  kc::tridiag_ws_destroy(tri);
+  for (auto& p : pending) { cudaEventDestroy(p.a); cudaEventDestroy(p.b); }
+  for (auto e : event_pool) cudaEventDestroy(e);
 }
+
+void kcma_destroy(kcma_t* h) { delete h; }
 
 int kcma_create(const kcma_cfg* cfg, kcma_t** out) {
   *out = nullptr;
-  g_create_err[0] = 0;
-  if (!cfg || cfg->abi_version != KCMA_ABI_VERSION) return fail(nullptr, "kcma_cfg ABI version mismatch");
-  if (cfg->n == 0) return fail(nullptr, "Optimization Evaluation problems require at least one variable.\n");
-  if (cfg->n > 32768) return fail(nullptr, "Variable Count %zu exceeds the supported maximum (32768)", (size_t)cfg->n);
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0)
-    return fail(nullptr, "libkcma needs a CUDA device (sm_100a); none is visible. There is no CPU fallback.");
-  if (cfg->device < 0 || cfg->device >= ndev) return fail(nullptr, "invalid CUDA device %d", cfg->device);
+  kcma::create_err[0] = 0;
+  if (!cfg || cfg->abi_version != KCMA_ABI_VERSION) return fail<kcma>(nullptr, "kcma_cfg ABI version mismatch");
+  if (cfg->n == 0) return fail<kcma>(nullptr, "Optimization Evaluation problems require at least one variable.\n");
+  if (cfg->n > 32768) return fail<kcma>(nullptr, "Variable Count %zu exceeds the supported maximum (32768)", (size_t)cfg->n);
+  if (open_device<kcma>(cfg->device)) return 1;
   kcma* h = new kcma();
   h->cfg = *cfg;
   h->device = cfg->device;
-#define CREATE_FAIL(...) do { fail(nullptr, __VA_ARGS__); kcma_destroy(h); return 1; } while (0)
-#define CREATE_CUDA(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) CREATE_FAIL("CUDA error %s (%s)", cudaGetErrorString(e_), #call); } while (0)
-  CREATE_CUDA(cudaSetDevice(h->device));
   cudaDeviceGetAttribute(&h->num_sms, cudaDevAttrMultiProcessorCount, h->device);
   const int N = h->N = (int)cfg->n;
   const int ld = h->ld = round_up(N, 16);
@@ -1153,12 +1098,12 @@ int kcma_create(const kcma_cfg* cfg, kcma_t** out) {
   h->gran = copyv(cfg->granularity, N, 0.0);
   h->cfg.granularity = nullptr;
   for (int i = 0; i < N; i++) {   // CMAES.cpp.base:44-50
-    if (h->gran[i] < 0.0) { char msg[96]; snprintf(msg, sizeof(msg), "Negative granularity for variable %d.\n", i); CREATE_FAIL(msg); }
+    if (h->gran[i] < 0.0) return create_fail(h, "Negative granularity for variable %d.\n", i);
     if (h->gran[i] > 0.0) h->has_discrete = true;
   }
   if (h->has_discrete) {
-    if (cfg->n_constraints > 0) CREATE_FAIL("discrete variables together with constraints are not supported");
-    if (cfg->max_infeasible_resamplings != 0) CREATE_FAIL("discrete variables with resampling rounds (Max Infeasible Resamplings > 0) are not supported");
+    if (cfg->n_constraints > 0) return create_fail(h, "discrete variables together with constraints are not supported");
+    if (cfg->max_infeasible_resamplings != 0) return create_fail(h, "discrete variables with resampling rounds (Max Infeasible Resamplings > 0) are not supported");
     h->cfg.keep_population = 1;   // after the discrete mutations X is no longer mean + sigma * y: it is materialised
   }
   h->coef.resize(N);
@@ -1173,49 +1118,46 @@ int kcma_create(const kcma_cfg* cfg, kcma_t** out) {
   }
   // ref :26-31
   uint64_t lambda = cfg->population_size, mu = cfg->mu_value, vlambda = cfg->viability_population_size, vmu = cfg->viability_mu_value;
-  if (cfg->use_gradient_information && cfg->gradient_step_size <= 0.) {   // CMAES.cpp.base:86
-    char msg[128];
-    snprintf(msg, sizeof(msg), "Gradient Step Size must be larger than 0.0 (is %f)", cfg->gradient_step_size);
-    CREATE_FAIL(msg);
-  }
-  if (lambda <= 1) CREATE_FAIL("'Population Size' must be larger 1.");
+  if (cfg->use_gradient_information && cfg->gradient_step_size <= 0.)   // CMAES.cpp.base:86
+    return create_fail(h, "Gradient Step Size must be larger than 0.0 (is %f)", cfg->gradient_step_size);
+  if (lambda <= 1) return create_fail(h, "'Population Size' must be larger 1.");
   if (mu == 0) mu = lambda / 2;
   if (vmu == 0) vmu = vlambda / 2;
-  if (mu > lambda) CREATE_FAIL("'Mu Value' (%zu) must not exceed 'Population Size' (%zu).", (size_t)mu, (size_t)lambda);
+  if (mu > lambda) return create_fail(h, "'Mu Value' (%zu) must not exceed 'Population Size' (%zu).", (size_t)mu, (size_t)lambda);
   h->lambda = lambda; h->mu = mu; h->vlambda = vlambda; h->vmu = vmu;
   h->cfg.mu_value = mu; h->cfg.viability_mu_value = vmu;
   h->has_constraints = h->n_con > 0;
   h->s_max = std::max(lambda, h->has_constraints ? vlambda : lambda);
   h->mu_max = std::max(mu, h->has_constraints ? vmu : mu);
-  if (h->s_max >= (1ull << 31)) CREATE_FAIL("'Population Size' too large");
+  if (h->s_max >= (1ull << 31)) return create_fail(h, "'Population Size' too large");
   h->chi_n = sqrt((double)N) * (1. - 1. / (4. * N) + 1. / (21. * N * N));
   h->is_viability = h->has_constraints;
   if (cfg->mirrored_sampling) {  // ref :89-93
-    if (lambda % 2 == 1) CREATE_FAIL("Mirrored Sampling can only be applied with an even Sample Population (is %zu)", (size_t)lambda);
-    if (h->has_constraints) CREATE_FAIL("Mirrored Sampling not applicable to problems with constraints");
+    if (lambda % 2 == 1) return create_fail(h, "Mirrored Sampling can only be applied with an even Sample Population (is %zu)", (size_t)lambda);
+    if (h->has_constraints) return create_fail(h, "Mirrored Sampling not applicable to problems with constraints");
   }
-  if (cfg->nranks < 1 || cfg->rank < 0 || cfg->rank >= cfg->nranks) CREATE_FAIL("invalid rank %d of %d", cfg->rank, cfg->nranks);
+  if (cfg->nranks < 1 || cfg->rank < 0 || cfg->rank >= cfg->nranks) return create_fail(h, "invalid rank %d of %d", cfg->rank, cfg->nranks);
   if (cfg->nranks > 1) {
     const uint64_t unit = (cfg->mirrored_sampling ? 2 : 1) * (uint64_t)cfg->nranks;
     if (lambda % unit || (h->has_constraints && vlambda % unit))
-      CREATE_FAIL("population size must be divisible by %zu to shard it across %d GPUs", (size_t)unit, cfg->nranks);
+      return create_fail(h, "population size must be divisible by %zu to shard it across %d GPUs", (size_t)unit, cfg->nranks);
   }
   for (int i = 0; i < N; ++i) {  // ref :111-126
     if (!std::isfinite(h->init_val[i])) {
-      if (!std::isfinite(h->lower[i])) CREATE_FAIL("'Initial Value' of variable 'X%d' not defined, and cannot be inferred because variable lower bound is not finite.\n", i);
-      if (!std::isfinite(h->upper[i])) CREATE_FAIL("'Initial Value' of variable 'X%d' not defined, and cannot be inferred because variable upper bound is not finite.\n", i);
+      if (!std::isfinite(h->lower[i])) return create_fail(h, "'Initial Value' of variable 'X%d' not defined, and cannot be inferred because variable lower bound is not finite.\n", i);
+      if (!std::isfinite(h->upper[i])) return create_fail(h, "'Initial Value' of variable 'X%d' not defined, and cannot be inferred because variable upper bound is not finite.\n", i);
       h->init_val[i] = (h->upper[i] + h->lower[i]) * 0.5;
     }
     if (!std::isfinite(h->init_sd[i])) {
-      if (!std::isfinite(h->lower[i])) CREATE_FAIL("Initial (Mean) Value of variable 'X%d' not defined, and cannot be inferred because variable lower bound is not finite.\n", i);
-      if (!std::isfinite(h->upper[i])) CREATE_FAIL("Initial Standard Deviation 'X%d' not defined, and cannot be inferred because variable upper bound is not finite.\n", i);
+      if (!std::isfinite(h->lower[i])) return create_fail(h, "Initial (Mean) Value of variable 'X%d' not defined, and cannot be inferred because variable lower bound is not finite.\n", i);
+      if (!std::isfinite(h->upper[i])) return create_fail(h, "Initial Standard Deviation 'X%d' not defined, and cannot be inferred because variable upper bound is not finite.\n", i);
       h->init_sd[i] = (h->upper[i] - h->lower[i]) * 0.3;
     }
   }
   if (h->has_constraints) {
-    if ((cfg->global_success_learning_rate <= 0.0) || (cfg->global_success_learning_rate > 1.0)) CREATE_FAIL("Invalid Global Success Learning Rate (%f), must be greater than 0.0 and less than 1.0\n", cfg->global_success_learning_rate);
-    if ((cfg->target_success_rate <= 0.0) || (cfg->target_success_rate > 1.0)) CREATE_FAIL("Invalid Target Success Rate (%f), must be greater than 0.0 and less than 1.0\n", cfg->target_success_rate);
-    if (cfg->covariance_matrix_adaption_strength <= 0.0) CREATE_FAIL("Invalid Adaption Size (%f), must be greater than 0.0\n", cfg->covariance_matrix_adaption_strength);
+    if ((cfg->global_success_learning_rate <= 0.0) || (cfg->global_success_learning_rate > 1.0)) return create_fail(h, "Invalid Global Success Learning Rate (%f), must be greater than 0.0 and less than 1.0\n", cfg->global_success_learning_rate);
+    if ((cfg->target_success_rate <= 0.0) || (cfg->target_success_rate > 1.0)) return create_fail(h, "Invalid Target Success Rate (%f), must be greater than 0.0 and less than 1.0\n", cfg->target_success_rate);
+    if (cfg->covariance_matrix_adaption_strength <= 0.0) return create_fail(h, "Invalid Adaption Size (%f), must be greater than 0.0\n", cfg->covariance_matrix_adaption_strength);
   }
   h->repl = h->has_constraints && cfg->nranks > 1;
   set_population(h, h->is_viability ? vlambda : lambda, h->is_viability ? vmu : mu);
@@ -1227,59 +1169,59 @@ int kcma_create(const kcma_cfg* cfg, kcma_t** out) {
     h->max_zrows = cfg->mirrored_sampling ? h->max_local / 2 : h->max_local;
   }
   const size_t nn = (size_t)N * ld;
-  CREATE_CUDA(dmalloc(&h->dC, nn)); CREATE_CUDA(dmalloc(&h->dB, nn)); CREATE_CUDA(dmalloc(&h->dA, nn));
-  CREATE_CUDA(dmalloc(&h->dVT, nn)); CREATE_CUDA(dmalloc(&h->dVTw, nn)); CREATE_CUDA(dmalloc(&h->dGT, nn));
-  CREATE_CUDA(dmalloc(&h->dD, ld)); CREATE_CUDA(dmalloc(&h->dEv, ld)); CREATE_CUDA(dmalloc(&h->dPerm, ld));
-  CREATE_CUDA(dmalloc(&h->dMean, ld)); CREATE_CUDA(dmalloc(&h->dMeanOld, ld)); CREATE_CUDA(dmalloc(&h->dMeanUpd, ld));
-  CREATE_CUDA(dmalloc(&h->dT, ld)); CREATE_CUDA(dmalloc(&h->dPs, ld)); CREATE_CUDA(dmalloc(&h->dPc, ld));
-  CREATE_CUDA(dmalloc(&h->dBestEver, ld)); CREATE_CUDA(dmalloc(&h->dCurBest, ld));
-  CREATE_CUDA(dmalloc(&h->dZ, h->max_zrows * ld)); CREATE_CUDA(dmalloc(&h->dY, h->max_zrows * ld));
-  CREATE_CUDA(dmalloc(&h->dX, (h->cfg.keep_population ? h->max_local : 1) * (size_t)ld));
-  if (cfg->use_gradient_information) CREATE_CUDA(dmalloc(&h->dGrad, h->max_local * (size_t)ld));
+  Allocations& m = h->mem;
+  CREATE_OK(h, alloc(m, &h->dC, nn)); CREATE_OK(h, alloc(m, &h->dB, nn)); CREATE_OK(h, alloc(m, &h->dA, nn));
+  CREATE_OK(h, alloc(m, &h->dVT, nn)); CREATE_OK(h, alloc(m, &h->dVTw, nn)); CREATE_OK(h, alloc(m, &h->dGT, nn));
+  CREATE_OK(h, alloc(m, &h->dD, ld)); CREATE_OK(h, alloc(m, &h->dEv, ld)); CREATE_OK(h, alloc(m, &h->dPerm, ld));
+  CREATE_OK(h, alloc(m, &h->dMean, ld)); CREATE_OK(h, alloc(m, &h->dMeanOld, ld)); CREATE_OK(h, alloc(m, &h->dMeanUpd, ld));
+  CREATE_OK(h, alloc(m, &h->dT, ld)); CREATE_OK(h, alloc(m, &h->dPs, ld)); CREATE_OK(h, alloc(m, &h->dPc, ld));
+  CREATE_OK(h, alloc(m, &h->dBestEver, ld)); CREATE_OK(h, alloc(m, &h->dCurBest, ld));
+  CREATE_OK(h, alloc(m, &h->dZ, h->max_zrows * ld)); CREATE_OK(h, alloc(m, &h->dY, h->max_zrows * ld));
+  CREATE_OK(h, alloc(m, &h->dX, (h->cfg.keep_population ? h->max_local : 1) * (size_t)ld));
+  if (cfg->use_gradient_information) CREATE_OK(h, alloc(m, &h->dGrad, h->max_local * (size_t)ld));
   if (h->has_discrete) {
-    CREATE_CUDA(dmalloc(&h->dGran, ld)); CREATE_CUDA(dmalloc(&h->dMask, ld)); CREATE_CUDA(dmalloc(&h->dMaskSigma, ld));
-    CREATE_CUDA(dmalloc(&h->dDiscMut, h->max_local * (size_t)ld));
-    CREATE_CUDA(cudaMemcpy(h->dGran, h->gran.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
+    CREATE_OK(h, alloc(m, &h->dGran, ld)); CREATE_OK(h, alloc(m, &h->dMask, ld)); CREATE_OK(h, alloc(m, &h->dMaskSigma, ld));
+    CREATE_OK(h, alloc(m, &h->dDiscMut, h->max_local * (size_t)ld));
+    CREATE_OK(h, cudaMemcpy(h->dGran, h->gran.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
   }
-  CREATE_CUDA(dmalloc(&h->dF, h->s_max)); CREATE_CUDA(dmalloc(&h->dIdx, h->s_max));
-  CREATE_CUDA(cudaMalloc(&h->dSortWs, sort_workspace_bytes((int)h->s_max)));
-  CREATE_CUDA(dmalloc(&h->dW, h->mu_max));
+  CREATE_OK(h, alloc(m, &h->dF, h->s_max)); CREATE_OK(h, alloc(m, &h->dIdx, h->s_max));
+  CREATE_OK(h, alloc(m, &h->dSortWs, sort_workspace_bytes((int)h->s_max)));
+  CREATE_OK(h, alloc(m, &h->dW, h->mu_max));
   const uint64_t max_sel = std::max<uint64_t>(std::min(h->mu_max, h->max_local), h->max_zrows);
-  CREATE_CUDA(dmalloc(&h->dSelW, max_sel + 16)); CREATE_CUDA(dmalloc(&h->dSelS, max_sel + 16)); CREATE_CUDA(dmalloc(&h->dCount, 4));
+  CREATE_OK(h, alloc(m, &h->dSelW, max_sel + 16)); CREATE_OK(h, alloc(m, &h->dSelS, max_sel + 16)); CREATE_OK(h, alloc(m, &h->dCount, 4));
   h->s_rows_padded = round_up((int)std::min(h->mu_max, h->max_local), 16) + 16;
-  CREATE_CUDA(dmalloc(&h->dS, (size_t)h->s_rows_padded * ld));
-  CREATE_CUDA(dmalloc(&h->dPartial, ((size_t)h->s_rows_padded / h->rows_per_cta + 2) * ld));
-  CREATE_CUDA(dmalloc(&h->dWsplit, (size_t)h->max_splits * nn));
-  CREATE_CUDA(dmalloc(&h->dRed, nn + 2 * (size_t)ld + 16));
-  CREATE_CUDA(dmalloc(&h->dLower, ld)); CREATE_CUDA(dmalloc(&h->dUpper, ld)); CREATE_CUDA(dmalloc(&h->dMinSd, ld));
-  CREATE_CUDA(dmalloc(&h->dCoef, ld)); CREATE_CUDA(dmalloc(&h->dShift, h->n_con + 1));
-  CREATE_CUDA(dmalloc(&h->dSigmaSampling, 2)); CREATE_CUDA(dmalloc(&h->dInfeasible, h->max_local + 16));
-  CREATE_CUDA(dmalloc(&h->dSc, 1));
-  CREATE_CUDA(dmalloc(&h->dAttempt, h->max_zrows + 16));
+  CREATE_OK(h, alloc(m, &h->dS, (size_t)h->s_rows_padded * ld));
+  CREATE_OK(h, alloc(m, &h->dPartial, ((size_t)h->s_rows_padded / h->rows_per_cta + 2) * ld));
+  CREATE_OK(h, alloc(m, &h->dWsplit, (size_t)h->max_splits * nn));
+  CREATE_OK(h, alloc(m, &h->dRed, nn + 2 * (size_t)ld + 16));
+  CREATE_OK(h, alloc(m, &h->dLower, ld)); CREATE_OK(h, alloc(m, &h->dUpper, ld)); CREATE_OK(h, alloc(m, &h->dMinSd, ld));
+  CREATE_OK(h, alloc(m, &h->dCoef, ld)); CREATE_OK(h, alloc(m, &h->dShift, h->n_con + 1));
+  CREATE_OK(h, alloc(m, &h->dSigmaSampling, 2)); CREATE_OK(h, alloc(m, &h->dInfeasible, h->max_local + 16));
+  CREATE_OK(h, alloc(m, &h->dSc, 1));
+  CREATE_OK(h, alloc(m, &h->dAttempt, h->max_zrows + 16));
   if (h->has_constraints) {
-    if (cfg->constraint_family != KCMA_CON_HALFSPACE && cfg->constraint_family != KCMA_CON_EXTERNAL) CREATE_FAIL("unknown constraint family %d", cfg->constraint_family);
-    if (cfg->nranks > 1 && cfg->use_gradient_information) CREATE_FAIL("Use Gradient Information together with constraints runs on one GPU (nranks must be 1)");
+    if (cfg->constraint_family != KCMA_CON_HALFSPACE && cfg->constraint_family != KCMA_CON_EXTERNAL) return create_fail(h, "unknown constraint family %d", cfg->constraint_family);
+    if (cfg->nranks > 1 && cfg->use_gradient_information) return create_fail(h, "Use Gradient Information together with constraints runs on one GPU (nranks must be 1)");
     h->ldg = (long long)h->s_max;
     h->u_rows = round_up((int)std::min<uint64_t>(h->n_con * h->s_max, 1u << 22), 16) + 32;
-    CREATE_CUDA(dmalloc(&h->dG, h->n_con * h->s_max)); CREATE_CUDA(dmalloc(&h->dBounds, h->n_con)); CREATE_CUDA(dmalloc(&h->dNormal, h->n_con * ld));
-    CREATE_CUDA(dmalloc(&h->dCaux, nn)); CREATE_CUDA(dmalloc(&h->dBestCon, h->n_con)); CREATE_CUDA(dmalloc(&h->dU, (size_t)h->u_rows * ld));
-    CREATE_CUDA(dmalloc(&h->dViol, h->s_max)); CREATE_CUDA(dmalloc(&h->dIndicator, h->n_con * h->s_max));
-    CREATE_CUDA(dmalloc(&h->dEvSample, h->n_con * h->s_max + 16)); CREATE_CUDA(dmalloc(&h->dEvCon, h->n_con * h->s_max + 16));
-    CREATE_CUDA(dmalloc(&h->dVioRows, h->s_max + 16));
+    CREATE_OK(h, alloc(m, &h->dG, h->n_con * h->s_max)); CREATE_OK(h, alloc(m, &h->dBounds, h->n_con)); CREATE_OK(h, alloc(m, &h->dNormal, h->n_con * ld));
+    CREATE_OK(h, alloc(m, &h->dCaux, nn)); CREATE_OK(h, alloc(m, &h->dBestCon, h->n_con)); CREATE_OK(h, alloc(m, &h->dU, (size_t)h->u_rows * ld));
+    CREATE_OK(h, alloc(m, &h->dViol, h->s_max)); CREATE_OK(h, alloc(m, &h->dIndicator, h->n_con * h->s_max));
+    CREATE_OK(h, alloc(m, &h->dEvSample, h->n_con * h->s_max + 16)); CREATE_OK(h, alloc(m, &h->dEvCon, h->n_con * h->s_max + 16));
+    CREATE_OK(h, alloc(m, &h->dVioRows, h->s_max + 16));
     h->normal_lr = 1.0 / (2.0 + N);                                           // ref :154
     h->cov_adaption_factor = cfg->covariance_matrix_adaption_strength / (N + 2.);  // ref :155
   }
-  CREATE_CUDA(cudaMallocHost((void**)&h->hSc, sizeof(DevScalars)));
-  CREATE_CUDA(cudaMallocHost((void**)&h->hCount, 4 * sizeof(int)));
-  CREATE_CUDA(cudaMallocHost((void**)&h->hRound, 2 * sizeof(unsigned long long)));
-  CREATE_CUDA(dmalloc(&h->dRound, 2)); CREATE_CUDA(dmalloc(&h->dFresh, h->max_local + 16));
-  CREATE_CUDA(dmalloc(&h->dRoundV, (size_t)(h->cfg.nranks > 0 ? h->cfg.nranks : 1)));
-  memset(h->hSc, 0, sizeof(DevScalars));
-  CREATE_CUDA(cudaMemcpy(h->dLower, h->lower.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
-  CREATE_CUDA(cudaMemcpy(h->dUpper, h->upper.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
-  CREATE_CUDA(cudaMemcpy(h->dMinSd, h->min_sd.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
-  CREATE_CUDA(cudaMemcpy(h->dCoef, h->coef.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
-  if (h->n_con) CREATE_CUDA(cudaMemcpy(h->dShift, h->con_shift.data(), sizeof(double) * h->n_con, cudaMemcpyHostToDevice));
+  CREATE_OK(h, alloc_host(m, &h->hSc, 1));
+  CREATE_OK(h, alloc_host(m, &h->hCount, 4));
+  CREATE_OK(h, alloc_host(m, &h->hRound, 2));
+  CREATE_OK(h, alloc(m, &h->dRound, 2)); CREATE_OK(h, alloc(m, &h->dFresh, h->max_local + 16));
+  CREATE_OK(h, alloc(m, &h->dRoundV, (size_t)(h->cfg.nranks > 0 ? h->cfg.nranks : 1)));
+  CREATE_OK(h, cudaMemcpy(h->dLower, h->lower.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
+  CREATE_OK(h, cudaMemcpy(h->dUpper, h->upper.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
+  CREATE_OK(h, cudaMemcpy(h->dMinSd, h->min_sd.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
+  CREATE_OK(h, cudaMemcpy(h->dCoef, h->coef.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
+  if (h->n_con) CREATE_OK(h, cudaMemcpy(h->dShift, h->con_shift.data(), sizeof(double) * h->n_con, cudaMemcpyHostToDevice));
   // ref :20-24, :138/159, :175-183
   DevScalars s; memset(&s, 0, sizeof(s));
   s.best_ever_value = s.previous_best_ever_value = s.previous_best_value = s.current_best_value = -INFINITY;
@@ -1288,28 +1230,26 @@ int kcma_create(const kcma_cfg* cfg, kcma_t** out) {
   s.global_success_rate = h->has_constraints ? 0.5 : -1.0;
   s.best_valid_sample = h->has_constraints ? ~0ull : 0ull;
   *h->hSc = s;
-  CREATE_CUDA(cudaMemcpy(h->dSc, h->hSc, sizeof(DevScalars), cudaMemcpyHostToDevice));
+  CREATE_OK(h, cudaMemcpy(h->dSc, h->hSc, sizeof(DevScalars), cudaMemcpyHostToDevice));
   h->h_weights.assign(h->mu_max, 0.0);
-  if (init_mu_weights(h, h->is_viability ? vmu : mu)) { strncpy(g_create_err, h->err.c_str(), sizeof(g_create_err) - 1); kcma_destroy(h); return 1; }
+  if (init_mu_weights(h, h->is_viability ? vmu : mu)) return create_fail(h, "%s", h->err.c_str());
   init_covariance(h);
-  CREATE_CUDA(cudaMemcpy(h->dMean, h->init_val.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
-  CREATE_CUDA(cudaMemcpy(h->dMeanOld, h->init_val.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
-  CREATE_CUDA(cudaDeviceSynchronize());
-#undef CREATE_FAIL
-#undef CREATE_CUDA
+  CREATE_OK(h, cudaMemcpy(h->dMean, h->init_val.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
+  CREATE_OK(h, cudaMemcpy(h->dMeanOld, h->init_val.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
+  CREATE_OK(h, cudaDeviceSynchronize());
   *out = h;
   return 0;
 }
 
 int kcma_set_host_objective(kcma_t* h, kcma_host_objective_fn fn, void* user) {
-  if (!h) return fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   invalidate_graph(h);
   if (fn && !h->cfg.keep_population) return fail(h, "a host objective needs keep_population = 1 (X is copied to the host every generation)");
   h->host_obj = fn; h->host_obj_user = user;
   return 0;
 }
 int kcma_set_host_objective_grad(kcma_t* h, kcma_host_objective_grad_fn fn, void* user) {
-  if (!h) return fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   invalidate_graph(h);
   if (fn && !h->cfg.use_gradient_information) return fail(h, "a gradient-returning host objective needs Use Gradient Information");
   if (fn && !h->cfg.keep_population) return fail(h, "a host objective needs keep_population = 1 (X is copied to the host every generation)");
@@ -1317,7 +1257,7 @@ int kcma_set_host_objective_grad(kcma_t* h, kcma_host_objective_grad_fn fn, void
   return 0;
 }
 int kcma_set_device_objective(kcma_t* h, kcma_device_objective_fn fn, void* user) {
-  if (!h) return fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   invalidate_graph(h);
   if (fn && !h->cfg.keep_population) return fail(h, "a device objective needs keep_population = 1 (it reads the materialised X)");
   if (fn && h->cfg.use_gradient_information) return fail(h, "a device objective cannot return gradients: use kcma_set_host_objective_grad");
@@ -1325,7 +1265,7 @@ int kcma_set_device_objective(kcma_t* h, kcma_device_objective_fn fn, void* user
   return 0;
 }
 int kcma_set_host_constraints(kcma_t* h, kcma_host_constraints_fn fn, void* user) {
-  if (!h) return fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   invalidate_graph(h);
   if (!h->has_constraints) return fail(h, "the problem has no constraints (n_constraints = 0)");
   if (fn && !h->cfg.keep_population) return fail(h, "host constraints need keep_population = 1 (X is copied to the host)");
@@ -1335,15 +1275,15 @@ int kcma_set_host_constraints(kcma_t* h, kcma_host_constraints_fn fn, void* user
 
 int kcma_comm_unique_id(uint8_t id_out[128]) {
   std::string err;
-  if (!g_nccl.load(err)) return fail(nullptr, "%s", err.c_str());
+  if (!g_nccl.load(err)) return fail<kcma>(nullptr, "%s", err.c_str());
   ncclUniqueId id;
-  if (g_nccl.GetUniqueId(&id) != ncclSuccess) return fail(nullptr, "ncclGetUniqueId failed");
+  if (g_nccl.GetUniqueId(&id) != ncclSuccess) return fail<kcma>(nullptr, "ncclGetUniqueId failed");
   memcpy(id_out, id.internal, 128);
   return 0;
 }
 
 int kcma_comm_init(kcma_t* h, const uint8_t id_in[128]) {
-  if (!h) return fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   std::string err;
   if (!g_nccl.load(err)) return fail(h, "%s", err.c_str());
   CUDA_OK(h, cudaSetDevice(h->device));
@@ -1354,11 +1294,11 @@ int kcma_comm_init(kcma_t* h, const uint8_t id_in[128]) {
 
 // All ranks of ONE process (one handle per device, rank r = handles[r]): the communicator is built inside an NCCL group.
 int kcma_comm_init_all(kcma_t** handles, int count) {
-  if (!handles || count < 1) return fail(nullptr, "kcma_comm_init_all: no handles");
+  if (!handles || count < 1) return fail<kcma>(nullptr, "kcma_comm_init_all: no handles");
   std::string err;
   if (!g_nccl.load(err)) return fail(handles[0], "%s", err.c_str());
   for (int r = 0; r < count; r++) {
-    if (!handles[r]) return fail(nullptr, "null solver handle");
+    if (!handles[r]) return fail(handles[r], "null solver handle");
     if (handles[r]->cfg.nranks != count || handles[r]->cfg.rank != r)
       return fail(handles[r], "kcma_comm_init_all: handle %d was created as rank %d of %d, expected rank %d of %d", r, handles[r]->cfg.rank,
                   handles[r]->cfg.nranks, r, count);
@@ -1378,16 +1318,16 @@ int kcma_comm_init_all(kcma_t** handles, int count) {
 }
 
 int kcma_ask(kcma_t* h) {
-  if (!h) return fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   CUDA_OK(h, cudaSetDevice(h->device));
   return do_ask(h);
 }
 
 int kcma_eval(kcma_t* h) {
-  if (!h) return fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   CUDA_OK(h, cudaSetDevice(h->device));
   if (do_eval(h)) return 1;
-  if (pull_scalars(h)) return 1;
+  if (pull_cached(h)) return 1;
   if (h->hSc->nonfinite) {
     h->hSc->nonfinite = 0;
     push_scalars(h);
@@ -1397,7 +1337,7 @@ int kcma_eval(kcma_t* h) {
 }
 
 int kcma_tell(kcma_t* h) {
-  if (!h) return fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   CUDA_OK(h, cudaSetDevice(h->device));
   if (do_tell(h)) return 1;
   return end_of_generation(h);
@@ -1473,7 +1413,7 @@ bool build_graph(kcma* h) {
 }  // namespace
 
 int kcma_run_generation(kcma_t* h) {
-  if (!h) return fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   CUDA_OK(h, cudaSetDevice(h->device));
   if (graph_eligible(h) && (h->gexec || build_graph(h))) {
     // The replay takes the generation from DevScalars::gen (inc_gen_kernel is its first node). Eager generations in between
@@ -1495,8 +1435,8 @@ int kcma_run_generation(kcma_t* h) {
 }
 
 int kcma_check_termination(kcma_t* h, int* finished, const char** reason) {
-  if (!h) return fail(nullptr, "null solver handle");
-  if (pull_scalars(h)) return 1;
+  if (!h) return fail(h, "null solver handle");
+  if (pull_cached(h)) return 1;
   const DevScalars& s = *h->hSc;
   int fin = 0;
   h->reason.clear();
@@ -1520,17 +1460,7 @@ int kcma_check_termination(kcma_t* h, int* finished, const char** reason) {
 }
 
 int kcma_run(kcma_t* h, uint64_t max_generations, uint64_t* done) {
-  if (!h) return fail(nullptr, "null solver handle");
-  uint64_t n = 0;
-  int fin = 0;
-  while (n < max_generations) {
-    if (kcma_check_termination(h, &fin, nullptr)) { if (done) *done = n; return 1; }
-    if (fin) break;
-    if (kcma_run_generation(h)) { if (done) *done = n; return 1; }
-    n++;
-  }
-  if (done) *done = n;
-  return 0;
+  return run(h, max_generations, done, kcma_check_termination, kcma_run_generation);
 }
 
 // ---- injection ---------------------------------------------------------------------------------------------
@@ -1542,7 +1472,7 @@ static int upload_rows(kcma* h, double* dst, const double* src, size_t rows) {
 }
 
 int kcma_inject(kcma_t* h, int kind, const double* src, size_t count) {
-  if (!h) return fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   invalidate_graph(h);
   CUDA_OK(h, cudaSetDevice(h->device));
   const size_t N = h->N;
@@ -1592,7 +1522,7 @@ int kcma_inject(kcma_t* h, int kind, const double* src, size_t count) {
       if (count != N * N + N) return fail(h, "inject BD: expected N*N+N values");
       if (upload_rows(h, h->dB, src, N)) return 1;
       CUDA_OK(h, cudaMemcpy(h->dD, src + N * N, sizeof(double) * N, cudaMemcpyHostToDevice));
-      if (pull_scalars(h)) return 1;
+      if (pull_cached(h)) return 1;
       double mn = INFINITY, mx = -INFINITY;
       for (size_t d = 0; d < N; d++) { const double ev = src[N * N + d] * src[N * N + d]; mn = std::min(mn, ev); mx = std::max(mx, ev); }
       h->hSc->min_eig = mn; h->hSc->max_eig = mx;
@@ -1607,30 +1537,29 @@ int kcma_inject(kcma_t* h, int kind, const double* src, size_t count) {
 
 // ---- state access ---------------------------------------------------------------------------------------------
 namespace {
-struct ArrRef { double* p; size_t rows, cols; int ld; };  // rows x cols with leading dimension ld (ld = cols: dense)
-bool find_array(kcma* h, const char* key, ArrRef* r) {
-  const size_t N = h->N; const int ld = h->ld;
-#define A(K, P, R, C, LD) if (!strcmp(key, K)) { r->p = (P); r->rows = (R); r->cols = (C); r->ld = (LD); return true; }
-  A("Covariance Matrix", h->dC, N, N, ld)
-  A("Covariance Eigenvector Matrix", h->dB, N, N, ld)
-  A("Axis Lengths", h->dD, 1, N, ld)
-  A("Current Mean", h->dMean, 1, N, ld)
-  A("Previous Mean", h->dMeanOld, 1, N, ld)
-  A("Mean Update", h->dMeanUpd, 1, N, ld)
-  A("Evolution Path", h->dPc, 1, N, ld)
-  A("Conjugate Evolution Path", h->dPs, 1, N, ld)
-  A("Auxiliar BDZ Matrix", h->dT, 1, N, ld)
-  A("Mu Weights", h->dW, 1, h->cur_mu, (int)h->cur_mu)
-  A("Value Vector", h->dF, 1, h->cur_lambda, (int)h->cur_lambda)
-  A("Best Ever Variables", h->dBestEver, 1, N, ld)
-  A("Current Best Variables", h->dCurBest, 1, N, ld)
-  A("Objective Coefficients", h->dCoef, 1, N, ld)
+bool find_array(kcma* h, const char* key, Array* r) {
+  const size_t N = h->N, ld = h->ld;
+#define A(K, ARR) if (!strcmp(key, K)) { *r = ARR; return true; }
+  A("Covariance Matrix", pitched(h->dC, N, N, ld))
+  A("Covariance Eigenvector Matrix", pitched(h->dB, N, N, ld))
+  A("Axis Lengths", dense(h->dD, N))
+  A("Current Mean", dense(h->dMean, N))
+  A("Previous Mean", dense(h->dMeanOld, N))
+  A("Mean Update", dense(h->dMeanUpd, N))
+  A("Evolution Path", dense(h->dPc, N))
+  A("Conjugate Evolution Path", dense(h->dPs, N))
+  A("Auxiliar BDZ Matrix", dense(h->dT, N))
+  A("Mu Weights", dense(h->dW, h->cur_mu))
+  A("Value Vector", dense(h->dF, h->cur_lambda))
+  A("Best Ever Variables", dense(h->dBestEver, N))
+  A("Current Best Variables", dense(h->dCurBest, N))
+  A("Objective Coefficients", dense(h->dCoef, N))
   if (h->has_constraints) {
-    A("Viability Boundaries", h->dBounds, 1, h->n_con, (int)h->n_con)
-    A("Normal Constraint Approximation", h->dNormal, h->n_con, N, ld)
-    A("Best Constraint Evaluations", h->dBestCon, 1, h->n_con, (int)h->n_con)
-    A("Constraint Evaluations", h->dG, h->n_con, h->s_max, (int)h->s_max)
-    A("Auxiliar Covariance Matrix", h->dCaux, N, N, ld)
+    A("Viability Boundaries", dense(h->dBounds, h->n_con))
+    A("Normal Constraint Approximation", pitched(h->dNormal, h->n_con, N, ld))
+    A("Best Constraint Evaluations", dense(h->dBestCon, h->n_con))
+    A("Constraint Evaluations", pitched(h->dG, h->n_con, h->s_max, h->s_max))
+    A("Auxiliar Covariance Matrix", pitched(h->dCaux, N, N, ld))
   }
 #undef A
   return false;
@@ -1638,7 +1567,7 @@ bool find_array(kcma* h, const char* key, ArrRef* r) {
 }  // namespace
 
 int kcma_get_array(kcma_t* h, const char* key, double* out, size_t cap, size_t* count) {
-  if (!h) return fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   CUDA_OK(h, cudaSetDevice(h->device));
   const size_t N = h->N;
   if (!strcmp(key, "BDZ Matrix") || !strcmp(key, "Sample Population")) {
@@ -1647,80 +1576,52 @@ int kcma_get_array(kcma_t* h, const char* key, double* out, size_t cap, size_t* 
     if (count) *count = n;
     if (!out) return 0;
     if (cap < n) return fail(h, "buffer too small for '%s'", key);
-    double* tmp = nullptr;
-    CUDA_OK(h, cudaMalloc(&tmp, sizeof(double) * (n ? n : 1)));
-    if (!strcmp(key, "BDZ Matrix")) {
-      if (h->cfg.mirrored_sampling) expand_mirrored_kernel<<<h->num_sms * 4, 256, 0, h->stream>>>(h->dY, tmp, h->ld, (long long)ls, (int)N);
-      else cudaMemcpy2DAsync(tmp, sizeof(double) * N, h->dY, sizeof(double) * h->ld, sizeof(double) * N, ls, cudaMemcpyDeviceToDevice, h->stream);
-    } else if (h->cfg.keep_population) {
-      cudaMemcpy2DAsync(tmp, sizeof(double) * N, h->dX, sizeof(double) * h->ld, sizeof(double) * N, ls, cudaMemcpyDeviceToDevice, h->stream);
-    } else {
-      cudaFree(tmp);
+    if (strcmp(key, "BDZ Matrix") && !h->cfg.keep_population)
       return fail(h, "'Sample Population' is not materialised: create the handle with keep_population = 1");
-    }
+    Allocations scratch;
+    double* tmp = nullptr;
+    CUDA_OK(h, alloc(scratch, &tmp, n));
+    if (strcmp(key, "BDZ Matrix"))
+      cudaMemcpy2DAsync(tmp, sizeof(double) * N, h->dX, sizeof(double) * h->ld, sizeof(double) * N, ls, cudaMemcpyDeviceToDevice, h->stream);
+    else if (h->cfg.mirrored_sampling)
+      expand_mirrored_kernel<<<h->num_sms * 4, 256, 0, h->stream>>>(h->dY, tmp, h->ld, (long long)ls, (int)N);
+    else
+      cudaMemcpy2DAsync(tmp, sizeof(double) * N, h->dY, sizeof(double) * h->ld, sizeof(double) * N, ls, cudaMemcpyDeviceToDevice, h->stream);
     cudaError_t e = cudaMemcpyAsync(out, tmp, sizeof(double) * n, cudaMemcpyDeviceToHost, h->stream);
     cudaStreamSynchronize(h->stream);
-    cudaFree(tmp);
     CUDA_OK(h, e);
     return 0;
   }
-  ArrRef r;
-  if (!strcmp(key, "Gradients") && h->dGrad) {   // LOCAL shard rows, like "Sample Population"
-    r.p = h->dGrad; r.rows = local_samples(h); r.cols = N; r.ld = h->ld;
-  } else if (!strcmp(key, "Discrete Mutations") && h->dDiscMut) {
-    r.p = h->dDiscMut; r.rows = local_samples(h); r.cols = N; r.ld = h->ld;
-  } else if (!strcmp(key, "Masking Matrix") && h->dMask) {
-    r.p = h->dMask; r.rows = 1; r.cols = N; r.ld = h->ld;
-  } else if (!strcmp(key, "Masking Matrix Sigma") && h->dMaskSigma) {
-    r.p = h->dMaskSigma; r.rows = 1; r.cols = N; r.ld = h->ld;
-  } else if (!find_array(h, key, &r)) return fail(h, "unknown array key '%s'", key);
-  const size_t n = r.rows * r.cols;
-  if (count) *count = n;
-  if (!out) return 0;
-  if (cap < n) return fail(h, "buffer too small for '%s' (%zu < %zu)", key, cap, n);
-  if (n == 0) return 0;
-  CUDA_OK(h, cudaMemcpy2DAsync(out, sizeof(double) * r.cols, r.p, sizeof(double) * r.ld, sizeof(double) * r.cols, r.rows,
-                               cudaMemcpyDeviceToHost, h->stream));
-  CUDA_OK(h, cudaStreamSynchronize(h->stream));
-  return 0;
+  Array r;
+  if (!strcmp(key, "Gradients") && h->dGrad) r = pitched(h->dGrad, local_samples(h), N, h->ld);   // LOCAL shard rows, like "Sample Population"
+  else if (!strcmp(key, "Discrete Mutations") && h->dDiscMut) r = pitched(h->dDiscMut, local_samples(h), N, h->ld);
+  else if (!strcmp(key, "Masking Matrix") && h->dMask) r = dense(h->dMask, N);
+  else if (!strcmp(key, "Masking Matrix Sigma") && h->dMaskSigma) r = dense(h->dMaskSigma, N);
+  else if (!find_array(h, key, &r)) return fail(h, "unknown array key '%s'", key);
+  return copy_out(h, key, r, out, cap, count, "buffer too small for '%s' (%zu < %zu)");
 }
 
 int kcma_set_array(kcma_t* h, const char* key, const double* in, size_t count) {
-  if (!h) return fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   invalidate_graph(h);
   CUDA_OK(h, cudaSetDevice(h->device));
-  ArrRef r;
+  Array r;
   if (!find_array(h, key, &r)) return fail(h, "unknown array key '%s'", key);
-  if (count != r.rows * r.cols) return fail(h, "size mismatch for '%s' (%zu != %zu)", key, count, r.rows * r.cols);
-  CUDA_OK(h, cudaMemcpy2DAsync(r.p, sizeof(double) * r.ld, in, sizeof(double) * r.cols, sizeof(double) * r.cols, r.rows,
-                               cudaMemcpyHostToDevice, h->stream));
-  CUDA_OK(h, cudaStreamSynchronize(h->stream));
+  if (copy_in(h, key, r, in, count)) return 1;
   if (!strcmp(key, "Covariance Eigenvector Matrix") || !strcmp(key, "Axis Lengths")) h->vt_valid = false;
   if (!strcmp(key, "Mu Weights")) std::copy(in, in + count, h->h_weights.begin());
   return 0;
 }
 
 int kcma_get_index_array(kcma_t* h, const char* key, uint64_t* out, size_t cap, size_t* count) {
-  if (!h) return fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   CUDA_OK(h, cudaSetDevice(h->device));
   const size_t n = h->cur_lambda;
-  if (!strcmp(key, "Sample Constraint Violation Counts")) {
-    const size_t m = h->has_constraints ? n : 0;
-    if (count) *count = m;
-    if (!out) return 0;
-    if (cap < m) return fail(h, "buffer too small for '%s'", key);
-    if (m) { CUDA_OK(h, cudaMemcpyAsync(out, h->dViol, sizeof(uint64_t) * m, cudaMemcpyDeviceToHost, h->stream)); CUDA_OK(h, cudaStreamSynchronize(h->stream)); }
-    return 0;
-  }
-  if (strcmp(key, "Sorting Index")) return fail(h, "unknown index key '%s'", key);
-  if (count) *count = n;
-  if (!out) return 0;
-  if (cap < n) return fail(h, "buffer too small for '%s'", key);
-  std::vector<unsigned> tmp(n);
-  CUDA_OK(h, cudaMemcpyAsync(tmp.data(), h->dIdx, sizeof(unsigned) * n, cudaMemcpyDeviceToHost, h->stream));
-  CUDA_OK(h, cudaStreamSynchronize(h->stream));
-  for (size_t i = 0; i < n; i++) out[i] = tmp[i];
-  return 0;
+  Array r;
+  if (!strcmp(key, "Sample Constraint Violation Counts")) r = dense(h->dViol, h->has_constraints ? n : 0, Elem::u64);
+  else if (!strcmp(key, "Sorting Index")) r = dense(h->dIdx, n, Elem::u32);
+  else return fail(h, "unknown index key '%s'", key);
+  return copy_out(h, key, r, out, cap, count, "buffer too small for '%s'");
 }
 
 namespace {
@@ -1737,27 +1638,28 @@ double* find_dev_scalar(kcma* h, const char* key) {
 #undef S
   return nullptr;
 }
-double* find_host_scalar(kcma* h, const char* key) {
-#define S(K, F) if (!strcmp(key, K)) return &h->F;
-  S("Trace", trace) S("Effective Mu", mueff) S("Sigma Cumulation Factor", cs) S("Damp Factor", damp)
-  S("Cumulative Covariance", cc) S("Chi Square Number", chi_n)
-  S("Termination Criteria/Max Condition Covariance Matrix", tc_max_condition)
-  S("Termination Criteria/Min Standard Deviation", tc_min_sd)
-  S("Termination Criteria/Max Standard Deviation", tc_max_sd)
-  S("Termination Criteria/Max Value", tc_max_value)
-  S("Termination Criteria/Min Value Difference Threshold", tc_min_value_diff)
-  S("Termination Criteria/Max Model Evaluations", tc_max_model_evaluations)
-  S("Termination Criteria/Max Generations", tc_max_generations)
-#undef S
-  return nullptr;
-}
+const HostScalar<kcma> kHostScalars[] = {
+    {"Trace", &kcma::trace, true},
+    {"Effective Mu", &kcma::mueff, true},
+    {"Sigma Cumulation Factor", &kcma::cs, true},
+    {"Damp Factor", &kcma::damp, true},
+    {"Cumulative Covariance", &kcma::cc, true},
+    {"Chi Square Number", &kcma::chi_n, true},
+    {"Termination Criteria/Max Condition Covariance Matrix", &kcma::tc_max_condition, true},
+    {"Termination Criteria/Min Standard Deviation", &kcma::tc_min_sd, true},
+    {"Termination Criteria/Max Standard Deviation", &kcma::tc_max_sd, true},
+    {"Termination Criteria/Max Value", &kcma::tc_max_value, true},
+    {"Termination Criteria/Min Value Difference Threshold", &kcma::tc_min_value_diff, true},
+    {"Termination Criteria/Max Model Evaluations", &kcma::tc_max_model_evaluations, true},
+    {"Termination Criteria/Max Generations", &kcma::tc_max_generations, true},
+};
 }  // namespace
 
 int kcma_get_scalar(kcma_t* h, const char* key, double* out) {
-  if (!h) return fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   CUDA_OK(h, cudaSetDevice(h->device));
-  if (double* p = find_host_scalar(h, key)) { *out = *p; return 0; }
-  if (pull_scalars(h)) return 1;
+  if (double* p = host_scalar(h, kHostScalars, key, false)) { *out = *p; return 0; }
+  if (pull_cached(h)) return 1;
   if (double* p = find_dev_scalar(h, key)) { *out = *p; return 0; }
 #define U(K, V) if (!strcmp(key, K)) { *out = (double)(V); return 0; }
   U("Current Generation", h->gen - 1) U("Model Evaluation Count", h->model_evals) U("Variable Count", h->N)
@@ -1778,11 +1680,11 @@ int kcma_get_scalar(kcma_t* h, const char* key, double* out) {
 }
 
 int kcma_set_scalar(kcma_t* h, const char* key, double v) {
-  if (!h) return fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   invalidate_graph(h);
   CUDA_OK(h, cudaSetDevice(h->device));
-  if (double* p = find_host_scalar(h, key)) { *p = v; return 0; }
-  if (pull_scalars(h)) return 1;
+  if (double* p = host_scalar(h, kHostScalars, key, true)) { *p = v; return 0; }
+  if (pull_cached(h)) return 1;
   if (double* p = find_dev_scalar(h, key)) { *p = v; return push_scalars(h); }
 #define U(K, STMT) if (!strcmp(key, K)) { STMT; return 0; }
   U("Current Generation", h->gen = (uint64_t)v + 1)
@@ -1813,80 +1715,82 @@ extern "C" int kcma_debug_jacobi_timestamps(long long* out3584) {
   if (!kc::g_jacobi_dbg) return 1;
   return cudaMemcpy(out3584, kc::g_jacobi_dbg, sizeof(long long) * 3584, cudaMemcpyDeviceToHost) != cudaSuccess;
 }
-int kcma_timing_enable(kcma_t* h, int on) { if (!h) return fail(nullptr, "null solver handle"); h->timing = on != 0; return 0; }   // the graph path is skipped while timing
+int kcma_timing_enable(kcma_t* h, int on) { if (!h) return fail(h, "null solver handle"); h->timing = on != 0; return 0; }   // the graph path is skipped while timing
 int kcma_timing_get(kcma_t* h, const char* phase, double* ms, uint64_t* calls) {
-  if (!h) return fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   resolve_timers(h);
   auto it = h->phases.find(phase);
   if (ms) *ms = it == h->phases.end() ? 0.0 : it->second.ms;
   if (calls) *calls = it == h->phases.end() ? 0 : it->second.calls;
   if (calls && !strcmp(phase, "eigen_sweeps")) {   // persistent kernel: counted on the device; per-step path: counted by the host loop
     h->scalars_fresh = false;
-    if (pull_scalars(h)) return 1;
+    if (pull_cached(h)) return 1;
     *calls += h->hSc->jacobi_sweeps_total - h->sweeps_base;
   }
   return 0;
 }
 int kcma_timing_reset(kcma_t* h) {
-  if (!h) return fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   resolve_timers(h);
   h->phases.clear();
   h->scalars_fresh = false;
-  if (pull_scalars(h)) return 1;
+  if (pull_cached(h)) return 1;
   h->sweeps_base = h->hSc->jacobi_sweeps_total;
   return 0;
 }
-uint64_t kcma_launch_count(const kcma_t* h) { return h->launches; }
+uint64_t kcma_launch_count(const kcma_t* h) { return h ? h->launches : 0; }
 int kcma_flush_l2(kcma_t* h) {
-  if (!h) return fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   CUDA_OK(h, cudaSetDevice(h->device));
-  if (!h->dFlush) { h->flush_bytes = 256ull << 20; CUDA_OK(h, cudaMalloc(&h->dFlush, h->flush_bytes)); }
-  flush_kernel<<<h->num_sms * 8, 256, 0, h->stream>>>((double*)h->dFlush, h->flush_bytes / sizeof(double));
+  if (!h->dFlush) { h->flush_bytes = 256ull << 20; CUDA_OK(h, alloc(h->mem, &h->dFlush, h->flush_bytes / sizeof(double))); }
+  flush_kernel<<<h->num_sms * 8, 256, 0, h->stream>>>(h->dFlush, h->flush_bytes / sizeof(double));
   return 0;
 }
 
 // ---- single kernels on host buffers -----------------------------------------------------------------------
-#define K_CUDA(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return fail(nullptr, "CUDA error %s (%s)", cudaGetErrorString(e_), #call); } while (0)
+// They have no handle: failures are reported through kcma_last_error(NULL), and each call's buffers are freed on every return.
+static kcma* const kNoHandle = nullptr;
 
 int kcma_k_sort_index(int device, const double* f, uint64_t n, uint64_t* index_out) {
   if (n == 0) return 0;
-  K_CUDA(cudaSetDevice(device));
+  CUDA_OK(kNoHandle, cudaSetDevice(device));
   int sms; cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
-  double* df; unsigned* di; void* ws;
-  K_CUDA(cudaMalloc(&df, sizeof(double) * n)); K_CUDA(cudaMalloc(&di, sizeof(unsigned) * n));
-  K_CUDA(cudaMalloc(&ws, sort_workspace_bytes((int)n)));
-  K_CUDA(cudaMemcpy(df, f, sizeof(double) * n, cudaMemcpyHostToDevice));
+  Allocations scratch;
+  double* df; unsigned* di; unsigned char* ws;
+  CUDA_OK(kNoHandle, alloc(scratch, &df, n)); CUDA_OK(kNoHandle, alloc(scratch, &di, n));
+  CUDA_OK(kNoHandle, alloc(scratch, &ws, sort_workspace_bytes((int)n)));
+  CUDA_OK(kNoHandle, cudaMemcpy(df, f, sizeof(double) * n, cudaMemcpyHostToDevice));
   launch_sort_index(0, df, (int)n, ws, di, sms);
   std::vector<unsigned> tmp(n);
-  K_CUDA(cudaMemcpy(tmp.data(), di, sizeof(unsigned) * n, cudaMemcpyDeviceToHost));
+  CUDA_OK(kNoHandle, cudaMemcpy(tmp.data(), di, sizeof(unsigned) * n, cudaMemcpyDeviceToHost));
   for (uint64_t i = 0; i < n; i++) index_out[i] = tmp[i];
-  cudaFree(df); cudaFree(di); cudaFree(ws);
   return 0;
 }
 
 int kcma_k_sample(int device, uint64_t n, uint64_t rows, const double* z, const double* b, const double* d, const double* mean,
                   double sigma, double* y_out, double* x_out) {
-  K_CUDA(cudaSetDevice(device));
+  CUDA_OK(kNoHandle, cudaSetDevice(device));
   const int N = (int)n, ld = round_up(N, 16);
+  Allocations scratch;
   double *dZ, *dB, *dA, *dD, *dY;
-  K_CUDA(dmalloc(&dZ, rows * ld)); K_CUDA(dmalloc(&dY, rows * ld)); K_CUDA(dmalloc(&dB, (size_t)N * ld)); K_CUDA(dmalloc(&dA, (size_t)N * ld));
-  K_CUDA(dmalloc(&dD, ld));
-  K_CUDA(cudaMemcpy2D(dZ, sizeof(double) * ld, z, sizeof(double) * N, sizeof(double) * N, rows, cudaMemcpyHostToDevice));
-  K_CUDA(cudaMemcpy2D(dB, sizeof(double) * ld, b, sizeof(double) * N, sizeof(double) * N, N, cudaMemcpyHostToDevice));
-  K_CUDA(cudaMemcpy(dD, d, sizeof(double) * N, cudaMemcpyHostToDevice));
+  CUDA_OK(kNoHandle, alloc(scratch, &dZ, rows * ld)); CUDA_OK(kNoHandle, alloc(scratch, &dY, rows * ld));
+  CUDA_OK(kNoHandle, alloc(scratch, &dB, (size_t)N * ld)); CUDA_OK(kNoHandle, alloc(scratch, &dA, (size_t)N * ld));
+  CUDA_OK(kNoHandle, alloc(scratch, &dD, ld));
+  CUDA_OK(kNoHandle, cudaMemcpy2D(dZ, sizeof(double) * ld, z, sizeof(double) * N, sizeof(double) * N, rows, cudaMemcpyHostToDevice));
+  CUDA_OK(kNoHandle, cudaMemcpy2D(dB, sizeof(double) * ld, b, sizeof(double) * N, sizeof(double) * N, N, cudaMemcpyHostToDevice));
+  CUDA_OK(kNoHandle, cudaMemcpy(dD, d, sizeof(double) * N, cudaMemcpyHostToDevice));
   launch_scale_bd(0, dB, ld, dD, dA, ld, N);
   launch_gemm_tn(0, (int)rows, N, N, dZ, ld, dA, ld, dY, ld);
-  K_CUDA(cudaMemcpy2D(y_out, sizeof(double) * N, dY, sizeof(double) * ld, sizeof(double) * N, rows, cudaMemcpyDeviceToHost));
+  CUDA_OK(kNoHandle, cudaMemcpy2D(y_out, sizeof(double) * N, dY, sizeof(double) * ld, sizeof(double) * N, rows, cudaMemcpyDeviceToHost));
   if (x_out)
     for (uint64_t i = 0; i < rows; i++)
       for (int k = 0; k < N; k++) x_out[i * N + k] = mean[k] + sigma * y_out[i * N + k];
-  cudaFree(dZ); cudaFree(dY); cudaFree(dB); cudaFree(dA); cudaFree(dD);
-  K_CUDA(cudaGetLastError());
+  CUDA_OK(kNoHandle, cudaGetLastError());
   return 0;
 }
 
 int kcma_k_rank_mu(int device, uint64_t n, uint64_t rows, const double* t, const double* w, double* p_out) {
-  K_CUDA(cudaSetDevice(device));
+  CUDA_OK(kNoHandle, cudaSetDevice(device));
   int sms; cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
   const int N = (int)n, ld = round_up(N, 16);
   const size_t rp = round_up((int)rows, 16) + 16;
@@ -1895,60 +1799,61 @@ int kcma_k_rank_mu(int device, uint64_t n, uint64_t rows, const double* t, const
     const double rw = sqrt(w[k]);
     for (int d = 0; d < N; d++) s[k * N + d] = rw * t[k * N + d];
   }
+  Allocations scratch;
   double *dS, *dW, *dP;
-  K_CUDA(dmalloc(&dS, rp * ld));
-  K_CUDA(dmalloc(&dW, (size_t)16 * N * ld)); K_CUDA(dmalloc(&dP, (size_t)N * ld));
-  K_CUDA(cudaMemcpy2D(dS, sizeof(double) * ld, s.data(), sizeof(double) * N, sizeof(double) * N, rows, cudaMemcpyHostToDevice));
+  CUDA_OK(kNoHandle, alloc(scratch, &dS, rp * ld));
+  CUDA_OK(kNoHandle, alloc(scratch, &dW, (size_t)16 * N * ld)); CUDA_OK(kNoHandle, alloc(scratch, &dP, (size_t)N * ld));
+  CUDA_OK(kNoHandle, cudaMemcpy2D(dS, sizeof(double) * ld, s.data(), sizeof(double) * N, sizeof(double) * N, rows, cudaMemcpyHostToDevice));
   const int splits = launch_syrk(0, N, (int)rows, nullptr, dS, ld, (long long)rp, dW, ld, (int)rows, sms, 16);
   launch_reduce_splits(0, dW, ld, splits, N, dP);
   std::vector<double> p((size_t)N * N);
-  K_CUDA(cudaMemcpy2D(p.data(), sizeof(double) * N, dP, sizeof(double) * ld, sizeof(double) * N, N, cudaMemcpyDeviceToHost));
+  CUDA_OK(kNoHandle, cudaMemcpy2D(p.data(), sizeof(double) * N, dP, sizeof(double) * ld, sizeof(double) * N, N, cudaMemcpyDeviceToHost));
   for (int d = 0; d < N; d++)
     for (int e = 0; e <= d; e++) p_out[(size_t)d * N + e] = p_out[(size_t)e * N + d] = p[(size_t)d * N + e];
-  cudaFree(dS); cudaFree(dW); cudaFree(dP);
-  K_CUDA(cudaGetLastError());
+  CUDA_OK(kNoHandle, cudaGetLastError());
   return 0;
 }
 
 int kcma_k_philox_normal(int device, uint64_t seed, uint64_t generation, uint64_t row_begin, uint64_t rows, uint64_t n, double* z_out) {
-  K_CUDA(cudaSetDevice(device));
+  CUDA_OK(kNoHandle, cudaSetDevice(device));
   int sms; cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
   const int N = (int)n, ld = round_up(N, 16);
+  Allocations scratch;
   double* dZ;
-  K_CUDA(dmalloc(&dZ, rows * ld));
+  CUDA_OK(kNoHandle, alloc(scratch, &dZ, rows * ld));
   launch_philox_normal(0, dZ, ld, (long long)rows, N, seed, (unsigned)generation, row_begin, nullptr, nullptr, sms);
-  K_CUDA(cudaMemcpy2D(z_out, sizeof(double) * N, dZ, sizeof(double) * ld, sizeof(double) * N, rows, cudaMemcpyDeviceToHost));
-  cudaFree(dZ);
-  K_CUDA(cudaGetLastError());
+  CUDA_OK(kNoHandle, cudaMemcpy2D(z_out, sizeof(double) * N, dZ, sizeof(double) * ld, sizeof(double) * N, rows, cudaMemcpyDeviceToHost));
+  CUDA_OK(kNoHandle, cudaGetLastError());
   return 0;
 }
 
 int kcma_k_philox_raw(int device, const uint32_t ctr[4], const uint32_t key[2], uint32_t out[4]) {
-  K_CUDA(cudaSetDevice(device));
+  CUDA_OK(kNoHandle, cudaSetDevice(device));
   uint32_t in[6] = {ctr[0], ctr[1], ctr[2], ctr[3], key[0], key[1]};
+  Allocations scratch;
   uint32_t *din, *dout;
-  K_CUDA(cudaMalloc(&din, sizeof(in))); K_CUDA(cudaMalloc(&dout, 16));
-  K_CUDA(cudaMemcpy(din, in, sizeof(in), cudaMemcpyHostToDevice));
+  CUDA_OK(kNoHandle, alloc(scratch, &din, 6)); CUDA_OK(kNoHandle, alloc(scratch, &dout, 4));
+  CUDA_OK(kNoHandle, cudaMemcpy(din, in, sizeof(in), cudaMemcpyHostToDevice));
   launch_philox_raw(0, din, dout);
-  K_CUDA(cudaMemcpy(out, dout, 16, cudaMemcpyDeviceToHost));
-  cudaFree(din); cudaFree(dout);
+  CUDA_OK(kNoHandle, cudaMemcpy(out, dout, 16, cudaMemcpyDeviceToHost));
   return 0;
 }
 
 int kcma_k_objective(int device, int objective, uint64_t n, uint64_t rows, const double* x, const double* coef, double* f_out) {
-  K_CUDA(cudaSetDevice(device));
+  CUDA_OK(kNoHandle, cudaSetDevice(device));
   int sms; cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device);
   const int N = (int)n, ld = round_up(N, 16);
+  Allocations scratch;
   double *dX, *dCoef, *dF; DevScalars* dSc;
-  K_CUDA(dmalloc(&dX, rows * ld)); K_CUDA(dmalloc(&dCoef, ld)); K_CUDA(dmalloc(&dF, rows)); K_CUDA(dmalloc(&dSc, 1));
-  K_CUDA(cudaMemcpy2D(dX, sizeof(double) * ld, x, sizeof(double) * N, sizeof(double) * N, rows, cudaMemcpyHostToDevice));
+  CUDA_OK(kNoHandle, alloc(scratch, &dX, rows * ld)); CUDA_OK(kNoHandle, alloc(scratch, &dCoef, ld));
+  CUDA_OK(kNoHandle, alloc(scratch, &dF, rows)); CUDA_OK(kNoHandle, alloc(scratch, &dSc, 1));
+  CUDA_OK(kNoHandle, cudaMemcpy2D(dX, sizeof(double) * ld, x, sizeof(double) * N, sizeof(double) * N, rows, cudaMemcpyHostToDevice));
   std::vector<double> c(N);
   for (int i = 0; i < N; i++) c[i] = coef ? coef[i] : (N > 1 ? pow(10.0, 6.0 * (double)i / (double)(N - 1)) : 1.0);
-  K_CUDA(cudaMemcpy(dCoef, c.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
-  if (launch_objective(0, objective, dX, ld, (long long)rows, N, 0, 1, dCoef, dSc, dCoef, dF, sms)) return fail(nullptr, "unknown objective id %d", objective);
-  K_CUDA(cudaMemcpy(f_out, dF, sizeof(double) * rows, cudaMemcpyDeviceToHost));
-  cudaFree(dX); cudaFree(dCoef); cudaFree(dF); cudaFree(dSc);
-  K_CUDA(cudaGetLastError());
+  CUDA_OK(kNoHandle, cudaMemcpy(dCoef, c.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
+  if (launch_objective(0, objective, dX, ld, (long long)rows, N, 0, 1, dCoef, dSc, dCoef, dF, sms)) return fail(kNoHandle, "unknown objective id %d", objective);
+  CUDA_OK(kNoHandle, cudaMemcpy(f_out, dF, sizeof(double) * rows, cudaMemcpyDeviceToHost));
+  CUDA_OK(kNoHandle, cudaGetLastError());
   return 0;
 }
 
@@ -1962,16 +1867,16 @@ int kcma_k_eigen(int device, uint64_t n, const double* c, double* eigenvalues, d
   if (kcma_create(&cfg, &h)) return 1;
   int rc = kcma_set_array(h, "Covariance Matrix", c, n * n);
   if (!rc) rc = update_eigensystem(h, h->dC);
-  if (!rc) rc = pull_scalars(h);
-  if (!rc) { cudaError_t e = cudaGetLastError(); if (e != cudaSuccess) rc = fail(nullptr, "CUDA error in the eigensolver: %s", cudaGetErrorString(e)); }
+  if (!rc) rc = pull_cached(h);
+  if (!rc) { cudaError_t e = cudaGetLastError(); if (e != cudaSuccess) rc = fail(kNoHandle, "CUDA error in the eigensolver: %s", cudaGetErrorString(e)); }
   if (!rc && h->hSc->eig_rejected) {  // report the raw spectrum anyway (unsorted acceptance is the caller's business)
-    rc = fail(nullptr, "matrix is not positive definite: eigensystem rejected (CMAES.cpp.base:876-880)");
+    rc = fail(kNoHandle, "matrix is not positive definite: eigensystem rejected (CMAES.cpp.base:876-880)");
   }
   if (!rc) rc = kcma_get_array(h, "Covariance Eigenvector Matrix", q, n * n, nullptr);
   if (!rc) {
     rc = kcma_get_array(h, "Axis Lengths", eigenvalues, n, nullptr);
     for (uint64_t i = 0; i < n; i++) eigenvalues[i] *= eigenvalues[i];
-  } else if (h->err.size()) strncpy(g_create_err, h->err.c_str(), sizeof(g_create_err) - 1);
+  } else if (h->err.size()) fail(kNoHandle, "%s", h->err.c_str());
   kcma_destroy(h);
   return rc;
 }
@@ -1981,27 +1886,26 @@ int kcma_k_eigen(int device, uint64_t n, const double* c, double* eigenvalues, d
 // mode 0: C (n x n) -> d, e, tau, reflector rows vr (n x n); mode 1: (d, e) -> eigenvalues lam, eigenvectors as rows zt (n x n).
 int kcma_k_tridiag_stage(int device, int mode, uint64_t n, const double* c, double* d, double* e, double* tau, double* vr,
                          double* lam, double* zt) {
-  if (cudaSetDevice(device) != cudaSuccess) return fail(nullptr, "no CUDA device %d (libkcma has no CPU fallback)", device);
+  if (cudaSetDevice(device) != cudaSuccess) return fail(kNoHandle, "no CUDA device %d (libkcma has no CPU fallback)", device);
   cudaDeviceProp prop;
   cudaGetDeviceProperties(&prop, device);
   const int N = (int)n, ld = round_up(N, 16);
   char msg[512] = "";
   TridiagWs* ws = tridiag_ws_create(N, ld, prop.multiProcessorCount, msg, sizeof(msg));
-  if (!ws) return fail(nullptr, "%s", msg);
+  if (!ws) return fail(kNoHandle, "%s", msg);
   int rc = 0, l = 0;
   if (mode == 0) {
+    Allocations scratch;
     double* dM = nullptr;
-    cudaMalloc(&dM, sizeof(double) * (size_t)N * ld);
-    cudaMemset(dM, 0, sizeof(double) * (size_t)N * ld);
+    alloc(scratch, &dM, (size_t)N * ld);
     cudaMemcpy2D(dM, sizeof(double) * ld, c, sizeof(double) * N, sizeof(double) * N, N, cudaMemcpyHostToDevice);
-    if (!tridiag_stage_sytrd(0, ws, dM)) rc = fail(nullptr, "sytrd launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-    if (!rc && cudaDeviceSynchronize() != cudaSuccess) rc = fail(nullptr, "sytrd failed: %s", cudaGetErrorString(cudaGetLastError()));
+    if (!tridiag_stage_sytrd(0, ws, dM)) rc = fail(kNoHandle, "sytrd launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    if (!rc && cudaDeviceSynchronize() != cudaSuccess) rc = fail(kNoHandle, "sytrd failed: %s", cudaGetErrorString(cudaGetLastError()));
     if (!rc) { tridiag_get_tridiagonal(ws, d, e, tau, vr); tridiag_dump_prof(ws); }
-    cudaFree(dM);
   } else {
     tridiag_set_tridiagonal(ws, d, e);
-    if (!tridiag_stage_dc(0, ws, &l)) rc = fail(nullptr, "divide & conquer launch failed: %s", cudaGetErrorString(cudaGetLastError()));
-    if (!rc && cudaDeviceSynchronize() != cudaSuccess) rc = fail(nullptr, "divide & conquer failed: %s", cudaGetErrorString(cudaGetLastError()));
+    if (!tridiag_stage_dc(0, ws, &l)) rc = fail(kNoHandle, "divide & conquer launch failed: %s", cudaGetErrorString(cudaGetLastError()));
+    if (!rc && cudaDeviceSynchronize() != cudaSuccess) rc = fail(kNoHandle, "divide & conquer failed: %s", cudaGetErrorString(cudaGetLastError()));
     if (!rc) {
       cudaMemcpy(lam, tridiag_result_values(ws), sizeof(double) * N, cudaMemcpyDeviceToHost);
       cudaMemcpy2D(zt, sizeof(double) * N, tridiag_result_vectors(ws), sizeof(double) * ld, sizeof(double) * N, N, cudaMemcpyDeviceToHost);

@@ -11,7 +11,6 @@
 //                                running maximum), dea_mean_kernel (mean in sample order, max - min per dimension)
 // All arithmetic with explicit roundings (no FMA contraction): populations are bit-identical to oracle/odea.c.
 #include <math.h>
-#include <stdarg.h>
 #include <stdio.h>
 #include <string.h>
 
@@ -21,6 +20,7 @@
 
 #include "../../include/kdea.h"
 #include "common.cuh"
+#include "handle.cuh"
 #include "kernels.h"
 
 namespace kc {
@@ -298,55 +298,57 @@ void launch_dea_mean(cudaStream_t st, const double* X, int ld, long long lambda,
   dea_mean_kernel<<<(n + 31) / 32, DM_NT, smem, st>>>(X, ld, lambda, n, mean, prev_mean, maxdist);
 }
 
-char g_dea_create_err[512] = "";
-
 }  // namespace
 }  // namespace kc
 
 using namespace kc;
 
-struct kdea {
+struct kdea : Handle<kdea, DeaScalars> {
   kdea_cfg cfg;
-  int N = 0, ld = 0, device = 0, num_sms = 148;
+  int N = 0, ld = 0, num_sms = 148;
   long long lambda = 0;
-  cudaStream_t stream = 0;
   std::vector<double> lower, upper, coef;
   double *dX = nullptr, *dXc = nullptr, *dF = nullptr, *dFprev = nullptr, *dMean = nullptr, *dPrevMean = nullptr, *dBestEver = nullptr,
          *dCurBest = nullptr, *dMaxDist = nullptr, *dLower = nullptr, *dUpper = nullptr, *dCoef = nullptr;
   int* dRows = nullptr;
   unsigned* dAttempt = nullptr;
   unsigned char *dInfeasible = nullptr, *dIterAccept = nullptr;
-  DeaScalars *dSc = nullptr, *hSc = nullptr;
   DevScalars* dObjSc = nullptr;   // sigma / nonfinite block the objective kernels expect
-  uint64_t gen = 1, model_evals = 0, launches = 0;
-  bool have_inj_f = false, scalars_fresh = false;
+  uint64_t model_evals = 0;
+  bool have_inj_f = false;
   kcma_host_objective_fn host_obj = nullptr; void* host_obj_user = nullptr;
   std::vector<double> hX, hF;
   double tc_max_infeasible = 1e7, tc_min_value = -INFINITY, tc_min_step = -INFINITY, tc_max_value = INFINITY, tc_min_value_diff = -INFINITY,
          tc_max_generations = 1e10, tc_max_model_evaluations = 1e9;
-  std::string err, reason;
 };
 
 namespace {
-int dfail(kdea* h, const char* fmt, ...) {
-  char buf[512];
-  va_list ap; va_start(ap, fmt); vsnprintf(buf, sizeof(buf), fmt, ap); va_end(ap);
-  if (h) h->err = buf; else { strncpy(g_dea_create_err, buf, sizeof(g_dea_create_err) - 1); g_dea_create_err[sizeof(g_dea_create_err) - 1] = 0; }
-  return 1;
+const HostScalar<kdea> kHostScalars[] = {
+    {"Termination Criteria/Max Infeasible Resamplings", &kdea::tc_max_infeasible, true},
+    {"Termination Criteria/Min Value", &kdea::tc_min_value, true},
+    {"Termination Criteria/Min Step Size", &kdea::tc_min_step, true},
+    {"Termination Criteria/Max Value", &kdea::tc_max_value, true},
+    {"Termination Criteria/Min Value Difference Threshold", &kdea::tc_min_value_diff, true},
+    {"Termination Criteria/Max Generations", &kdea::tc_max_generations, true},
+    {"Termination Criteria/Max Model Evaluations", &kdea::tc_max_model_evaluations, true},
+};
+bool find_array(kdea* h, const char* key, Array* r) {
+  const size_t N = h->N, L = (size_t)h->lambda, ld = h->ld;
+#define A(K, ARR) if (!strcmp(key, K)) { *r = ARR; return true; }
+  A("Sample Population", pitched(h->dX, L, N, ld)) A("Candidate Population", pitched(h->dXc, L, N, ld))
+  A("Value Vector", dense(h->dF, L)) A("Previous Value Vector", dense(h->dFprev, L))
+  A("Current Mean", dense(h->dMean, N)) A("Previous Mean", dense(h->dPrevMean, N)) A("Best Ever Variables", dense(h->dBestEver, N))
+  A("Current Best Variables", dense(h->dCurBest, N)) A("Max Distances", dense(h->dMaxDist, N))
+#undef A
+  return false;
 }
-#define DEA_CUDA(h, call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return dfail(h, "CUDA error %s (%s)", cudaGetErrorString(e_), #call); } while (0)
-
-int dea_pull(kdea* h) {
-  if (h->scalars_fresh) return 0;
-  DEA_CUDA(h, cudaMemcpyAsync(h->hSc, h->dSc, sizeof(DeaScalars), cudaMemcpyDeviceToHost, h->stream));
-  DEA_CUDA(h, cudaStreamSynchronize(h->stream));
-  h->scalars_fresh = true;
-  return 0;
-}
-int dea_push(kdea* h) {
-  DEA_CUDA(h, cudaMemcpyAsync(h->dSc, h->hSc, sizeof(DeaScalars), cudaMemcpyHostToDevice, h->stream));
-  DEA_CUDA(h, cudaStreamSynchronize(h->stream));
-  return 0;
+double* find_dev_scalar(kdea* h, const char* key) {
+  DeaScalars* s = h->hSc;
+#define S(K, F) if (!strcmp(key, K)) return &s->F;
+  S("Best Ever Value", best_ever_value) S("Current Best Value", cur_best_value) S("Previous Best Value", prev_best_value)
+  S("Previous Best Ever Value", prev_best_ever_value) S("Current Minimum Step Size", min_step)
+#undef S
+  return nullptr;
 }
 }  // namespace
 
@@ -360,35 +362,23 @@ void kdea_cfg_defaults(kdea_cfg* c) {
   c->fix_infeasible = 1;
 }
 
-const char* kdea_last_error(const kdea_t* h) { return h ? h->err.c_str() : g_dea_create_err; }
+const char* kdea_last_error(const kdea_t* h) { return h ? h->err.c_str() : kdea::create_err; }
 
-void kdea_destroy(kdea_t* h) {
-  if (!h) return;
-  cudaSetDevice(h->device);
-  void* ptrs[] = {h->dX, h->dXc, h->dF, h->dFprev, h->dMean, h->dPrevMean, h->dBestEver, h->dCurBest, h->dMaxDist, h->dLower, h->dUpper, h->dCoef,
-                  h->dRows, h->dAttempt, h->dInfeasible, h->dIterAccept, h->dSc, h->dObjSc};
-  for (void* p : ptrs) if (p) cudaFree(p);
-  if (h->hSc) cudaFreeHost(h->hSc);
-  delete h;
-}
+void kdea_destroy(kdea_t* h) { delete h; }
 
 // setInitialConfiguration (:15-64)
 int kdea_create(const kdea_cfg* cfg, kdea_t** out) {
-  if (!cfg || !out) return dfail(nullptr, "kdea_create: null argument");
-  if (cfg->abi_version != KDEA_ABI_VERSION) return dfail(nullptr, "kdea_cfg ABI version %u, library %u", cfg->abi_version, KDEA_ABI_VERSION);
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-    cudaGetLastError();
-    return dfail(nullptr, "libkcma needs a CUDA device (sm_100a); none is visible. There is no CPU fallback.");
-  }
-  if (cfg->n == 0) return dfail(nullptr, "Optimization Evaluation problems require at least one variable.\n");
-  if (cfg->n > (1u << 20)) return dfail(nullptr, "too many variables for the Philox sub-streams of DEA (%lu > 2^20)", (unsigned long)cfg->n);
-  if (cfg->population_size < 4) return dfail(nullptr, "DEA needs a Population Size of at least 4 (three distinct partners per sample, DEA.cpp.base:125-166)");
-  if (cfg->population_size > 0x7fffffffull) return dfail(nullptr, "Population Size too large");
-  if (cfg->mutation_rule != KDEA_MUTATION_FIXED) return dfail(nullptr, "Mutation Rule 'Self Adaptive' is not built (its rates are global state updated sample by sample, DEA.cpp.base:136-156)");
-  if (cfg->parent_selection_rule != KDEA_PARENT_RANDOM && cfg->parent_selection_rule != KDEA_PARENT_BEST) return dfail(nullptr, "Parent Selection Rule not recognized");
-  if (cfg->accept_rule < KDEA_ACCEPT_BEST || cfg->accept_rule > KDEA_ACCEPT_ITERATIVE) return dfail(nullptr, "Accept Rule (%d) not recognized.\n", cfg->accept_rule);
-  if (!cfg->lower_bound || !cfg->upper_bound) return dfail(nullptr, "DEA needs Lower Bound and Upper Bound for every variable (the initial population is uniform in the box)");
+  if (!cfg || !out) return fail<kdea>(nullptr, "kdea_create: null argument");
+  if (cfg->abi_version != KDEA_ABI_VERSION) return fail<kdea>(nullptr, "kdea_cfg ABI version %u, library %u", cfg->abi_version, KDEA_ABI_VERSION);
+  if (open_device<kdea>(cfg->device)) return 1;
+  if (cfg->n == 0) return fail<kdea>(nullptr, "Optimization Evaluation problems require at least one variable.\n");
+  if (cfg->n > (1u << 20)) return fail<kdea>(nullptr, "too many variables for the Philox sub-streams of DEA (%lu > 2^20)", (unsigned long)cfg->n);
+  if (cfg->population_size < 4) return fail<kdea>(nullptr, "DEA needs a Population Size of at least 4 (three distinct partners per sample, DEA.cpp.base:125-166)");
+  if (cfg->population_size > 0x7fffffffull) return fail<kdea>(nullptr, "Population Size too large");
+  if (cfg->mutation_rule != KDEA_MUTATION_FIXED) return fail<kdea>(nullptr, "Mutation Rule 'Self Adaptive' is not built (its rates are global state updated sample by sample, DEA.cpp.base:136-156)");
+  if (cfg->parent_selection_rule != KDEA_PARENT_RANDOM && cfg->parent_selection_rule != KDEA_PARENT_BEST) return fail<kdea>(nullptr, "Parent Selection Rule not recognized");
+  if (cfg->accept_rule < KDEA_ACCEPT_BEST || cfg->accept_rule > KDEA_ACCEPT_ITERATIVE) return fail<kdea>(nullptr, "Accept Rule (%d) not recognized.\n", cfg->accept_rule);
+  if (!cfg->lower_bound || !cfg->upper_bound) return fail<kdea>(nullptr, "DEA needs Lower Bound and Upper Bound for every variable (the initial population is uniform in the box)");
   kdea* h = new kdea();
   h->cfg = *cfg;
   h->N = (int)cfg->n; h->ld = (h->N + 15) / 16 * 16; h->lambda = (long long)cfg->population_size; h->device = cfg->device;
@@ -396,61 +386,57 @@ int kdea_create(const kdea_cfg* cfg, kdea_t** out) {
   h->lower.assign(cfg->lower_bound, cfg->lower_bound + N);
   h->upper.assign(cfg->upper_bound, cfg->upper_bound + N);
   for (int d = 0; d < N; d++) {
-    if (!std::isfinite(h->lower[d]) || !std::isfinite(h->upper[d])) { delete h; return dfail(nullptr, "DEA: variable %d needs finite bounds", d); }
-    if (h->upper[d] < h->lower[d]) { const double lo = h->lower[d], up = h->upper[d]; delete h; return dfail(nullptr, "Lower Bound (%.4f) of variable %d exceeds Upper Bound (%.4f).\n", lo, d, up); }
+    if (!std::isfinite(h->lower[d]) || !std::isfinite(h->upper[d])) return create_fail(h, "DEA: variable %d needs finite bounds", d);
+    if (h->upper[d] < h->lower[d]) return create_fail(h, "Lower Bound (%.4f) of variable %d exceeds Upper Bound (%.4f).\n", h->lower[d], d, h->upper[d]);
   }
   h->coef.resize(N);
   for (int d = 0; d < N; d++) h->coef[d] = cfg->objective_coef ? cfg->objective_coef[d] : pow(10.0, 6.0 * (double)d / (double)(N > 1 ? N - 1 : 1));
   h->cfg.lower_bound = h->cfg.upper_bound = h->cfg.objective_coef = nullptr;
-#define DC(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { dfail(nullptr, "CUDA error %s (%s)", cudaGetErrorString(e_), #call); kdea_destroy(h); return 1; } } while (0)
-  DC(cudaSetDevice(h->device));
   cudaDeviceProp prop;
-  DC(cudaGetDeviceProperties(&prop, h->device));
+  CREATE_OK(h, cudaGetDeviceProperties(&prop, h->device));
   h->num_sms = prop.multiProcessorCount;
   const size_t L = (size_t)h->lambda, mat = L * ld;
-  auto dalloc = [&](void** p, size_t bytes) { cudaError_t e = cudaMalloc(p, bytes ? bytes : 8); if (e == cudaSuccess) e = cudaMemset(*p, 0, bytes ? bytes : 8); return e; };
-  DC(dalloc((void**)&h->dX, sizeof(double) * mat)); DC(dalloc((void**)&h->dXc, sizeof(double) * mat));
-  DC(dalloc((void**)&h->dF, sizeof(double) * L)); DC(dalloc((void**)&h->dFprev, sizeof(double) * L));
-  DC(dalloc((void**)&h->dMean, sizeof(double) * ld)); DC(dalloc((void**)&h->dPrevMean, sizeof(double) * ld));
-  DC(dalloc((void**)&h->dBestEver, sizeof(double) * ld)); DC(dalloc((void**)&h->dCurBest, sizeof(double) * ld));
-  DC(dalloc((void**)&h->dMaxDist, sizeof(double) * ld)); DC(dalloc((void**)&h->dLower, sizeof(double) * ld));
-  DC(dalloc((void**)&h->dUpper, sizeof(double) * ld)); DC(dalloc((void**)&h->dCoef, sizeof(double) * ld));
-  DC(dalloc((void**)&h->dRows, sizeof(int) * L)); DC(dalloc((void**)&h->dAttempt, sizeof(unsigned) * L));
-  DC(dalloc((void**)&h->dInfeasible, L)); DC(dalloc((void**)&h->dIterAccept, L));
-  DC(dalloc((void**)&h->dSc, sizeof(DeaScalars))); DC(dalloc((void**)&h->dObjSc, sizeof(DevScalars)));
-  DC(cudaMallocHost((void**)&h->hSc, sizeof(DeaScalars)));
-  DC(cudaMemcpy(h->dLower, h->lower.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
-  DC(cudaMemcpy(h->dUpper, h->upper.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
-  DC(cudaMemcpy(h->dCoef, h->coef.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
-  memset(h->hSc, 0, sizeof(DeaScalars));
+  Allocations& m = h->mem;
+  CREATE_OK(h, alloc(m, &h->dX, mat)); CREATE_OK(h, alloc(m, &h->dXc, mat));
+  CREATE_OK(h, alloc(m, &h->dF, L)); CREATE_OK(h, alloc(m, &h->dFprev, L));
+  CREATE_OK(h, alloc(m, &h->dMean, ld)); CREATE_OK(h, alloc(m, &h->dPrevMean, ld));
+  CREATE_OK(h, alloc(m, &h->dBestEver, ld)); CREATE_OK(h, alloc(m, &h->dCurBest, ld));
+  CREATE_OK(h, alloc(m, &h->dMaxDist, ld)); CREATE_OK(h, alloc(m, &h->dLower, ld));
+  CREATE_OK(h, alloc(m, &h->dUpper, ld)); CREATE_OK(h, alloc(m, &h->dCoef, ld));
+  CREATE_OK(h, alloc(m, &h->dRows, L)); CREATE_OK(h, alloc(m, &h->dAttempt, L));
+  CREATE_OK(h, alloc(m, &h->dInfeasible, L)); CREATE_OK(h, alloc(m, &h->dIterAccept, L));
+  CREATE_OK(h, alloc(m, &h->dSc, 1)); CREATE_OK(h, alloc(m, &h->dObjSc, 1));
+  CREATE_OK(h, alloc_host(m, &h->hSc, 1));
+  CREATE_OK(h, cudaMemcpy(h->dLower, h->lower.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
+  CREATE_OK(h, cudaMemcpy(h->dUpper, h->upper.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
+  CREATE_OK(h, cudaMemcpy(h->dCoef, h->coef.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
   h->hSc->best_ever_value = h->hSc->prev_best_ever_value = h->hSc->cur_best_value = h->hSc->prev_best_value = -INFINITY;
   h->hSc->min_step = INFINITY;
-  DC(cudaMemcpy(h->dSc, h->hSc, sizeof(DeaScalars), cudaMemcpyHostToDevice));
+  CREATE_OK(h, cudaMemcpy(h->dSc, h->hSc, sizeof(DeaScalars), cudaMemcpyHostToDevice));
   std::vector<double> ninf(L, -INFINITY);   // _valueVector = -Inf (:37)
-  DC(cudaMemcpy(h->dF, ninf.data(), sizeof(double) * L, cudaMemcpyHostToDevice));
-  DC(cudaMemcpy(h->dFprev, ninf.data(), sizeof(double) * L, cudaMemcpyHostToDevice));
+  CREATE_OK(h, cudaMemcpy(h->dF, ninf.data(), sizeof(double) * L, cudaMemcpyHostToDevice));
+  CREATE_OK(h, cudaMemcpy(h->dFprev, ninf.data(), sizeof(double) * L, cudaMemcpyHostToDevice));
   dea_init_kernel<<<h->num_sms * 4, 256, 0, h->stream>>>(h->dX, h->dXc, ld, h->lambda, N, h->dLower, h->dUpper, cfg->seed);
   launch_dea_mean(h->stream, h->dX, ld, h->lambda, N, h->dMean, h->dPrevMean, h->dMaxDist);   // :60-63
-  DC(cudaMemset(h->dPrevMean, 0, sizeof(double) * ld));
-  DC(cudaMemset(h->dMaxDist, 0, sizeof(double) * ld));
+  CREATE_OK(h, cudaMemset(h->dPrevMean, 0, sizeof(double) * ld));
+  CREATE_OK(h, cudaMemset(h->dMaxDist, 0, sizeof(double) * ld));
   h->launches += 2;
-  DC(cudaDeviceSynchronize());
-#undef DC
+  CREATE_OK(h, cudaDeviceSynchronize());
   *out = h;
   return 0;
 }
 
 int kdea_set_host_objective(kdea_t* h, kcma_host_objective_fn fn, void* user) {
-  if (!h) return dfail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   h->host_obj = fn; h->host_obj_user = user;
   return 0;
 }
 
 int kdea_inject_f(kdea_t* h, const double* f, size_t count) {
-  if (!h) return dfail(nullptr, "null solver handle");
-  if (count != (size_t)h->lambda) return dfail(h, "inject F: expected %zu values", (size_t)h->lambda);
-  for (size_t i = 0; i < count; i++) if (!std::isfinite(f[i])) return dfail(h, "Non finite value of function evaluation detected: %f\n", f[i]);
-  DEA_CUDA(h, cudaSetDevice(h->device));
+  if (!h) return fail(h, "null solver handle");
+  if (count != (size_t)h->lambda) return fail(h, "inject F: expected %zu values", (size_t)h->lambda);
+  for (size_t i = 0; i < count; i++) if (!std::isfinite(f[i])) return fail(h, "Non finite value of function evaluation detected: %f\n", f[i]);
+  CUDA_OK(h, cudaSetDevice(h->device));
   h->hF.assign(f, f + count);
   h->have_inj_f = true;
   return 0;
@@ -458,12 +444,12 @@ int kdea_inject_f(kdea_t* h, const double* f, size_t count) {
 
 // prepareGeneration (:103-121)
 int kdea_ask(kdea_t* h) {
-  if (!h) return dfail(nullptr, "null solver handle");
-  DEA_CUDA(h, cudaSetDevice(h->device));
+  if (!h) return fail(h, "null solver handle");
+  CUDA_OK(h, cudaSetDevice(h->device));
   const int N = h->N, ld = h->ld;
   const long long L = h->lambda;
   if (h->gen > 1) {
-    DEA_CUDA(h, cudaMemsetAsync(h->dAttempt, 0, sizeof(unsigned) * (size_t)L, h->stream));
+    CUDA_OK(h, cudaMemsetAsync(h->dAttempt, 0, sizeof(unsigned) * (size_t)L, h->stream));
     const int wpb = 8;
     dea_mutate_kernel<<<(unsigned)((L + wpb - 1) / wpb), 256, 0, h->stream>>>(h->dX, h->dXc, ld, L, N, nullptr, (int)L, nullptr, h->dLower, h->dUpper,
                                                                             h->cfg.crossover_rate, h->cfg.mutation_rate, h->cfg.parent_selection_rule,
@@ -474,62 +460,62 @@ int kdea_ask(kdea_t* h) {
       dea_compact_kernel<<<(unsigned)std::min<long long>((L + 255) / 256, (long long)h->num_sms * 4), 256, 0, h->stream>>>(h->dInfeasible, L, h->dRows, h->dAttempt, h->dSc);
       h->launches += 2;
       h->scalars_fresh = false;
-      if (dea_pull(h)) return 1;
+      if (pull_cached(h)) return 1;
       const int cnt = h->hSc->redo_count;
       if (cnt == 0) break;
-      if (round >= 100000) return dfail(h, "a sample never becomes feasible (100000 mutations)");
+      if (round >= 100000) return fail(h, "a sample never becomes feasible (100000 mutations)");
       dea_mutate_kernel<<<(unsigned)((cnt + wpb - 1) / wpb), 256, 0, h->stream>>>(h->dX, h->dXc, ld, L, N, h->dRows, cnt, h->dAttempt, h->dLower, h->dUpper,
                                                                                 h->cfg.crossover_rate, h->cfg.mutation_rate, h->cfg.parent_selection_rule,
                                                                                 h->cfg.fix_infeasible, h->cfg.seed, (unsigned)h->gen, h->dSc, h->dInfeasible);
       h->launches++;
     }
   }
-  DEA_CUDA(h, cudaMemcpyAsync(h->dFprev, h->dF, sizeof(double) * (size_t)L, cudaMemcpyDeviceToDevice, h->stream));   // :120
+  CUDA_OK(h, cudaMemcpyAsync(h->dFprev, h->dF, sizeof(double) * (size_t)L, cudaMemcpyDeviceToDevice, h->stream));   // :120
   return 0;
 }
 
 // runGeneration :72-85 as one batched evaluation
 int kdea_eval(kdea_t* h) {
-  if (!h) return dfail(nullptr, "null solver handle");
-  DEA_CUDA(h, cudaSetDevice(h->device));
+  if (!h) return fail(h, "null solver handle");
+  CUDA_OK(h, cudaSetDevice(h->device));
   const int N = h->N, ld = h->ld;
   const size_t L = (size_t)h->lambda;
   h->model_evals += L;
   if (h->have_inj_f) {
     h->have_inj_f = false;
-    DEA_CUDA(h, cudaMemcpyAsync(h->dF, h->hF.data(), sizeof(double) * L, cudaMemcpyHostToDevice, h->stream));
-    DEA_CUDA(h, cudaStreamSynchronize(h->stream));
+    CUDA_OK(h, cudaMemcpyAsync(h->dF, h->hF.data(), sizeof(double) * L, cudaMemcpyHostToDevice, h->stream));
+    CUDA_OK(h, cudaStreamSynchronize(h->stream));
     return 0;
   }
   if (h->host_obj) {
     h->hX.resize(L * N); h->hF.resize(L);
-    DEA_CUDA(h, cudaMemcpy2DAsync(h->hX.data(), sizeof(double) * N, h->dXc, sizeof(double) * ld, sizeof(double) * N, L, cudaMemcpyDeviceToHost, h->stream));
-    DEA_CUDA(h, cudaStreamSynchronize(h->stream));
+    CUDA_OK(h, cudaMemcpy2DAsync(h->hX.data(), sizeof(double) * N, h->dXc, sizeof(double) * ld, sizeof(double) * N, L, cudaMemcpyDeviceToHost, h->stream));
+    CUDA_OK(h, cudaStreamSynchronize(h->stream));
     h->host_obj(h->host_obj_user, h->hX.data(), (uint64_t)L, (uint64_t)N, h->hF.data());
     for (size_t i = 0; i < L; i++)
-      if (!std::isfinite(h->hF[i])) return dfail(h, "Non finite value of function evaluation detected: %f\n", h->hF[i]);
-    DEA_CUDA(h, cudaMemcpyAsync(h->dF, h->hF.data(), sizeof(double) * L, cudaMemcpyHostToDevice, h->stream));
-    DEA_CUDA(h, cudaStreamSynchronize(h->stream));
+      if (!std::isfinite(h->hF[i])) return fail(h, "Non finite value of function evaluation detected: %f\n", h->hF[i]);
+    CUDA_OK(h, cudaMemcpyAsync(h->dF, h->hF.data(), sizeof(double) * L, cudaMemcpyHostToDevice, h->stream));
+    CUDA_OK(h, cudaStreamSynchronize(h->stream));
     return 0;
   }
-  if (h->cfg.objective == KCMA_OBJ_EXTERNAL) return dfail(h, "objective is External: set a host objective or inject the Value Vector before eval");
+  if (h->cfg.objective == KCMA_OBJ_EXTERNAL) return fail(h, "objective is External: set a host objective or inject the Value Vector before eval");
   if (launch_objective(h->stream, h->cfg.objective, h->dXc, ld, (long long)L, N, 0, 1, h->dMean, h->dObjSc, h->dCoef, h->dF, h->num_sms))
-    return dfail(h, "unknown objective id %d", h->cfg.objective);
+    return fail(h, "unknown objective id %d", h->cfg.objective);
   h->launches++;
   int bad = 0;
-  DEA_CUDA(h, cudaMemcpyAsync(&bad, &h->dObjSc->nonfinite, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
-  DEA_CUDA(h, cudaStreamSynchronize(h->stream));
+  CUDA_OK(h, cudaMemcpyAsync(&bad, &h->dObjSc->nonfinite, sizeof(int), cudaMemcpyDeviceToHost, h->stream));
+  CUDA_OK(h, cudaStreamSynchronize(h->stream));
   if (bad) {
     cudaMemsetAsync(&h->dObjSc->nonfinite, 0, sizeof(int), h->stream);
-    return dfail(h, "Non finite value of function evaluation detected: nan\n");
+    return fail(h, "Non finite value of function evaluation detected: nan\n");
   }
   return 0;
 }
 
 // updateSolver (:203-282)
 int kdea_tell(kdea_t* h) {
-  if (!h) return dfail(nullptr, "null solver handle");
-  DEA_CUDA(h, cudaSetDevice(h->device));
+  if (!h) return fail(h, "null solver handle");
+  CUDA_OK(h, cudaSetDevice(h->device));
   const int N = h->N, ld = h->ld;
   const long long L = h->lambda;
   dea_best_kernel<<<1, 1024, 0, h->stream>>>(h->dF, L, h->dSc);
@@ -542,7 +528,7 @@ int kdea_tell(kdea_t* h) {
   h->scalars_fresh = false;
   h->gen++;
   cudaError_t e = cudaGetLastError();
-  if (e != cudaSuccess) return dfail(h, "CUDA error after generation: %s", cudaGetErrorString(e));
+  if (e != cudaSuccess) return fail(h, "CUDA error after generation: %s", cudaGetErrorString(e));
   return 0;
 }
 
@@ -550,9 +536,9 @@ int kdea_run_generation(kdea_t* h) { return kdea_ask(h) || kdea_eval(h) || kdea_
 
 // generated checkTermination: DEA.config:62-83, optimizer.config, solver.config
 int kdea_check_termination(kdea_t* h, int* finished, const char** reason) {
-  if (!h) return dfail(nullptr, "null solver handle");
-  DEA_CUDA(h, cudaSetDevice(h->device));
-  if (dea_pull(h)) return 1;
+  if (!h) return fail(h, "null solver handle");
+  CUDA_OK(h, cudaSetDevice(h->device));
+  if (pull_cached(h)) return 1;
   const DeaScalars& s = *h->hSc;
   int fin = 0;
   h->reason.clear();
@@ -570,100 +556,50 @@ int kdea_check_termination(kdea_t* h, int* finished, const char** reason) {
 }
 
 int kdea_run(kdea_t* h, uint64_t max_generations, uint64_t* done) {
-  if (!h) return dfail(nullptr, "null solver handle");
-  uint64_t n = 0;
-  int fin = 0;
-  while (n < max_generations) {
-    if (kdea_check_termination(h, &fin, nullptr)) { if (done) *done = n; return 1; }
-    if (fin) break;
-    if (kdea_run_generation(h)) { if (done) *done = n; return 1; }
-    n++;
-  }
-  if (done) *done = n;
-  return 0;
+  return run(h, max_generations, done, kdea_check_termination, kdea_run_generation);
 }
-
-namespace {
-struct DArr { double* p; size_t rows, cols; int ld; };
-bool dea_find_array(kdea* h, const char* key, DArr* r) {
-  const size_t N = h->N, L = (size_t)h->lambda; const int ld = h->ld;
-#define A(K, P, R, C, LD) if (!strcmp(key, K)) { r->p = (P); r->rows = (R); r->cols = (C); r->ld = (LD); return true; }
-  A("Sample Population", h->dX, L, N, ld) A("Candidate Population", h->dXc, L, N, ld)
-  A("Value Vector", h->dF, 1, L, (int)L) A("Previous Value Vector", h->dFprev, 1, L, (int)L)
-  A("Current Mean", h->dMean, 1, N, ld) A("Previous Mean", h->dPrevMean, 1, N, ld) A("Best Ever Variables", h->dBestEver, 1, N, ld)
-  A("Current Best Variables", h->dCurBest, 1, N, ld) A("Max Distances", h->dMaxDist, 1, N, ld)
-#undef A
-  return false;
-}
-double* dea_find_host_scalar(kdea* h, const char* key) {
-#define S(K, F) if (!strcmp(key, K)) return &h->F;
-  S("Termination Criteria/Max Infeasible Resamplings", tc_max_infeasible) S("Termination Criteria/Min Value", tc_min_value)
-  S("Termination Criteria/Min Step Size", tc_min_step) S("Termination Criteria/Max Value", tc_max_value)
-  S("Termination Criteria/Min Value Difference Threshold", tc_min_value_diff) S("Termination Criteria/Max Generations", tc_max_generations)
-  S("Termination Criteria/Max Model Evaluations", tc_max_model_evaluations)
-#undef S
-  return nullptr;
-}
-double* dea_find_dev_scalar(kdea* h, const char* key) {
-  DeaScalars* s = h->hSc;
-#define S(K, F) if (!strcmp(key, K)) return &s->F;
-  S("Best Ever Value", best_ever_value) S("Current Best Value", cur_best_value) S("Previous Best Value", prev_best_value)
-  S("Previous Best Ever Value", prev_best_ever_value) S("Current Minimum Step Size", min_step)
-#undef S
-  return nullptr;
-}
-}  // namespace
 
 int kdea_get_array(kdea_t* h, const char* key, double* out, size_t cap, size_t* count) {
-  if (!h) return dfail(nullptr, "null solver handle");
-  DEA_CUDA(h, cudaSetDevice(h->device));
-  DArr r;
-  if (!dea_find_array(h, key, &r)) return dfail(h, "unknown array key '%s'", key);
-  const size_t n = r.rows * r.cols;
-  if (count) *count = n;
-  if (!out) return 0;
-  if (cap < n) return dfail(h, "buffer too small for '%s' (%zu < %zu)", key, cap, n);
-  DEA_CUDA(h, cudaMemcpy2DAsync(out, sizeof(double) * r.cols, r.p, sizeof(double) * r.ld, sizeof(double) * r.cols, r.rows, cudaMemcpyDeviceToHost, h->stream));
-  DEA_CUDA(h, cudaStreamSynchronize(h->stream));
-  return 0;
+  if (!h) return fail(h, "null solver handle");
+  CUDA_OK(h, cudaSetDevice(h->device));
+  Array r;
+  if (!find_array(h, key, &r)) return fail(h, "unknown array key '%s'", key);
+  return copy_out(h, key, r, out, cap, count, "buffer too small for '%s' (%zu < %zu)");
 }
 
 int kdea_set_array(kdea_t* h, const char* key, const double* in, size_t count) {
-  if (!h) return dfail(nullptr, "null solver handle");
-  DEA_CUDA(h, cudaSetDevice(h->device));
-  DArr r;
-  if (!dea_find_array(h, key, &r)) return dfail(h, "unknown array key '%s'", key);
-  if (count != r.rows * r.cols) return dfail(h, "size mismatch for '%s' (%zu != %zu)", key, count, r.rows * r.cols);
-  DEA_CUDA(h, cudaMemcpy2DAsync(r.p, sizeof(double) * r.ld, in, sizeof(double) * r.cols, sizeof(double) * r.cols, r.rows, cudaMemcpyHostToDevice, h->stream));
-  DEA_CUDA(h, cudaStreamSynchronize(h->stream));
-  return 0;
+  if (!h) return fail(h, "null solver handle");
+  CUDA_OK(h, cudaSetDevice(h->device));
+  Array r;
+  if (!find_array(h, key, &r)) return fail(h, "unknown array key '%s'", key);
+  return copy_in(h, key, r, in, count);
 }
 
 int kdea_get_scalar(kdea_t* h, const char* key, double* out) {
-  if (!h) return dfail(nullptr, "null solver handle");
-  DEA_CUDA(h, cudaSetDevice(h->device));
-  if (double* p = dea_find_host_scalar(h, key)) { *out = *p; return 0; }
-  if (dea_pull(h)) return 1;
-  if (double* p = dea_find_dev_scalar(h, key)) { *out = *p; return 0; }
+  if (!h) return fail(h, "null solver handle");
+  CUDA_OK(h, cudaSetDevice(h->device));
+  if (double* p = host_scalar(h, kHostScalars, key, false)) { *out = *p; return 0; }
+  if (pull_cached(h)) return 1;
+  if (double* p = find_dev_scalar(h, key)) { *out = *p; return 0; }
   if (!strcmp(key, "Best Sample Index")) { *out = (double)h->hSc->best_idx; return 0; }
   if (!strcmp(key, "Infeasible Sample Count")) { *out = (double)h->hSc->infeasible; return 0; }
   if (!strcmp(key, "Current Generation")) { *out = (double)(h->gen - 1); return 0; }
   if (!strcmp(key, "Model Evaluation Count")) { *out = (double)h->model_evals; return 0; }
   if (!strcmp(key, "Variable Count")) { *out = (double)h->N; return 0; }
-  return dfail(h, "unknown scalar key '%s'", key);
+  return fail(h, "unknown scalar key '%s'", key);
 }
 
 int kdea_set_scalar(kdea_t* h, const char* key, double v) {
-  if (!h) return dfail(nullptr, "null solver handle");
-  DEA_CUDA(h, cudaSetDevice(h->device));
-  if (double* p = dea_find_host_scalar(h, key)) { *p = v; return 0; }
-  if (dea_pull(h)) return 1;
-  if (double* p = dea_find_dev_scalar(h, key)) { *p = v; return dea_push(h); }
-  if (!strcmp(key, "Best Sample Index")) { h->hSc->best_idx = (unsigned long long)v; return dea_push(h); }
-  if (!strcmp(key, "Infeasible Sample Count")) { h->hSc->infeasible = (unsigned long long)v; return dea_push(h); }
+  if (!h) return fail(h, "null solver handle");
+  CUDA_OK(h, cudaSetDevice(h->device));
+  if (double* p = host_scalar(h, kHostScalars, key, true)) { *p = v; return 0; }
+  if (pull_cached(h)) return 1;
+  if (double* p = find_dev_scalar(h, key)) { *p = v; return push(h); }
+  if (!strcmp(key, "Best Sample Index")) { h->hSc->best_idx = (unsigned long long)v; return push(h); }
+  if (!strcmp(key, "Infeasible Sample Count")) { h->hSc->infeasible = (unsigned long long)v; return push(h); }
   if (!strcmp(key, "Current Generation")) { h->gen = (uint64_t)v + 1; return 0; }
   if (!strcmp(key, "Model Evaluation Count")) { h->model_evals = (uint64_t)v; return 0; }
-  return dfail(h, "unknown scalar key '%s'", key);
+  return fail(h, "unknown scalar key '%s'", key);
 }
 
 uint64_t kdea_launch_count(const kdea_t* h) { return h ? h->launches : 0; }

@@ -16,7 +16,6 @@
 // Compiled with --fmad=false: the arithmetic rounds like the reference's scalar code and like oracle/omocma.c (bit-identical given
 // the same z; the device's log / sincospi / exp may differ from libm in the last bit, so device vs oracle is compared to 1e-9 over a free run).
 #include <math.h>
-#include <stdarg.h>
 #include <stdio.h>
 #include <string.h>
 
@@ -26,6 +25,7 @@
 
 #include "../../include/kmocma.h"
 #include "common.cuh"
+#include "handle.cuh"
 
 namespace {
 
@@ -356,12 +356,11 @@ mo_stats_kernel(int n, int lambda, int K, const double* __restrict__ F, const do
 
 }  // namespace
 
-struct kmocma {
+struct kmocma : Handle<kmocma, MoScalars> {
   kmocma_cfg cfg;
-  int N = 0, lambda = 0, mu = 0, K = 0, device = 0;
-  uint64_t gen = 1, model_evals = 0, launches = 0;
+  int N = 0, lambda = 0, mu = 0, K = 0;
+  uint64_t model_evals = 0;
   double cc = 0, ccov = 0, cp = 0, target = 0;
-  cudaStream_t stream = 0;
   double *dLower = nullptr, *dUpper = nullptr;
   double *dX[3] = {}, *dS[3] = {}, *dC[3] = {}, *dP[3] = {}, *dPS[3] = {};
   double *dF = nullptr, *dFprev = nullptr, *dParentIndex = nullptr;
@@ -369,41 +368,51 @@ struct kmocma {
   double *dBestEver = nullptr, *dBestEverX = nullptr, *dPrevBest = nullptr, *dPrevBestX = nullptr, *dCurBest = nullptr, *dCurBestX = nullptr,
          *dValDiff = nullptr, *dVarDiff = nullptr, *dMinSd = nullptr, *dMaxSd = nullptr;
   unsigned char* dFlag = nullptr;
-  MoScalars* dSc = nullptr;
   std::vector<double> coll_x, coll_f;   // archive of non-dominated samples (host)
   std::vector<double> hX, hF;
   double tc_min_value_diff = -INFINITY, tc_min_var_diff = -INFINITY, tc_min_sd = -INFINITY, tc_max_sd = INFINITY, tc_max_generations = 1e10,
          tc_max_model_evaluations = 1e9;
   kmocma_host_objective_fn host_obj = nullptr; void* host_obj_user = nullptr;
   bool have_inj_f = false;
-  std::string err, reason;
-  std::vector<void*> allocs;
 };
 enum { CUR = 0, PREV = 1, PAR = 2 };
 
 namespace {
-char g_mo_err[512] = "";
-int mo_fail(kmocma* h, const char* fmt, ...) {
-  char buf[512];
-  va_list ap; va_start(ap, fmt);
-  vsnprintf(buf, sizeof(buf), fmt, ap);
-  va_end(ap);
-  if (h) h->err = buf; else { strncpy(g_mo_err, buf, sizeof(g_mo_err) - 1); }
-  return 1;
-}
-#define MO_CUDA(h, call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return mo_fail(h, "CUDA error %s at %s:%d", cudaGetErrorString(e_), __FILE__, __LINE__); } while (0)
-template <typename T>
-cudaError_t mo_alloc(kmocma* h, T** p, size_t count) {
-  cudaError_t e = cudaMalloc((void**)p, sizeof(T) * (count ? count : 1));
-  if (e == cudaSuccess) { h->allocs.push_back(*p); e = cudaMemset(*p, 0, sizeof(T) * (count ? count : 1)); }
-  return e;
-}
-int mo_pull_scalars(kmocma* h, MoScalars* out) {
-  MO_CUDA(h, cudaMemcpyAsync(out, h->dSc, sizeof(MoScalars), cudaMemcpyDeviceToHost, h->stream));
-  MO_CUDA(h, cudaStreamSynchronize(h->stream));
-  return 0;
-}
 size_t sample_smem(int n) { return sizeof(double) * ((size_t)n * n + 2 * (size_t)n + 2); }
+const HostScalar<kmocma> kHostScalars[] = {
+    {"Evolution Path Adaption Strength", &kmocma::cc, false},
+    {"Covariance Learning Rate", &kmocma::ccov, false},
+    {"Termination Criteria/Min Value Difference Threshold", &kmocma::tc_min_value_diff, true},
+    {"Termination Criteria/Min Variable Difference Threshold", &kmocma::tc_min_var_diff, true},
+    {"Termination Criteria/Min Standard Deviation", &kmocma::tc_min_sd, true},
+    {"Termination Criteria/Max Standard Deviation", &kmocma::tc_max_sd, true},
+    {"Termination Criteria/Max Generations", &kmocma::tc_max_generations, true},
+    {"Termination Criteria/Max Model Evaluations", &kmocma::tc_max_model_evaluations, true},
+};
+bool find_array(kmocma* h, const char* key, Array* r) {
+  const size_t N = h->N, L = h->lambda, mu = h->mu, K = h->K;
+  static const char* pop[3] = {"Current", "Previous", "Parent"};
+  for (int s = 0; s < 3; s++) {
+    const size_t rows = s == PAR ? mu : L;
+    const std::string p = pop[s];
+    if (p + " Sample Population" == key) { *r = dense(h->dX[s], rows * N); return true; }
+    if (p + " Sigma" == key) { *r = dense(h->dS[s], rows); return true; }
+    if (p + " Covariance Matrix" == key) { *r = dense(h->dC[s], rows * N * N); return true; }
+    if (p + " Evolution Paths" == key) { *r = dense(h->dP[s], rows * N); return true; }
+    if (p + " Success Probabilities" == key) { *r = dense(h->dPS[s], rows); return true; }
+  }
+#define A(KEY, ARR) if (!strcmp(key, KEY)) { *r = ARR; return true; }
+  A("Current Values", dense(h->dF, L * K)) A("Previous Values", dense(h->dFprev, L * K)) A("Parent Index", dense(h->dParentIndex, L))
+  A("Best Ever Values", dense(h->dBestEver, K)) A("Current Best Values", dense(h->dCurBest, K)) A("Previous Best Values", dense(h->dPrevBest, K))
+  A("Best Ever Variables Vector", dense(h->dBestEverX, K * N)) A("Current Best Variables Vector", dense(h->dCurBestX, K * N))
+  A("Current Best Value Differences", dense(h->dValDiff, K)) A("Current Best Variable Differences", dense(h->dVarDiff, K))
+  A("Current Min Standard Deviations", dense(h->dMinSd, L)) A("Current Max Standard Deviations", dense(h->dMaxSd, L))
+  A("Sorted Indices", dense(h->dSorted, 2 * L, Elem::i32))
+#undef A
+  if (!strcmp(key, "Sample Collection")) { *r = dense(h->coll_x.data(), h->coll_x.size()); r->host = true; return true; }
+  if (!strcmp(key, "Sample Value Collection")) { *r = dense(h->coll_f.data(), h->coll_f.size()); r->host = true; return true; }
+  return false;
+}
 }  // namespace
 
 extern "C" {
@@ -416,38 +425,33 @@ void kmocma_cfg_defaults(kmocma_cfg* c) {
   c->target_success_rate = 0.175; c->threshold_probability = 0.44; c->success_learning_rate = 0.08;
 }
 
-const char* kmocma_last_error(const kmocma_t* h) { return h ? h->err.c_str() : g_mo_err; }
+const char* kmocma_last_error(const kmocma_t* h) { return h ? h->err.c_str() : kmocma::create_err; }
 
-void kmocma_destroy(kmocma_t* h) {
-  if (!h) return;
-  cudaSetDevice(h->device);
-  for (void* p : h->allocs) cudaFree(p);
-  delete h;
-}
+void kmocma_destroy(kmocma_t* h) { delete h; }
 
 // setInitialConfiguration :10-144
 int kmocma_create(const kmocma_cfg* cfg, kmocma_t** out) {
-  if (!cfg || !out) return mo_fail(nullptr, "null argument");
-  if (cfg->abi_version != KMOCMA_ABI_VERSION) return mo_fail(nullptr, "kmocma_cfg ABI version mismatch");
-  if (cfg->n < 1) return mo_fail(nullptr, "no variables");
+  if (!cfg || !out) return fail<kmocma>(nullptr, "null argument");
+  if (cfg->abi_version != KMOCMA_ABI_VERSION) return fail<kmocma>(nullptr, "kmocma_cfg ABI version mismatch");
+  if (cfg->n < 1) return fail<kmocma>(nullptr, "no variables");
   if (cfg->num_objectives < 2 || cfg->num_objectives > KMOCMA_MAX_OBJECTIVES)
-    return mo_fail(nullptr, "Problem requires multiple objectives, 'Num Objectives' is set to %zu\n.", (size_t)cfg->num_objectives);
+    return fail<kmocma>(nullptr, "Problem requires multiple objectives, 'Num Objectives' is set to %zu\n.", (size_t)cfg->num_objectives);
   const uint64_t N = cfg->n, K = cfg->num_objectives;
   uint64_t lambda = cfg->population_size, mu = cfg->mu_value;
   if (lambda == 0) lambda = (uint64_t)ceil(4. + floor(3. * log((double)N)));
   if (mu == 0) mu = (uint64_t)(lambda / 2.);
-  if (mu > lambda) return mo_fail(nullptr, "Number of parents ('Mu Value' %zu) must be smaller or equal with population size (%zu).\n", (size_t)mu, (size_t)lambda);
+  if (mu > lambda) return fail<kmocma>(nullptr, "Number of parents ('Mu Value' %zu) must be smaller or equal with population size (%zu).\n", (size_t)mu, (size_t)lambda);
   if (cfg->success_learning_rate <= 0. || cfg->success_learning_rate > 1.)
-    return mo_fail(nullptr, "Invalid Global Success Learning Rate (%f), must be greater than 0.0 and less or equal to 1.0\n", cfg->success_learning_rate);
+    return fail<kmocma>(nullptr, "Invalid Global Success Learning Rate (%f), must be greater than 0.0 and less or equal to 1.0\n", cfg->success_learning_rate);
   if (cfg->target_success_rate <= 0. || cfg->target_success_rate > 1.)
-    return mo_fail(nullptr, "Invalid Target Success Rate (%f), must be greater than 0.0 and less or equal to 1.0\n", cfg->target_success_rate);
-  if (sample_smem((int)N) > 200 * 1024) return mo_fail(nullptr, "Optimizer/MOCMAES on the device holds one covariance factor per CTA in shared memory: n <= 158");
-  if (2 * lambda * (sizeof(double) + 3 * sizeof(int)) > 200 * 1024) return mo_fail(nullptr, "Optimizer/MOCMAES: the ranking of the 2 lambda merged samples runs in one CTA's shared memory: population size <= 5120");
+    return fail<kmocma>(nullptr, "Invalid Target Success Rate (%f), must be greater than 0.0 and less or equal to 1.0\n", cfg->target_success_rate);
+  if (sample_smem((int)N) > 200 * 1024) return fail<kmocma>(nullptr, "Optimizer/MOCMAES on the device holds one covariance factor per CTA in shared memory: n <= 158");
+  if (2 * lambda * (sizeof(double) + 3 * sizeof(int)) > 200 * 1024) return fail<kmocma>(nullptr, "Optimizer/MOCMAES: the ranking of the 2 lambda merged samples runs in one CTA's shared memory: population size <= 5120");
   if (cfg->objective != KMOCMA_OBJ_EXTERNAL) {
     const uint64_t want = cfg->objective == KMOCMA_OBJ_NEG_ROSENBROCK_AND_TWO_SPHERES ? 3 : 2;
     if (cfg->objective != KMOCMA_OBJ_NEG_ROSENBROCK_AND_SPHERE && cfg->objective != KMOCMA_OBJ_NEG_ROSENBROCK_AND_TWO_SPHERES)
-      return mo_fail(nullptr, "unknown objective id %d", cfg->objective);
-    if (K != want) return mo_fail(nullptr, "the built-in objective has %zu objectives, 'Num Objectives' is %zu", (size_t)want, (size_t)K);
+      return fail<kmocma>(nullptr, "unknown objective id %d", cfg->objective);
+    if (K != want) return fail<kmocma>(nullptr, "the built-in objective has %zu objectives, 'Num Objectives' is %zu", (size_t)want, (size_t)K);
   }
   std::vector<double> lower(N), upper(N), sd(N);
   double trace = 0., min_sdev = INFINITY, max_sdev = -INFINITY;
@@ -457,10 +461,10 @@ int kmocma_create(const kmocma_cfg* cfg, kmocma_t** out) {
     const double iv = cfg->initial_value ? cfg->initial_value[i] : NAN;
     double s = cfg->initial_stddev ? cfg->initial_stddev[i] : NAN;
     if (!std::isfinite(iv) && (!std::isfinite(lower[i]) || !std::isfinite(upper[i])))
-      return mo_fail(nullptr, "Initial (Mean) Value of variable %zu not defined, and cannot be inferred because a variable bound is not finite.\n", (size_t)i);
+      return fail<kmocma>(nullptr, "Initial (Mean) Value of variable %zu not defined, and cannot be inferred because a variable bound is not finite.\n", (size_t)i);
     if (!std::isfinite(s)) {
       if (!std::isfinite(lower[i]) || !std::isfinite(upper[i]))
-        return mo_fail(nullptr, "Initial Standard Deviation of variable %zu not defined, and cannot be inferred because a variable bound is not finite.\n", (size_t)i);
+        return fail<kmocma>(nullptr, "Initial Standard Deviation of variable %zu not defined, and cannot be inferred because a variable bound is not finite.\n", (size_t)i);
       s = (upper[i] - lower[i]) * 0.3;
     }
     sd[i] = s;
@@ -469,9 +473,7 @@ int kmocma_create(const kmocma_cfg* cfg, kmocma_t** out) {
     if (s > max_sdev) max_sdev = s;
   }
   // (the configuration checks above come first, like the reference's; the device is needed from here on)
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) return mo_fail(nullptr, "no CUDA device: korali_b200 has no CPU fallback");
-  if (cfg->device < 0 || cfg->device >= ndev) return mo_fail(nullptr, "invalid device %d", cfg->device);
+  if (open_device<kmocma>(cfg->device)) return 1;
   kmocma* h = new kmocma();
   h->cfg = *cfg;
   h->cfg.lower_bound = h->cfg.upper_bound = h->cfg.initial_value = h->cfg.initial_stddev = nullptr;
@@ -479,112 +481,107 @@ int kmocma_create(const kmocma_cfg* cfg, kmocma_t** out) {
   h->cp = cfg->success_learning_rate; h->target = cfg->target_success_rate;
   h->cc = cfg->evolution_path_adaption_strength < 0. ? 2. / ((double)N + 2.) : cfg->evolution_path_adaption_strength;
   h->ccov = cfg->covariance_learning_rate < 0. ? 2. / ((double)N * (double)N + 6.) : cfg->covariance_learning_rate;
-#define CREATE_CUDA(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { mo_fail(nullptr, "CUDA error %s at %s:%d", cudaGetErrorString(e_), __FILE__, __LINE__); kmocma_destroy(h); return 1; } } while (0)
-  CREATE_CUDA(cudaSetDevice(h->device));
-  CREATE_CUDA(cudaFuncSetAttribute(mo_sample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sample_smem((int)N)));
-  CREATE_CUDA(cudaFuncSetAttribute(mo_sort_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(2 * lambda * (sizeof(double) + 3 * sizeof(int)))));
+  CREATE_OK(h, cudaFuncSetAttribute(mo_sample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sample_smem((int)N)));
+  CREATE_OK(h, cudaFuncSetAttribute(mo_sort_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(2 * lambda * (sizeof(double) + 3 * sizeof(int)))));
   const uint64_t rows[3] = {lambda, lambda, mu};
   for (int s = 0; s < 3; s++) {
-    CREATE_CUDA(mo_alloc(h, &h->dX[s], rows[s] * N)); CREATE_CUDA(mo_alloc(h, &h->dS[s], rows[s])); CREATE_CUDA(mo_alloc(h, &h->dC[s], rows[s] * N * N));
-    CREATE_CUDA(mo_alloc(h, &h->dP[s], rows[s] * N)); CREATE_CUDA(mo_alloc(h, &h->dPS[s], rows[s]));
+    CREATE_OK(h, alloc(h->mem, &h->dX[s], rows[s] * N)); CREATE_OK(h, alloc(h->mem, &h->dS[s], rows[s])); CREATE_OK(h, alloc(h->mem, &h->dC[s], rows[s] * N * N));
+    CREATE_OK(h, alloc(h->mem, &h->dP[s], rows[s] * N)); CREATE_OK(h, alloc(h->mem, &h->dPS[s], rows[s]));
   }
-  CREATE_CUDA(mo_alloc(h, &h->dLower, N)); CREATE_CUDA(mo_alloc(h, &h->dUpper, N));
-  CREATE_CUDA(mo_alloc(h, &h->dF, lambda * K)); CREATE_CUDA(mo_alloc(h, &h->dFprev, lambda * K)); CREATE_CUDA(mo_alloc(h, &h->dParentIndex, lambda));
-  CREATE_CUDA(mo_alloc(h, &h->dSorted, 2 * lambda));
-  CREATE_CUDA(mo_alloc(h, &h->dBestEver, K)); CREATE_CUDA(mo_alloc(h, &h->dPrevBest, K)); CREATE_CUDA(mo_alloc(h, &h->dCurBest, K));
-  CREATE_CUDA(mo_alloc(h, &h->dBestEverX, K * N)); CREATE_CUDA(mo_alloc(h, &h->dPrevBestX, K * N)); CREATE_CUDA(mo_alloc(h, &h->dCurBestX, K * N));
-  CREATE_CUDA(mo_alloc(h, &h->dValDiff, K)); CREATE_CUDA(mo_alloc(h, &h->dVarDiff, K)); CREATE_CUDA(mo_alloc(h, &h->dMinSd, lambda)); CREATE_CUDA(mo_alloc(h, &h->dMaxSd, lambda));
-  CREATE_CUDA(mo_alloc(h, &h->dFlag, lambda)); CREATE_CUDA(mo_alloc(h, &h->dSc, 1));
+  CREATE_OK(h, alloc(h->mem, &h->dLower, N)); CREATE_OK(h, alloc(h->mem, &h->dUpper, N));
+  CREATE_OK(h, alloc(h->mem, &h->dF, lambda * K)); CREATE_OK(h, alloc(h->mem, &h->dFprev, lambda * K)); CREATE_OK(h, alloc(h->mem, &h->dParentIndex, lambda));
+  CREATE_OK(h, alloc(h->mem, &h->dSorted, 2 * lambda));
+  CREATE_OK(h, alloc(h->mem, &h->dBestEver, K)); CREATE_OK(h, alloc(h->mem, &h->dPrevBest, K)); CREATE_OK(h, alloc(h->mem, &h->dCurBest, K));
+  CREATE_OK(h, alloc(h->mem, &h->dBestEverX, K * N)); CREATE_OK(h, alloc(h->mem, &h->dPrevBestX, K * N)); CREATE_OK(h, alloc(h->mem, &h->dCurBestX, K * N));
+  CREATE_OK(h, alloc(h->mem, &h->dValDiff, K)); CREATE_OK(h, alloc(h->mem, &h->dVarDiff, K)); CREATE_OK(h, alloc(h->mem, &h->dMinSd, lambda)); CREATE_OK(h, alloc(h->mem, &h->dMaxSd, lambda));
+  CREATE_OK(h, alloc(h->mem, &h->dFlag, lambda)); CREATE_OK(h, alloc(h->mem, &h->dSc, 1)); CREATE_OK(h, alloc_host(h->mem, &h->hSc, 1));
   auto up = [&](double* d, const std::vector<double>& v) { return cudaMemcpy(d, v.data(), sizeof(double) * v.size(), cudaMemcpyHostToDevice); };
-  CREATE_CUDA(up(h->dLower, lower)); CREATE_CUDA(up(h->dUpper, upper));
+  CREATE_OK(h, up(h->dLower, lower)); CREATE_OK(h, up(h->dUpper, upper));
   std::vector<double> ninf(lambda * K, -INFINITY), kinf(K, INFINITY), kninf(K, -INFINITY);
-  CREATE_CUDA(up(h->dF, ninf)); CREATE_CUDA(up(h->dFprev, ninf));
-  CREATE_CUDA(up(h->dBestEver, kninf)); CREATE_CUDA(up(h->dPrevBest, kninf)); CREATE_CUDA(up(h->dCurBest, kninf));
-  CREATE_CUDA(up(h->dValDiff, kinf)); CREATE_CUDA(up(h->dVarDiff, kinf));
-  CREATE_CUDA(up(h->dMinSd, std::vector<double>(lambda, min_sdev))); CREATE_CUDA(up(h->dMaxSd, std::vector<double>(lambda, max_sdev)));
+  CREATE_OK(h, up(h->dF, ninf)); CREATE_OK(h, up(h->dFprev, ninf));
+  CREATE_OK(h, up(h->dBestEver, kninf)); CREATE_OK(h, up(h->dPrevBest, kninf)); CREATE_OK(h, up(h->dCurBest, kninf));
+  CREATE_OK(h, up(h->dValDiff, kinf)); CREATE_OK(h, up(h->dVarDiff, kinf));
+  CREATE_OK(h, up(h->dMinSd, std::vector<double>(lambda, min_sdev))); CREATE_OK(h, up(h->dMaxSd, std::vector<double>(lambda, max_sdev)));
   const double sigma0 = sqrt(trace / (double)N);
   std::vector<double> pc((size_t)mu * N * N, 0.0);
   for (uint64_t i = 0; i < mu; i++)
     for (uint64_t d = 0; d < N; d++) pc[i * N * N + d * N + d] = sd[d] * sd[d] / (sigma0 * sigma0);
-  CREATE_CUDA(up(h->dC[PAR], pc));
-  CREATE_CUDA(up(h->dS[PAR], std::vector<double>(mu, sigma0))); CREATE_CUDA(up(h->dPS[PAR], std::vector<double>(mu, h->target)));
-  MoScalars s0; memset(&s0, 0, sizeof(s0)); s0.nondom = 1;
-  CREATE_CUDA(cudaMemcpy(h->dSc, &s0, sizeof(s0), cudaMemcpyHostToDevice));
-#undef CREATE_CUDA
+  CREATE_OK(h, up(h->dC[PAR], pc));
+  CREATE_OK(h, up(h->dS[PAR], std::vector<double>(mu, sigma0))); CREATE_OK(h, up(h->dPS[PAR], std::vector<double>(mu, h->target)));
+  h->hSc->nondom = 1;
+  CREATE_OK(h, cudaMemcpy(h->dSc, h->hSc, sizeof(MoScalars), cudaMemcpyHostToDevice));
   *out = h;
   return 0;
 }
 
 // prepareGeneration :177-189 + sampleSingle :191-230
 int kmocma_ask(kmocma_t* h) {
-  if (!h) return mo_fail(nullptr, "null solver handle");
-  MO_CUDA(h, cudaSetDevice(h->device));
+  if (!h) return fail(h, "null solver handle");
+  CUDA_OK(h, cudaSetDevice(h->device));
   const size_t N = h->N, L = h->lambda;
-  MO_CUDA(h, cudaMemcpyAsync(h->dFprev, h->dF, sizeof(double) * L * h->K, cudaMemcpyDeviceToDevice, h->stream));
-  MO_CUDA(h, cudaMemcpyAsync(h->dX[PREV], h->dX[CUR], sizeof(double) * L * N, cudaMemcpyDeviceToDevice, h->stream));
-  MO_CUDA(h, cudaMemcpyAsync(h->dS[PREV], h->dS[CUR], sizeof(double) * L, cudaMemcpyDeviceToDevice, h->stream));
-  MO_CUDA(h, cudaMemcpyAsync(h->dC[PREV], h->dC[CUR], sizeof(double) * L * N * N, cudaMemcpyDeviceToDevice, h->stream));
-  MO_CUDA(h, cudaMemcpyAsync(h->dP[PREV], h->dP[CUR], sizeof(double) * L * N, cudaMemcpyDeviceToDevice, h->stream));
-  MO_CUDA(h, cudaMemcpyAsync(h->dPS[PREV], h->dPS[CUR], sizeof(double) * L, cudaMemcpyDeviceToDevice, h->stream));
+  CUDA_OK(h, cudaMemcpyAsync(h->dFprev, h->dF, sizeof(double) * L * h->K, cudaMemcpyDeviceToDevice, h->stream));
+  CUDA_OK(h, cudaMemcpyAsync(h->dX[PREV], h->dX[CUR], sizeof(double) * L * N, cudaMemcpyDeviceToDevice, h->stream));
+  CUDA_OK(h, cudaMemcpyAsync(h->dS[PREV], h->dS[CUR], sizeof(double) * L, cudaMemcpyDeviceToDevice, h->stream));
+  CUDA_OK(h, cudaMemcpyAsync(h->dC[PREV], h->dC[CUR], sizeof(double) * L * N * N, cudaMemcpyDeviceToDevice, h->stream));
+  CUDA_OK(h, cudaMemcpyAsync(h->dP[PREV], h->dP[CUR], sizeof(double) * L * N, cudaMemcpyDeviceToDevice, h->stream));
+  CUDA_OK(h, cudaMemcpyAsync(h->dPS[PREV], h->dPS[CUR], sizeof(double) * L, cudaMemcpyDeviceToDevice, h->stream));
   mo_sample_kernel<<<h->lambda, 128, sample_smem(h->N), h->stream>>>(h->N, h->lambda, h->mu, h->cfg.seed, (unsigned)h->gen, h->dLower, h->dUpper,
                                                                     h->dX[PAR], h->dS[PAR], h->dC[PAR], h->dP[PAR], h->dPS[PAR], h->dX[CUR], h->dS[CUR],
                                                                     h->dC[CUR], h->dP[CUR], h->dPS[CUR], h->dParentIndex, h->dSc);
   h->launches++;
-  MoScalars s;
-  if (mo_pull_scalars(h, &s)) return 1;
-  if (s.chol_failed) return mo_fail(h, "Error during Cholesky decomposition of covariance matrix.\n");
-  if (s.no_feasible) return mo_fail(h, "no feasible sample after 10^6 draws");
+  if (pull(h)) return 1;
+  if (h->hSc->chol_failed) return fail(h, "Error during Cholesky decomposition of covariance matrix.\n");
+  if (h->hSc->no_feasible) return fail(h, "no feasible sample after 10^6 draws");
   return 0;
 }
 
 int kmocma_set_host_objective(kmocma_t* h, kmocma_host_objective_fn fn, void* user) {
-  if (!h) return mo_fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   h->host_obj = fn; h->host_obj_user = user;
   return 0;
 }
 
 int kmocma_inject_f(kmocma_t* h, const double* f, size_t count) {
-  if (!h) return mo_fail(nullptr, "null solver handle");
-  if (count != (size_t)h->lambda * h->K) return mo_fail(h, "inject_f: %zu values for %d x %d", count, h->lambda, h->K);
-  MO_CUDA(h, cudaSetDevice(h->device));
-  MO_CUDA(h, cudaMemcpyAsync(h->dF, f, sizeof(double) * count, cudaMemcpyHostToDevice, h->stream));
-  MO_CUDA(h, cudaStreamSynchronize(h->stream));
+  if (!h) return fail(h, "null solver handle");
+  if (count != (size_t)h->lambda * h->K) return fail(h, "inject_f: %zu values for %d x %d", count, h->lambda, h->K);
+  CUDA_OK(h, cudaSetDevice(h->device));
+  CUDA_OK(h, cudaMemcpyAsync(h->dF, f, sizeof(double) * count, cudaMemcpyHostToDevice, h->stream));
+  CUDA_OK(h, cudaStreamSynchronize(h->stream));
   h->have_inj_f = true;
   return 0;
 }
 
 // runGeneration :152-170
 int kmocma_eval(kmocma_t* h) {
-  if (!h) return mo_fail(nullptr, "null solver handle");
-  MO_CUDA(h, cudaSetDevice(h->device));
+  if (!h) return fail(h, "null solver handle");
+  CUDA_OK(h, cudaSetDevice(h->device));
   h->model_evals += h->lambda;
   const int L = h->lambda, K = h->K, N = h->N;
   if (h->have_inj_f) {
     h->have_inj_f = false;
   } else if (h->host_obj) {
     h->hX.resize((size_t)L * N); h->hF.resize((size_t)L * K);
-    MO_CUDA(h, cudaMemcpyAsync(h->hX.data(), h->dX[CUR], sizeof(double) * L * N, cudaMemcpyDeviceToHost, h->stream));
-    MO_CUDA(h, cudaStreamSynchronize(h->stream));
+    CUDA_OK(h, cudaMemcpyAsync(h->hX.data(), h->dX[CUR], sizeof(double) * L * N, cudaMemcpyDeviceToHost, h->stream));
+    CUDA_OK(h, cudaStreamSynchronize(h->stream));
     h->host_obj(h->host_obj_user, h->hX.data(), (uint64_t)L, (uint64_t)N, h->hF.data(), (uint64_t)K);
-    MO_CUDA(h, cudaMemcpyAsync(h->dF, h->hF.data(), sizeof(double) * L * K, cudaMemcpyHostToDevice, h->stream));
+    CUDA_OK(h, cudaMemcpyAsync(h->dF, h->hF.data(), sizeof(double) * L * K, cudaMemcpyHostToDevice, h->stream));
   } else if (h->cfg.objective == KMOCMA_OBJ_EXTERNAL) {
-    return mo_fail(h, "objective is External: inject the values or set a host objective before eval");
+    return fail(h, "objective is External: inject the values or set a host objective before eval");
   } else {
     mo_objective_kernel<<<(L + 127) / 128, 128, 0, h->stream>>>(h->cfg.objective, N, L, K, h->dX[CUR], h->dF, h->dSc);
     h->launches++;
   }
   mo_check_finite_kernel<<<(L * K + 255) / 256, 256, 0, h->stream>>>(h->dF, L * K, h->dSc);
   h->launches++;
-  MoScalars s;
-  if (mo_pull_scalars(h, &s)) return 1;
-  if (s.nonfinite) return mo_fail(h, "Non finite value of function evaluation detected\n");
+  if (pull(h)) return 1;
+  if (h->hSc->nonfinite) return fail(h, "Non finite value of function evaluation detected\n");
   return 0;
 }
 
 // updateDistribution :344-418 + updateStatistics :420-520
 int kmocma_tell(kmocma_t* h) {
-  if (!h) return mo_fail(nullptr, "null solver handle");
-  MO_CUDA(h, cudaSetDevice(h->device));
+  if (!h) return fail(h, "null solver handle");
+  CUDA_OK(h, cudaSetDevice(h->device));
   const int L = h->lambda, K = h->K, N = h->N, mu = h->mu;
   mo_sort_kernel<<<1, 1024, (size_t)2 * L * (sizeof(double) + 3 * sizeof(int)), h->stream>>>(h->dF, h->dFprev, L, K, h->dSorted);
   mo_update_kernel<<<L, 128, sizeof(double) * N, h->stream>>>(N, L, mu, h->cc, h->ccov, h->cp, h->target, h->dSorted, h->dParentIndex, h->dX[PAR],
@@ -598,11 +595,11 @@ int kmocma_tell(kmocma_t* h) {
   // archive of non-dominated samples (:483-519) on the host
   std::vector<unsigned char> flag(L);
   h->hX.resize((size_t)L * N); h->hF.resize((size_t)L * K);
-  MO_CUDA(h, cudaMemcpyAsync(flag.data(), h->dFlag, L, cudaMemcpyDeviceToHost, h->stream));
-  MO_CUDA(h, cudaMemcpyAsync(h->hX.data(), h->dX[CUR], sizeof(double) * L * N, cudaMemcpyDeviceToHost, h->stream));
-  MO_CUDA(h, cudaMemcpyAsync(h->hF.data(), h->dF, sizeof(double) * L * K, cudaMemcpyDeviceToHost, h->stream));
-  MO_CUDA(h, cudaStreamSynchronize(h->stream));
-  MO_CUDA(h, cudaGetLastError());
+  CUDA_OK(h, cudaMemcpyAsync(flag.data(), h->dFlag, L, cudaMemcpyDeviceToHost, h->stream));
+  CUDA_OK(h, cudaMemcpyAsync(h->hX.data(), h->dX[CUR], sizeof(double) * L * N, cudaMemcpyDeviceToHost, h->stream));
+  CUDA_OK(h, cudaMemcpyAsync(h->hF.data(), h->dF, sizeof(double) * L * K, cudaMemcpyDeviceToHost, h->stream));
+  CUDA_OK(h, cudaStreamSynchronize(h->stream));
+  CUDA_OK(h, cudaGetLastError());
   std::vector<int> cand;
   for (int i = 0; i < L; i++) if (flag[i]) cand.push_back(i);
   const size_t ncoll = h->coll_f.size() / K;
@@ -633,17 +630,18 @@ int kmocma_tell(kmocma_t* h) {
 int kmocma_run_generation(kmocma_t* h) { return kmocma_ask(h) || kmocma_eval(h) || kmocma_tell(h); }
 
 int kmocma_check_termination(kmocma_t* h, int* finished, const char** reason) {
-  if (!h || !finished) return mo_fail(h, "null argument");
-  MO_CUDA(h, cudaSetDevice(h->device));
+  if (!h) return fail(h, "null solver handle");
+  if (!finished) return fail(h, "null argument");
+  CUDA_OK(h, cudaSetDevice(h->device));
   h->reason.clear();
   int fin = 0;
   const int K = h->K, L = h->lambda;
   if (h->gen > 1) {
     std::vector<double> vd(K), xd(K), mn(L), mx(L);
-    MO_CUDA(h, cudaMemcpy(vd.data(), h->dValDiff, sizeof(double) * K, cudaMemcpyDeviceToHost));
-    MO_CUDA(h, cudaMemcpy(xd.data(), h->dVarDiff, sizeof(double) * K, cudaMemcpyDeviceToHost));
-    MO_CUDA(h, cudaMemcpy(mn.data(), h->dMinSd, sizeof(double) * L, cudaMemcpyDeviceToHost));
-    MO_CUDA(h, cudaMemcpy(mx.data(), h->dMaxSd, sizeof(double) * L, cudaMemcpyDeviceToHost));
+    CUDA_OK(h, cudaMemcpy(vd.data(), h->dValDiff, sizeof(double) * K, cudaMemcpyDeviceToHost));
+    CUDA_OK(h, cudaMemcpy(xd.data(), h->dVarDiff, sizeof(double) * K, cudaMemcpyDeviceToHost));
+    CUDA_OK(h, cudaMemcpy(mn.data(), h->dMinSd, sizeof(double) * L, cudaMemcpyDeviceToHost));
+    CUDA_OK(h, cudaMemcpy(mx.data(), h->dMaxSd, sizeof(double) * L, cudaMemcpyDeviceToHost));
     // (the first criterion reads the BASE class threshold _minValueDifferenceThreshold, MOCMAES.config "Termination Criteria")
     if (fabs(*std::max_element(vd.begin(), vd.end())) < h->tc_min_value_diff) { h->reason += "Min Max Value Difference Threshold;"; fin = 1; }
     if (*std::max_element(xd.begin(), xd.end()) < h->tc_min_var_diff) { h->reason += "Min Variable Difference Threshold;"; fin = 1; }
@@ -658,104 +656,42 @@ int kmocma_check_termination(kmocma_t* h, int* finished, const char** reason) {
 }
 
 int kmocma_run(kmocma_t* h, uint64_t max_generations, uint64_t* done) {
-  if (!h) return mo_fail(nullptr, "null solver handle");
-  uint64_t g = 0;
-  for (; g < max_generations; g++) {
-    int fin; const char* why;
-    if (kmocma_check_termination(h, &fin, &why)) return 1;
-    if (fin) break;
-    if (kmocma_run_generation(h)) return 1;
-  }
-  if (done) *done = g;
-  return 0;
+  return run(h, max_generations, done, kmocma_check_termination, kmocma_run_generation);
 }
 
 int kmocma_get_array(kmocma_t* h, const char* key, double* out, size_t cap, size_t* count) {
-  if (!h || !key) return mo_fail(h, "null argument");
-  MO_CUDA(h, cudaSetDevice(h->device));
-  const size_t N = h->N, L = h->lambda, mu = h->mu, K = h->K;
-  const double* src = nullptr; size_t n = 0; bool host = false, found = false;
-  static const char* pop[3] = {"Current", "Previous", "Parent"};
-  for (int s = 0; s < 3 && !found; s++) {
-    const size_t rows = s == PAR ? mu : L;
-    const std::string p = pop[s];
-    if (p + " Sample Population" == key) { src = h->dX[s]; n = rows * N; found = true; }
-    else if (p + " Sigma" == key) { src = h->dS[s]; n = rows; found = true; }
-    else if (p + " Covariance Matrix" == key) { src = h->dC[s]; n = rows * N * N; found = true; }
-    else if (p + " Evolution Paths" == key) { src = h->dP[s]; n = rows * N; found = true; }
-    else if (p + " Success Probabilities" == key) { src = h->dPS[s]; n = rows; found = true; }
-  }
-  if (!found) {
-    found = true;
-    if (!strcmp(key, "Current Values")) { src = h->dF; n = L * K; }
-    else if (!strcmp(key, "Previous Values")) { src = h->dFprev; n = L * K; }
-    else if (!strcmp(key, "Parent Index")) { src = h->dParentIndex; n = L; }
-    else if (!strcmp(key, "Best Ever Values")) { src = h->dBestEver; n = K; }
-    else if (!strcmp(key, "Current Best Values")) { src = h->dCurBest; n = K; }
-    else if (!strcmp(key, "Previous Best Values")) { src = h->dPrevBest; n = K; }
-    else if (!strcmp(key, "Best Ever Variables Vector")) { src = h->dBestEverX; n = K * N; }
-    else if (!strcmp(key, "Current Best Variables Vector")) { src = h->dCurBestX; n = K * N; }
-    else if (!strcmp(key, "Current Best Value Differences")) { src = h->dValDiff; n = K; }
-    else if (!strcmp(key, "Current Best Variable Differences")) { src = h->dVarDiff; n = K; }
-    else if (!strcmp(key, "Current Min Standard Deviations")) { src = h->dMinSd; n = L; }
-    else if (!strcmp(key, "Current Max Standard Deviations")) { src = h->dMaxSd; n = L; }
-    else if (!strcmp(key, "Sample Collection")) { src = h->coll_x.data(); n = h->coll_x.size(); host = true; }
-    else if (!strcmp(key, "Sample Value Collection")) { src = h->coll_f.data(); n = h->coll_f.size(); host = true; }
-    else if (!strcmp(key, "Sorted Indices")) {
-      n = 2 * L;
-      if (count) *count = n;
-      if (!out) return 0;
-      if (cap < n) return mo_fail(h, "get_array(%s): capacity %zu < %zu", key, cap, n);
-      std::vector<int> tmp(n);
-      MO_CUDA(h, cudaMemcpy(tmp.data(), h->dSorted, sizeof(int) * n, cudaMemcpyDeviceToHost));
-      for (size_t i = 0; i < n; i++) out[i] = (double)tmp[i];
-      return 0;
-    } else found = false;
-  }
-  if (!found) return mo_fail(h, "unknown array key '%s'", key);
-  if (count) *count = n;
-  if (!out) return 0;
-  if (cap < n) return mo_fail(h, "get_array(%s): capacity %zu < %zu", key, cap, n);
-  if (n == 0) return 0;
-  if (host) memcpy(out, src, sizeof(double) * n);
-  else MO_CUDA(h, cudaMemcpy(out, src, sizeof(double) * n, cudaMemcpyDeviceToHost));
-  return 0;
+  if (!h) return fail(h, "null solver handle");
+  if (!key) return fail(h, "null argument");
+  CUDA_OK(h, cudaSetDevice(h->device));
+  Array r;
+  if (!find_array(h, key, &r)) return fail(h, "unknown array key '%s'", key);
+  return copy_out(h, key, r, out, cap, count, "get_array(%s): capacity %zu < %zu");
 }
 
 int kmocma_get_scalar(kmocma_t* h, const char* key, double* out) {
-  if (!h || !key || !out) return mo_fail(h, "null argument");
-  if (!strcmp(key, "Current Non Dominated Sample Count")) {
-    MO_CUDA(h, cudaSetDevice(h->device));
-    MoScalars s;
-    if (mo_pull_scalars(h, &s)) return 1;
-    *out = (double)s.nondom;
+  if (!h) return fail(h, "null solver handle");
+  if (!key || !out) return fail(h, "null argument");
+  if (double* p = host_scalar(h, kHostScalars, key, false)) *out = *p;
+  else if (!strcmp(key, "Current Non Dominated Sample Count")) {
+    CUDA_OK(h, cudaSetDevice(h->device));
+    if (pull(h)) return 1;
+    *out = (double)h->hSc->nondom;
   } else if (!strcmp(key, "Infeasible Sample Count")) *out = 0.0;   // :216 counts nothing (the increment is commented out in the reference)
   else if (!strcmp(key, "Model Evaluation Count")) *out = (double)h->model_evals;
   else if (!strcmp(key, "Current Generation")) *out = (double)h->gen;
   else if (!strcmp(key, "Sample Collection Size")) *out = (double)(h->coll_f.size() / h->K);
   else if (!strcmp(key, "Population Size")) *out = (double)h->lambda;
   else if (!strcmp(key, "Mu Value")) *out = (double)h->mu;
-  else if (!strcmp(key, "Evolution Path Adaption Strength")) *out = h->cc;
-  else if (!strcmp(key, "Covariance Learning Rate")) *out = h->ccov;
-  else if (!strcmp(key, "Termination Criteria/Min Value Difference Threshold")) *out = h->tc_min_value_diff;
-  else if (!strcmp(key, "Termination Criteria/Min Variable Difference Threshold")) *out = h->tc_min_var_diff;
-  else if (!strcmp(key, "Termination Criteria/Min Standard Deviation")) *out = h->tc_min_sd;
-  else if (!strcmp(key, "Termination Criteria/Max Standard Deviation")) *out = h->tc_max_sd;
-  else if (!strcmp(key, "Termination Criteria/Max Generations")) *out = h->tc_max_generations;
-  else if (!strcmp(key, "Termination Criteria/Max Model Evaluations")) *out = h->tc_max_model_evaluations;
-  else return mo_fail(h, "unknown scalar key '%s'", key);
+  else return fail(h, "unknown scalar key '%s'", key);
   return 0;
 }
 
 int kmocma_set_scalar(kmocma_t* h, const char* key, double v) {
-  if (!h || !key) return mo_fail(h, "null argument");
-  if (!strcmp(key, "Termination Criteria/Min Value Difference Threshold")) h->tc_min_value_diff = v;
-  else if (!strcmp(key, "Termination Criteria/Min Variable Difference Threshold")) h->tc_min_var_diff = v;
-  else if (!strcmp(key, "Termination Criteria/Min Standard Deviation")) h->tc_min_sd = v;
-  else if (!strcmp(key, "Termination Criteria/Max Standard Deviation")) h->tc_max_sd = v;
-  else if (!strcmp(key, "Termination Criteria/Max Generations")) h->tc_max_generations = v;
-  else if (!strcmp(key, "Termination Criteria/Max Model Evaluations")) h->tc_max_model_evaluations = v;
-  else return mo_fail(h, "unknown scalar key '%s'", key);
+  if (!h) return fail(h, "null solver handle");
+  if (!key) return fail(h, "null argument");
+  double* p = host_scalar(h, kHostScalars, key, true);
+  if (!p) return fail(h, "unknown scalar key '%s'", key);
+  *p = v;
   return 0;
 }
 

@@ -19,7 +19,6 @@
 // Compiled with --fmad=false: the arithmetic rounds like oracle/otmcmc.c (the device's exp / log / sincospi may differ from libm in
 // the last bit; the GEMM and the SYRK sum in their own order).
 #include <math.h>
-#include <stdarg.h>
 #include <stdio.h>
 #include <string.h>
 
@@ -29,6 +28,7 @@
 
 #include "../../include/ktmcmc.h"
 #include "common.cuh"
+#include "handle.cuh"
 #include "kernels.h"
 
 namespace {
@@ -478,12 +478,10 @@ unsigned grid_for(long long threads, int per) { return (unsigned)std::max<long l
 
 }  // namespace
 
-struct ktmcmc {
+struct ktmcmc : Handle<ktmcmc, TmScalars> {
   ktmcmc_cfg cfg;
-  int N = 0, ld = 0, lambda = 0, device = 0, num_sms = 148, L = 1;
-  uint64_t gen = 1, launches = 0;
+  int N = 0, ld = 0, lambda = 0, num_sms = 148, L = 1;
   std::vector<uint64_t> burn_in;
-  cudaStream_t stream = 0;
   int *dType = nullptr, *dCounts = nullptr, *dLeader = nullptr, *dLen = nullptr, *dDbStart = nullptr, *dFlag = nullptr, *dSlot = nullptr,
       *dAcc = nullptr, *dPerm = nullptr;
   double *dPa = nullptr, *dPb = nullptr, *dCoef = nullptr;
@@ -495,8 +493,6 @@ struct ktmcmc {
   double *dVT = nullptr, *dGT = nullptr, *dB = nullptr, *dA = nullptr, *dD = nullptr, *dSign = nullptr;
   long long s_rows = 0;
   DevScalars* dDsc = nullptr;
-  TmScalars* dSc = nullptr;
-  TmScalars* hSc = nullptr;          // pinned
   TridiagWs* tri = nullptr;
   // generation state on the host
   int chains = 0, steps = 0, step = 0, burn = 0, eval_rows = 0;
@@ -513,31 +509,23 @@ struct ktmcmc {
   ktmcmc_host_reference_fn host_ref_fn = nullptr; void* host_ref_user = nullptr;
   ktmcmc_device_reference_fn dev_ref_fn = nullptr; void* dev_ref_user = nullptr;
   std::vector<double> hX, hF, hG, hP;
-  std::string err, reason;
-  std::vector<void*> allocs;
+  ~ktmcmc() {
+    cudaSetDevice(device);
+    cudaStreamSynchronize(stream);
+    if (tri) tridiag_ws_destroy(tri);
+  }
 };
 
 namespace {
-char g_tm_err[512] = "";
-int tm_fail(ktmcmc* h, const char* fmt, ...) {
-  char buf[512];
-  va_list ap; va_start(ap, fmt);
-  vsnprintf(buf, sizeof(buf), fmt, ap);
-  va_end(ap);
-  if (h) h->err = buf; else snprintf(g_tm_err, sizeof(g_tm_err), "%s", buf);
-  return 1;
-}
-#define TM_CUDA(h, call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) return tm_fail(h, "CUDA error %s at %s:%d", cudaGetErrorString(e_), __FILE__, __LINE__); } while (0)
-template <typename T>
-cudaError_t tm_alloc(ktmcmc* h, T** p, size_t count) {
-  cudaError_t e = cudaMalloc((void**)p, sizeof(T) * (count ? count : 1));
-  if (e == cudaSuccess) { h->allocs.push_back(*p); e = cudaMemset(*p, 0, sizeof(T) * (count ? count : 1)); }
-  return e;
-}
+const HostScalar<ktmcmc> kHostScalars[] = {
+    {"Termination Criteria/Target Annealing Exponent", &ktmcmc::tc_target, true},
+    {"Termination Criteria/Max Generations", &ktmcmc::tc_max_generations, true},
+    {"Termination Criteria/Max Model Evaluations", &ktmcmc::tc_max_model_evaluations, true},
+};
+// every pull also reports a failed launch since the last one
 int tm_pull(ktmcmc* h) {
-  TM_CUDA(h, cudaMemcpyAsync(h->hSc, h->dSc, sizeof(TmScalars), cudaMemcpyDeviceToHost, h->stream));
-  TM_CUDA(h, cudaStreamSynchronize(h->stream));
-  TM_CUDA(h, cudaGetLastError());
+  if (pull(h)) return 1;
+  CUDA_OK(h, cudaGetLastError());
   return 0;
 }
 const char* tm_param_key(int lik) { return lik == KTMCMC_LIK_STUDENT_T ? "Degrees Of Freedom" : "Standard Deviation"; }
@@ -547,13 +535,13 @@ int tm_check_flags(ktmcmc* h) {
     const long long row = (long long)(e >> 2);
     const int code = (int)(e & 3);
     if (code == kRefNonFinite)
-      return tm_fail(h, "Bayesian/Reference: 'Reference Evaluations' of sample %lld contains a non-finite value\n", row);
+      return fail(h, "Bayesian/Reference: 'Reference Evaluations' of sample %lld contains a non-finite value\n", row);
     if (code == kRefParameter)
-      return tm_fail(h, "Bayesian/Reference: '%s' of sample %lld contains a value that is not positive and finite\n", tm_param_key(h->lik), row);
-    return tm_fail(h, "Bayesian/Reference: 'Reference Evaluations' of sample %lld contains a negative Poisson mean\n", row);
+      return fail(h, "Bayesian/Reference: '%s' of sample %lld contains a value that is not positive and finite\n", tm_param_key(h->lik), row);
+    return fail(h, "Bayesian/Reference: 'Reference Evaluations' of sample %lld contains a negative Poisson mean\n", row);
   }
-  if (h->hSc->nan_flag) return tm_fail(h, "A NaN log-likelihood was produced by the likelihood model\n");
-  if (h->hSc->allinf_flag) return tm_fail(h, "Every sample of the population has a log-likelihood of -inf: the annealing step is undefined\n");
+  if (h->hSc->nan_flag) return fail(h, "A NaN log-likelihood was produced by the likelihood model\n");
+  if (h->hSc->allinf_flag) return fail(h, "Every sample of the population has a log-likelihood of -inf: the annealing step is undefined\n");
   return 0;
 }
 }  // namespace
@@ -572,153 +560,139 @@ void ktmcmc_cfg_defaults(ktmcmc_cfg* c) {
   c->loglik = KCMA_OBJ_EXTERNAL;
 }
 
-const char* ktmcmc_last_error(const ktmcmc_t* h) { return h ? h->err.c_str() : g_tm_err; }
+const char* ktmcmc_last_error(const ktmcmc_t* h) { return h ? h->err.c_str() : ktmcmc::create_err; }
 
-void ktmcmc_destroy(ktmcmc_t* h) {
-  if (!h) return;
-  cudaSetDevice(h->device);
-  cudaStreamSynchronize(h->stream);
-  if (h->tri) tridiag_ws_destroy(h->tri);
-  for (void* p : h->allocs) cudaFree(p);
-  if (h->hSc) cudaFreeHost(h->hSc);
-  delete h;
-}
+void ktmcmc_destroy(ktmcmc_t* h) { delete h; }
 
 int ktmcmc_create(const ktmcmc_cfg* cfg, ktmcmc_t** out) {
-  if (!cfg || !out) return tm_fail(nullptr, "null argument");
-  if (cfg->abi_version != KTMCMC_ABI_VERSION) return tm_fail(nullptr, "ktmcmc_cfg ABI version mismatch");
-  if (cfg->n < 1) return tm_fail(nullptr, "Bayesian problems require at least one variable.\n");
-  if (cfg->population_size < 2) return tm_fail(nullptr, "Sampler/TMCMC: 'Population Size' must be at least 2 (got %zu)\n", (size_t)cfg->population_size);
-  if (cfg->population_size > (1u << 30)) return tm_fail(nullptr, "Sampler/TMCMC: 'Population Size' above 2^30 is not supported\n");
-  if (cfg->max_chain_length < 1) return tm_fail(nullptr, "Sampler/TMCMC: 'Max Chain Length' must be at least 1\n");
-  if (!(cfg->target_cov > 0.0)) return tm_fail(nullptr, "Sampler/TMCMC: 'Target Coefficient Of Variation' must be positive\n");
-  if (!(cfg->covariance_scaling > 0.0)) return tm_fail(nullptr, "Sampler/TMCMC: 'Covariance Scaling' must be positive\n");
+  if (!cfg || !out) return fail<ktmcmc>(nullptr, "null argument");
+  if (cfg->abi_version != KTMCMC_ABI_VERSION) return fail<ktmcmc>(nullptr, "ktmcmc_cfg ABI version mismatch");
+  if (cfg->n < 1) return fail<ktmcmc>(nullptr, "Bayesian problems require at least one variable.\n");
+  if (cfg->population_size < 2) return fail<ktmcmc>(nullptr, "Sampler/TMCMC: 'Population Size' must be at least 2 (got %zu)\n", (size_t)cfg->population_size);
+  if (cfg->population_size > (1u << 30)) return fail<ktmcmc>(nullptr, "Sampler/TMCMC: 'Population Size' above 2^30 is not supported\n");
+  if (cfg->max_chain_length < 1) return fail<ktmcmc>(nullptr, "Sampler/TMCMC: 'Max Chain Length' must be at least 1\n");
+  if (!(cfg->target_cov > 0.0)) return fail<ktmcmc>(nullptr, "Sampler/TMCMC: 'Target Coefficient Of Variation' must be positive\n");
+  if (!(cfg->covariance_scaling > 0.0)) return fail<ktmcmc>(nullptr, "Sampler/TMCMC: 'Covariance Scaling' must be positive\n");
   if (!(cfg->min_annealing_update > 0.0) || !(cfg->max_annealing_update >= cfg->min_annealing_update))
-    return tm_fail(nullptr, "Sampler/TMCMC: need 0 < 'Min Annealing Exponent Update' <= 'Max Annealing Exponent Update'\n");
-  if (!cfg->prior_type || !cfg->prior_a || !cfg->prior_b) return tm_fail(nullptr, "Sampler/TMCMC: every variable needs a prior distribution\n");
+    return fail<ktmcmc>(nullptr, "Sampler/TMCMC: need 0 < 'Min Annealing Exponent Update' <= 'Max Annealing Exponent Update'\n");
+  if (!cfg->prior_type || !cfg->prior_a || !cfg->prior_b) return fail<ktmcmc>(nullptr, "Sampler/TMCMC: every variable needs a prior distribution\n");
   const int N = (int)cfg->n;
   for (int d = 0; d < N; d++) {
     const int t = cfg->prior_type[d];
     const double a = cfg->prior_a[d], b = cfg->prior_b[d];
     if (t == KTMCMC_PRIOR_UNIFORM) {
-      if (!std::isfinite(a) || !std::isfinite(b) || !(b > a)) return tm_fail(nullptr, "Univariate/Uniform prior of variable %d: need finite Minimum < Maximum\n", d);
+      if (!std::isfinite(a) || !std::isfinite(b) || !(b > a)) return fail<ktmcmc>(nullptr, "Univariate/Uniform prior of variable %d: need finite Minimum < Maximum\n", d);
     } else if (t == KTMCMC_PRIOR_NORMAL) {
-      if (!std::isfinite(a) || !std::isfinite(b) || !(b > 0.0)) return tm_fail(nullptr, "Univariate/Normal prior of variable %d: need a finite Mean and a positive Standard Deviation\n", d);
-    } else return tm_fail(nullptr, "unknown prior type %d of variable %d", t, d);
+      if (!std::isfinite(a) || !std::isfinite(b) || !(b > 0.0)) return fail<ktmcmc>(nullptr, "Univariate/Normal prior of variable %d: need a finite Mean and a positive Standard Deviation\n", d);
+    } else return fail<ktmcmc>(nullptr, "unknown prior type %d of variable %d", t, d);
   }
   if (cfg->loglik != KCMA_OBJ_EXTERNAL && (cfg->loglik < KCMA_OBJ_NEG_SPHERE || cfg->loglik > KCMA_OBJ_NEG_SPHERE_SIN2))
-    return tm_fail(nullptr, "unknown log-likelihood model id %d", cfg->loglik);
-  if (!eigen_use_small(N) && !eigen_tridiag_fits(N)) return tm_fail(nullptr, "Sampler/TMCMC: n = %d is above the tridiagonal eigensolver's size\n", N);
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev <= 0) return tm_fail(nullptr, "no CUDA device: korali_b200 has no CPU fallback");
-  if (cfg->device < 0 || cfg->device >= ndev) return tm_fail(nullptr, "invalid device %d", cfg->device);
+    return fail<ktmcmc>(nullptr, "unknown log-likelihood model id %d", cfg->loglik);
+  if (!eigen_use_small(N) && !eigen_tridiag_fits(N)) return fail<ktmcmc>(nullptr, "Sampler/TMCMC: n = %d is above the tridiagonal eigensolver's size\n", N);
+  if (open_device<ktmcmc>(cfg->device)) return 1;
   ktmcmc* h = new ktmcmc();
   h->cfg = *cfg;
   h->burn_in.assign(cfg->per_generation_burn_in, cfg->per_generation_burn_in + (cfg->per_generation_burn_in ? cfg->burn_in_count : 0));
   h->cfg.per_generation_burn_in = nullptr; h->cfg.prior_type = nullptr; h->cfg.prior_a = h->cfg.prior_b = h->cfg.loglik_coef = nullptr;
   h->N = N; h->ld = (N + 15) / 16 * 16; h->lambda = (int)cfg->population_size; h->device = cfg->device;
   h->L = (int)std::min<uint64_t>(cfg->max_chain_length, cfg->population_size);
-#define CREATE_CUDA(call) do { cudaError_t e_ = (call); if (e_ != cudaSuccess) { tm_fail(nullptr, "CUDA error %s at %s:%d", cudaGetErrorString(e_), __FILE__, __LINE__); ktmcmc_destroy(h); return 1; } } while (0)
-  CREATE_CUDA(cudaSetDevice(h->device));
   cudaDeviceGetAttribute(&h->num_sms, cudaDevAttrMultiProcessorCount, h->device);
   const size_t ld = h->ld, lam = h->lambda, rows = (lam + 15) / 16 * 16 + 16;
   h->s_rows = (long long)rows;
-  CREATE_CUDA(tm_alloc(h, &h->dType, N)); CREATE_CUDA(tm_alloc(h, &h->dPa, N)); CREATE_CUDA(tm_alloc(h, &h->dPb, N)); CREATE_CUDA(tm_alloc(h, &h->dCoef, N));
-  for (double** p : {&h->dX, &h->dDX, &h->dCX, &h->dZ, &h->dY, &h->dXP, &h->dEX, &h->dS}) CREATE_CUDA(tm_alloc(h, p, rows * ld));
-  for (double** p : {&h->dLL, &h->dLP, &h->dDLL, &h->dDLP, &h->dCLL, &h->dCLP, &h->dLPP, &h->dEF, &h->dW, &h->dCum}) CREATE_CUDA(tm_alloc(h, p, lam));
-  for (int** p : {&h->dCounts, &h->dLeader, &h->dLen, &h->dDbStart, &h->dFlag, &h->dSlot, &h->dAcc}) CREATE_CUDA(tm_alloc(h, p, lam));
-  CREATE_CUDA(tm_alloc(h, &h->dPerm, 2 * (size_t)N + 64));
-  CREATE_CUDA(tm_alloc(h, &h->dPart, (size_t)kMeanChunks * ld)); CREATE_CUDA(tm_alloc(h, &h->dMean, ld));
-  CREATE_CUDA(tm_alloc(h, &h->dWs, (size_t)16 * N * ld));
-  for (double** p : {&h->dP, &h->dCov, &h->dVT, &h->dGT, &h->dB, &h->dA}) CREATE_CUDA(tm_alloc(h, p, (size_t)N * ld));
-  CREATE_CUDA(tm_alloc(h, &h->dD, ld)); CREATE_CUDA(tm_alloc(h, &h->dSign, ld));
-  CREATE_CUDA(tm_alloc(h, &h->dDsc, 1)); CREATE_CUDA(tm_alloc(h, &h->dSc, 1));
-  CREATE_CUDA(cudaMallocHost((void**)&h->hSc, sizeof(TmScalars)));
-  memset(h->hSc, 0, sizeof(TmScalars));
+  CREATE_OK(h, alloc(h->mem, &h->dType, N)); CREATE_OK(h, alloc(h->mem, &h->dPa, N)); CREATE_OK(h, alloc(h->mem, &h->dPb, N)); CREATE_OK(h, alloc(h->mem, &h->dCoef, N));
+  for (double** p : {&h->dX, &h->dDX, &h->dCX, &h->dZ, &h->dY, &h->dXP, &h->dEX, &h->dS}) CREATE_OK(h, alloc(h->mem, p, rows * ld));
+  for (double** p : {&h->dLL, &h->dLP, &h->dDLL, &h->dDLP, &h->dCLL, &h->dCLP, &h->dLPP, &h->dEF, &h->dW, &h->dCum}) CREATE_OK(h, alloc(h->mem, p, lam));
+  for (int** p : {&h->dCounts, &h->dLeader, &h->dLen, &h->dDbStart, &h->dFlag, &h->dSlot, &h->dAcc}) CREATE_OK(h, alloc(h->mem, p, lam));
+  CREATE_OK(h, alloc(h->mem, &h->dPerm, 2 * (size_t)N + 64));
+  CREATE_OK(h, alloc(h->mem, &h->dPart, (size_t)kMeanChunks * ld)); CREATE_OK(h, alloc(h->mem, &h->dMean, ld));
+  CREATE_OK(h, alloc(h->mem, &h->dWs, (size_t)16 * N * ld));
+  for (double** p : {&h->dP, &h->dCov, &h->dVT, &h->dGT, &h->dB, &h->dA}) CREATE_OK(h, alloc(h->mem, p, (size_t)N * ld));
+  CREATE_OK(h, alloc(h->mem, &h->dD, ld)); CREATE_OK(h, alloc(h->mem, &h->dSign, ld));
+  CREATE_OK(h, alloc(h->mem, &h->dDsc, 1)); CREATE_OK(h, alloc(h->mem, &h->dSc, 1));
+  CREATE_OK(h, alloc_host(h->mem, &h->hSc, 1));
   std::vector<int> type(cfg->prior_type, cfg->prior_type + N);
   std::vector<double> coef(N);
   for (int d = 0; d < N; d++) coef[d] = cfg->loglik_coef ? cfg->loglik_coef[d] : pow(10.0, 6.0 * d / (double)std::max(N - 1, 1));
-  CREATE_CUDA(cudaMemcpy(h->dType, type.data(), sizeof(int) * N, cudaMemcpyHostToDevice));
-  CREATE_CUDA(cudaMemcpy(h->dPa, cfg->prior_a, sizeof(double) * N, cudaMemcpyHostToDevice));
-  CREATE_CUDA(cudaMemcpy(h->dPb, cfg->prior_b, sizeof(double) * N, cudaMemcpyHostToDevice));
-  CREATE_CUDA(cudaMemcpy(h->dCoef, coef.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
+  CREATE_OK(h, cudaMemcpy(h->dType, type.data(), sizeof(int) * N, cudaMemcpyHostToDevice));
+  CREATE_OK(h, cudaMemcpy(h->dPa, cfg->prior_a, sizeof(double) * N, cudaMemcpyHostToDevice));
+  CREATE_OK(h, cudaMemcpy(h->dPb, cfg->prior_b, sizeof(double) * N, cudaMemcpyHostToDevice));
+  CREATE_OK(h, cudaMemcpy(h->dCoef, coef.data(), sizeof(double) * N, cudaMemcpyHostToDevice));
   DevScalars ds; memset(&ds, 0, sizeof(ds)); ds.sigma = 1.0;
-  CREATE_CUDA(cudaMemcpy(h->dDsc, &ds, sizeof(ds), cudaMemcpyHostToDevice));
+  CREATE_OK(h, cudaMemcpy(h->dDsc, &ds, sizeof(ds), cudaMemcpyHostToDevice));
   launch_set_identity(h->stream, h->dVT, (int)ld, N);
   launch_set_identity(h->stream, h->dB, (int)ld, N);
   if (!eigen_use_small(N)) {
     char msg[512] = "";
     h->tri = tridiag_ws_create(N, (int)ld, h->num_sms, msg, sizeof(msg));
-    if (!h->tri) { tm_fail(nullptr, "%s", msg); ktmcmc_destroy(h); return 1; }
+    if (!h->tri) return create_fail(h, "%s", msg);
   }
-  CREATE_CUDA(cudaStreamSynchronize(h->stream));
-  CREATE_CUDA(cudaGetLastError());
-#undef CREATE_CUDA
+  CREATE_OK(h, cudaStreamSynchronize(h->stream));
+  CREATE_OK(h, cudaGetLastError());
   *out = h;
   return 0;
 }
 
 int ktmcmc_set_host_loglik(ktmcmc_t* h, ktmcmc_host_loglik_fn fn, void* user) {
-  if (!h) return tm_fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   h->host_fn = fn; h->host_user = user;
   return 0;
 }
 int ktmcmc_set_device_loglik(ktmcmc_t* h, kcma_device_objective_fn fn, void* user) {
-  if (!h) return tm_fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   h->dev_fn = fn; h->dev_user = user;
   return 0;
 }
 
 int ktmcmc_set_reference(ktmcmc_t* h, int32_t likelihood, const double* data, uint64_t m) {
-  if (!h) return tm_fail(nullptr, "null solver handle");
-  if (h->lik) return tm_fail(h, "set_reference: the reference data are already set");
-  if (h->gen != 1 || h->proposed) return tm_fail(h, "set_reference: call it before generation 1");
-  if (h->cfg.loglik != KCMA_OBJ_EXTERNAL) return tm_fail(h, "set_reference: the log-likelihood must be External (KCMA_OBJ_EXTERNAL)");
-  if (likelihood < KTMCMC_LIK_NORMAL || likelihood > KTMCMC_LIK_POISSON) return tm_fail(h, "set_reference: unknown likelihood %d", likelihood);
-  if (!data || m < 1 || m > (uint64_t)INT32_MAX) return tm_fail(h, "set_reference: need 1 <= m < 2^31 reference data (got %zu)", (size_t)m);
+  if (!h) return fail(h, "null solver handle");
+  if (h->lik) return fail(h, "set_reference: the reference data are already set");
+  if (h->gen != 1 || h->proposed) return fail(h, "set_reference: call it before generation 1");
+  if (h->cfg.loglik != KCMA_OBJ_EXTERNAL) return fail(h, "set_reference: the log-likelihood must be External (KCMA_OBJ_EXTERNAL)");
+  if (likelihood < KTMCMC_LIK_NORMAL || likelihood > KTMCMC_LIK_POISSON) return fail(h, "set_reference: unknown likelihood %d", likelihood);
+  if (!data || m < 1 || m > (uint64_t)INT32_MAX) return fail(h, "set_reference: need 1 <= m < 2^31 reference data (got %zu)", (size_t)m);
   std::vector<double> dc(m, 0.0);
   for (uint64_t j = 0; j < m; j++) {
     const double d = data[j];
-    if (!std::isfinite(d)) return tm_fail(h, "Bayesian/Reference: 'Reference Data' %zu is not finite\n", (size_t)j);
+    if (!std::isfinite(d)) return fail(h, "Bayesian/Reference: 'Reference Data' %zu is not finite\n", (size_t)j);
     if (likelihood == KTMCMC_LIK_POISSON && (d < 0.0 || d != floor(d)))
-      return tm_fail(h, "Bayesian/Reference: 'Reference Data' %zu (%g) must be a non-negative integer for the Poisson likelihood\n", (size_t)j, d);
+      return fail(h, "Bayesian/Reference: 'Reference Data' %zu (%g) must be a non-negative integer for the Poisson likelihood\n", (size_t)j, d);
     if (likelihood == KTMCMC_LIK_POSITIVE_NORMAL && d < 0.0)
-      return tm_fail(h, "Bayesian/Reference: 'Reference Data' %zu (%g) must be >= 0 for the Positive Normal likelihood\n", (size_t)j, d);
+      return fail(h, "Bayesian/Reference: 'Reference Data' %zu (%g) must be >= 0 for the Positive Normal likelihood\n", (size_t)j, d);
     if (likelihood == KTMCMC_LIK_POISSON) dc[j] = lgamma(d + 1.0);
   }
-  TM_CUDA(h, cudaSetDevice(h->device));
+  CUDA_OK(h, cudaSetDevice(h->device));
   const long long ldm = ((long long)m + 3) / 4 * 4;   // 32-byte aligned rows
   const bool param = likelihood != KTMCMC_LIK_POISSON;
   const size_t each = (size_t)h->s_rows * ldm;
   const double gib = (double)each * sizeof(double) * (param ? 2 : 1) / (double)(1ull << 30);
-  if (tm_alloc(h, &h->dG, each) != cudaSuccess || (param && tm_alloc(h, &h->dPr, each) != cudaSuccess)) {
+  if (alloc(h->mem, &h->dG, each) != cudaSuccess || (param && alloc(h->mem, &h->dPr, each) != cudaSuccess)) {
     cudaGetLastError();
-    return tm_fail(h, "Bayesian/Reference: cannot allocate the model outputs of %d samples x %zu reference points (%.2f GiB)\n", h->lambda,
+    return fail(h, "Bayesian/Reference: cannot allocate the model outputs of %d samples x %zu reference points (%.2f GiB)\n", h->lambda,
                    (size_t)m, gib);
   }
-  TM_CUDA(h, tm_alloc(h, &h->dData, m));
-  TM_CUDA(h, tm_alloc(h, &h->dDataC, m));
-  TM_CUDA(h, cudaMemcpy(h->dData, data, sizeof(double) * m, cudaMemcpyHostToDevice));
-  TM_CUDA(h, cudaMemcpy(h->dDataC, dc.data(), sizeof(double) * m, cudaMemcpyHostToDevice));
+  CUDA_OK(h, alloc(h->mem, &h->dData, m));
+  CUDA_OK(h, alloc(h->mem, &h->dDataC, m));
+  CUDA_OK(h, cudaMemcpy(h->dData, data, sizeof(double) * m, cudaMemcpyHostToDevice));
+  CUDA_OK(h, cudaMemcpy(h->dDataC, dc.data(), sizeof(double) * m, cudaMemcpyHostToDevice));
   h->lik = likelihood; h->m = (long long)m; h->ldm = ldm;
   return 0;
 }
 int ktmcmc_set_host_reference_model(ktmcmc_t* h, ktmcmc_host_reference_fn fn, void* user) {
-  if (!h) return tm_fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   h->host_ref_fn = fn; h->host_ref_user = user;
   return 0;
 }
 int ktmcmc_set_device_reference_model(ktmcmc_t* h, ktmcmc_device_reference_fn fn, void* user) {
-  if (!h) return tm_fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   h->dev_ref_fn = fn; h->dev_ref_user = user;
   return 0;
 }
 
 // steps 1-3
 int ktmcmc_anneal(ktmcmc_t* h) {
-  if (!h) return tm_fail(nullptr, "null solver handle");
-  if (h->gen < 2 || h->in_generation) return tm_fail(h, "anneal: expected the start of a generation after the first");
-  TM_CUDA(h, cudaSetDevice(h->device));
+  if (!h) return fail(h, "null solver handle");
+  if (h->gen < 2 || h->in_generation) return fail(h, "anneal: expected the start of a generation after the first");
+  CUDA_OK(h, cudaSetDevice(h->device));
   const int N = h->N, ld = h->ld, lam = h->lambda;
   cudaStream_t st = h->stream;
   tm_anneal_kernel<<<1, kThreads, 0, st>>>(h->dLL, lam, h->cfg.target_cov, h->cfg.min_annealing_update, h->cfg.max_annealing_update, h->dW, h->dCum, h->dSc);
@@ -737,13 +711,13 @@ int ktmcmc_anneal(ktmcmc_t* h) {
     double *vt = nullptr, *ev = nullptr;
     int l = 0;
     if (!launch_eigen_tridiag(st, h->tri, h->dCov, &vt, &ev, &l))
-      return tm_fail(h, "the tridiagonal eigensolver could not be launched: %s", cudaGetErrorString(cudaGetLastError()));
+      return fail(h, "the tridiagonal eigensolver could not be launched: %s", cudaGetErrorString(cudaGetLastError()));
     launch_eig_sign(st, vt, ld, N, h->dSign);
     launch_eig_order(st, ev, N, h->dPerm, h->dDsc);
     tm_commit_kernel<<<dim3((N + 127) / 128, N), 128, 0, st>>>(vt, ld, N, h->dPerm, ev, h->dSign, h->dA);
     h->launches += l + 4;
   }
-  TM_CUDA(h, cudaGetLastError());
+  CUDA_OK(h, cudaGetLastError());
   h->in_generation = true;
   h->chains = 0;
   return 0;
@@ -751,12 +725,12 @@ int ktmcmc_anneal(ktmcmc_t* h) {
 
 // step 4; reads the chain count and the longest chain (the number of MCMC steps)
 int ktmcmc_resample(ktmcmc_t* h) {
-  if (!h) return tm_fail(nullptr, "null solver handle");
-  if (!h->in_generation || h->chains) return tm_fail(h, "resample: call ktmcmc_anneal first");
-  TM_CUDA(h, cudaSetDevice(h->device));
+  if (!h) return fail(h, "null solver handle");
+  if (!h->in_generation || h->chains) return fail(h, "resample: call ktmcmc_anneal first");
+  CUDA_OK(h, cudaSetDevice(h->device));
   const int lam = h->lambda;
   cudaStream_t st = h->stream;
-  TM_CUDA(h, cudaMemsetAsync(h->dCounts, 0, sizeof(int) * lam, st));
+  CUDA_OK(h, cudaMemsetAsync(h->dCounts, 0, sizeof(int) * lam, st));
   tm_draw_kernel<<<grid_for(lam, 256), 256, 0, st>>>(h->dCum, lam, h->cfg.seed, (unsigned)h->gen, h->dSc, h->dCounts);
   tm_chains_kernel<<<1, kThreads, 0, st>>>(h->dCounts, lam, h->L, h->dLeader, h->dLen, h->dDbStart, h->dSc);
   tm_chain_init_kernel<<<grid_for((long long)lam * 32, 256), 256, 0, st>>>(h->dSc, h->dLeader, h->dX, h->dLL, h->dLP, h->ld, h->N, h->dCX, h->dCLL, h->dCLP);
@@ -772,17 +746,17 @@ int ktmcmc_resample(ktmcmc_t* h) {
 }
 
 int ktmcmc_propose(ktmcmc_t* h) {
-  if (!h) return tm_fail(nullptr, "null solver handle");
-  TM_CUDA(h, cudaSetDevice(h->device));
+  if (!h) return fail(h, "null solver handle");
+  CUDA_OK(h, cudaSetDevice(h->device));
   const int N = h->N, ld = h->ld;
   cudaStream_t st = h->stream;
   if (h->gen == 1) {
-    if (h->proposed) return tm_fail(h, "propose: the prior draws of generation 1 are waiting for eval / accept");
+    if (h->proposed) return fail(h, "propose: the prior draws of generation 1 are waiting for eval / accept");
     tm_prior_kernel<<<grid_for((long long)h->lambda * 32, 256), 256, 0, st>>>(N, h->lambda, h->cfg.seed, h->dType, h->dPa, h->dPb, h->dEX, ld, h->dLP);
     h->launches++;
     h->eval_rows = h->lambda;
   } else {
-    if (!h->in_generation || !h->chains || h->step >= h->steps || h->proposed) return tm_fail(h, "propose: no MCMC step pending (anneal and resample first)");
+    if (!h->in_generation || !h->chains || h->step >= h->steps || h->proposed) return fail(h, "propose: no MCMC step pending (anneal and resample first)");
     const int K = h->chains;
     const long long pairs = (long long)K * ((N + 1) / 2);
     tm_z_kernel<<<std::min(grid_for(pairs, 256), (unsigned)h->num_sms * 16), 256, 0, st>>>(h->dZ, ld, K, N, h->cfg.seed, (unsigned)h->step, (unsigned)h->gen);
@@ -794,55 +768,55 @@ int ktmcmc_propose(ktmcmc_t* h) {
     h->launches += 5;
     h->eval_rows = -1;   // known on the device; read only when a host or device conduit needs it
   }
-  TM_CUDA(h, cudaGetLastError());
+  CUDA_OK(h, cudaGetLastError());
   h->proposed = true;
   h->evaluated = false;
   return 0;
 }
 
 int ktmcmc_inject_loglik(ktmcmc_t* h, const double* l, size_t count) {
-  if (!h) return tm_fail(nullptr, "null solver handle");
-  if (!h->proposed || h->evaluated) return tm_fail(h, "inject_loglik: no proposals waiting for an evaluation");
-  TM_CUDA(h, cudaSetDevice(h->device));
+  if (!h) return fail(h, "null solver handle");
+  if (!h->proposed || h->evaluated) return fail(h, "inject_loglik: no proposals waiting for an evaluation");
+  CUDA_OK(h, cudaSetDevice(h->device));
   if (h->eval_rows < 0) { if (tm_pull(h)) return 1; h->eval_rows = (int)h->hSc->step_evals; }
-  if (count != (size_t)h->eval_rows) return tm_fail(h, "inject_loglik: %zu values for %d evaluation rows", count, h->eval_rows);
-  if (count) TM_CUDA(h, cudaMemcpyAsync(h->dEF, l, sizeof(double) * count, cudaMemcpyHostToDevice, h->stream));
-  TM_CUDA(h, cudaStreamSynchronize(h->stream));
+  if (count != (size_t)h->eval_rows) return fail(h, "inject_loglik: %zu values for %d evaluation rows", count, h->eval_rows);
+  if (count) CUDA_OK(h, cudaMemcpyAsync(h->dEF, l, sizeof(double) * count, cudaMemcpyHostToDevice, h->stream));
+  CUDA_OK(h, cudaStreamSynchronize(h->stream));
   h->have_inj = true;
   return 0;
 }
 
 int ktmcmc_inject_reference(ktmcmc_t* h, const double* g, const double* p, size_t count) {
-  if (!h) return tm_fail(nullptr, "null solver handle");
-  if (!h->lik) return tm_fail(h, "inject_reference: no reference data (ktmcmc_set_reference)");
-  if (!h->proposed || h->evaluated) return tm_fail(h, "inject_reference: no proposals waiting for an evaluation");
-  if (!g || (h->lik != KTMCMC_LIK_POISSON) != (p != nullptr)) return tm_fail(h, "inject_reference: need g, and p exactly when the likelihood has a parameter");
-  TM_CUDA(h, cudaSetDevice(h->device));
+  if (!h) return fail(h, "null solver handle");
+  if (!h->lik) return fail(h, "inject_reference: no reference data (ktmcmc_set_reference)");
+  if (!h->proposed || h->evaluated) return fail(h, "inject_reference: no proposals waiting for an evaluation");
+  if (!g || (h->lik != KTMCMC_LIK_POISSON) != (p != nullptr)) return fail(h, "inject_reference: need g, and p exactly when the likelihood has a parameter");
+  CUDA_OK(h, cudaSetDevice(h->device));
   if (h->eval_rows < 0) { if (tm_pull(h)) return 1; h->eval_rows = (int)h->hSc->step_evals; }
-  if (count != (size_t)h->eval_rows * h->m) return tm_fail(h, "inject_reference: %zu values for %d evaluation rows x %lld", count, h->eval_rows, h->m);
+  if (count != (size_t)h->eval_rows * h->m) return fail(h, "inject_reference: %zu values for %d evaluation rows x %lld", count, h->eval_rows, h->m);
   const size_t row = sizeof(double) * h->m, pitch = sizeof(double) * h->ldm;
   if (count) {
-    TM_CUDA(h, cudaMemcpy2DAsync(h->dG, pitch, g, row, row, h->eval_rows, cudaMemcpyHostToDevice, h->stream));
-    if (p) TM_CUDA(h, cudaMemcpy2DAsync(h->dPr, pitch, p, row, row, h->eval_rows, cudaMemcpyHostToDevice, h->stream));
+    CUDA_OK(h, cudaMemcpy2DAsync(h->dG, pitch, g, row, row, h->eval_rows, cudaMemcpyHostToDevice, h->stream));
+    if (p) CUDA_OK(h, cudaMemcpy2DAsync(h->dPr, pitch, p, row, row, h->eval_rows, cudaMemcpyHostToDevice, h->stream));
   }
-  TM_CUDA(h, cudaStreamSynchronize(h->stream));
+  CUDA_OK(h, cudaStreamSynchronize(h->stream));
   h->have_ref_inj = true;
   return 0;
 }
 
 int ktmcmc_inject_factor(ktmcmc_t* h, const double* a, size_t count) {
-  if (!h) return tm_fail(nullptr, "null solver handle");
-  if (count != (size_t)h->N * h->N) return tm_fail(h, "inject_factor: %zu values for %d x %d", count, h->N, h->N);
-  TM_CUDA(h, cudaSetDevice(h->device));
-  TM_CUDA(h, cudaMemcpy2DAsync(h->dA, sizeof(double) * h->ld, a, sizeof(double) * h->N, sizeof(double) * h->N, h->N, cudaMemcpyHostToDevice, h->stream));
-  TM_CUDA(h, cudaStreamSynchronize(h->stream));
+  if (!h) return fail(h, "null solver handle");
+  if (count != (size_t)h->N * h->N) return fail(h, "inject_factor: %zu values for %d x %d", count, h->N, h->N);
+  CUDA_OK(h, cudaSetDevice(h->device));
+  CUDA_OK(h, cudaMemcpy2DAsync(h->dA, sizeof(double) * h->ld, a, sizeof(double) * h->N, sizeof(double) * h->N, h->N, cudaMemcpyHostToDevice, h->stream));
+  CUDA_OK(h, cudaStreamSynchronize(h->stream));
   return 0;
 }
 
 int ktmcmc_eval(ktmcmc_t* h) {
-  if (!h) return tm_fail(nullptr, "null solver handle");
-  if (!h->proposed || h->evaluated) return tm_fail(h, "eval: call ktmcmc_propose first");
-  TM_CUDA(h, cudaSetDevice(h->device));
+  if (!h) return fail(h, "null solver handle");
+  if (!h->proposed || h->evaluated) return fail(h, "eval: call ktmcmc_propose first");
+  CUDA_OK(h, cudaSetDevice(h->device));
   const int N = h->N, ld = h->ld;
   cudaStream_t st = h->stream;
   h->ef_rows = h->eval_rows;
@@ -861,13 +835,13 @@ int ktmcmc_eval(ktmcmc_t* h) {
     } else if (rows > 0 && h->host_ref_fn) {
       const size_t row = sizeof(double) * m, pitch = sizeof(double) * ldm;
       h->hX.resize((size_t)rows * N); h->hG.resize((size_t)rows * m); h->hP.resize(dp ? (size_t)rows * m : 0);
-      TM_CUDA(h, cudaMemcpy2DAsync(h->hX.data(), sizeof(double) * N, h->dEX, sizeof(double) * ld, sizeof(double) * N, rows, cudaMemcpyDeviceToHost, st));
-      TM_CUDA(h, cudaStreamSynchronize(st));
+      CUDA_OK(h, cudaMemcpy2DAsync(h->hX.data(), sizeof(double) * N, h->dEX, sizeof(double) * ld, sizeof(double) * N, rows, cudaMemcpyDeviceToHost, st));
+      CUDA_OK(h, cudaStreamSynchronize(st));
       h->host_ref_fn(h->host_ref_user, h->hX.data(), (uint64_t)rows, (uint64_t)N, h->hG.data(), dp ? h->hP.data() : nullptr, (uint64_t)m);
-      TM_CUDA(h, cudaMemcpy2DAsync(h->dG, pitch, h->hG.data(), row, row, rows, cudaMemcpyHostToDevice, st));
-      if (dp) TM_CUDA(h, cudaMemcpy2DAsync(dp, pitch, h->hP.data(), row, row, rows, cudaMemcpyHostToDevice, st));
+      CUDA_OK(h, cudaMemcpy2DAsync(h->dG, pitch, h->hG.data(), row, row, rows, cudaMemcpyHostToDevice, st));
+      if (dp) CUDA_OK(h, cudaMemcpy2DAsync(dp, pitch, h->hP.data(), row, row, rows, cudaMemcpyHostToDevice, st));
     } else if (rows > 0) {
-      return tm_fail(h, "Bayesian/Reference: inject the model outputs or set a host / device computational model before eval");
+      return fail(h, "Bayesian/Reference: inject the model outputs or set a host / device computational model before eval");
     }
     if (rows > 0) {
       switch (h->lik) {
@@ -890,30 +864,30 @@ int ktmcmc_eval(ktmcmc_t* h) {
         h->dev_fn(h->dev_user, h->dEX, (uint64_t)rows, (uint64_t)N, (uint64_t)ld, h->dEF, (void*)st);
       } else {
         h->hX.resize((size_t)rows * N); h->hF.resize(rows);
-        TM_CUDA(h, cudaMemcpy2DAsync(h->hX.data(), sizeof(double) * N, h->dEX, sizeof(double) * ld, sizeof(double) * N, rows, cudaMemcpyDeviceToHost, st));
-        TM_CUDA(h, cudaStreamSynchronize(st));
+        CUDA_OK(h, cudaMemcpy2DAsync(h->hX.data(), sizeof(double) * N, h->dEX, sizeof(double) * ld, sizeof(double) * N, rows, cudaMemcpyDeviceToHost, st));
+        CUDA_OK(h, cudaStreamSynchronize(st));
         h->host_fn(h->host_user, h->hX.data(), (uint64_t)rows, (uint64_t)N, h->hF.data());
-        TM_CUDA(h, cudaMemcpyAsync(h->dEF, h->hF.data(), sizeof(double) * rows, cudaMemcpyHostToDevice, st));
+        CUDA_OK(h, cudaMemcpyAsync(h->dEF, h->hF.data(), sizeof(double) * rows, cudaMemcpyHostToDevice, st));
       }
     }
   } else {
-    return tm_fail(h, "the log-likelihood is External: inject the values or set a host / device model before eval");
+    return fail(h, "the log-likelihood is External: inject the values or set a host / device model before eval");
   }
-  TM_CUDA(h, cudaGetLastError());
+  CUDA_OK(h, cudaGetLastError());
   h->evaluated = true;
   return 0;
 }
 
 int ktmcmc_accept(ktmcmc_t* h) {
-  if (!h) return tm_fail(nullptr, "null solver handle");
-  if (!h->evaluated) return tm_fail(h, "accept: call ktmcmc_eval first");
-  TM_CUDA(h, cudaSetDevice(h->device));
+  if (!h) return fail(h, "null solver handle");
+  if (!h->evaluated) return fail(h, "accept: call ktmcmc_eval first");
+  CUDA_OK(h, cudaSetDevice(h->device));
   const int N = h->N, ld = h->ld, lam = h->lambda;
   cudaStream_t st = h->stream;
   h->proposed = h->evaluated = false;
   if (h->gen == 1) {
-    TM_CUDA(h, cudaMemcpyAsync(h->dX, h->dEX, sizeof(double) * lam * ld, cudaMemcpyDeviceToDevice, st));
-    TM_CUDA(h, cudaMemcpyAsync(h->dLL, h->dEF, sizeof(double) * lam, cudaMemcpyDeviceToDevice, st));
+    CUDA_OK(h, cudaMemcpyAsync(h->dX, h->dEX, sizeof(double) * lam * ld, cudaMemcpyDeviceToDevice, st));
+    CUDA_OK(h, cudaMemcpyAsync(h->dLL, h->dEF, sizeof(double) * lam, cudaMemcpyDeviceToDevice, st));
     tm_check_nan_kernel<<<grid_for(lam, 256), 256, 0, st>>>(h->dLL, lam, h->dSc);
     h->launches++;
     h->init_evals = lam;
@@ -926,7 +900,7 @@ int ktmcmc_accept(ktmcmc_t* h) {
                                                                     h->dSlot, h->dXP, h->dLPP, h->dEF, h->dCX, h->dCLL, h->dCLP, h->dDX, h->dDLL,
                                                                     h->dDLP, h->dAcc, h->dSc);
   h->launches++;
-  TM_CUDA(h, cudaGetLastError());
+  CUDA_OK(h, cudaGetLastError());
   if (++h->step < h->steps) return 0;
   std::swap(h->dX, h->dDX); std::swap(h->dLL, h->dDLL); std::swap(h->dLP, h->dDLP);
   h->in_generation = false;
@@ -936,7 +910,7 @@ int ktmcmc_accept(ktmcmc_t* h) {
 }
 
 int ktmcmc_run_generation(ktmcmc_t* h) {
-  if (!h) return tm_fail(nullptr, "null solver handle");
+  if (!h) return fail(h, "null solver handle");
   if (h->gen == 1) return ktmcmc_propose(h) || ktmcmc_eval(h) || ktmcmc_accept(h);
   if (ktmcmc_anneal(h) || ktmcmc_resample(h)) return 1;
   while (h->in_generation)
@@ -945,8 +919,9 @@ int ktmcmc_run_generation(ktmcmc_t* h) {
 }
 
 int ktmcmc_check_termination(ktmcmc_t* h, int* finished, const char** reason) {
-  if (!h || !finished) return tm_fail(h, "null argument");
-  TM_CUDA(h, cudaSetDevice(h->device));
+  if (!h) return fail(h, "null solver handle");
+  if (!finished) return fail(h, "null argument");
+  CUDA_OK(h, cudaSetDevice(h->device));
   if (tm_pull(h)) return 1;
   h->reason.clear();
   int fin = 0;
@@ -959,66 +934,46 @@ int ktmcmc_check_termination(ktmcmc_t* h, int* finished, const char** reason) {
 }
 
 int ktmcmc_run(ktmcmc_t* h, uint64_t max_generations, uint64_t* done) {
-  if (!h) return tm_fail(nullptr, "null solver handle");
-  uint64_t g = 0;
-  for (; g < max_generations; g++) {
-    int fin; const char* why;
-    if (ktmcmc_check_termination(h, &fin, &why)) return 1;
-    if (fin) break;
-    if (ktmcmc_run_generation(h)) return 1;
-  }
-  if (done) *done = g;
-  return 0;
+  return run(h, max_generations, done, ktmcmc_check_termination, ktmcmc_run_generation);
 }
 
 int ktmcmc_get_array(ktmcmc_t* h, const char* key, double* out, size_t cap, size_t* count) {
-  if (!h || !key) return tm_fail(h, "null argument");
-  TM_CUDA(h, cudaSetDevice(h->device));
-  TM_CUDA(h, cudaStreamSynchronize(h->stream));
-  const size_t N = h->N, ld = h->ld, lam = h->lambda;
-  const double* src = nullptr;
-  const int* isrc = nullptr;
-  size_t rows = 0, width = 1, pitch = 1;
-  if (!strcmp(key, "Sample Database")) { src = h->dX; rows = lam; width = N; pitch = ld; }
-  else if (!strcmp(key, "Sample LogLikelihood Database")) { src = h->dLL; rows = lam; }
-  else if (!strcmp(key, "Sample LogPrior Database")) { src = h->dLP; rows = lam; }
-  else if (!strcmp(key, "Covariance Matrix")) { src = h->dCov; rows = N; width = N; pitch = ld; }
-  else if (!strcmp(key, "Proposal Factor")) { src = h->dA; rows = N; width = N; pitch = ld; }
-  else if (!strcmp(key, "Mean Theta")) { src = h->dMean; rows = 1; width = N; pitch = ld; }
-  else if (!strcmp(key, "Weights")) { src = h->dW; rows = lam; }
-  else if (!strcmp(key, "Selection Counts")) { isrc = h->dCounts; rows = lam; }
-  else if (!strcmp(key, "Chain Leaders")) { isrc = h->dLeader; rows = h->chains; }
-  else if (!strcmp(key, "Chain Lengths")) { isrc = h->dLen; rows = h->chains; }
-  else if (!strcmp(key, "Proposal Support")) { isrc = h->dFlag; rows = h->chains; }
-  else if (!strcmp(key, "Accept Flags")) { isrc = h->dAcc; rows = h->chains; }
+  if (!h) return fail(h, "null solver handle");
+  if (!key) return fail(h, "null argument");
+  CUDA_OK(h, cudaSetDevice(h->device));
+  CUDA_OK(h, cudaStreamSynchronize(h->stream));
+  const size_t N = h->N, ld = h->ld, lam = h->lambda, chains = h->chains;
+  Array r;
+  if (!strcmp(key, "Sample Database")) r = pitched(h->dX, lam, N, ld);
+  else if (!strcmp(key, "Sample LogLikelihood Database")) r = dense(h->dLL, lam);
+  else if (!strcmp(key, "Sample LogPrior Database")) r = dense(h->dLP, lam);
+  else if (!strcmp(key, "Covariance Matrix")) r = pitched(h->dCov, N, N, ld);
+  else if (!strcmp(key, "Proposal Factor")) r = pitched(h->dA, N, N, ld);
+  else if (!strcmp(key, "Mean Theta")) r = dense(h->dMean, N);
+  else if (!strcmp(key, "Weights")) r = dense(h->dW, lam);
+  else if (!strcmp(key, "Selection Counts")) r = dense(h->dCounts, lam, Elem::i32);
+  else if (!strcmp(key, "Chain Leaders")) r = dense(h->dLeader, chains, Elem::i32);
+  else if (!strcmp(key, "Chain Lengths")) r = dense(h->dLen, chains, Elem::i32);
+  else if (!strcmp(key, "Proposal Support")) r = dense(h->dFlag, chains, Elem::i32);
+  else if (!strcmp(key, "Accept Flags")) r = dense(h->dAcc, chains, Elem::i32);
   else if (!strcmp(key, "Evaluation Rows")) {
     if (h->proposed && h->eval_rows < 0) { if (tm_pull(h)) return 1; h->eval_rows = (int)h->hSc->step_evals; }
-    src = h->dEX; rows = h->proposed ? (size_t)h->eval_rows : 0; width = N; pitch = ld;
+    r = pitched(h->dEX, h->proposed ? (size_t)h->eval_rows : 0, N, ld);
   } else if (!strcmp(key, "Evaluation LogLikelihoods")) {
     if (h->ef_rows < 0) { if (tm_pull(h)) return 1; h->ef_rows = (int)h->hSc->step_evals; }
-    src = h->dEF; rows = (size_t)h->ef_rows;
-  } else return tm_fail(h, "unknown array key '%s'", key);
-  const size_t n = rows * width;
-  if (count) *count = n;
-  if (!out) return 0;
-  if (cap < n) return tm_fail(h, "get_array(%s): capacity %zu < %zu", key, cap, n);
-  if (n == 0) return 0;
-  if (isrc) {
-    std::vector<int> tmp(n);
-    TM_CUDA(h, cudaMemcpy(tmp.data(), isrc, sizeof(int) * n, cudaMemcpyDeviceToHost));
-    for (size_t i = 0; i < n; i++) out[i] = (double)tmp[i];
-  } else {
-    TM_CUDA(h, cudaMemcpy2D(out, sizeof(double) * width, src, sizeof(double) * pitch, sizeof(double) * width, rows, cudaMemcpyDeviceToHost));
-  }
-  return 0;
+    r = dense(h->dEF, (size_t)h->ef_rows);
+  } else return fail(h, "unknown array key '%s'", key);
+  return copy_out(h, key, r, out, cap, count, "get_array(%s): capacity %zu < %zu");
 }
 
 int ktmcmc_get_scalar(ktmcmc_t* h, const char* key, double* out) {
-  if (!h || !key || !out) return tm_fail(h, "null argument");
-  TM_CUDA(h, cudaSetDevice(h->device));
+  if (!h) return fail(h, "null solver handle");
+  if (!key || !out) return fail(h, "null argument");
+  CUDA_OK(h, cudaSetDevice(h->device));
   if (tm_pull(h)) return 1;
   const TmScalars& s = *h->hSc;
-  if (!strcmp(key, "Annealing Exponent")) *out = s.rho;
+  if (double* p = host_scalar(h, kHostScalars, key, false)) *out = *p;
+  else if (!strcmp(key, "Annealing Exponent")) *out = s.rho;
   else if (!strcmp(key, "Previous Annealing Exponent")) *out = s.rho_prev;
   else if (!strcmp(key, "Annealing Exponent Update")) *out = s.delta;
   else if (!strcmp(key, "Coefficient Of Variation")) *out = s.cov;
@@ -1033,19 +988,16 @@ int ktmcmc_get_scalar(ktmcmc_t* h, const char* key, double* out) {
   else if (!strcmp(key, "Current Generation")) *out = (double)h->gen;
   else if (!strcmp(key, "Population Size")) *out = (double)h->lambda;
   else if (!strcmp(key, "Burn In")) *out = (double)h->burn;
-  else if (!strcmp(key, "Termination Criteria/Target Annealing Exponent")) *out = h->tc_target;
-  else if (!strcmp(key, "Termination Criteria/Max Generations")) *out = h->tc_max_generations;
-  else if (!strcmp(key, "Termination Criteria/Max Model Evaluations")) *out = h->tc_max_model_evaluations;
-  else return tm_fail(h, "unknown scalar key '%s'", key);
+  else return fail(h, "unknown scalar key '%s'", key);
   return 0;
 }
 
 int ktmcmc_set_scalar(ktmcmc_t* h, const char* key, double v) {
-  if (!h || !key) return tm_fail(h, "null argument");
-  if (!strcmp(key, "Termination Criteria/Target Annealing Exponent")) h->tc_target = v;
-  else if (!strcmp(key, "Termination Criteria/Max Generations")) h->tc_max_generations = v;
-  else if (!strcmp(key, "Termination Criteria/Max Model Evaluations")) h->tc_max_model_evaluations = v;
-  else return tm_fail(h, "unknown scalar key '%s'", key);
+  if (!h) return fail(h, "null solver handle");
+  if (!key) return fail(h, "null argument");
+  double* p = host_scalar(h, kHostScalars, key, true);
+  if (!p) return fail(h, "unknown scalar key '%s'", key);
+  *p = v;
   return 0;
 }
 

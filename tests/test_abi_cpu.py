@@ -5,6 +5,7 @@ import ctypes as C
 import os
 import re
 import subprocess
+import sys
 import tempfile
 import numpy as np
 import pytest
@@ -74,18 +75,42 @@ def test_no_cpu_fallback():
         _lib.k_sort_index(np.arange(4.0))
 
 
+ABIS = [("kcma_", "kcma.h"), ("kdea_", "kdea.h"), ("kmocma_", "kmocma.h"), ("ktmcmc_", "ktmcmc.h")]
+
+
+def _handle_entry_points(prefix, header):
+    """(name, ctypes argument types) of every int-returning entry point of include/<header> whose first argument is the handle."""
+    src = open(os.path.join(ROOT, "include", header)).read()
+    found = []
+    for name, args in re.findall(r"\bint (%s[a-z0-9_]+)\(%st\* h,?([^)]*)\);" % (prefix, prefix), src):
+        types = [C.c_void_p]
+        for a in filter(None, (x.strip() for x in args.split(","))):
+            types.append(C.c_double if a.startswith("double ") else C.c_void_p if ("*" in a or "[" in a or "_fn " in a) else C.c_uint64)
+        found.append((name, types))
+    return found
+
+
 def test_null_handle_is_an_error_not_a_crash():
-    """Every entry point that takes a handle returns non-zero for NULL (kcma_last_error(NULL) explains), and the Python
-    wrapper refuses to pass a closed handle into the library."""
-    import ctypes as C
+    """In each of the four ABIs, every entry point that takes a handle returns non-zero for NULL and <prefix>last_error(NULL)
+    explains; <prefix>launch_count(NULL) is 0 (run in a subprocess: it used to dereference NULL in kcma_)."""
     lib = _lib.lib()
-    for name, extra in [("kcma_run_generation", []), ("kcma_ask", []), ("kcma_eval", []), ("kcma_tell", []),
-                        ("kcma_timing_enable", [C.c_int(1)]), ("kcma_timing_reset", []), ("kcma_flush_l2", [])]:
-        fn = getattr(lib, name)
-        fn.restype, fn.argtypes = C.c_int, [C.c_void_p] + [type(a) for a in extra]
-        assert fn(None, *extra) != 0, name
-    out = C.c_double()
-    lib.kcma_get_scalar.restype, lib.kcma_get_scalar.argtypes = C.c_int, [C.c_void_p, C.c_char_p, C.POINTER(C.c_double)]
-    assert lib.kcma_get_scalar(None, b"Sigma", C.byref(out)) != 0
-    lib.kcma_last_error.restype, lib.kcma_last_error.argtypes = C.c_char_p, [C.c_void_p]
-    assert b"null solver handle" in lib.kcma_last_error(None)
+    for prefix, header in ABIS:
+        last_error = getattr(lib, prefix + "last_error")
+        last_error.restype, last_error.argtypes = C.c_char_p, [C.c_void_p]
+        create = getattr(lib, prefix + "create")
+        create.restype, create.argtypes = C.c_int, [C.c_void_p, C.c_void_p]
+        entry_points = _handle_entry_points(prefix, header)
+        assert len(entry_points) >= 10, prefix
+        for name, types in entry_points:
+            assert create(None, C.byref(C.c_void_p())) != 0                      # leaves a different message behind
+            assert b"null solver handle" not in last_error(None)
+            fn = getattr(lib, name)
+            fn.restype, fn.argtypes = C.c_int, types
+            assert fn(*[t(0) if t in (C.c_double, C.c_uint64) else None for t in types]) != 0, name
+            assert b"null solver handle" in last_error(None), name
+    code = ("import ctypes, sys; sys.path.insert(0, %r); from korali_b200 import _lib\n"
+            "for p in %r:\n"
+            "    f = getattr(_lib.lib(), p + 'launch_count'); f.restype, f.argtypes = ctypes.c_uint64, [ctypes.c_void_p]; print(p, f(None))"
+            % (ROOT, [p for p, _ in ABIS]))
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300)
+    assert r.returncode == 0 and r.stdout.split() == [w for p, _ in ABIS for w in (p, "0")], (r.returncode, r.stdout, r.stderr)
