@@ -56,7 +56,7 @@ enum {
   KCMA_INJ_Z = 0,   /* lambda_z x N standard normals used instead of Philox for the NEXT ask   */
   KCMA_INJ_BDZ = 1, /* lambda x N "BDZ Matrix" (y_i); X is recomputed as m + sigma*y            */
   KCMA_INJ_X = 2,   /* lambda x N "Sample Population" overriding the sampled X                  */
-  KCMA_INJ_F = 3,   /* lambda "Value Vector"                                                    */
+  KCMA_INJ_F = 3,   /* lambda "Value Vector"; taken as F as it is (on a Bayesian handle: as the log-posterior, no prior added) */
   KCMA_INJ_GRAD = 5, /* lambda*N gradients dF/dx of the current population ("Gradients", row-major); with KCMA_INJ_F */
   KCMA_INJ_BD = 4   /* N*N eigenvectors (row-major, columns = vectors) followed by N axis lengths; skips the eigensolver for the NEXT ask */
 };
@@ -182,6 +182,41 @@ int kcma_set_host_constraints(kcma_t* h, kcma_host_constraints_fn fn, void* user
 typedef void (*kcma_device_objective_fn)(void* user, const double* x_dev, uint64_t rows, uint64_t n, uint64_t ldx, double* f_dev, void* stream);
 int kcma_set_device_objective(kcma_t* h, kcma_device_objective_fn fn, void* user);
 
+/* ---- Bayesian problems: F(x) is the log-posterior and CMA-ES returns the maximum a posteriori estimate -----------------
+ * For a sample x with log-prior p = sum_d prior_d(x_d) and log-likelihood l:
+ *   p = -inf (x outside the prior's support): F = -inf. The model is still called on the whole batch; its output for that row is
+ *            ignored and is never an error.
+ *   p finite: l = -inf gives F = -inf, a finite l gives F = p + l, l = NaN or +inf is an error naming the sample. On Bayesian/Reference
+ *            problems the model-output errors of include/ktmcmc.h (a non-finite prediction, a per-point parameter <= 0 or non-finite, a
+ *            Poisson mean < 0) apply to these rows only.
+ * F = -inf ranks last (ties by ascending index); a generation in which every F is -inf completes. Optimization problems are unchanged:
+ * there every non-finite F, -inf included, is an error.
+ * The log-prior is summed like TMCMC's (include/ktmcmc.h): lane d % 32 of one warp sums its variables ascending, then the xor butterfly.
+ * Uniform(a, b): -log(b - a) on [a, b], -inf outside; Normal(a = mean, b = standard deviation): -((x - a) / b)^2 / 2 - log b - log(2 pi) / 2.
+ * The prior enters only through F: it does not set the bounds. Not defined on Bayesian problems (rejected by kcma_set_priors):
+ * Mu Type Proportional (its weights are computed from F), Use Gradient Information, constraints.
+ * Built-in device objectives (KCMA_OBJ_*) are read as log-likelihoods; the log-prior is reduced in the same pass over the samples. */
+enum { KCMA_PRIOR_UNIFORM = 0, KCMA_PRIOR_NORMAL = 1 };
+/* Bayesian/Reference likelihoods (definitions in include/ktmcmc.h) */
+enum { KCMA_LIK_NORMAL = 1, KCMA_LIK_POSITIVE_NORMAL = 2, KCMA_LIK_STUDENT_T = 3, KCMA_LIK_POISSON = 4 };
+/* Once, after create and before the first ask: type[n] (KCMA_PRIOR_*), a[n] = Minimum / Mean, b[n] = Maximum / Standard Deviation.
+ * From then on F is the log-posterior. */
+int kcma_set_priors(kcma_t* h, const int32_t* type, const double* a, const double* b);
+/* Bayesian/Reference: once, after kcma_set_priors and before the first ask; needs objective = KCMA_OBJ_EXTERNAL and keep_population = 1.
+ * Copies data[m] and allocates the model outputs of this rank's samples (rows x m, and as many per-point parameters unless the
+ * likelihood has none). The computational model is set with one of the two setters below. */
+int kcma_set_reference(kcma_t* h, int32_t likelihood, const double* data, uint64_t m);
+/* g_out / p_out: rows x m, row-major, packed; p_out is NULL for a likelihood without a per-point parameter (Poisson) */
+typedef void (*kcma_host_reference_fn)(void* user, const double* x, uint64_t rows, uint64_t n, double* g_out, double* p_out, uint64_t m);
+/* x_dev: rows x n with leading dimension ldx; g_dev / p_dev: rows x m with leading dimension ldm (p_dev NULL as above); the model
+ * writes them on `stream` (a cudaStream_t) */
+typedef void (*kcma_device_reference_fn)(void* user, const double* x_dev, uint64_t rows, uint64_t n, uint64_t ldx, double* g_dev,
+                                         double* p_dev, uint64_t m, uint64_t ldm, void* stream);
+/* Both need kcma_set_reference first. Like the objective setters they may be called between generations; the model set last is the
+ * one the next evaluation calls (the device model when both are set). */
+int kcma_set_host_reference_model(kcma_t* h, kcma_host_reference_fn fn, void* user);
+int kcma_set_device_reference_model(kcma_t* h, kcma_device_reference_fn fn, void* user);
+
 /* ---- parity hooks ------------------------------------------------------------------- */
 int kcma_inject(kcma_t* h, int kind, const double* host, size_t count);
 
@@ -200,7 +235,9 @@ int kcma_set_scalar(kcma_t* h, const char* key, double value);
 
 /* ---- measurement -------------------------------------------------------------------- */
 /* Accumulated CUDA-event time (ms) and call count of a phase since the last reset. Phases:
- * "eigen", "rng", "sample_gemm", "objective", "sort", "gather_mean", "rank_mu", "paths", "collectives", "generation". */
+ * "eigen", "rng", "sample_gemm", "objective", "sort", "gather_mean", "rank_mu", "paths", "collectives", "generation";
+ * Bayesian problems with a host / device model add "posterior" (the log-posterior kernel) and "reference_model" (the computational
+ * model's call). */
 int kcma_timing_enable(kcma_t* h, int on);
 int kcma_timing_get(kcma_t* h, const char* phase, double* ms, uint64_t* calls);
 int kcma_timing_reset(kcma_t* h);

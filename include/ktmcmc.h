@@ -72,7 +72,7 @@ extern "C" {
 
 #define KTMCMC_ABI_VERSION 1u
 
-enum { KTMCMC_PRIOR_UNIFORM = 0, KTMCMC_PRIOR_NORMAL = 1 };
+enum { KTMCMC_PRIOR_UNIFORM = KCMA_PRIOR_UNIFORM, KTMCMC_PRIOR_NORMAL = KCMA_PRIOR_NORMAL };
 
 /* Log-likelihood models: the built-in CMA-ES device objectives read as log-likelihoods (KCMA_OBJ_*, e.g. KCMA_OBJ_NEG_SPHERE gives
  * -1/2 sum x^2), or KCMA_OBJ_EXTERNAL: the host conduit, a device callback or ktmcmc_inject_loglik. */
@@ -126,16 +126,14 @@ int ktmcmc_set_host_loglik(ktmcmc_t* h, ktmcmc_host_loglik_fn fn, void* user);
 int ktmcmc_set_device_loglik(ktmcmc_t* h, kcma_device_objective_fn fn, void* user);
 
 /* Bayesian/Reference: the log-likelihood is reduced on the device from the outputs of a computational model (definitions above). */
-enum { KTMCMC_LIK_NORMAL = 1, KTMCMC_LIK_POSITIVE_NORMAL = 2, KTMCMC_LIK_STUDENT_T = 3, KTMCMC_LIK_POISSON = 4 };
+enum { KTMCMC_LIK_NORMAL = KCMA_LIK_NORMAL, KTMCMC_LIK_POSITIVE_NORMAL = KCMA_LIK_POSITIVE_NORMAL, KTMCMC_LIK_STUDENT_T = KCMA_LIK_STUDENT_T,
+       KTMCMC_LIK_POISSON = KCMA_LIK_POISSON };
 /* Once, after create and before generation 1; cfg.loglik must be KCMA_OBJ_EXTERNAL. Copies data[m]. Allocates the model outputs
  * (lambda x m, and as many per-point parameters unless the likelihood has none); an allocation failure names the GiB needed. */
 int ktmcmc_set_reference(ktmcmc_t* h, int32_t likelihood, const double* data, uint64_t m);
-/* g_out / p_out: rows x m, row-major, packed; p_out is NULL for a likelihood without a per-point parameter (Poisson) */
-typedef void (*ktmcmc_host_reference_fn)(void* user, const double* x, uint64_t rows, uint64_t n, double* g_out, double* p_out, uint64_t m);
-/* x_dev: rows x n with leading dimension ldx; g_dev / p_dev: rows x m with leading dimension ldm (p_dev NULL as above); the model
- * writes them on `stream` (a cudaStream_t) */
-typedef void (*ktmcmc_device_reference_fn)(void* user, const double* x_dev, uint64_t rows, uint64_t n, uint64_t ldx,
-                                           double* g_dev, double* p_dev, uint64_t m, uint64_t ldm, void* stream);
+/* the computational models of kcma.h (kcma_host_reference_fn, kcma_device_reference_fn) */
+typedef kcma_host_reference_fn ktmcmc_host_reference_fn;
+typedef kcma_device_reference_fn ktmcmc_device_reference_fn;
 int ktmcmc_set_host_reference_model(ktmcmc_t* h, ktmcmc_host_reference_fn fn, void* user);
 int ktmcmc_set_device_reference_model(ktmcmc_t* h, ktmcmc_device_reference_fn fn, void* user);
 /* The model outputs of the rows the next ktmcmc_eval evaluates (parity tests); count = rows * m; p is NULL for Poisson. */

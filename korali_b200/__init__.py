@@ -6,7 +6,8 @@
 Served: `"Solver": {"Type": "Optimizer/CMAES"}` (the hot path) and its sibling population solvers `Optimizer/DEA`, `Optimizer/MOCMAES`
 of `"Problem": {"Type": "Optimization"}`, the transitional MCMC sampler `Sampler/TMCMC` of `"Problem": {"Type": "Bayesian/Custom"}`
 and `"Bayesian/Reference"` (priors from `e["Distributions"]`; Reference: "Reference Data", a "Computational Model" that sets
-`sample["Reference Evaluations"]`, and the Normal, Positive Normal, StudentT or Poisson "Likelihood Model", reduced on the device),
+`sample["Reference Evaluations"]`, and the Normal, Positive Normal, StudentT or Poisson "Likelihood Model", reduced on the device) —
+the same Bayesian problems also run with `Optimizer/CMAES`, which maximises the log-posterior and returns the MAP estimate,
 plus the float ask/tell class `fCMAES` (SURVEY.md scope).
 Layers: korali_b200._host (pybind11, C++: Engine / Experiment, mirrors python/korali/__init__.py:9-20 + source/engine.cpp:201-254)
  -> include/kcma.h (C ABI) -> korali_b200/libkcma.so (hand-written sm_100a CUDA). There is no CPU fallback.

@@ -14,8 +14,11 @@ OBJECTIVES = {"NegSphere": 0, "NegRosenbrock": 1, "NegAckley": 2, "NegEllipsoid"
               "NegSphereSin2": 5, "External": 100}
 CONSTRAINTS = {"None": 0, "HalfSpace": 1, "External": 100}
 INJ_Z, INJ_BDZ, INJ_X, INJ_F, INJ_BD, INJ_GRAD = 0, 1, 2, 3, 4, 5
+PRIORS = {"Uniform": 0, "Normal": 1}                                                # KCMA_PRIOR_*
+LIKELIHOODS = {"Normal": 1, "Positive Normal": 2, "StudentT": 3, "Poisson": 4}   # KCMA_LIK_* of Bayesian/Reference
 
 _dp = C.POINTER(C.c_double)
+HOST_REFERENCE_CB = C.CFUNCTYPE(None, C.c_void_p, _dp, C.c_uint64, C.c_uint64, _dp, _dp, C.c_uint64)
 
 
 class KcmaCfg(C.Structure):
@@ -140,6 +143,27 @@ class HandleBase:
             self._live(), C.byref(fin), C.byref(reason)))
         return bool(fin.value), (reason.value or b"").decode()
 
+    def _set_reference(self, reference):
+        """Bayesian/Reference: reference = (likelihood name of LIKELIHOODS, data) through <prefix>set_reference."""
+        name, data = reference
+        d = np.ascontiguousarray(data, dtype=np.float64).ravel()
+        self.likelihood, self.m = LIKELIHOODS[name], d.size
+        self._keep.append(d)
+        self._check(self._fn("set_reference", C.c_int, [C.c_void_p, C.c_int32, _dp, C.c_uint64])(self._live(), self.likelihood, _as_dp(d), d.size))
+
+    def set_host_reference(self, fn):
+        """Bayesian/Reference: fn(X: ndarray[rows, n]) -> (G, P) of rows x m predictions and per-point parameters (broadcast), or G
+        alone for Poisson."""
+        def tramp(_u, x, rows, n, g_out, p_out, m):
+            out = fn(np.ctypeslib.as_array(x, shape=(rows, n)))
+            g, p = (out, None) if not p_out else out
+            np.ctypeslib.as_array(g_out, shape=(rows, m))[:] = np.broadcast_to(np.asarray(g, dtype=np.float64), (rows, m))
+            if p_out:
+                np.ctypeslib.as_array(p_out, shape=(rows, m))[:] = np.broadcast_to(np.asarray(p, dtype=np.float64), (rows, m))
+        cb = HOST_REFERENCE_CB(tramp)
+        self._keep.append(cb)
+        self._check(self._fn("set_host_reference_model", C.c_int, [C.c_void_p, HOST_REFERENCE_CB, C.c_void_p])(self._live(), cb, None))
+
     def _inject(self, name, data):
         a = np.ascontiguousarray(data, dtype=np.float64).ravel()
         self._check(self._fn(name, C.c_int, [C.c_void_p, _dp, C.c_size_t])(self._live(), _as_dp(a), a.size))
@@ -182,17 +206,34 @@ class HandleBase:
 
 
 class Handle(HandleBase):
-    """A CMA-ES solver handle of libkcma.so (prefix 'kcma_') — or of the oracle (prefix 'okcma_') in tests."""
+    """A CMA-ES solver handle of libkcma.so (prefix 'kcma_') — or of the oracle (prefix 'okcma_') in tests.
+    Bayesian problems (F = the log-posterior): priors = [(type, a, b)] * n (type "Uniform" | "Normal"), and for Bayesian/Reference
+    reference = (likelihood name of LIKELIHOODS, data) with objective "External" and keep_population = 1."""
     CFG = KcmaCfg
     ARRAYS = ("lower_bound", "upper_bound", "initial_value", "initial_stddev", "min_stddev_update", "objective_coef", "granularity")
     ENUMS = {"mu_type": MU_TYPES, "objective": OBJECTIVES, "constraint_family": CONSTRAINTS}
+    priors = reference = None
 
     def _field(self, cfg, k, v, kw):
-        if k != "constraint_shift":
+        if k == "priors":
+            self.priors = v
+        elif k == "reference":
+            self.reference = v
+        elif k == "constraint_shift":
+            if v is not None:
+                cfg.constraint_shift = self._array(v, int(kw.get("n_constraints", 0)))
+        else:
             return False
-        if v is not None:
-            cfg.constraint_shift = self._array(v, int(kw.get("n_constraints", 0)))
         return True
+
+    def _created(self, cfg):
+        if self.priors is not None:
+            v = self.priors
+            t = self._array([PRIORS[p[0]] for p in v], len(v), np.int32)
+            a, b = self._array([p[1] for p in v], len(v)), self._array([p[2] for p in v], len(v))
+            self._check(self._fn("set_priors", C.c_int, [C.c_void_p, C.POINTER(C.c_int32), _dp, _dp])(self._live(), t, a, b))
+        if self.reference is not None:
+            self._set_reference(self.reference)
 
     def take_warnings(self):
         return self._fn("take_warnings", C.c_char_p, [C.c_void_p])(self._live()).decode()

@@ -16,7 +16,8 @@ EXPORTS = [
     "kcma_cfg_defaults", "kcma_create", "kcma_destroy", "kcma_last_error", "kcma_take_warnings",
     "kcma_comm_unique_id", "kcma_comm_init", "kcma_comm_init_all", "kcma_shard_range",
     "kcma_run_generation", "kcma_ask", "kcma_eval", "kcma_tell", "kcma_check_termination", "kcma_run",
-    "kcma_set_host_objective", "kcma_set_host_objective_grad", "kcma_set_device_objective", "kcma_set_host_constraints", "kcma_inject", "kcma_get_array", "kcma_set_array", "kcma_get_index_array", "kcma_get_scalar", "kcma_set_scalar",
+    "kcma_set_host_objective", "kcma_set_host_objective_grad", "kcma_set_device_objective", "kcma_set_host_constraints", "kcma_set_priors", "kcma_set_reference",
+    "kcma_set_host_reference_model", "kcma_set_device_reference_model", "kcma_inject", "kcma_get_array", "kcma_set_array", "kcma_get_index_array", "kcma_get_scalar", "kcma_set_scalar",
     "kcma_timing_enable", "kcma_timing_get", "kcma_timing_reset", "kcma_launch_count", "kcma_flush_l2",
     "kcma_k_sort_index", "kcma_k_eigen", "kcma_k_tridiag_stage", "kcma_k_sample", "kcma_k_rank_mu", "kcma_k_philox_normal",
     "kcma_k_philox_raw", "kcma_k_objective",

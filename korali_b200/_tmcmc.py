@@ -2,14 +2,11 @@
 (oracle/libokcma.so, prefix ``otmcmc_``; test infrastructure only) can be driven with the same vocabulary. Nothing here loads the oracle."""
 import ctypes as C
 import numpy as np
-from ._abi import HandleBase, OBJECTIVES, _as_dp, _dp
+from ._abi import HandleBase, HOST_REFERENCE_CB, LIKELIHOODS, OBJECTIVES, PRIORS, _as_dp, _dp   # noqa: F401 (re-exported)
 
 KTMCMC_ABI_VERSION = 1
 KCMA_OBJ_EXTERNAL = 100
-PRIORS = {"Uniform": 0, "Normal": 1}
-LIKELIHOODS = {"Normal": 1, "Positive Normal": 2, "StudentT": 3, "Poisson": 4}   # KTMCMC_LIK_* of Bayesian/Reference
 HOST_CB = C.CFUNCTYPE(None, C.c_void_p, _dp, C.c_uint64, C.c_uint64, _dp)
-HOST_REFERENCE_CB = C.CFUNCTYPE(None, C.c_void_p, _dp, C.c_uint64, C.c_uint64, _dp, _dp, C.c_uint64)
 
 # every symbol include/ktmcmc.h declares
 EXPORTS = [
@@ -57,10 +54,7 @@ class TmcmcHandle(HandleBase):
     def _created(self, cfg):
         self.population_size = int(cfg.population_size)
         if self.reference is not None:
-            name, data = self.reference
-            d = np.ascontiguousarray(data, dtype=np.float64).ravel()
-            self.likelihood, self.m = LIKELIHOODS[name], d.size
-            self._check(self._fn("set_reference", C.c_int, [C.c_void_p, C.c_int32, _dp, C.c_uint64])(self._live(), self.likelihood, _as_dp(d), d.size))
+            self._set_reference(self.reference)
 
     def anneal(self): self._call("anneal")
     def resample(self): self._call("resample")
@@ -72,19 +66,6 @@ class TmcmcHandle(HandleBase):
     def set_host_loglik(self, fn):
         """fn(X: ndarray[rows, n]) -> ndarray[rows] of log-likelihoods."""
         self._set_callback("set_host_loglik", HOST_CB, fn, lambda rows, n: (rows,))
-
-    def set_host_reference(self, fn):
-        """Bayesian/Reference: fn(X: ndarray[rows, n]) -> (G, P) of rows x m predictions and per-point parameters (broadcast), or G
-        alone for Poisson."""
-        def tramp(_u, x, rows, n, g_out, p_out, m):
-            out = fn(np.ctypeslib.as_array(x, shape=(rows, n)))
-            g, p = (out, None) if not p_out else out
-            np.ctypeslib.as_array(g_out, shape=(rows, m))[:] = np.broadcast_to(np.asarray(g, dtype=np.float64), (rows, m))
-            if p_out:
-                np.ctypeslib.as_array(p_out, shape=(rows, m))[:] = np.broadcast_to(np.asarray(p, dtype=np.float64), (rows, m))
-        cb = HOST_REFERENCE_CB(tramp)
-        self._keep.append(cb)
-        self._check(self._fn("set_host_reference_model", C.c_int, [C.c_void_p, HOST_REFERENCE_CB, C.c_void_p])(self._live(), cb, None))
 
     def inject_reference(self, g, p=None):
         """The model outputs (rows x m, and the parameters unless Poisson) of the rows the next eval evaluates."""

@@ -13,6 +13,7 @@
 #include <vector>
 
 #include "../../include/kcma.h"
+#include "bayes.cuh"
 #include "common.cuh"
 #include "handle.cuh"
 #include "kernels.h"
@@ -116,6 +117,18 @@ struct kcma : Handle<kcma, DevScalars> {
   kcma_host_constraints_fn host_con = nullptr; void* host_con_user = nullptr;
   kcma_device_objective_fn dev_obj = nullptr; void* dev_obj_user = nullptr;   // user objective on the device pointer of X
   std::vector<double> hX, hF, hG;
+  // Bayesian problems (kcma_set_priors): F is the log-posterior. Priors on the device (dPrior*: type, a, b, prior_const); Bayesian/
+  // Reference (kcma_set_reference): the likelihood, data and lgamma(data + 1) (Poisson), the model outputs of this rank's samples
+  // (max_local x ldm) and the computational model
+  bool bayes = false;
+  int* dPriorType = nullptr;
+  double *dPriorA = nullptr, *dPriorB = nullptr, *dPriorC = nullptr;
+  int lik = 0;
+  long long m = 0, ldm = 0;
+  double *dData = nullptr, *dDataC = nullptr, *dRefG = nullptr, *dRefP = nullptr;
+  kcma_host_reference_fn host_ref = nullptr; void* host_ref_user = nullptr;
+  kcma_device_reference_fn dev_ref = nullptr; void* dev_ref_user = nullptr;
+  std::vector<double> hRefP;
   // tridiagonalisation-based eigensolver (created on first use)
   kc::TridiagWs* tri = nullptr;
   // nccl
@@ -281,6 +294,39 @@ __global__ void check_finite_kernel(const double* __restrict__ f, long long n, D
 }
 void launch_check_finite(cudaStream_t st, const double* f, long long n, DevScalars* sc) {
   if (n > 0) check_finite_kernel<<<(int)std::min<long long>((n + 255) / 256, 1024), 256, 0, st>>>(f, n, sc);
+}
+
+// The error of a set nonfinite flag (pulled into hSc); clears it. Bayesian problems name the sample of the first bad log-likelihood
+// (DevScalars::post_err) when this rank recorded it.
+int nonfinite_error(kcma* h) {
+  const unsigned long long e = ~h->hSc->post_err;
+  const bool named = h->hSc->post_err != 0;
+  h->hSc->nonfinite = 0;
+  h->hSc->post_err = 0;
+  push_scalars(h);
+  if (!named) return fail(h, "Non finite value of function evaluation detected: nan\n");
+  const long long sample = (long long)(e >> 3);
+  switch ((int)(e & 7)) {
+    case kRefNonFinite: return fail(h, "Bayesian/Reference: 'Reference Evaluations' of sample %lld contains a non-finite value\n", sample);
+    case kRefParameter:
+      return fail(h, "Bayesian/Reference: '%s' of sample %lld contains a value that is not positive and finite\n",
+                  h->lik == KCMA_LIK_STUDENT_T ? "Degrees Of Freedom" : "Standard Deviation", sample);
+    case kRefPoissonMean: return fail(h, "Bayesian/Reference: 'Reference Evaluations' of sample %lld contains a negative Poisson mean\n", sample);
+    case kPostPosInf: return fail(h, "Non finite value of function evaluation detected: the log-likelihood of sample %lld is +inf\n", sample);
+    default: return fail(h, "Non finite value of function evaluation detected: the log-likelihood of sample %lld is nan\n", sample);
+  }
+}
+
+PriorCols prior_cols(const kcma* h) { return PriorCols{h->dPriorType, h->dPriorA, h->dPriorB, h->dPriorC}; }
+
+// Bayesian problems: F of the evaluated rows from the materialised X, after a host / device model wrote the log-likelihoods into F
+// (lik = 0) or a computational model wrote its outputs
+void launch_posterior_of_rows(kcma* h, int lik) {
+  PhaseTimer t(h, "posterior");
+  const long long ls = (long long)(h->eval_hi - h->eval_lo);
+  launch_posterior_rows(h->stream, lik, ls, h->N, h->dX + (h->eval_lo - h->shard_lo) * h->ld, h->ld, prior_cols(h), (int)h->m, h->ldm, h->dRefG,
+                        h->dRefP, h->dData, h->dDataC, h->dF + h->eval_lo, h->eval_lo, h->dSc, h->num_sms);
+  h->launches++;
 }
 
 // infeasible flags -> list of z-rows to resample + counters (prepareGeneration :455-459, :484-490). Single block.
@@ -829,6 +875,30 @@ int do_eval(kcma* h) {
   const bool have_grad = h->inj_grad;
   h->inj_grad = false;
   if (h->inj_f) { h->inj_f = false; return 0; }
+  if (h->lik) {   // Bayesian/Reference: the computational model's outputs of this rank's samples, then the log-posterior
+    {   // the model call (timed apart from the log-posterior kernel)
+      PhaseTimer t(h, "reference_model");
+      const size_t ls = eval_samples(h), N = h->N, m = h->m;
+      const double* x = h->dX + eval_row0(h) * h->ld;
+      double* p = h->lik == KCMA_LIK_POISSON ? nullptr : h->dRefP;
+      if (h->dev_ref) {
+        h->dev_ref(h->dev_ref_user, x, ls, N, h->ld, h->dRefG, p, m, h->ldm, (void*)h->stream);
+      } else if (h->host_ref) {
+        const size_t row = sizeof(double) * m, pitch = sizeof(double) * h->ldm;
+        h->hX.resize(ls * N); h->hG.resize(ls * m); h->hRefP.resize(p ? ls * m : 0);
+        CUDA_OK(h, cudaMemcpy2DAsync(h->hX.data(), sizeof(double) * N, x, sizeof(double) * h->ld, sizeof(double) * N, ls, cudaMemcpyDeviceToHost, h->stream));
+        CUDA_OK(h, cudaStreamSynchronize(h->stream));
+        h->host_ref(h->host_ref_user, h->hX.data(), ls, N, h->hG.data(), p ? h->hRefP.data() : nullptr, m);
+        CUDA_OK(h, cudaMemcpy2DAsync(h->dRefG, pitch, h->hG.data(), row, row, ls, cudaMemcpyHostToDevice, h->stream));
+        if (p) CUDA_OK(h, cudaMemcpy2DAsync(p, pitch, h->hRefP.data(), row, row, ls, cudaMemcpyHostToDevice, h->stream));
+      } else {
+        return fail(h, "Bayesian/Reference: set a host / device computational model before eval");
+      }
+    }
+    launch_posterior_of_rows(h, h->lik);
+    h->scalars_fresh = false;
+    return 0;
+  }
   if (want_grad && h->host_obj_grad) {  // batched host conduit, model returns F and dF/dx
     PhaseTimer t(h, "host_objective");
     const size_t ls = eval_samples(h), N = h->N;
@@ -849,8 +919,12 @@ int do_eval(kcma* h) {
     PhaseTimer t(h, "device_objective");
     const long long ls = (long long)eval_samples(h);
     h->dev_obj(h->dev_obj_user, h->dX + eval_row0(h) * h->ld, (uint64_t)ls, (uint64_t)h->N, (uint64_t)h->ld, h->dF + h->eval_lo, (void*)h->stream);
-    launch_check_finite(h->stream, h->dF + h->eval_lo, ls, h->dSc);
-    h->launches++;
+    if (h->bayes) {
+      launch_posterior_of_rows(h, 0);
+    } else {
+      launch_check_finite(h->stream, h->dF + h->eval_lo, ls, h->dSc);
+      h->launches++;
+    }
     h->scalars_fresh = false;
     return 0;
   }
@@ -861,6 +935,12 @@ int do_eval(kcma* h) {
     CUDA_OK(h, cudaMemcpy2DAsync(h->hX.data(), sizeof(double) * N, h->dX + eval_row0(h) * h->ld, sizeof(double) * h->ld, sizeof(double) * N, ls, cudaMemcpyDeviceToHost, h->stream));
     CUDA_OK(h, cudaStreamSynchronize(h->stream));
     h->host_obj(h->host_obj_user, h->hX.data(), (uint64_t)ls, (uint64_t)N, h->hF.data());
+    if (h->bayes) {   // the log-likelihoods are checked with the log-prior on the device
+      CUDA_OK(h, cudaMemcpyAsync(h->dF + h->eval_lo, h->hF.data(), sizeof(double) * ls, cudaMemcpyHostToDevice, h->stream));
+      launch_posterior_of_rows(h, 0);
+      h->scalars_fresh = false;
+      return 0;
+    }
     for (size_t i = 0; i < ls; i++)  // ref: optimization.cpp.base:32-33
       if (!std::isfinite(h->hF[i])) {
         if (h->cfg.nranks == 1) return fail(h, "Non finite value of function evaluation detected: %f\n", h->hF[i]);
@@ -877,8 +957,10 @@ int do_eval(kcma* h) {
   const long long ls = (long long)eval_samples(h);
   double* f_local = h->dF + h->eval_lo;
   const double* src = (h->inj_x ? h->dX : h->dY) + eval_row0(h) * h->ld;
-  if (launch_objective(h->stream, h->cfg.objective, src, h->ld, ls, h->N, h->cfg.mirrored_sampling, h->inj_x ? 1 : 0, h->dMean,
-                       h->dSc, h->dCoef, f_local, h->num_sms))
+  if (h->bayes ? launch_posterior_objective(h->stream, h->cfg.objective, src, h->ld, ls, h->N, h->cfg.mirrored_sampling, h->inj_x ? 1 : 0,
+                                            h->dMean, h->dSc, h->dCoef, prior_cols(h), f_local, h->eval_lo, h->num_sms)
+               : launch_objective(h->stream, h->cfg.objective, src, h->ld, ls, h->N, h->cfg.mirrored_sampling, h->inj_x ? 1 : 0, h->dMean,
+                                  h->dSc, h->dCoef, f_local, h->num_sms))
     return fail(h, "unknown objective id %d", h->cfg.objective);
   h->launches++;
   if (want_grad && !have_grad) {
@@ -995,11 +1077,7 @@ int end_of_generation(kcma* h) {
   if (h->timing) resolve_timers(h);
   cudaError_t e = cudaGetLastError();
   if (e != cudaSuccess) return fail(h, "CUDA error after generation: %s", cudaGetErrorString(e));
-  if (h->hSc->nonfinite) {
-    h->hSc->nonfinite = 0;
-    push_scalars(h);
-    return fail(h, "Non finite value of function evaluation detected: nan\n");
-  }
+  if (h->hSc->nonfinite) return nonfinite_error(h);
   if (h->hSc->warn_no_valid) {
     h->warn += "No sample without constraint violations in this generation: using the best-ranked sample (the reference reads out of bounds here).\n";
     h->hSc->warn_no_valid = 0;
@@ -1273,6 +1351,95 @@ int kcma_set_host_constraints(kcma_t* h, kcma_host_constraints_fn fn, void* user
   return 0;
 }
 
+int kcma_set_priors(kcma_t* h, const int32_t* type, const double* a, const double* b) {
+  if (!h) return fail(h, "null solver handle");
+  if (h->bayes) return fail(h, "set_priors: the priors are already set");
+  if (h->gen != 1 || h->sampled_pending) return fail(h, "set_priors: call it before the first generation");
+  if (!type || !a || !b) return fail(h, "set_priors: every variable needs a prior distribution");
+  if (h->cfg.mu_type == KCMA_MU_PROPORTIONAL)
+    return fail(h, "Optimizer/CMAES: 'Mu Type' Proportional is not defined on Bayesian problems (its weights are computed from F(x), "
+                   "which is -inf outside the prior's support)\n");
+  if (h->cfg.use_gradient_information) return fail(h, "Optimizer/CMAES: 'Use Gradient Information' is not built for Bayesian problems\n");
+  if (h->has_constraints) return fail(h, "Optimizer/CMAES: 'Constraints' are not defined on Bayesian problems\n");
+  const int N = h->N;
+  for (int d = 0; d < N; d++) {
+    if (type[d] == KCMA_PRIOR_UNIFORM) {
+      if (!std::isfinite(a[d]) || !std::isfinite(b[d]) || !(b[d] > a[d])) return fail(h, "Univariate/Uniform prior of variable %d: need finite Minimum < Maximum\n", d);
+    } else if (type[d] == KCMA_PRIOR_NORMAL) {
+      if (!std::isfinite(a[d]) || !std::isfinite(b[d]) || !(b[d] > 0.0))
+        return fail(h, "Univariate/Normal prior of variable %d: need a finite Mean and a positive Standard Deviation\n", d);
+    } else {
+      return fail(h, "unknown prior type %d of variable %d", type[d], d);
+    }
+  }
+  CUDA_OK(h, cudaSetDevice(h->device));
+  invalidate_graph(h);
+  if (!h->dPriorType) {
+    CUDA_OK(h, alloc(h->mem, &h->dPriorType, N));
+    for (double** p : {&h->dPriorA, &h->dPriorB, &h->dPriorC}) CUDA_OK(h, alloc(h->mem, p, N));
+  }
+  CUDA_OK(h, cudaMemcpyAsync(h->dPriorType, type, sizeof(int32_t) * N, cudaMemcpyHostToDevice, h->stream));
+  CUDA_OK(h, cudaMemcpyAsync(h->dPriorA, a, sizeof(double) * N, cudaMemcpyHostToDevice, h->stream));
+  CUDA_OK(h, cudaMemcpyAsync(h->dPriorB, b, sizeof(double) * N, cudaMemcpyHostToDevice, h->stream));
+  launch_prior_constants(h->stream, N, h->dPriorType, h->dPriorA, h->dPriorB, h->dPriorC);
+  h->launches++;
+  CUDA_OK(h, cudaStreamSynchronize(h->stream));
+  CUDA_OK(h, cudaGetLastError());
+  h->bayes = true;
+  return 0;
+}
+
+int kcma_set_reference(kcma_t* h, int32_t likelihood, const double* data, uint64_t m) {
+  if (!h) return fail(h, "null solver handle");
+  if (h->lik) return fail(h, "set_reference: the reference data are already set");
+  if (!h->bayes) return fail(h, "set_reference: set the priors first (kcma_set_priors)");
+  if (h->gen != 1 || h->sampled_pending) return fail(h, "set_reference: call it before the first generation");
+  if (h->cfg.objective != KCMA_OBJ_EXTERNAL) return fail(h, "set_reference: the objective must be External (KCMA_OBJ_EXTERNAL)");
+  if (!h->cfg.keep_population) return fail(h, "set_reference: needs keep_population = 1 (the computational model reads the materialised X)");
+  if (likelihood < KCMA_LIK_NORMAL || likelihood > KCMA_LIK_POISSON) return fail(h, "set_reference: unknown likelihood %d", likelihood);
+  if (!data || m < 1 || m > (uint64_t)INT32_MAX) return fail(h, "set_reference: need 1 <= m < 2^31 reference data (got %zu)", (size_t)m);
+  std::vector<double> dc(m, 0.0);
+  for (uint64_t j = 0; j < m; j++) {
+    const double d = data[j];
+    if (!std::isfinite(d)) return fail(h, "Bayesian/Reference: 'Reference Data' %zu is not finite\n", (size_t)j);
+    if (likelihood == KCMA_LIK_POISSON && (d < 0.0 || d != floor(d)))
+      return fail(h, "Bayesian/Reference: 'Reference Data' %zu (%g) must be a non-negative integer for the Poisson likelihood\n", (size_t)j, d);
+    if (likelihood == KCMA_LIK_POSITIVE_NORMAL && d < 0.0)
+      return fail(h, "Bayesian/Reference: 'Reference Data' %zu (%g) must be >= 0 for the Positive Normal likelihood\n", (size_t)j, d);
+    if (likelihood == KCMA_LIK_POISSON) dc[j] = lgamma(d + 1.0);
+  }
+  CUDA_OK(h, cudaSetDevice(h->device));
+  invalidate_graph(h);
+  const long long ldm = ((long long)m + 3) / 4 * 4;   // 32-byte aligned rows
+  const bool param = likelihood != KCMA_LIK_POISSON;
+  const size_t each = (size_t)h->max_local * ldm;
+  if (alloc(h->mem, &h->dRefG, each) != cudaSuccess || (param && alloc(h->mem, &h->dRefP, each) != cudaSuccess)) {
+    cudaGetLastError();
+    return fail(h, "Bayesian/Reference: cannot allocate the model outputs of %zu samples x %zu reference points (%.2f GiB)\n", (size_t)h->max_local,
+                (size_t)m, (double)each * sizeof(double) * (param ? 2 : 1) / (double)(1ull << 30));
+  }
+  CUDA_OK(h, alloc(h->mem, &h->dData, m));
+  CUDA_OK(h, alloc(h->mem, &h->dDataC, m));
+  CUDA_OK(h, cudaMemcpy(h->dData, data, sizeof(double) * m, cudaMemcpyHostToDevice));
+  CUDA_OK(h, cudaMemcpy(h->dDataC, dc.data(), sizeof(double) * m, cudaMemcpyHostToDevice));
+  h->lik = likelihood; h->m = (long long)m; h->ldm = ldm;
+  return 0;
+}
+int kcma_set_host_reference_model(kcma_t* h, kcma_host_reference_fn fn, void* user) {
+  if (!h) return fail(h, "null solver handle");
+  if (!h->lik) return fail(h, "set_host_reference_model: set the reference data first (kcma_set_reference)");
+  invalidate_graph(h);
+  h->host_ref = fn; h->host_ref_user = user;
+  return 0;
+}
+int kcma_set_device_reference_model(kcma_t* h, kcma_device_reference_fn fn, void* user) {
+  if (!h) return fail(h, "null solver handle");
+  if (!h->lik) return fail(h, "set_device_reference_model: set the reference data first (kcma_set_reference)");
+  invalidate_graph(h);
+  h->dev_ref = fn; h->dev_ref_user = user;
+  return 0;
+}
+
 int kcma_comm_unique_id(uint8_t id_out[128]) {
   std::string err;
   if (!g_nccl.load(err)) return fail<kcma>(nullptr, "%s", err.c_str());
@@ -1328,11 +1495,7 @@ int kcma_eval(kcma_t* h) {
   CUDA_OK(h, cudaSetDevice(h->device));
   if (do_eval(h)) return 1;
   if (pull_cached(h)) return 1;
-  if (h->hSc->nonfinite) {
-    h->hSc->nonfinite = 0;
-    push_scalars(h);
-    return fail(h, "Non finite value of function evaluation detected: nan\n");
-  }
+  if (h->hSc->nonfinite) return nonfinite_error(h);
   return 0;
 }
 

@@ -83,10 +83,23 @@ struct DevScalars {
   int n_disc_mut;            // _numberOfDiscreteMutations
   unsigned long long jacobi_sweeps_total;   // sweeps of the persistent Jacobi kernel since creation (read once by the timers)
   unsigned long long gen;    // generation counter for CUDA-graph replays (kernels launched with generation == kGenFromDevice read it)
+  unsigned long long post_err;   // Bayesian problems: ~(sample << 3 | code) of the first bad log-likelihood (atomicMax), 0 = none
 };
 
 // Sentinel for the by-value `generation` kernel argument: take the counter from DevScalars::gen instead. A captured CUDA graph
 // bakes its kernel arguments, so the replayed generation loop keeps the one argument that changes per generation on the device.
 constexpr unsigned kGenFromDevice = 0xffffffffu;
+
+// Codes of DevScalars::post_err beyond the model-output codes of bayes.cuh (kRefNonFinite, kRefParameter, kRefPoissonMean)
+enum { kPostNaN = 3, kPostPosInf = 4 };
+
+// The priors of a Bayesian problem on the device (kcma_set_priors): per variable its KCMA_PRIOR_* type, parameters and
+// prior_const(type, a, b)
+struct PriorCols {
+  const int* type;
+  const double* a;
+  const double* b;
+  const double* c;
+};
 
 }  // namespace kc

@@ -17,6 +17,7 @@ inline bool first_call_on_device(std::atomic<unsigned long long>& mask) {
   return !(mask.fetch_or(bit) & bit);
 }
 struct DevScalars;
+struct PriorCols;
 
 // gemm.cu
 size_t gemm_tn_smem_bytes();
@@ -83,6 +84,16 @@ void launch_philox_raw(cudaStream_t st, const uint32_t* in6, uint32_t* out4);
 // objective.cu
 int launch_objective(cudaStream_t st, int objective, const double* Y, int ldy, long long samples, int n, int mirrored, int from_x,
                      const double* mean, DevScalars* sc, const double* coef, double* f, int num_sms);
+// Bayesian problems (include/kcma.h): the per-variable constants of the priors; F = the log-posterior of a built-in log-likelihood
+// (the log-prior reduced in the same pass over Y; row0 = global index of the first sample, for the error); the log-posterior of
+// materialised rows X whose log-likelihood is in F already (lik = 0) or is reduced from the model outputs G, P (KCMA_LIK_*)
+void launch_prior_constants(cudaStream_t st, int n, const int* type, const double* a, const double* b, double* c);
+int launch_posterior_objective(cudaStream_t st, int objective, const double* Y, int ldy, long long samples, int n, int mirrored, int from_x,
+                               const double* mean, DevScalars* sc, const double* coef, const PriorCols& pr, double* f,
+                               unsigned long long row0, int num_sms);
+void launch_posterior_rows(cudaStream_t st, int lik, long long rows, int n, const double* X, int ldx, const PriorCols& pr, int m,
+                           long long ldm, const double* G, const double* P, const double* D, const double* DC, double* f,
+                           unsigned long long row0, DevScalars* sc, int num_sms);
 void launch_feasibility(cudaStream_t st, const double* Y, int ldy, long long samples, int n, int mirrored, const double* mean,
                         const DevScalars* sc, const double* lower, const double* upper, unsigned char* infeasible, double* X,
                         int ldx, const int* row_list, int num_sms);

@@ -27,6 +27,7 @@
 #include <vector>
 
 #include "../../include/ktmcmc.h"
+#include "bayes.cuh"
 #include "common.cuh"
 #include "handle.cuh"
 #include "kernels.h"
@@ -38,7 +39,6 @@ using namespace kc;
 constexpr int kThreads = 1024;        // one-CTA reductions and scans: thread t owns a fixed slice (restated by the oracle)
 constexpr int kMeanChunks = 64;       // row chunks of the weighted mean
 constexpr uint32_t kKeyTag = 0x544d434du;   // "TMCM"
-constexpr double kHalfLog2Pi = 0.91893853320467274178;
 
 __device__ __forceinline__ void tm_philox(uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, unsigned long long seed, uint32_t out[4]) {
   uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32) ^ kKeyTag;
@@ -73,20 +73,6 @@ struct TmScalars {
   int nan_flag, allinf_flag;
   unsigned long long ref_err;        // Bayesian/Reference: ~(row << 2 | code) of the first bad model output (atomicMax), 0 = none
 };
-enum { kRefNonFinite = 0, kRefParameter = 1, kRefPoissonMean = 2 };
-
-__device__ __forceinline__ double prior_term(int type, double a, double b, double x) {
-  if (type == KTMCMC_PRIOR_UNIFORM) return (x >= a && x <= b) ? -log(b - a) : -INFINITY;
-  const double z = (x - a) / b;
-  return -0.5 * (z * z) - log(b) - kHalfLog2Pi;
-}
-// log-prior of one row: lane-strided partials, xor butterfly (all lanes return the same bits)
-__device__ __forceinline__ double log_prior_row(const double* __restrict__ x, int n, const int* __restrict__ type,
-                                                const double* __restrict__ pa, const double* __restrict__ pb, int lane) {
-  double p = 0.0;
-  for (int d = lane; d < n; d += 32) p = p + prior_term(type[d], pa[d], pb[d], x[d]);
-  return warp_sum_butterfly(p);
-}
 
 // Generation 1: one warp per sample; lanes over the Box-Muller pairs, then the log-prior of the row.
 __global__ void __launch_bounds__(256)
@@ -419,18 +405,6 @@ __global__ void tm_check_nan_kernel(const double* __restrict__ F, int count, TmS
   if (i < count && F[i] != F[i]) sc->nan_flag = 1;
 }
 
-// Bayesian/Reference terms (include/ktmcmc.h; tests/helpers/otmcmc_reference.c restates them in the same operation order)
-constexpr double kInvSqrt2 = 0.70710678118654752440;
-constexpr double kPi = 3.14159265358979323846;
-__device__ __forceinline__ double log_ndtr(double u) {
-  if (u >= -1.0) return log(0.5 * erfc(-u * kInvSqrt2));
-  return log(0.5 * erfcx(-u * kInvSqrt2)) - 0.5 * (u * u);
-}
-__device__ __forceinline__ double student_t_const(double nu) {   // lgamma((nu + 1) / 2) - lgamma(nu / 2) - log(nu pi) / 2
-  if (nu < 50.0) return lgamma(0.5 * (nu + 1.0)) - lgamma(0.5 * nu) - 0.5 * log(nu * kPi);
-  const double ix = 1.0 / (0.5 * nu), y = ix * ix;
-  return ix * (-0.125 + y * (1.0 / 192.0 + y * (-1.0 / 640.0 + y * (17.0 / 14336.0)))) - kHalfLog2Pi;
-}
 // l of each evaluated row from its M predictions G (and parameters P): one warp per row, lane k sums j = k, k + 32, ... ascending,
 // then the xor butterfly. Reads rows * M * 8 bytes of G (and of P) once, coalesced; the data (and, for Poisson, lgamma(d + 1) in
 // DC) through the read-only path. A bad output is recorded in sc->ref_err and leaves its term NaN.
@@ -445,25 +419,7 @@ tm_reference_loglik_kernel(int rows, int m, long long ldm, const double* __restr
   const double* p = LIK == KTMCMC_LIK_POISSON ? nullptr : P + i * ldm;
   double s = 0.0;
   int bad = 4;
-  for (int j = lane; j < m; j += 32) {
-    const double gj = g[j], dj = __ldg(D + j);
-    double t;
-    if (!isfinite(gj)) { bad = min(bad, (int)kRefNonFinite); t = NAN; }
-    else if (LIK == KTMCMC_LIK_POISSON) {
-      if (gj < 0.0) { bad = min(bad, (int)kRefPoissonMean); t = NAN; }
-      else t = dj == 0.0 ? -gj : (gj == 0.0 ? -INFINITY : dj * log(gj) - gj - __ldg(DC + j));
-    } else {
-      const double pj = p[j], r = dj - gj;
-      if (!(pj > 0.0) || !isfinite(pj)) { bad = min(bad, (int)kRefParameter); t = NAN; }
-      else if (LIK == KTMCMC_LIK_STUDENT_T) t = student_t_const(pj) - 0.5 * (pj + 1.0) * log1p(r * r / pj);
-      else {
-        const double z = r / pj;
-        t = -kHalfLog2Pi - log(pj) - 0.5 * (z * z);
-        if (LIK == KTMCMC_LIK_POSITIVE_NORMAL) { t = t - log_ndtr(gj / pj); if (t != t) t = -INFINITY; }
-      }
-    }
-    s = s + t;
-  }
+  for (int j = lane; j < m; j += 32) s = s + reference_term<LIK>(g[j], p, j, __ldg(D + j), DC, bad);
   if (bad < 4) atomicMax(&sc->ref_err, ~(((unsigned long long)i << 2) | (unsigned)bad));
   s = warp_sum_butterfly(s);
   if (lane == 0) EF[i] = s;

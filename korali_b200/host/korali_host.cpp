@@ -568,6 +568,113 @@ class Plugin : public SolverBase {
   }
 };
 
+// ---- Bayesian problems (bayesian/custom.config, bayesian/reference.config), shared by Sampler/TMCMC and Optimizer/CMAES (which maximises
+// the log-posterior): the priors from e["Distributions"] and each variable's "Prior Distribution", and the likelihood model
+struct Bayesian {
+  std::vector<int32_t> prior_type;   // per variable: KCMA_PRIOR_*, Minimum / Mean, Maximum / Standard Deviation
+  std::vector<double> prior_a, prior_b;
+  Model model;                       // the Python likelihood model when loglik is KCMA_OBJ_EXTERNAL, or the Bayesian/Reference computational model
+  int32_t loglik = KCMA_OBJ_EXTERNAL;   // Bayesian/Custom: a built-in device model read as the log-likelihood, or External
+  int32_t likelihood = 0;            // Bayesian/Reference: KCMA_LIK_*, 0 for Bayesian/Custom
+  std::vector<double> ref_data;      // its "Reference Data"
+  std::vector<std::string> dname, dtype;   // e["Distributions"]
+  std::vector<double> da, db;
+
+  // bayesian/custom.config: "Likelihood Model" is a callable setting sample["logLikelihood"] or the name of a device model
+  void setCustom(Settings& p, std::string* pending) {
+    if (!p.has("Likelihood Model")) korali_error(" + Object: [ Bayesian/Custom ] \n + Key:    ['Likelihood Model']\n + Reason: mandatory setting missing\n");
+    py::object model_fn = p.take("Likelihood Model");
+    p.finish();
+    if (py::isinstance<py::str>(model_fn)) {
+      loglik = deviceObjective(model_fn.cast<std::string>(), "likelihood model");
+    } else if (PyCallable_Check(model_fn.ptr())) {
+      loglik = KCMA_OBJ_EXTERNAL;
+      model.set(model_fn, pending);
+      model.output = "logLikelihood";   // Bayesian/Custom "Evaluate": the model sets sample["logLikelihood"]
+      model.fill = 0.0;
+    } else {
+      korali_error(" + Object: [ Bayesian/Custom ] \n + Key:    ['Likelihood Model']\n + Reason: neither a callable nor the name of a device model\n");
+    }
+  }
+
+  // bayesian/reference.config: "Likelihood Model", "Reference Data" and a "Computational Model" that sets sample["Reference
+  // Evaluations"] (and the likelihood's per-point parameter); the log-likelihood is reduced on the device (include/ktmcmc.h)
+  void setReference(Settings& p, std::string* pending) {
+    p.module = "Bayesian/Reference";
+    for (const char* k : {"Likelihood Model", "Reference Data", "Computational Model"})
+      if (!p.has(k)) korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['%s']\n + Reason: mandatory setting missing\n", k);
+    const std::string name = p.str("Likelihood Model", "");
+    const std::string lik = canon(name);
+    if (lik == "normal") likelihood = KCMA_LIK_NORMAL;
+    else if (lik == "positivenormal") likelihood = KCMA_LIK_POSITIVE_NORMAL;
+    else if (lik == "studentt") likelihood = KCMA_LIK_STUDENT_T;
+    else if (lik == "poisson") likelihood = KCMA_LIK_POISSON;
+    else if (lik == "positivestudentt" || lik == "geometric" || lik == "negativebinomial")
+      korali_error("Bayesian/Reference: 'Likelihood Model' '%s' is not built on the B200 path (Normal, Positive Normal, StudentT and Poisson are)\n", name.c_str());
+    else korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Likelihood Model']\n + Reason: unknown value '%s' (Normal, Positive Normal, StudentT, Poisson)\n", name.c_str());
+    py::object data = p.take("Reference Data");
+    if (!py::isinstance<py::list>(data) || py::len(data) == 0)
+      korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Reference Data']\n + Reason: a non-empty array of numbers was expected\n");
+    ref_data.clear();
+    for (auto x : data) {
+      const size_t j = ref_data.size();
+      if (!is_number(x) || !std::isfinite(x.cast<double>()))
+        korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Reference Data']\n + Reason: entry %zu is not a finite number\n", j);
+      const double d = x.cast<double>();
+      if (likelihood == KCMA_LIK_POISSON && (d < 0.0 || d != std::floor(d)))
+        korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Reference Data']\n + Reason: entry %zu (%g) must be a non-negative integer for the Poisson likelihood\n", j, d);
+      if (likelihood == KCMA_LIK_POSITIVE_NORMAL && d < 0.0)
+        korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Reference Data']\n + Reason: entry %zu (%g) must be >= 0 for the Positive Normal likelihood\n", j, d);
+      ref_data.push_back(d);
+    }
+    py::object model_fn = p.take("Computational Model");
+    if (py::isinstance<py::str>(model_fn))
+      korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Computational Model']\n + Reason: a callable was expected (there is no built-in device computational model)\n");
+    if (!PyCallable_Check(model_fn.ptr()))
+      korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Computational Model']\n + Reason: a callable was expected\n");
+    p.finish();
+    loglik = KCMA_OBJ_EXTERNAL;
+    model.set(model_fn, pending);
+    model.output = "Reference Evaluations";
+    model.param = likelihood == KCMA_LIK_POISSON ? nullptr : likelihood == KCMA_LIK_STUDENT_T ? "Degrees Of Freedom" : "Standard Deviation";
+  }
+
+  // priors: e["Distributions"][k] = {"Name", "Type", parameters}; solver names the plug-in in errors
+  void setDistributions(py::object distributions, const char* solver) {
+    dname.clear(); dtype.clear(); da.clear(); db.clear();
+    if (!distributions.is_none()) {
+      if (!py::isinstance<py::list>(distributions)) korali_error(" + Object: [ Experiment ] \n + Key:    ['Distributions']\n + Reason: an array was expected\n");
+      for (auto item : distributions) {
+        Settings d = object(item, "Distribution", "Distributions: every entry must be an object\n");
+        const std::string nm = d.str("Name", ""), ty = d.str("Type", "");
+        const std::string ct = canon(ty);
+        double a = NAN, b = NAN;
+        if (ct == "univariate/uniform") { a = d.num("Minimum", NAN); b = d.num("Maximum", NAN); dtype.push_back("uniform"); }
+        else if (ct == "univariate/normal") { a = d.num("Mean", NAN); b = d.num("Standard Deviation", NAN); dtype.push_back("normal"); }
+        else korali_error("%s: prior distribution type '%s' of '%s' is not built (Univariate/Uniform, Univariate/Normal)\n", solver, ty.c_str(), nm.c_str());
+        if (d.has("Random Seed")) d.take("Random Seed");
+        d.finish();
+        if (!std::isfinite(a) || !std::isfinite(b)) korali_error("Distribution '%s' (%s): its parameters must be set to finite numbers\n", nm.c_str(), ty.c_str());
+        dname.push_back(nm); da.push_back(a); db.push_back(b);
+      }
+    }
+  }
+
+  void resize(size_t n) { prior_type.assign(n, 0); prior_a.assign(n, 0.0); prior_b.assign(n, 0.0); }
+  // the "Prior Distribution" of variable i (consumed from v)
+  std::string takePrior(Settings& v, size_t i, const std::string& vname) {
+    if (!v.has("Prior Distribution")) korali_error("Variable %zu ('%s') has no 'Prior Distribution'\n", i, vname.c_str());
+    return v.str("Prior Distribution", "");
+  }
+  void resolvePrior(size_t i, const std::string& vname, const std::string& pd) {
+    size_t k = 0;
+    while (k < dname.size() && dname[k] != pd) k++;
+    if (k == dname.size()) korali_error("Variable %zu ('%s'): prior distribution '%s' is not defined in e['Distributions']\n", i, vname.c_str(), pd.c_str());
+    prior_type[i] = dtype[k] == "uniform" ? KCMA_PRIOR_UNIFORM : KCMA_PRIOR_NORMAL;
+    prior_a[i] = da[k]; prior_b[i] = db[k];
+  }
+};
+
 // ---- the solver plug-in: Optimizer/CMAES on libkcma ----------------------------------------------------------
 class CMAES : public Plugin<kcma_t, kcma_cfg> {
  public:
@@ -577,6 +684,10 @@ class CMAES : public Plugin<kcma_t, kcma_cfg> {
   std::vector<std::string> names;
   Model objective;                      // the Python model when cfg.objective is KCMA_OBJ_EXTERNAL
   std::vector<py::object> constraints;  // Python callables
+  // Bayesian/Custom and Bayesian/Reference: F(x) is the log-posterior (include/kcma.h), the run returns the maximum a posteriori estimate
+  bool bayesian = false;
+  py::object distributions = py::none();   // the experiment's top-level "Distributions" (the priors)
+  Bayesian bayes;
 
   CMAES() : Plugin({kcma_create, kcma_destroy, kcma_last_error, kcma_run_generation, kcma_check_termination, kcma_get_array, kcma_get_scalar,
                     kcma_set_scalar},
@@ -672,15 +783,29 @@ class CMAES : public Plugin<kcma_t, kcma_cfg> {
     if (s.has("Is Diagonal")) { const int v = s.boolean("Is Diagonal", 0); if (v) cfg.diagonal_covariance = 1; }
     for (const char* k : {"Are Constraints Defined", "Best Sample Index", "Previous Value Vector"})
       if (s.has(k)) s.take(k);
+    // Bayesian problems: a problem keyed for Optimization first names the Problem Type; then the settings whose meaning needs a finite F
+    const std::string ptype_raw = problem.contains("Type") && py::isinstance<py::str>(problem["Type"]) ? problem["Type"].cast<std::string>() : "";
+    bayesian = canon(ptype_raw) == "bayesian/custom" || canon(ptype_raw) == "bayesian/reference";
+    if (bayesian) {
+      if (!problem.contains("Likelihood Model"))
+        korali_error("Problem Type '%s' needs a 'Likelihood Model' (an 'Objective Function' belongs to Problem Type 'Optimization')\n", ptype_raw.c_str());
+      if (cfg.mu_type == KCMA_MU_PROPORTIONAL)
+        korali_error("Optimizer/CMAES: 'Mu Type' Proportional is not defined on Bayesian problems (its weights are computed from F(x), which is "
+                     "-inf outside the prior's support)\n");
+      if (cfg.use_gradient_information) korali_error("Optimizer/CMAES: 'Use Gradient Information' is not built for Bayesian problems\n");
+      if (problem.contains("Constraints")) korali_error("Optimizer/CMAES: 'Constraints' are not defined on Bayesian problems\n");
+    }
     // variables (optimizer.config:45-82, CMAES.config Variable Defaults: Granularity 0.0)
     const size_t n = py::len(variables);
     if (n == 0) korali_error("Optimization Evaluation problems require at least one variable.\n");
+    std::vector<std::string> prior_of(n);   // Bayesian: each variable's "Prior Distribution", resolved with the problem
     lower.assign(n, -INFINITY); upper.assign(n, INFINITY); init_val.assign(n, NAN); init_sd.assign(n, NAN); min_sd.assign(n, 0.0);
     gran.assign(n, 0.0);
     names.assign(n, "");
     for (size_t i = 0; i < n; i++) {
       Settings v = variable(variables, i);
       names[i] = v.str("Name", "");
+      if (bayesian) prior_of[i] = bayes.takePrior(v, i, names[i]);
       lower[i] = v.num("Lower Bound", -INFINITY);
       upper[i] = v.num("Upper Bound", INFINITY);
       init_val[i] = v.num("Initial Value", NAN);
@@ -696,6 +821,19 @@ class CMAES : public Plugin<kcma_t, kcma_cfg> {
     cfg.lower_bound = lower.data(); cfg.upper_bound = upper.data(); cfg.initial_value = init_val.data();
     cfg.initial_stddev = init_sd.data(); cfg.min_stddev_update = min_sd.data(); cfg.granularity = gran.data();
     cfg.seed = seed;
+    if (bayesian) {   // bayesian/custom.config, bayesian/reference.config and the priors, as Sampler/TMCMC reads them
+      Settings p = object(problem, "Bayesian/Custom", "'Problem' is not an object\n");
+      const std::string ptype = canon(p.str("Type", ""));
+      if (ptype == "bayesian/reference") bayes.setReference(p, &pending_error);
+      else bayes.setCustom(p, &pending_error);
+      bayes.setDistributions(distributions, name());
+      bayes.resize(n);
+      for (size_t i = 0; i < n; i++) bayes.resolvePrior(i, names[i], prior_of[i]);
+      cfg.objective = bayes.loglik;
+      cfg.keep_population = cfg.objective == KCMA_OBJ_EXTERNAL ? 1 : 0;
+      s.finish();
+      return;
+    }
     // problem (optimization.config)
     Settings p = object(problem, "Optimization", "'Problem' is not an object\n");
     const std::string ptype = canon(p.str("Type", ""));
@@ -780,7 +918,18 @@ class CMAES : public Plugin<kcma_t, kcma_cfg> {
       if (kcma_comm_init_all(hs.data(), G)) korali_error("%s", kcma_last_error(h));
       pool = std::make_unique<RankPool>(G);
     }
-    if (cfg.objective == KCMA_OBJ_EXTERNAL) {
+    if (bayesian) {
+      each([&](kcma_t* x) { return kcma_set_priors(x, bayes.prior_type.data(), bayes.prior_a.data(), bayes.prior_b.data()); });
+      if (bayes.likelihood) {
+        Model& model = bayes.model;
+        check(kcma_set_reference(h, bayes.likelihood, bayes.ref_data.data(), bayes.ref_data.size()));
+        if (model.flavour == "device") check(kcma_set_device_reference_model(h, &Model::deviceReference, &model));
+        else check(kcma_set_host_reference_model(h, &Model::hostReference, &model));
+      } else if (cfg.objective == KCMA_OBJ_EXTERNAL) {
+        if (bayes.model.flavour == "device") check(kcma_set_device_objective(h, &Model::device, &bayes.model));
+        else check(kcma_set_host_objective(h, &Model::host, &bayes.model));
+      }
+    } else if (cfg.objective == KCMA_OBJ_EXTERNAL) {
       if (cfg.use_gradient_information) check(kcma_set_host_objective_grad(h, &CMAES::host_objective_grad, this));
       else if (objective.flavour == "device") check(kcma_set_device_objective(h, &Model::device, &objective));
       else check(kcma_set_host_objective(h, &Model::host, &objective));
@@ -1200,13 +1349,8 @@ class MOCMAES : public Plugin<kmocma_t, kmocma_cfg> {
 class TMCMC : public Plugin<ktmcmc_t, ktmcmc_cfg> {
  public:
   py::object distributions = py::none();   // the experiment's top-level "Distributions" (the priors)
-  std::vector<int32_t> prior_type;
-  std::vector<double> prior_a, prior_b;
   std::vector<uint64_t> burn_in;
-  std::vector<std::string> prior_name;
-  Model model;   // the Python likelihood model when cfg.loglik is KCMA_OBJ_EXTERNAL, or the Bayesian/Reference computational model
-  int32_t likelihood = 0;          // Bayesian/Reference: KTMCMC_LIK_*, 0 for Bayesian/Custom
-  std::vector<double> ref_data;    // its "Reference Data"
+  Bayesian bayes;
 
   TMCMC() : Plugin({ktmcmc_create, ktmcmc_destroy, ktmcmc_last_error, ktmcmc_run_generation, ktmcmc_check_termination, ktmcmc_get_array,
                     ktmcmc_get_scalar, ktmcmc_set_scalar},
@@ -1215,65 +1359,6 @@ class TMCMC : public Plugin<ktmcmc_t, ktmcmc_cfg> {
                     {"Max Model Evaluations", 1e9, false, true}}) {}
   const char* name() const override { return "Sampler/TMCMC"; }
   size_t variableCount() const override { return cfg.n; }
-
-  // bayesian/custom.config: "Likelihood Model" is a callable setting sample["logLikelihood"] or the name of a device model
-  void setCustom(Settings& p) {
-    if (!p.has("Likelihood Model")) korali_error(" + Object: [ Bayesian/Custom ] \n + Key:    ['Likelihood Model']\n + Reason: mandatory setting missing\n");
-    py::object model_fn = p.take("Likelihood Model");
-    p.finish();
-    if (py::isinstance<py::str>(model_fn)) {
-      cfg.loglik = deviceObjective(model_fn.cast<std::string>(), "likelihood model");
-    } else if (PyCallable_Check(model_fn.ptr())) {
-      cfg.loglik = KCMA_OBJ_EXTERNAL;
-      model.set(model_fn, &pending_error);
-      model.output = "logLikelihood";   // Bayesian/Custom "Evaluate": the model sets sample["logLikelihood"]
-      model.fill = 0.0;
-    } else {
-      korali_error(" + Object: [ Bayesian/Custom ] \n + Key:    ['Likelihood Model']\n + Reason: neither a callable nor the name of a device model\n");
-    }
-  }
-
-  // bayesian/reference.config: "Likelihood Model", "Reference Data" and a "Computational Model" that sets sample["Reference
-  // Evaluations"] (and the likelihood's per-point parameter); the log-likelihood is reduced on the device (include/ktmcmc.h)
-  void setReference(Settings& p) {
-    p.module = "Bayesian/Reference";
-    for (const char* k : {"Likelihood Model", "Reference Data", "Computational Model"})
-      if (!p.has(k)) korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['%s']\n + Reason: mandatory setting missing\n", k);
-    const std::string name = p.str("Likelihood Model", "");
-    const std::string lik = canon(name);
-    if (lik == "normal") likelihood = KTMCMC_LIK_NORMAL;
-    else if (lik == "positivenormal") likelihood = KTMCMC_LIK_POSITIVE_NORMAL;
-    else if (lik == "studentt") likelihood = KTMCMC_LIK_STUDENT_T;
-    else if (lik == "poisson") likelihood = KTMCMC_LIK_POISSON;
-    else if (lik == "positivestudentt" || lik == "geometric" || lik == "negativebinomial")
-      korali_error("Bayesian/Reference: 'Likelihood Model' '%s' is not built on the B200 path (Normal, Positive Normal, StudentT and Poisson are)\n", name.c_str());
-    else korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Likelihood Model']\n + Reason: unknown value '%s' (Normal, Positive Normal, StudentT, Poisson)\n", name.c_str());
-    py::object data = p.take("Reference Data");
-    if (!py::isinstance<py::list>(data) || py::len(data) == 0)
-      korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Reference Data']\n + Reason: a non-empty array of numbers was expected\n");
-    ref_data.clear();
-    for (auto x : data) {
-      const size_t j = ref_data.size();
-      if (!is_number(x) || !std::isfinite(x.cast<double>()))
-        korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Reference Data']\n + Reason: entry %zu is not a finite number\n", j);
-      const double d = x.cast<double>();
-      if (likelihood == KTMCMC_LIK_POISSON && (d < 0.0 || d != std::floor(d)))
-        korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Reference Data']\n + Reason: entry %zu (%g) must be a non-negative integer for the Poisson likelihood\n", j, d);
-      if (likelihood == KTMCMC_LIK_POSITIVE_NORMAL && d < 0.0)
-        korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Reference Data']\n + Reason: entry %zu (%g) must be >= 0 for the Positive Normal likelihood\n", j, d);
-      ref_data.push_back(d);
-    }
-    py::object model_fn = p.take("Computational Model");
-    if (py::isinstance<py::str>(model_fn))
-      korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Computational Model']\n + Reason: a callable was expected (there is no built-in device computational model)\n");
-    if (!PyCallable_Check(model_fn.ptr()))
-      korali_error(" + Object: [ Bayesian/Reference ] \n + Key:    ['Computational Model']\n + Reason: a callable was expected\n");
-    p.finish();
-    cfg.loglik = KCMA_OBJ_EXTERNAL;
-    model.set(model_fn, &pending_error);
-    model.output = "Reference Evaluations";
-    model.param = likelihood == KTMCMC_LIK_POISSON ? nullptr : likelihood == KTMCMC_LIK_STUDENT_T ? "Degrees Of Freedom" : "Standard Deviation";
-  }
 
   // generated TMCMC::setConfiguration (TMCMC.config) + Sampler:: + Solver:: (strict); priors from e["Distributions"]
   void setConfiguration(py::dict solver, py::list variables, py::dict problem, uint64_t seed) override {
@@ -1310,57 +1395,35 @@ class TMCMC : public Plugin<ktmcmc_t, ktmcmc_cfg> {
     // problem (bayesian/custom.config, bayesian/reference.config)
     Settings p = object(problem, "Bayesian/Custom", "'Problem' is not an object\n");
     const std::string ptype = canon(p.str("Type", ""));
-    if (ptype == "bayesian/reference") setReference(p);
-    else if (ptype == "bayesian/custom") setCustom(p);
+    if (ptype == "bayesian/reference") bayes.setReference(p, &pending_error);
+    else if (ptype == "bayesian/custom") bayes.setCustom(p, &pending_error);
     else korali_error("Sampler/TMCMC: only Problem Type 'Bayesian/Custom' or 'Bayesian/Reference' is served (got '%s')\n", ptype.c_str());
-    // priors: e["Distributions"][k] = {"Name", "Type", parameters}
-    std::vector<std::string> dname, dtype;
-    std::vector<double> da, db;
-    if (!distributions.is_none()) {
-      if (!py::isinstance<py::list>(distributions)) korali_error(" + Object: [ Experiment ] \n + Key:    ['Distributions']\n + Reason: an array was expected\n");
-      for (auto item : distributions) {
-        Settings d = object(item, "Distribution", "Distributions: every entry must be an object\n");
-        const std::string nm = d.str("Name", ""), ty = d.str("Type", "");
-        const std::string ct = canon(ty);
-        double a = NAN, b = NAN;
-        if (ct == "univariate/uniform") { a = d.num("Minimum", NAN); b = d.num("Maximum", NAN); dtype.push_back("uniform"); }
-        else if (ct == "univariate/normal") { a = d.num("Mean", NAN); b = d.num("Standard Deviation", NAN); dtype.push_back("normal"); }
-        else korali_error("Sampler/TMCMC: prior distribution type '%s' of '%s' is not built (Univariate/Uniform, Univariate/Normal)\n", ty.c_str(), nm.c_str());
-        if (d.has("Random Seed")) d.take("Random Seed");
-        d.finish();
-        if (!std::isfinite(a) || !std::isfinite(b)) korali_error("Distribution '%s' (%s): its parameters must be set to finite numbers\n", nm.c_str(), ty.c_str());
-        dname.push_back(nm); da.push_back(a); db.push_back(b);
-      }
-    }
+    cfg.loglik = bayes.loglik;
+    bayes.setDistributions(distributions, name());
     const size_t n = py::len(variables);
     if (n == 0) korali_error("Bayesian problems require at least one variable.\n");
     lower.assign(n, -INFINITY); upper.assign(n, INFINITY);
-    prior_type.assign(n, 0); prior_a.assign(n, 0.0); prior_b.assign(n, 0.0); prior_name.assign(n, "");
+    bayes.resize(n);
     for (size_t i = 0; i < n; i++) {
       Settings v = variable(variables, i);
       const std::string vname = v.str("Name", "");
-      if (!v.has("Prior Distribution")) korali_error("Variable %zu ('%s') has no 'Prior Distribution'\n", i, vname.c_str());
-      const std::string pd = v.str("Prior Distribution", "");
+      const std::string pd = bayes.takePrior(v, i, vname);
       v.num("Lower Bound", -INFINITY); v.num("Upper Bound", INFINITY);   // written back by getConfiguration
       v.finish();
-      size_t k = 0;
-      while (k < dname.size() && dname[k] != pd) k++;
-      if (k == dname.size()) korali_error("Variable %zu ('%s'): prior distribution '%s' is not defined in e['Distributions']\n", i, vname.c_str(), pd.c_str());
-      prior_name[i] = pd;
-      prior_type[i] = dtype[k] == "uniform" ? KTMCMC_PRIOR_UNIFORM : KTMCMC_PRIOR_NORMAL;
-      prior_a[i] = da[k]; prior_b[i] = db[k];
-      if (prior_type[i] == KTMCMC_PRIOR_UNIFORM) { lower[i] = da[k]; upper[i] = db[k]; }
+      bayes.resolvePrior(i, vname, pd);
+      if (bayes.prior_type[i] == KCMA_PRIOR_UNIFORM) { lower[i] = bayes.prior_a[i]; upper[i] = bayes.prior_b[i]; }
     }
     cfg.n = n; cfg.seed = seed;
-    cfg.prior_type = prior_type.data(); cfg.prior_a = prior_a.data(); cfg.prior_b = prior_b.data();
+    cfg.prior_type = bayes.prior_type.data(); cfg.prior_a = bayes.prior_a.data(); cfg.prior_b = bayes.prior_b.data();
     cfg.per_generation_burn_in = burn_in.empty() ? nullptr : burn_in.data(); cfg.burn_in_count = burn_in.size();
   }
 
   void initialize(const std::vector<int>& device_ids) override {
     requireOneDevice(device_ids);
     create(device_ids[0]);
-    if (likelihood) {
-      check(ktmcmc_set_reference(h, likelihood, ref_data.data(), ref_data.size()));
+    Model& model = bayes.model;
+    if (bayes.likelihood) {
+      check(ktmcmc_set_reference(h, bayes.likelihood, bayes.ref_data.data(), bayes.ref_data.size()));
       if (model.flavour == "device") check(ktmcmc_set_device_reference_model(h, &Model::deviceReference, &model));
       else check(ktmcmc_set_host_reference_model(h, &Model::hostReference, &model));
     } else if (cfg.loglik == KCMA_OBJ_EXTERNAL) {
@@ -1445,7 +1508,7 @@ class Experiment : public KoraliJson {
     py::dict d = py::reinterpret_borrow<py::dict>(loaded);
     if (_js.contains("Problem") && py::isinstance<py::dict>(_js["Problem"]) && d.contains("Problem")) {
       py::dict oldp = py::reinterpret_borrow<py::dict>(_js["Problem"]), newp = py::reinterpret_borrow<py::dict>(d["Problem"]);
-      for (const char* k : {"Objective Function", "Constraints"}) if (oldp.contains(k)) newp[k] = oldp[k];
+      for (const char* k : {"Objective Function", "Constraints", "Likelihood Model", "Computational Model"}) if (oldp.contains(k)) newp[k] = oldp[k];
     }
     if (d.contains("Solver") && py::isinstance<py::dict>(d["Solver"])) {   // .npy side-cars of large N x N arrays (saveState)
       py::dict sj = py::reinterpret_borrow<py::dict>(d["Solver"]);
@@ -1487,10 +1550,11 @@ class Experiment : public KoraliJson {
     py::dict problem_js = py::reinterpret_borrow<py::dict>(top.take("Problem"));
     py::list variables = py::reinterpret_borrow<py::list>(top.take("Variables"));
     const std::string stype = canon(solver_js.contains("Type") && py::isinstance<py::str>(solver_js["Type"]) ? solver_js["Type"].cast<std::string>() : "");
-    // the solver types, by canonical name and short name; TMCMC reads its priors from e["Distributions"], the optimizers ignore the key
+    // the solver types, by canonical name and short name; TMCMC and CMAES (Bayesian problems) read the priors from e["Distributions"],
+    // the other optimizers ignore the key
     using Factory = std::unique_ptr<SolverBase> (*)(py::object distributions);
     static const struct { const char* type; const char* alias; Factory make; } kSolvers[] = {
-        {"optimizer/cmaes", "cmaes", [](py::object) -> std::unique_ptr<SolverBase> { return std::make_unique<CMAES>(); }},
+        {"optimizer/cmaes", "cmaes", [](py::object d) -> std::unique_ptr<SolverBase> { auto c = std::make_unique<CMAES>(); c->distributions = d; return c; }},
         {"optimizer/dea", "dea", [](py::object) -> std::unique_ptr<SolverBase> { return std::make_unique<DEA>(); }},
         {"optimizer/mocmaes", "mocmaes", [](py::object) -> std::unique_ptr<SolverBase> { return std::make_unique<MOCMAES>(); }},
         {"sampler/tmcmc", "tmcmc", [](py::object d) -> std::unique_ptr<SolverBase> { auto t = std::make_unique<TMCMC>(); t->distributions = d; return t; }}};
